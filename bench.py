@@ -81,7 +81,14 @@ def parse():
     ap.add_argument('--no-profile', action='store_true')
     ap.add_argument('--no-file', action='store_true', help='skip the FITS-file-inclusive measurement')
     ap.add_argument('--no-alt', action='store_true', help='skip the informational run in the other 16-bit format')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the timed path returned in its last timed step as DIR/<name>.npy (float32 / '
+                         'float64; integer fields as float64) so that two builds can be compared output for output: '
+                         'the merged catalog (the same for any GPU count), or with --config 5 the outputs of rank 0\'s '
+                         '256 tiles (the same head maps for any GPU count; other ranks draw their own)')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     if a.mosaic is None:
         a.mosaic = 32768 if a.config == 4 else 16384
     if a.step is None:
@@ -215,11 +222,14 @@ def run_reference(args):
     img = synth.make_mosaic(n, n, seed=1234, nan_border_frac=0.0)
     vals = []
     for i in range(args.warmup + args.steps):
-        v, dt, nt, _ = cpu_reference(args, img, threads)
+        v, dt, nt, cat = cpu_reference(args, img, threads, keep_catalog=bool(args.dump_outputs))
         if i >= args.warmup:
             vals.append((v, dt, nt))
-        if sum(x[1] for x in vals) > 240:
-            break
+    if args.dump_outputs:      # the oracle's catalog under the field names of the b200 dump (it has no tile ids)
+        out = {'sources_' + k: np.array([s[k] for s in cat], np.float64) for k in ('x1', 'y1', 'x2', 'y2', 'score')}
+        out['sources_cls'] = np.array([s['class_id'] for s in cat])
+        out['sources_flags'] = np.array([int(bool(s['edge'])) | 2 * int(bool(s.get('merged', False))) for s in cat])
+        dump_outputs(args.dump_outputs, out)
     v = float(np.mean([x[0] for x in vals]))
     ms = float(np.mean([x[1] for x in vals])) * 1e3
     nt = vals[0][2]
@@ -235,6 +245,8 @@ def run_reference(args):
             "cpu_baseline": {"value": v, "unit": "tiles/s", "cores": threads, "kind": "port", "sample": sample},
             "e2e": {"value": v, "unit": "tiles/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "mpix_per_s": v * args.tile * args.tile / 1e6}
+    if args.dump_outputs:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "outputs": "oracle catalog of the %d-tile sample" % nt}
     emit(line)
     return 0
 
@@ -256,6 +268,33 @@ def workload_config(args, n, T=None, mosaic=None):
 def catalog_crc(src):
     """crc32 of the catalog bytes (cy_source records in catalog order): identical across GPU counts iff the catalogs are."""
     return "%08x" % (zlib.crc32(np.ascontiguousarray(src).view(np.uint8).tobytes()) & 0xffffffff)
+
+
+DUMP_BYTES = 64 << 20      # cap on everything --dump-outputs writes
+
+
+def dump_outputs(d, arrays):
+    """Writes {name: array} as d/<name>.npy.  float32 / float64 arrays are written as they are, integer arrays as
+    float64 (exact for int32)."""
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)
+        np.save(os.path.join(d, name + '.npy'), a)
+
+
+def catalog_arrays(src, nrec):
+    """The catalog (cy_source array, catalog order) as one array per field plus the record count.  A catalog too large
+    for DUMP_BYTES is cut to a fixed, seeded sample of its rows; `sources_row` then holds the rows kept."""
+    out = {'records': np.array([nrec])}
+    rows = DUMP_BYTES // (8 * (len(src.dtype.names) + 1))
+    if len(src) > rows:
+        keep = np.sort(np.random.default_rng(0).choice(len(src), rows, replace=False))
+        src = src[keep]
+        out['sources_row'] = keep
+    out.update(('sources_' + f, src[f]) for f in src.dtype.names)
+    return out
 
 
 def match_fraction(got, want, thr):
@@ -343,6 +382,13 @@ def run_nms_stress(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:      # rank 0's tiles: every rank draws its own head maps
+        ndh, nkh = nd.cpu().numpy(), nkeep.cpu().numpy()
+        dh, kh = dets.cpu().numpy(), keep.cpu().numpy()
+        dump_outputs(args.dump_outputs, {
+            'dets': np.concatenate([dh[i, :ndh[i]] for i in range(B)]), 'ndets': ndh,
+            'keep_idx': np.concatenate([kh[i, :nkh[i]] for i in range(B)]), 'nkeep': nkh,
+            'merge_status': mstat.cpu().numpy()})
     ms = float(t[0]) / args.steps
     # end to end: head maps from pinned host memory, kept indices back to the host
     hosts = [h.cpu().pin_memory() for h in heads]
@@ -381,6 +427,9 @@ def run_nms_stress(args):
                          "algorithmic_bytes_per_launch": alg,
                          "note": "latency/IoU-test bound: the suppression bitmask stays in shared memory"},
             "dets_per_tile": float(nd.float().mean()), "kept_after_merge_per_tile": float(nkeep.float().mean())}
+    if args.dump_outputs:
+        line["dump_outputs"] = {"dir": args.dump_outputs,
+                                "outputs": "rank 0's %d tiles (the same head maps for any GPU count)" % B}
     emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -461,6 +510,8 @@ def main():
     eng.stage_events = None
     launches = eng.launches - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, catalog_arrays(src, nrec))
     for _ in range(max(2, args.warmup - 1)):
         step_e2e()
     eng.stage_events = []
@@ -486,8 +537,8 @@ def main():
             return pipeline.run_image(eng, fimg, True, tiles, rank=rank, world=world, on_rank0_only=False)
         for _ in range(2):
             step_file()
-        ms_f, wall_f, (src3, _) = timed(step_file, max(2, args.steps // 2))
-        file_ms = max(ms_f, wall_f) / max(2, args.steps // 2)
+        ms_f, wall_f, (src3, _) = timed(step_file, args.steps)
+        file_ms = max(ms_f, wall_f) / args.steps
         # raw read rate of the same byte range with the same reader, nothing else running
         t0 = time.time()
         nbytes = pipeline.read_rows_benchmark(eng, fimg, y0b, y1b)
@@ -521,13 +572,12 @@ def main():
             return eng2.exchange_and_merge(world)
         for _ in range(2):
             step_alt()
-        k2 = max(2, args.steps // 2)
         eng2.stage_events = []
-        ms2, _, (src_alt, _) = timed(step_alt, k2)
-        st2 = {k: v / k2 for k, v in eng2.stage_times_ms().items()}
-        alt = {"dtype": altp, "value": T / (ms2 / k2 * 1e-3), "unit": "tiles/s", "ms_per_step": ms2 / k2,
+        ms2, _, (src_alt, _) = timed(step_alt, args.steps)
+        st2 = {k: v / args.steps for k, v in eng2.stage_times_ms().items()}
+        alt = {"dtype": altp, "value": T / (ms2 / args.steps * 1e-3), "unit": "tiles/s", "ms_per_step": ms2 / args.steps,
                "forward_ms_per_step": round(st2.get('forward', 0.0), 3), "sources": int(len(src_alt)),
-               "note": "same box, same workload, mosaic resident; %d timed steps" % k2}
+               "note": "same box, same workload, mosaic resident; %d timed steps" % args.steps}
         del eng2
 
     if rank != 0:
@@ -557,6 +607,9 @@ def main():
     if alt is not None:
         line["alt_precision"] = alt
     line["host_numa_node"] = numa_node       # node the rank-0 process (and its pinned staging) was bound to; None: not bound
+    if args.dump_outputs:
+        line["dump_outputs"] = {"dir": args.dump_outputs,
+                                "outputs": "merged catalog of the last timed step (the same for any GPU count)"}
     known = sum(stage_ms.get(k, 0.0) for k in ('preprocess', 'forward', 'decode_nms', 'merge_tile_records'))
     line["exchange_ms"] = round(stage_ms.get('exchange', 0.0), 3)
     line["unattributed_ms"] = round(ms_step - known - stage_ms.get('exchange', 0.0) - stage_ms.get('merge_global', 0.0), 3)
