@@ -77,6 +77,21 @@ class RunConfig(ctypes.Structure):
                 ("rank", ctypes.c_int32), ("world", ctypes.c_int32)]
 
 
+class SrcPartial(ctypes.Structure):
+    """cy_src_partial: one source's sums over one row range."""
+    _fields_ = [("npix", c_i64), ("peak_idx", c_i64), ("peak", c_double), ("sum", c_double), ("sw", c_double),
+                ("swx", c_double), ("swy", c_double), ("swxx", c_double), ("swyy", c_double), ("swxy", c_double)]
+
+
+class SrcMeas(ctypes.Structure):
+    """cy_src_meas: final per-source measurements."""
+    _fields_ = [("npix", c_i64), ("sum", c_double), ("peak", c_double), ("peak_x", c_double), ("peak_y", c_double),
+                ("xc", c_double), ("yc", c_double), ("a", c_double), ("b", c_double), ("theta", c_double)]
+
+
+assert ctypes.sizeof(SrcPartial) == 80 and ctypes.sizeof(SrcMeas) == 80
+
+
 ALLGATHER_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t,
                                 ctypes.c_size_t)
 
@@ -90,7 +105,7 @@ SYMBOLS = [
     "cy_model_create", "cy_model_set_tensor", "cy_model_set_precision", "cy_model_plan_summary", "cy_letterbox_resize_fmt", "cy_model_finalize", "cy_model_forward", "cy_model_info",
     "cy_stem_conv_nhwc4", "cy_model_profile", "cy_model_conv_bytes", "cy_model_destroy", "cy_num_anchors", "cy_decode_pred", "cy_postprocess_scratch_bytes",
     "cy_postprocess", "cy_nms_scratch_bytes", "cy_nms_batched", "cy_merge_tile", "cy_make_records",
-    "cy_compact_scratch_bytes", "cy_compact_records", "cy_merge_global",
+    "cy_compact_scratch_bytes", "cy_compact_records", "cy_merge_global", "cy_measure_sources", "cy_measure_combine",
     "cy_ctx_create", "cy_ctx_set_allgather", "cy_ctx_destroy", "cy_run_local", "cy_run_local_payload", "cy_ctx_records",
     "cy_ctx_pack_slot", "cy_ctx_unpack_slots", "cy_run_merge", "cy_run_mosaic", "cy_run_payload", "cy_ctx_info",
 ]

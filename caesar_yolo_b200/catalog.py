@@ -3,6 +3,7 @@
 (Analyzer.write_json_results, caesar_yolo/evaluation.py:472-483) and the DS9 region text the `regions` package emits
 (inference.py:1214-1287, evaluation.py:487-548; `regions` itself is not a dependency)."""
 import json
+import math
 
 CLASS_COLOR_DS9 = {  # SFinder (mosaic catalog), inference.py:334-342
     'bkg': "black", 'spurious': "red", 'compact': "blue", 'extended': "green", 'extended-multisland': "yellow",
@@ -14,9 +15,34 @@ CLASS_COLOR_DS9_ANALYZER = {  # Analyzer (single image / per-tile files), evalua
 }
 
 
-def sources_to_dicts(src, names):
+# per-source measurement keys (Engine.measure + fits metadata); written only when measurements are requested
+MEASURE_KEYS = ('npix', 'sum', 'peak', 'peak_x', 'peak_y', 'xc', 'yc', 'a', 'b', 'theta', 'flux', 'ra', 'dec')
+
+
+def _num(v):
+    v = float(v)
+    return v if math.isfinite(v) else None      # JSON null
+
+
+def measurement_dicts(meas, beam_area_pix=None, radec=None):
+    """ops.MEAS_DTYPE array -> one dict of MEASURE_KEYS per source.  flux = sum / beam_area_pix (None without a beam);
+    radec: (ra, dec) arrays of the centroids in degrees, or None.  Non-finite values become None (JSON null)."""
+    out = []
+    for i, m in enumerate(meas):
+        d = {"npix": int(m['npix'])}
+        for k in MEASURE_KEYS[1:10]:
+            d[k] = _num(m[k])
+        d["flux"] = _num(m['sum'] / beam_area_pix) if beam_area_pix else None
+        d["ra"] = _num(radec[0][i]) if radec is not None else None
+        d["dec"] = _num(radec[1][i]) if radec is not None else None
+        out.append(d)
+    return out
+
+
+def sources_to_dicts(src, names, meas=None):
     """cy_source array -> list of dicts with the reference's keys.  Pass-through sources keep the reference's mixed
-    `edge` typing (int 0 from make_json_results, True once find_sources_at_edge fired)."""
+    `edge` typing (int 0 from make_json_results, True once find_sources_at_edge fired).  meas: optional
+    measurement_dicts of the same sources, whose keys are added."""
     out = []
     for i, s in enumerate(src):
         edge = bool(int(s['flags']) & 1)
@@ -26,17 +52,22 @@ def sources_to_dicts(src, names):
             "class_id": int(s['cls']), "class_name": str(names[int(s['cls'])]), "score": float(s['score']),
             "edge": True if edge else 0, "merged": bool(int(s['flags']) & 2),
         })
+        if meas is not None:
+            out[-1].update(meas[i])
     return out
 
 
-def records_to_objs(recs, names, tag=""):
-    """cy_det_record array of ONE image/tile -> Analyzer.results['objs'] (evaluation.py:418-469)."""
+def records_to_objs(recs, names, tag="", meas=None):
+    """cy_det_record array of ONE image/tile -> Analyzer.results['objs'] (evaluation.py:418-469).  meas: optional
+    measurement_dicts of the same records, whose keys are added."""
     objs = []
     for i, r in enumerate(recs):
         name = 'S' + str(i + 1) if tag == "" else 'S' + str(i + 1) + "_" + tag
         objs.append({"name": name, "x1": float(r['x1']), "x2": float(r['x2']), "y1": float(r['y1']),
                      "y2": float(r['y2']), "class_id": int(r['cls']), "class_name": str(names[int(r['cls'])]),
                      "score": float(r['score']), "edge": int(int(r['flags']) & 1)})
+        if meas is not None:
+            objs[-1].update(meas[i])
     return objs
 
 

@@ -42,4 +42,6 @@ CONFIG = {
     'draw_plot': False,
     'draw_class_label_in_caption': True,
     'save_plot': False,
+    # - Per-source measurements (not in the reference): peak, flux density, centroid, shape, sky position
+    'measure_sources': False,
 }

@@ -77,6 +77,75 @@ class FitsImage(object):
         return out
 
 
+def pixel_scale_matrix(h):
+    """2x2 matrix (degrees per pixel) from intermediate world coordinates to pixel offsets of a FITS header dict: the CD
+    matrix when any CDi_j card is present, else CDELTi times the PCi_j matrix (identity when absent), else CDELTi with
+    the CROTA2 rotation (Calabretta & Greisen 2002, eq. 189).  None without CDELT1/2 or CD cards."""
+    if any(("CD%d_%d" % (i, j)) in h for i in (1, 2) for j in (1, 2)):
+        return np.array([[float(h.get("CD%d_%d" % (i, j), 0.0)) for j in (1, 2)] for i in (1, 2)])
+    if "CDELT1" not in h or "CDELT2" not in h:
+        return None
+    c1, c2 = float(h["CDELT1"]), float(h["CDELT2"])
+    if any(("PC%d_%d" % (i, j)) in h for i in (1, 2) for j in (1, 2)):
+        pc = np.array([[float(h.get("PC%d_%d" % (i, j), 1.0 if i == j else 0.0)) for j in (1, 2)] for i in (1, 2)])
+        return np.array([[c1], [c2]]) * pc
+    rho = np.radians(float(h.get("CROTA2", 0.0)))
+    return np.array([[c1 * np.cos(rho), -c2 * np.sin(rho)], [c1 * np.sin(rho), c2 * np.cos(rho)]])
+
+
+def beam_area_pix(h):
+    """Solid angle of the Gaussian restoring beam in pixels, pi * BMAJ * BMIN / (4 ln 2) / |det(pixel scale matrix)|
+    (BMAJ / BMIN: FWHM in degrees); None when the cards are missing or degenerate.  The flux density of a source is
+    its pixel sum divided by this (Jy for a Jy/beam image)."""
+    m = pixel_scale_matrix(h)
+    if m is None or "BMAJ" not in h or "BMIN" not in h:
+        return None
+    det = abs(float(np.linalg.det(m)))
+    area = np.pi * float(h["BMAJ"]) * float(h["BMIN"]) / (4.0 * np.log(2.0))
+    if not (det > 0 and area > 0 and np.isfinite(det) and np.isfinite(area)):
+        return None
+    return area / det
+
+
+def celestial_projection(h):
+    """'SIN' or 'TAN' when CTYPE1/2 are RA---SIN / DEC--SIN or RA---TAN / DEC--TAN, else None."""
+    t1, t2 = str(h.get("CTYPE1", "")).strip().upper(), str(h.get("CTYPE2", "")).strip().upper()
+    for proj in ("SIN", "TAN"):
+        if t1 == "RA---" + proj and t2 == "DEC--" + proj:
+            return proj
+    return None
+
+
+def pixel_to_world(h, x, y):
+    """(ra, dec) in degrees of 0-based pixel coordinates x (column), y (row) for the SIN and TAN projections (Calabretta
+    & Greisen 2002, sections 2-3 and 5.1: zenithal projections with the reference point at the native pole; SIN without
+    the PV obliqueness terms).  The native longitude of the celestial pole is the LONPOLE card, by default 180 deg, or 0
+    when CRVAL2 = 90 (C&G sect. 2.4).  FITS pixels are 1-based: p = x + 1.  Points outside the projection's domain give
+    NaN.  None when the header has no SIN / TAN celestial WCS."""
+    proj = celestial_projection(h)
+    m = pixel_scale_matrix(h)
+    if proj is None or m is None or any(k not in h for k in ("CRVAL1", "CRVAL2", "CRPIX1", "CRPIX2")):
+        return None
+    x = np.asarray(x, dtype=np.float64)
+    y = np.asarray(y, dtype=np.float64)
+    d1 = x + 1.0 - float(h["CRPIX1"])
+    d2 = y + 1.0 - float(h["CRPIX2"])
+    xi = np.radians(m[0, 0] * d1 + m[0, 1] * d2)          # intermediate world coordinates (projection plane)
+    eta = np.radians(m[1, 0] * d1 + m[1, 1] * d2)
+    r = np.hypot(xi, eta)
+    phi = np.arctan2(xi, -eta)                              # native longitude
+    with np.errstate(invalid="ignore"):
+        theta = np.arctan2(1.0, r) if proj == "TAN" else np.arccos(r)   # native latitude
+    a0, d0 = np.radians(float(h["CRVAL1"])), np.radians(float(h["CRVAL2"]))
+    # default LONPOLE (C&G 2002 eq. 8 with theta_0 = 90 deg): 0 for a reference point at the north pole, else 180
+    phi_p = np.radians(float(h.get("LONPOLE", 0.0 if float(h["CRVAL2"]) >= 90.0 else 180.0)))
+    dphi = phi - phi_p
+    st, ct = np.sin(theta), np.cos(theta)
+    ra = a0 + np.arctan2(-ct * np.sin(dphi), st * np.cos(d0) - ct * np.sin(d0) * np.cos(dphi))
+    dec = np.arcsin(np.clip(st * np.sin(d0) + ct * np.cos(d0) * np.cos(dphi), -1.0, 1.0))
+    return np.degrees(ra) % 360.0, np.degrees(dec)
+
+
 def write_fits(data, path):
     """Minimal primary-HDU writer (utils.write_fits, caesar_yolo/utils.py:126-134: `fits.PrimaryHDU(data)` with no
     header): 2-D float32 / float64 array -> big-endian payload padded to 2880-byte blocks."""

@@ -12,7 +12,7 @@ import time
 import numpy as np
 import torch
 
-from . import catalog, ops
+from . import catalog, fits as fitsmeta, ops
 from .fits import FitsImage
 from .pipeline import Engine, make_pp_config, run_image
 from .preprocessing import DataPreprocessor
@@ -25,6 +25,14 @@ def _dist_info():
     if dist.is_available() and dist.is_initialized():
         return dist.get_rank(), dist.get_world_size()
     return 0, 1
+
+
+def _as_sources(recs):
+    """cy_det_record array -> cy_source array with the same boxes (what Engine.measure takes)."""
+    src = np.zeros(len(recs), dtype=ops.SRC_DTYPE)
+    for k in ('x1', 'y1', 'x2', 'y2', 'score', 'cls', 'flags', 'tile_id'):
+        src[k] = recs[k]
+    return src
 
 
 class SFinder(object):
@@ -44,6 +52,7 @@ class SFinder(object):
         self.save_tile_json = config.get('save_tile_catalog', False)
         self.save_tile_regions = config.get('save_tile_region', False)
         self.save_tile_img = config.get('save_tile_img', False)
+        self.measure_sources = bool(config.get('measure_sources', False))   # per-source measurements (opt-in)
         self.procId, self.nproc = _dist_info()
         self.timing = {}
         self.engine = None
@@ -120,7 +129,8 @@ class SFinder(object):
         return self.engine
 
     def set_img_size_params(self):
-        """inference.py:354-477 (pixel geometry only; WCS/beam metadata are not used by the catalog)."""
+        """inference.py:354-477 (pixel geometry; the beam / WCS cards of the header are read by the per-source
+        measurements, fits.beam_area_pix / fits.pixel_to_world)."""
         c = self.config
         self.image_id = os.path.splitext(os.path.basename(os.path.abspath(c['image_path'])))[0]
         if os.path.splitext(c['image_path'])[1] in ('.png', '.jpg'):   # inference.py:396-404: size from PIL
@@ -173,11 +183,13 @@ class SFinder(object):
         tiles[0] = (x0, x1, y0, y1)
         t0 = time.time()
         eng.begin(tiles)
+        dev_img = None
+        if self._host_callable() is None or self.measure_sources:
+            img = self.fits.rows(y0, y1)
+            dev_img = torch.from_numpy(np.array(img, copy=True).view(np.int32)).to(eng.device)   # memmap rows are read-only
         if self._host_callable() is not None:
             self._process_tiles_host_callable(eng, tiles, [0], self._host_callable())
         else:
-            img = self.fits.rows(y0, y1)
-            dev_img = torch.from_numpy(np.array(img, copy=True).view(np.int32)).to(eng.device)   # memmap rows are read-only
             eng.process_tiles(dev_img, self.fits.nx, self.fits.is_raw_f32, 0, y0, [0])
         packed, n = eng.finish()
         recs = packed.cpu().numpy().view(ops.REC_DTYPE)
@@ -185,11 +197,25 @@ class SFinder(object):
         # predict() adds no offsets in the serial path (image_xmin/ymin default 0, inference.py:530)
         recs = recs.copy()
         recs['x1'] -= x0; recs['x2'] -= x0; recs['y1'] -= y0; recs['y2'] -= y0
+        meas = None
+        if self.measure_sources:   # in the coordinates of the catalog: the (sub-)image read, columns from x0
+            m = eng.measure(_as_sources(recs), dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0,
+                            y1 - y0)
+            meas = self._measurements(m, self.fits.header, x0, y0)
         self.timing['run_s'] = time.time() - t0
-        return self._save_serial(recs, status)
+        return self._save_serial(recs, status, meas)
 
-    def _save_serial(self, recs, status):
-        self.results = {"image_id": self.image_id, "objs": catalog.records_to_objs(recs, self.class_names)}
+    def _measurements(self, m, header, x0=0, y0=0):
+        """Engine.measure output -> catalog.measurement_dicts with flux (beam area of the header) and the sky position
+        of the centroid (SIN / TAN WCS; x0, y0: offset of the catalog's pixel grid in the file)."""
+        radec = fitsmeta.pixel_to_world(header, m['xc'] + x0, m['yc'] + y0)
+        if radec is None:
+            logger.warning("No RA---SIN/TAN, DEC--SIN/TAN celestial WCS in the image header (CTYPE1=%s, CTYPE2=%s): "
+                           "ra/dec are written as null", header.get('CTYPE1'), header.get('CTYPE2'))
+        return catalog.measurement_dicts(m, fitsmeta.beam_area_pix(header), radec)
+
+    def _save_serial(self, recs, status, meas=None):
+        self.results = {"image_id": self.image_id, "objs": catalog.records_to_objs(recs, self.class_names, meas=meas)}
         if self.write_to_json:
             catalog.write_json(self.results, os.path.join(self.outdir, 'out_' + str(self.image_id) + '.json'))
         if self.write_to_ds9:
@@ -222,10 +248,12 @@ class SFinder(object):
         tiles[0] = (0, W, 0, H)
         t0 = time.time()
         eng.begin(tiles)
+        plane_dev = None
         if gray:
             plane = np.ascontiguousarray(a if a.ndim == 2 else a[:, :, 0], dtype=np.float32)
             plane[~np.isfinite(plane)] = 0
-            eng.process_tiles(torch.from_numpy(plane).to(eng.device), W, False, 0, 0, [0])
+            plane_dev = torch.from_numpy(plane).to(eng.device)
+            eng.process_tiles(plane_dev, W, False, 0, 0, [0])
         else:
             if eng.pp_cfg.nstages > 0:
                 logger.error("Colour image with --preprocessing: the preprocessing chain of this build takes "
@@ -242,8 +270,14 @@ class SFinder(object):
             eng._run_batch(x, status, torch.zeros(1, dtype=torch.int32, device=eng.device), H, W, Sh, Sw, lb)
         packed, n = eng.finish()
         recs = packed.cpu().numpy().view(ops.REC_DTYPE).copy()
+        meas = None
+        if self.measure_sources:
+            if plane_dev is None:
+                logger.warning("Colour image: per-source measurements need a single-plane image and are not written")
+            else:
+                meas = self._measurements(eng.measure(_as_sources(recs), plane_dev, W, False, 0, W, 0, H), {})
         self.timing['run_s'] = time.time() - t0
-        return self._save_serial(recs, 0)
+        return self._save_serial(recs, 0, meas)
 
     def run_parallel(self):
         """Tiled path (inference.py:578-658)."""
@@ -284,19 +318,31 @@ class SFinder(object):
                 st = eng.tile_status[a:b].cpu().numpy()
                 catalog.write_tile_outputs(recs, tiles, np.arange(a, b), st, self.class_names, self.image_id,
                                            self.outdir, self.save_tile_json, self.save_tile_regions)
+        # measurements need the catalog on every rank (each measures its own rows)
+        rank0_only = not self.measure_sources
         if self._host_callable() is not None:
             from .pipeline import split_tile_rows
             eng.begin(tiles)
             a, b = split_tile_rows(tiles, self.nproc)[self.procId]
             eng._my_range = (a, b)
             self._process_tiles_host_callable(eng, tiles, range(a, b), self._host_callable())
-            src, n = eng.exchange_and_merge(self.nproc, rank0_only=True, rank=self.procId, on_local_records=hook)
+            src, n = eng.exchange_and_merge(self.nproc, rank0_only=rank0_only, rank=self.procId,
+                                            on_local_records=hook)
+            if self.measure_sources:   # the tiles went through the host: bring this rank's rows to the GPU
+                Y0, Y1 = (int(tiles['ymin'][a:b].min()), int(tiles['ymax'][a:b].max())) if b > a else (0, 0)
+                band = torch.from_numpy(np.array(self.fits.rows(Y0, Y1), copy=True).view(np.int32)).to(eng.device)
+                eng.band = (band if b > a else None, Y0, Y1, self.fits.nx, self.fits.is_raw_f32)
         else:
             src, n = run_image(eng, img, self.fits.is_raw_f32, tiles, rank=self.procId, world=self.nproc,
-                               on_local_records=hook)
+                               on_rank0_only=rank0_only, on_local_records=hook)
+        meas = None
+        if self.measure_sources:
+            m = eng.measure_band(src, tiles, self.procId, self.nproc)
+            if self.procId == 0:
+                meas = self._measurements(m, self.fits.header)
         self.timing['run_s'] = time.time() - t0
         if self.procId == 0:
-            self.sources = {"sources": catalog.sources_to_dicts(src, self.class_names)}
+            self.sources = {"sources": catalog.sources_to_dicts(src, self.class_names, meas)}
             self.save()
             logger.info("Run completed in %d seconds", int(time.time() - t0))
         return 0

@@ -352,5 +352,36 @@ def merge_global(recs, n, tiles_dev, T, nb_off_dev, nb_idx_dev, out=None):
     return out[:k * SRC_DTYPE.itemsize].cpu().numpy().view(SRC_DTYPE)
 
 
+# ------------------------------------------------------------------------------------------------ measurements
+
+PARTIAL_BYTES = ctypes.sizeof(_capi.SrcPartial)
+MEAS_DTYPE = np.dtype([('npix', '<i8'), ('sum', '<f8'), ('peak', '<f8'), ('peak_x', '<f8'), ('peak_y', '<f8'),
+                       ('xc', '<f8'), ('yc', '<f8'), ('a', '<f8'), ('b', '<f8'), ('theta', '<f8')])
+PARTIAL_DTYPE = np.dtype([('npix', '<i8'), ('peak_idx', '<i8'), ('peak', '<f8'), ('sum', '<f8'), ('sw', '<f8'),
+                          ('swx', '<f8'), ('swy', '<f8'), ('swxx', '<f8'), ('swyy', '<f8'), ('swxy', '<f8')])
+assert MEAS_DTYPE.itemsize == ctypes.sizeof(_capi.SrcMeas) and PARTIAL_DTYPE.itemsize == PARTIAL_BYTES
+
+
+def measure_sources(img, row_stride, big_endian, row0, ncols, src_dev, nsrc, row_begin, row_end, out=None):
+    """cy_measure_sources.  img: device tensor of 4-byte pixels whose first element is (row0, column 0); src_dev: uint8
+    device tensor of nsrc cy_source.  Returns the partials as a uint8 device tensor [nsrc * 80] (synchronises)."""
+    if out is None:
+        out = torch.empty((max(nsrc, 1) * PARTIAL_BYTES,), dtype=torch.uint8, device=src_dev.device)
+    check(lib.cy_measure_sources(ptr(img), c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0),
+                                 c_int(ncols), ptr(src_dev), c_int(nsrc), c_int(row_begin), c_int(row_end), ptr(out),
+                                 cur_stream()))
+    return out[:nsrc * PARTIAL_BYTES]
+
+
+def measure_combine(partials, world, src_dev, nsrc, ncols, out=None):
+    """cy_measure_combine: partials [world * nsrc * 80] uint8 device (rank-major) -> uint8 device tensor of nsrc
+    cy_src_meas."""
+    if out is None:
+        out = torch.empty((max(nsrc, 1) * MEAS_DTYPE.itemsize,), dtype=torch.uint8, device=partials.device)
+    check(lib.cy_measure_combine(ptr(partials), c_int(world), ptr(src_dev), c_int(nsrc), c_int(ncols), ptr(out),
+                                 cur_stream()))
+    return out[:nsrc * MEAS_DTYPE.itemsize]
+
+
 def to_device_bytes(np_array, device):
     return torch.from_numpy(np_array.view(np.uint8).reshape(-1).copy()).to(device)

@@ -127,6 +127,7 @@ class Engine(object):
         self.launches += 1
         self._my_range = (0, self.T)
         self.tile_status = None
+        self.band = None          # (device rows, first row, end row, columns, big_endian) of the last run_image
         if self.collect_tile_status:
             self.tile_status = torch.full((self.T,), -3, dtype=torch.int32, device=self.device)  # -3: not processed
 
@@ -320,6 +321,39 @@ class Engine(object):
         h = torch.cat([tot[:1], counts.max().view(1)]).cpu()
         return allp, int(h[0]), int(h[1])
 
+    def measure(self, sources, img, row_stride, big_endian, row0, ncols, row_begin, row_end, world=1):
+        """Per-source measurements of the catalog `sources` (ops.SRC_DTYPE) over rows [row_begin, row_end) of `img`, a
+        device tensor of 4-byte pixels whose first element is image row row0, column 0 (cy_measure_sources).  With
+        world > 1 every rank passes the same catalog and its own rows: the partials are all-gathered in the group of the
+        record exchange and folded in rank order (cy_measure_combine).  Returns a structured array (ops.MEAS_DTYPE)."""
+        src = np.ascontiguousarray(sources, dtype=ops.SRC_DTYPE)
+        n = len(src)
+        if n == 0:
+            return np.zeros(0, dtype=ops.MEAS_DTYPE)
+        src_dev = ops.to_device_bytes(src, self.device)
+        e = self._mark()
+        part = ops.measure_sources(img, row_stride, big_endian, row0, ncols, src_dev, n, row_begin, row_end,
+                                   out=self._get('meas_part', (n * ops.PARTIAL_BYTES,), torch.uint8))
+        if world > 1:
+            import torch.distributed as dist
+            allp = self._get('meas_gather', (world * n * ops.PARTIAL_BYTES,), torch.uint8)
+            dist.all_gather_into_tensor(allp, part)
+        else:
+            allp = part
+        meas = ops.measure_combine(allp, world, src_dev, n, ncols)
+        self._stage('measure', e)
+        self.launches += 4 + (1 if world > 1 else 0)
+        return meas.cpu().numpy().view(ops.MEAS_DTYPE)
+
+    def measure_band(self, sources, tiles, rank=0, world=1):
+        """Engine.measure over the rows this rank owns (measure_rows), read from the band of mosaic rows the last
+        run_image left in HBM: no second read of the file."""
+        r0, r1 = measure_rows(tiles, world)[rank]
+        band, Y0, _, nx, big_endian = self.band
+        if band is None:                     # a rank without tiles still takes part in the all-gather
+            band, Y0 = self._get('meas_noband', (1,), torch.int32), r0
+        return self.measure(sources, band, nx, big_endian, Y0, nx, r0, r1, world=world)
+
     def _exchange_cap(self, world, need=0):
         """Records per rank slot of the all-gather: 48 per tile of the largest band (the catalogs of the synthetic
         mosaics hold ~20 per tile), grown on demand; kept across steps so the buffers are allocated once."""
@@ -356,6 +390,23 @@ def lead_group_size(ymins, min_tiles=32):
         if k >= min_tiles:
             return k
     return 0
+
+
+def measure_rows(tiles, world):
+    """Row range [r0, r1) of the mosaic each rank measures, from the first row of its band (split_tile_rows) to the first
+    row of the next rank's band; the last rank's range ends with its band.  The ranges partition the rows the run read,
+    in rank order, and each lies inside its rank's band at any tile step, so a hull that crosses a band boundary is
+    measured in parts with no halo.  A rank without tiles gets an empty range."""
+    parts = split_tile_rows(tiles, world)
+    bands = [(int(tiles['ymin'][a:b].min()), int(tiles['ymax'][a:b].max())) if b > a else None for a, b in parts]
+    out = []
+    for r, bd in enumerate(bands):
+        if bd is None:
+            out.append((0, 0))
+            continue
+        nxt = next((b2[0] for b2 in bands[r + 1:] if b2 is not None), bd[1])
+        out.append((bd[0], max(bd[0], min(nxt, bd[1]))))
+    return out
 
 
 def bind_host_to_device_numa(device_index):
@@ -596,4 +647,7 @@ def run_image(engine, img_host, big_endian, tiles, rank=0, world=1, piece_bytes=
             engine.process_tiles(band, nx, big_endian, 0, Y0, ids, ready=ready, min_groups=2)
         finally:
             src.close()
+        engine.band = (band, Y0, Y1, nx, bool(big_endian))
+    else:
+        engine.band = (None, 0, 0, nx, bool(big_endian))
     return engine.exchange_and_merge(world, rank0_only=on_rank0_only, rank=rank, on_local_records=on_local_records)

@@ -242,6 +242,45 @@ int cy_compact_records(const cy_det_record* slots, const int32_t* counts, int T,
 int cy_merge_global(cy_det_record* recs, int n, const cy_tile* tiles, int T, const int32_t* nb_off,
                     const int32_t* nb_idx, cy_source* out, int64_t* nout, uintptr_t stream);
 
+/* ------------------------------------------------------------------------------------------------ source measurements
+ * Per-source numbers the reference catalog does not carry (not part of the reference).  Pixel (x, y) belongs to source
+ * s when x1 <= x <= x2 and y1 <= y <= y2 (catalog coordinates, inclusive), the pixel lies inside the image and the
+ * owned rows, and its value is finite and non-zero (0 = masked, utils.py:219,394).  w = max(v, 0).
+ *
+ * Partial record of one source over one row range.  Every field combines by addition, the peak by max on the key
+ * (peak, -peak_idx), so partials of disjoint row ranges fold into the partial of their union.  The first and second
+ * moments are taken about the box corner (cx, cy) = (ceil(x1), ceil(y1)) — dx = x - cx, dy = y - cy — which is the
+ * same on every rank and keeps fp64 free of the cancellation that absolute mosaic coordinates (~1e4 px) would bring
+ * into the central moments.  peak_idx = y * ncols + x of the first pixel (row-major) that reaches the peak;
+ * npix = 0: peak = -inf, peak_idx = INT64_MAX.  80 bytes. */
+typedef struct {
+    int64_t npix, peak_idx;
+    double peak;
+    double sum;                        /* sum of v */
+    double sw, swx, swy;               /* sum of w, w*dx, w*dy */
+    double swxx, swyy, swxy;           /* sum of w*dx^2, w*dy^2, w*dx*dy */
+} cy_src_partial;
+/* Final values.  xc, yc: w-weighted centroid (NaN when sum w = 0); a >= b: square roots of the eigenvalues of the
+ * w-weighted central second-moment matrix (for a Gaussian source, its sigmas along the major / minor axis); theta: angle
+ * of the major axis in degrees, in (-90, 90], measured from the +x (column) axis towards the +y (row) axis of the pixel
+ * grid — counter-clockwise on the usual FITS display with row 0 at the bottom; it is not a sky position angle.  peak_x,
+ * peak_y: pixel of the peak (NaN when npix = 0).  80 bytes. */
+typedef struct {
+    int64_t npix;
+    double sum, peak, peak_x, peak_y, xc, yc, a, b, theta;
+} cy_src_meas;
+/* img: 4-byte pixels as for cy_preprocess (row_stride elements per row, big_endian = raw FITS byte order); the buffer
+ * holds image rows from row0 on and columns [0, ncols).  Reads rows [row_begin, row_end) (row_begin >= row0, all inside
+ * the buffer) for the nsrc sources src[] (device) and writes partials[nsrc].  Work units are up to 32 rows of one box;
+ * the unit partials of a source are folded in unit order (deterministic for a given row range).  Synchronises the
+ * stream (the unit count is data dependent). */
+int cy_measure_sources(const void* img, long long row_stride, int big_endian, int row0, int ncols, const cy_source* src,
+                       int nsrc, int row_begin, int row_end, cy_src_partial* partials, uintptr_t stream);
+/* partials [world][nsrc] (e.g. all-gathered from `world` ranks that own disjoint row ranges) folded in rank order ->
+ * meas[nsrc].  src and ncols as given to cy_measure_sources. */
+int cy_measure_combine(const cy_src_partial* partials, int world, const cy_source* src, int nsrc, int ncols,
+                       cy_src_meas* meas, uintptr_t stream);
+
 /* ------------------------------------------------------------------------------------------------ whole path
  * FITS file -> merged catalog with no host-language orchestration: SFinder.run_parallel (caesar_yolo/inference.py:
  * 578-658; the serial SFinder.run :485-552 is the tile_x <= 0 case: the whole region is one tile), TileTask.find_sources

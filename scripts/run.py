@@ -67,6 +67,8 @@ def parse_args(argv=None):
     p.add_argument('--save_tile_img', dest='save_tile_img', action='store_true')
     p.add_argument('--precision', required=False, type=str, default=None, choices=['fp16', 'bf16'],
                    help='B200 build only: 16-bit storage of weights/activations (default fp16; same tensor-core rate)')
+    p.add_argument('--measure_sources', dest='measure_sources', action='store_true',
+                   help='B200 build only: add peak, flux density, centroid, shape and sky position to every catalog source')
     p.add_argument('--detect_outfile', required=False, type=str, default="")
     p.add_argument('--detect_outfile_json', required=False, type=str, default="")
     return p.parse_args(argv)
@@ -161,7 +163,7 @@ def main(argv=None):
         'outfile_json': args.detect_outfile_json, 'draw_plot': args.draw_plots,
         'draw_class_label_in_caption': args.draw_class_label_in_caption, 'save_plot': args.save_plots,
         'save_tile_catalog': args.save_tile_catalog, 'save_tile_region': args.save_tile_region,
-        'save_tile_img': args.save_tile_img, 'precision': args.precision,
+        'save_tile_img': args.save_tile_img, 'precision': args.precision, 'measure_sources': args.measure_sources,
     })
     model = YOLO(args.weights, precision=args.precision)
     sfinder = SFinder(model, CONFIG)

@@ -1,0 +1,94 @@
+#!/usr/bin/env python
+"""Per-source measurements split over ranks, under torchrun: every rank runs pipeline.run_image on its band of bench.py's
+16k synthetic mosaic (config 3: YOLOv8l, full preprocessing chain), then Engine.measure_band over the rows it owns with
+one all-gather of the partials, exactly as SFinder.run_parallel(measure_sources=True) does; every rank then repeats the
+run alone (world 1, all rows) and compares: the catalog byte for byte, npix / peak / peak_x / peak_y exactly, the
+floating-point fields within --rtol relative.  Relative differences are taken against max(|a|, |b|); `sum` is compared
+against the sum of |sum| over the catalog's sources when its own value is tiny against it (a near-zero sum of signed
+pixels differs by reassociation only).
+
+usage: python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/measure_multirank.py
+       (--backend gloo: the same with the ranks sharing one GPU)
+Prints one JSON line on rank 0 with the largest relative difference per field and the verdict of every rank."""
+import argparse
+import json
+import os
+import sys
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+import bench  # noqa: E402  (mosaic generator, model and thresholds of the benchmark)
+
+FLOATS = ('sum', 'xc', 'yc', 'a', 'b', 'theta')
+EXACT = ('npix', 'peak', 'peak_x', 'peak_y')
+
+
+def compare(m, r):
+    """Largest relative difference per float field (NaN positions must agree) and exactness of the integer fields."""
+    out = {}
+    for k in EXACT:
+        out[k + '_exact'] = bool(np.array_equal(m[k], r[k], equal_nan=True))
+    for k in FLOATS:
+        a, b = m[k].astype(np.float64), r[k].astype(np.float64)
+        if not np.array_equal(np.isnan(a), np.isnan(b)):
+            out[k] = float('inf')
+            continue
+        ok = ~np.isnan(a)
+        scale = np.maximum(np.abs(a[ok]), np.abs(b[ok]))
+        if k == 'sum':
+            scale = np.maximum(scale, 1e-6 * np.abs(b[ok]).sum())
+        d = np.abs(a[ok] - b[ok]) / np.where(scale > 0, scale, 1.0)
+        out[k] = float(d.max()) if d.size else 0.0
+    return out
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument('--mosaic', type=int, default=16384)
+    ap.add_argument('--variant', default='l')
+    ap.add_argument('--rtol', type=float, default=1e-12)
+    ap.add_argument('--backend', default='nccl', choices=['nccl', 'gloo'],
+                    help='gloo lets several ranks share one GPU (NCCL needs one GPU per rank)')
+    a = ap.parse_args()
+    import torch
+    import torch.distributed as dist
+    from caesar_yolo_b200 import ops, pipeline, weights as W
+    rank, world, local = int(os.environ['RANK']), int(os.environ['WORLD_SIZE']), int(os.environ['LOCAL_RANK'])
+    local %= torch.cuda.device_count()
+    torch.cuda.set_device(local)
+    dev = torch.device('cuda', local)
+    if a.backend == 'nccl':
+        dist.init_process_group('nccl', device_id=dev)
+    else:
+        dist.init_process_group('gloo')
+    _, host = bench.make_mosaic_pinned(argparse.Namespace(mosaic=a.mosaic))
+    n = a.mosaic
+    tiles = ops.generate_tiles(0, n - 1, 0, n - 1, 512, 512, 1.0, 1.0)
+    w = W.make_random_weights(a.variant, 5, seed=0, cls_bias=bench.CLS_BIAS.get(a.variant, -16.0))
+    eng = pipeline.Engine(w, pipeline.make_pp_config(**bench.PP_FLAGS), imgsz=640, score_thr=bench.SCORE_THR,
+                          iou_thr=bench.IOU_THR, thr_soft=bench.SOFT, thr_hard=bench.HARD, device=dev)
+    src, _ = pipeline.run_image(eng, host, True, tiles, rank=rank, world=world, on_rank0_only=False)
+    meas = eng.measure_band(src, tiles, rank, world)
+    rows = pipeline.measure_rows(tiles, world)[rank]
+    ref, _ = pipeline.run_image(eng, host, True, tiles)
+    ref_meas = eng.measure_band(ref, tiles)
+    res = compare(meas, ref_meas)
+    same_catalog = bool(src.tobytes() == ref.tobytes())
+    ok = same_catalog and all(res[k + '_exact'] for k in EXACT) and all(res[k] <= a.rtol for k in FLOATS)
+    flags = torch.tensor([1 if ok else 0], device=dev if a.backend == 'nccl' else 'cpu')
+    dist.all_reduce(flags, op=dist.ReduceOp.MIN)
+    if rank == 0:
+        print(json.dumps(dict(world=world, backend=a.backend, gpus=torch.cuda.device_count(), mosaic=n,
+                              sources=int(len(src)), rows_of_rank0=list(rows),
+                              catalog_identical=same_catalog, max_rel_diff={k: res[k] for k in FLOATS},
+                              exact={k: res[k + '_exact'] for k in EXACT}, rtol=a.rtol,
+                              matches_single_rank_on_every_rank=bool(int(flags[0])))), flush=True)
+    dist.destroy_process_group()
+    return 0 if int(flags[0]) else 1
+
+
+if __name__ == '__main__':
+    sys.exit(main())
