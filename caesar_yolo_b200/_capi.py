@@ -89,7 +89,19 @@ class SrcMeas(ctypes.Structure):
                 ("xc", c_double), ("yc", c_double), ("a", c_double), ("b", c_double), ("theta", c_double)]
 
 
+class NoisePartial(ctypes.Structure):
+    """cy_noise_partial: one source's clipped frame sums over one row range and one pass."""
+    _fields_ = [("n", c_i64), ("s1", c_double), ("s2", c_double)]
+
+
+class NoiseState(ctypes.Structure):
+    """cy_noise_state: clipping state of one source; bkg, rms, nbkg, iters are final once done."""
+    _fields_ = [("lo", c_double), ("hi", c_double), ("c", c_double), ("bkg", c_double), ("rms", c_double),
+                ("nbkg", c_i64), ("iters", ctypes.c_int32), ("done", ctypes.c_int32)]
+
+
 assert ctypes.sizeof(SrcPartial) == 80 and ctypes.sizeof(SrcMeas) == 80
+assert ctypes.sizeof(NoisePartial) == 24 and ctypes.sizeof(NoiseState) == 56
 
 
 ALLGATHER_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t,
@@ -106,6 +118,7 @@ SYMBOLS = [
     "cy_stem_conv_nhwc4", "cy_model_profile", "cy_model_conv_bytes", "cy_model_destroy", "cy_num_anchors", "cy_decode_pred", "cy_postprocess_scratch_bytes",
     "cy_postprocess", "cy_nms_scratch_bytes", "cy_nms_batched", "cy_merge_tile", "cy_make_records",
     "cy_compact_scratch_bytes", "cy_compact_records", "cy_merge_global", "cy_measure_sources", "cy_measure_combine",
+    "cy_noise_init", "cy_noise_pass", "cy_noise_update",
     "cy_ctx_create", "cy_ctx_set_allgather", "cy_ctx_destroy", "cy_run_local", "cy_run_local_payload", "cy_ctx_records",
     "cy_ctx_pack_slot", "cy_ctx_unpack_slots", "cy_run_merge", "cy_run_mosaic", "cy_run_payload", "cy_ctx_info",
 ]

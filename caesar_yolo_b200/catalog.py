@@ -24,9 +24,14 @@ def _num(v):
     return v if math.isfinite(v) else None      # JSON null
 
 
-def measurement_dicts(meas, beam_area_pix=None, radec=None):
+# local background / noise keys (Engine.measure_noise); written only when the noise is measured
+NOISE_KEYS = ('bkg', 'rms', 'nbkg', 'snr', 'flux_bkgsub', 'flux_err')
+
+
+def measurement_dicts(meas, beam_area_pix=None, radec=None, noise=None):
     """ops.MEAS_DTYPE array -> one dict of MEASURE_KEYS per source.  flux = sum / beam_area_pix (None without a beam);
-    radec: (ra, dec) arrays of the centroids in degrees, or None.  Non-finite values become None (JSON null)."""
+    radec: (ra, dec) arrays of the centroids in degrees, or None.  noise: ops.NOISE_DTYPE array of the same sources, or
+    None; with it the dicts also get NOISE_KEYS (noise_keys).  Non-finite values become None (JSON null)."""
     out = []
     for i, m in enumerate(meas):
         d = {"npix": int(m['npix'])}
@@ -35,8 +40,35 @@ def measurement_dicts(meas, beam_area_pix=None, radec=None):
         d["flux"] = _num(m['sum'] / beam_area_pix) if beam_area_pix else None
         d["ra"] = _num(radec[0][i]) if radec is not None else None
         d["dec"] = _num(radec[1][i]) if radec is not None else None
+        if noise is not None:
+            d.update(noise_keys(m, noise[i], beam_area_pix))
         out.append(d)
     return out
+
+
+def noise_keys(m, z, beam_area_pix=None):
+    """NOISE_KEYS of one source from its measurements m (ops.MEAS_DTYPE) and clipped frame statistics z
+    (ops.NOISE_DTYPE), A = beam_area_pix:
+      bkg, rms     clipped mean / std of the frame (None when nbkg = 0)
+      nbkg         pixels in the final kept set
+      snr          (peak - bkg) / rms (None without a peak, when nbkg = 0 or rms = 0)
+      flux_bkgsub  (sum - npix * bkg) / A
+      flux_err     rms * sqrt(npix * min(npix, A)) / A: the noise taken as correlated over one beam, so it is
+                   rms * sqrt(npix / A) for a box much larger than the beam and rms * npix / A for one smaller than it
+    (flux_bkgsub and flux_err are None without a beam area or when nbkg = 0)."""
+    nb = int(z['nbkg'])
+    d = {"nbkg": nb, "bkg": None, "rms": None, "snr": None, "flux_bkgsub": None, "flux_err": None}
+    if nb == 0:
+        return d
+    bkg, rms, npix = float(z['bkg']), float(z['rms']), int(m['npix'])
+    d["bkg"], d["rms"] = _num(bkg), _num(rms)
+    if npix > 0 and rms > 0:
+        d["snr"] = _num((float(m['peak']) - bkg) / rms)
+    if beam_area_pix:
+        A = float(beam_area_pix)
+        d["flux_bkgsub"] = _num((float(m['sum']) - npix * bkg) / A)
+        d["flux_err"] = _num(rms * math.sqrt(npix * min(npix, A)) / A)
+    return d
 
 
 def sources_to_dicts(src, names, meas=None):

@@ -44,4 +44,8 @@ CONFIG = {
     'save_plot': False,
     # - Per-source measurements (not in the reference): peak, flux density, centroid, shape, sky position
     'measure_sources': False,
+    # - Local background, noise and S/N of every source (not in the reference; implies measure_sources): sigma-clipped
+    #   mean / std of a frame of noise_frame pixels around each box
+    'measure_noise': False,
+    'noise_frame': 16,
 }

@@ -1,6 +1,7 @@
 // Per-source measurements over the catalog boxes (cy_measure_sources / cy_measure_combine, include/caesar_b200.h):
 // pixel count, flux sum, peak and weighted first / second moments of the box pixels, read straight from the mosaic
-// rows that are already in HBM.
+// rows that are already in HBM.  The local background and noise (cy_noise_init / cy_noise_pass / cy_noise_update) take
+// the sigma-clipped mean and standard deviation of a frame around each box from the same rows, one pass per clip.
 //
 // Work is split into units of up to kUnitRows rows of one box, so that a merged hull of thousands of rows spreads over
 // many CTAs.  Every unit writes its own partial; the partials of a source are then folded in unit order, and
@@ -91,28 +92,42 @@ __device__ __forceinline__ Acc acc_shfl_down(const Acc& a, int d) {
     return b;
 }
 
-// Pixel rectangle of source s inside the owned rows, inclusive bounds; false when empty.  Catalog coordinates are
-// integer valued; ceil / floor keep the membership rule x1 <= x <= x2 exact for any value.
+// Pixel rectangle of source s grown by `grow` pixels on every side (0: the box itself; the noise frame's outer edge),
+// inside the image columns and the owned rows, inclusive bounds; false when empty or when the box itself is empty.
+// Catalog coordinates are integer valued; ceil / floor keep the membership rule x1 <= x <= x2 exact for any value.
 struct Box {
     int x0, x1, y0, y1;
 };
-__device__ __forceinline__ bool source_box(const cy_source& s, int ncols, int row_begin, int row_end, Box& b) {
+__device__ __forceinline__ bool source_box(const cy_source& s, int grow, int ncols, int row_begin, int row_end, Box& b) {
     const double bx0 = ceil((double)s.x1), bx1 = floor((double)s.x2);
     const double by0 = ceil((double)s.y1), by1 = floor((double)s.y2);
     // the comparisons are false for NaN coordinates
-    if (!(bx0 <= bx1 && by0 <= by1 && bx0 <= ncols - 1.0 && bx1 >= 0.0 && by0 <= row_end - 1.0 && by1 >= row_begin))
-        return false;
-    b.x0 = (int)fmax(bx0, 0.0);
-    b.x1 = (int)fmin(bx1, ncols - 1.0);
-    b.y0 = (int)fmax(by0, (double)row_begin);
-    b.y1 = (int)fmin(by1, row_end - 1.0);
+    if (!(bx0 <= bx1 && by0 <= by1)) return false;
+    const double gx0 = bx0 - grow, gx1 = bx1 + grow, gy0 = by0 - grow, gy1 = by1 + grow;
+    if (!(gx0 <= ncols - 1.0 && gx1 >= 0.0 && gy0 <= row_end - 1.0 && gy1 >= row_begin)) return false;
+    b.x0 = (int)fmax(gx0, 0.0);
+    b.x1 = (int)fmin(gx1, ncols - 1.0);
+    b.y0 = (int)fmax(gy0, (double)row_begin);
+    b.y1 = (int)fmin(gy1, row_end - 1.0);
     return b.y0 <= b.y1;   // empty when row_begin == row_end
 }
 
-// units per source -> exclusive offsets off[0..nsrc] (one CTA, chunks of kScanThreads sources carried in order)
+// source of work unit u: s with off[s] <= u < off[s + 1] (empty sources share offsets: take the last)
+__device__ __forceinline__ int unit_source(const long long* __restrict__ off, int nsrc, long long u) {
+    int lo = 0, hi = nsrc - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (off[mid] <= u) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+
+// units per source (rows of the box grown by `grow`) -> exclusive offsets off[0..nsrc] (one CTA, chunks of
+// kScanThreads sources carried in order)
 __global__ void __launch_bounds__(kScanThreads) measure_units_scan_kernel(const cy_source* __restrict__ src, int nsrc,
-                                                                           int ncols, int row_begin, int row_end,
-                                                                           long long* __restrict__ off) {
+                                                                           int grow, int ncols, int row_begin,
+                                                                           int row_end, long long* __restrict__ off) {
     __shared__ long long warp_tot[kScanThreads / 32];
     __shared__ long long carry;
     const int t = threadIdx.x, lane = t & 31, w = t >> 5;
@@ -122,7 +137,7 @@ __global__ void __launch_bounds__(kScanThreads) measure_units_scan_kernel(const 
         const int s = base + t;
         long long c = 0;
         Box b;
-        if (s < nsrc && source_box(src[s], ncols, row_begin, row_end, b)) c = (b.y1 - b.y0) / kUnitRows + 1;
+        if (s < nsrc && source_box(src[s], grow, ncols, row_begin, row_end, b)) c = (b.y1 - b.y0) / kUnitRows + 1;
         long long inc = c;
         for (int d = 1; d < 32; d <<= 1) {
             const long long v = __shfl_up_sync(0xffffffffu, inc, d);
@@ -149,15 +164,9 @@ __global__ void __launch_bounds__(kThreads) measure_unit_kernel(const uint32_t* 
                                                                 cy_src_partial* __restrict__ unit_out) {
     __shared__ Acc warp_acc[kThreads / 32];
     const long long u = blockIdx.x;
-    int lo = 0, hi = nsrc - 1;   // source s with off[s] <= u < off[s + 1] (empty sources share offsets: take the last)
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (off[mid] <= u) lo = mid;
-        else hi = mid - 1;
-    }
-    const int s = lo;
+    const int s = unit_source(off, nsrc, u);
     Box b;
-    source_box(src[s], ncols, row_begin, row_end, b);
+    source_box(src[s], 0, ncols, row_begin, row_end, b);
     const int ya = b.y0 + (int)(u - off[s]) * kUnitRows;
     const int yb = min(b.y1, ya + kUnitRows - 1);
     const double cx = ceil((double)src[s].x1), cy = ceil((double)src[s].y1);   // moments about the box corner
@@ -251,6 +260,157 @@ __global__ void measure_combine_kernel(const cy_src_partial* __restrict__ part, 
     out[s] = m;
 }
 
+// ---------------------------------------------------------------------------------------------- frame noise
+// One pass of the iterative sigma clipping of every active source's frame (cy_noise_pass / cy_noise_update): the units
+// are the rows of the grown box (measure_units_scan_kernel with grow = frame), scanned once per measurement.
+
+constexpr double kClipSigma = 3.0;   // kappa
+constexpr int kClipMaxIters = 5;     // passes 0..5: the statistics of all pixels, then up to 5 clipped sets
+
+struct NAcc {
+    long long n;
+    double s1, s2;
+};
+
+__device__ __forceinline__ void nacc_merge(NAcc& a, const NAcc& b) {
+    a.n += b.n;
+    a.s1 += b.s1;
+    a.s2 += b.s2;
+}
+
+__global__ void noise_init_kernel(int nsrc, cy_noise_state* __restrict__ state) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= nsrc) return;
+    cy_noise_state t;
+    t.lo = -INFINITY;
+    t.hi = INFINITY;
+    t.c = 0.0;
+    t.bkg = t.rms = __longlong_as_double(0x7ff8000000000000ll);
+    t.nbkg = 0;
+    t.iters = 0;
+    t.done = 0;
+    state[s] = t;
+}
+
+// one CTA per unit: sums of (v - c), (v - c)^2 over the frame pixels of up to kUnitRows rows of one grown box that lie
+// inside the source's kept interval [lo, hi].  Rows inside the box's row span read the two side segments, packed into
+// one run of lane indices; other rows read the full grown width.  A converged source's units return at once.
+__global__ void __launch_bounds__(kThreads) noise_unit_kernel(const uint32_t* __restrict__ img, long long row_stride,
+                                                              int big_endian, int row0, int ncols,
+                                                              const cy_source* __restrict__ src, int nsrc,
+                                                              int row_begin, int row_end, int frame,
+                                                              const long long* __restrict__ off,
+                                                              const cy_noise_state* __restrict__ state,
+                                                              cy_noise_partial* __restrict__ unit_out) {
+    __shared__ NAcc warp_acc[kThreads / 32];
+    const long long u = blockIdx.x;
+    const int s = unit_source(off, nsrc, u);
+    if (state[s].done) return;
+    const double lo = state[s].lo, hi = state[s].hi, c = state[s].c;
+    Box g;
+    source_box(src[s], frame, ncols, row_begin, row_end, g);
+    const double bx0 = ceil((double)src[s].x1), bx1 = floor((double)src[s].x2);
+    const double by0 = ceil((double)src[s].y1), by1 = floor((double)src[s].y2);
+    // side segments of a box row: [g.x0, g.x0 + nl) and [r0, r0 + nr), both inside [g.x0, g.x1]
+    const int l1 = (int)fmax(fmin(bx0 - 1.0, (double)g.x1), g.x0 - 1.0);
+    const int r0 = (int)fmin(fmax(bx1 + 1.0, (double)g.x0), g.x1 + 1.0);
+    const int side_l = l1 - g.x0 + 1, side_r = g.x1 - r0 + 1;
+    const int ya = g.y0 + (int)(u - off[s]) * kUnitRows;
+    const int yb = min(g.y1, ya + kUnitRows - 1);
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    NAcc a = {0, 0.0, 0.0};
+    for (int y = ya + w; y <= yb; y += kThreads / 32) {
+        const uint32_t* row = img + (long long)(y - row0) * row_stride;
+        const bool in_box = (double)y >= by0 && (double)y <= by1;
+        const int nl = in_box ? side_l : g.x1 - g.x0 + 1, nr = in_box ? side_r : 0;
+        for (int i = lane; i < nl + nr; i += 32) {
+            const int x = i < nl ? g.x0 + i : r0 + (i - nl);
+            uint32_t raw = __ldg(row + x);
+            if (big_endian) raw = __byte_perm(raw, 0, 0x0123);
+            const float f = __uint_as_float(raw);
+            if (!isfinite(f) || f == 0.0f) continue;   // the masking rule of the box measurements
+            const double v = (double)f;
+            if (!(v >= lo && v <= hi)) continue;
+            const double d = v - c;
+            a.n += 1;
+            a.s1 += d;
+            a.s2 += d * d;
+        }
+    }
+    for (int d = 16; d > 0; d >>= 1) {
+        NAcc o;
+        o.n = __shfl_down_sync(0xffffffffu, a.n, d);
+        o.s1 = __shfl_down_sync(0xffffffffu, a.s1, d);
+        o.s2 = __shfl_down_sync(0xffffffffu, a.s2, d);
+        nacc_merge(a, o);
+    }
+    if (lane == 0) warp_acc[w] = a;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        NAcc t = warp_acc[0];
+        for (int k = 1; k < kThreads / 32; ++k) nacc_merge(t, warp_acc[k]);
+        unit_out[u].n = t.n;
+        unit_out[u].s1 = t.s1;
+        unit_out[u].s2 = t.s2;
+    }
+}
+
+// unit partials of each active source, folded in unit order -> one partial per source (zero without units)
+__global__ void noise_fold_kernel(const cy_noise_partial* __restrict__ unit, const long long* __restrict__ off,
+                                  int nsrc, const cy_noise_state* __restrict__ state,
+                                  cy_noise_partial* __restrict__ out) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= nsrc || state[s].done) return;
+    NAcc a = {0, 0.0, 0.0};
+    for (long long u = off[s]; u < off[s + 1]; ++u) {
+        const NAcc b = {unit[u].n, unit[u].s1, unit[u].s2};
+        nacc_merge(a, b);
+    }
+    out[s].n = a.n;
+    out[s].s1 = a.s1;
+    out[s].s2 = a.s2;
+}
+
+// partials [world][nsrc] folded in rank order -> statistics of the pass just run; either the source stops (final bkg,
+// rms, nbkg, iters) or its interval, shift and pass index advance.  *active counts the sources that go on.
+__global__ void noise_update_kernel(const cy_noise_partial* __restrict__ part, int world, int nsrc,
+                                    cy_noise_state* __restrict__ state, int* __restrict__ active) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= nsrc) return;
+    cy_noise_state t = state[s];
+    if (t.done) return;
+    NAcc a = {0, 0.0, 0.0};
+    for (int r = 0; r < world; ++r) {
+        const cy_noise_partial& p = part[(long long)r * nsrc + s];
+        const NAcc b = {p.n, p.s1, p.s2};
+        nacc_merge(a, b);
+    }
+    const int k = t.iters;   // index of the pass just run
+    if (a.n == 0) {          // empty frame (a clipped set is never empty: it holds the pixels within sigma of the mean)
+        t.nbkg = 0;
+        t.bkg = t.rms = __longlong_as_double(0x7ff8000000000000ll);
+        t.done = 1;
+        state[s] = t;
+        return;
+    }
+    const double m1 = a.s1 / (double)a.n;
+    const double mu = t.c + m1;
+    const double sd = sqrt(fmax(a.s2 / (double)a.n - m1 * m1, 0.0));
+    t.bkg = mu;
+    t.rms = sd;
+    if ((k >= 1 && a.n == t.nbkg) || k == kClipMaxIters) {
+        t.done = 1;
+    } else {
+        t.lo = fmax(t.lo, mu - kClipSigma * sd);
+        t.hi = fmin(t.hi, mu + kClipSigma * sd);
+        t.c = mu;
+        t.iters = k + 1;
+        atomicAdd(active, 1);
+    }
+    t.nbkg = a.n;
+    state[s] = t;
+}
+
 }  // namespace
 
 extern "C" int cy_measure_sources(const void* img, long long row_stride, int big_endian, int row0, int ncols,
@@ -263,7 +423,7 @@ extern "C" int cy_measure_sources(const void* img, long long row_stride, int big
     cudaStream_t st = (cudaStream_t)stream;
     long long* off = nullptr;
     CY_CUDA_CHECK(cudaMallocAsync(&off, (size_t)(nsrc + 1) * sizeof(long long), st));
-    measure_units_scan_kernel<<<1, kScanThreads, 0, st>>>(src, nsrc, ncols, row_begin, row_end, off);
+    measure_units_scan_kernel<<<1, kScanThreads, 0, st>>>(src, nsrc, 0, ncols, row_begin, row_end, off);
     // the unit count is data dependent: bring it to the host
     long long units = 0;
     cudaMemcpyAsync(&units, off + nsrc, sizeof(long long), cudaMemcpyDeviceToHost, st);
@@ -300,5 +460,69 @@ extern "C" int cy_measure_combine(const cy_src_partial* partials, int world, con
     measure_combine_kernel<<<(nsrc + 255) / 256, 256, 0, (cudaStream_t)stream>>>(partials, world, src, nsrc, ncols, meas);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_measure_combine: %s", cudaGetErrorString(e));
+    return CY_OK;
+}
+
+extern "C" int cy_noise_init(const cy_source* src, int nsrc, int ncols, int row_begin, int row_end, int frame,
+                             cy_noise_state* state, long long* unit_off, long long* units, uintptr_t stream) {
+    if (nsrc < 0 || ncols <= 0 || row_end < row_begin || frame < 1 || !units)
+        return set_error(CY_ERR_INVALID, "cy_noise_init: invalid image geometry, row range or frame width");
+    *units = 0;
+    if (nsrc == 0) return CY_OK;
+    if (!src || !state || !unit_off) return set_error(CY_ERR_INVALID, "cy_noise_init: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    noise_init_kernel<<<(nsrc + 255) / 256, 256, 0, st>>>(nsrc, state);
+    measure_units_scan_kernel<<<1, kScanThreads, 0, st>>>(src, nsrc, frame, ncols, row_begin, row_end, unit_off);
+    long long n = 0;   // the unit count is data dependent: bring it to the host
+    cudaMemcpyAsync(&n, unit_off + nsrc, sizeof(long long), cudaMemcpyDeviceToHost, st);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_noise_init: %s", cudaGetErrorString(e));
+    if (n > 2147483647ll) return set_error(CY_ERR_INVALID, "cy_noise_init: %lld work units exceed one grid", n);
+    *units = n;
+    return CY_OK;
+}
+
+extern "C" int cy_noise_pass(const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                             const cy_source* src, int nsrc, int row_begin, int row_end, int frame,
+                             const long long* unit_off, long long units, const cy_noise_state* state,
+                             cy_noise_partial* partials, uintptr_t stream) {
+    if (nsrc < 0 || ncols <= 0 || row_stride < ncols || row_begin < row0 || row_end < row_begin || frame < 1 ||
+        units < 0 || units > 2147483647ll)
+        return set_error(CY_ERR_INVALID, "cy_noise_pass: invalid image geometry, row range, frame or unit count");
+    if (nsrc == 0) return CY_OK;
+    if (!src || !unit_off || !state || !partials || (units > 0 && !img))
+        return set_error(CY_ERR_INVALID, "cy_noise_pass: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    cy_noise_partial* unit = nullptr;
+    if (units > 0 && cudaMallocAsync(&unit, (size_t)units * sizeof(cy_noise_partial), st) != cudaSuccess)
+        return set_error(CY_ERR_NOMEM, "cy_noise_pass: no memory for %lld unit partials", units);
+    if (units > 0)
+        noise_unit_kernel<<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian, row0,
+                                                                ncols, src, nsrc, row_begin, row_end, frame, unit_off,
+                                                                state, unit);
+    noise_fold_kernel<<<(nsrc + 255) / 256, 256, 0, st>>>(unit, unit_off, nsrc, state, partials);
+    const cudaError_t e = cudaGetLastError();
+    if (unit) cudaFreeAsync(unit, st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_noise_pass: %s", cudaGetErrorString(e));
+    return CY_OK;
+}
+
+extern "C" int cy_noise_update(const cy_noise_partial* partials, int world, int nsrc, cy_noise_state* state,
+                               int* active, uintptr_t stream) {
+    if (world < 1 || nsrc < 0 || !active) return set_error(CY_ERR_INVALID, "cy_noise_update: invalid arguments");
+    *active = 0;
+    if (nsrc == 0) return CY_OK;
+    if (!partials || !state) return set_error(CY_ERR_INVALID, "cy_noise_update: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    int* cnt = nullptr;
+    CY_CUDA_CHECK(cudaMallocAsync(&cnt, sizeof(int), st));
+    cudaMemsetAsync(cnt, 0, sizeof(int), st);
+    noise_update_kernel<<<(nsrc + 255) / 256, 256, 0, st>>>(partials, world, nsrc, state, cnt);
+    int n = 0;
+    cudaMemcpyAsync(&n, cnt, sizeof(int), cudaMemcpyDeviceToHost, st);
+    cudaFreeAsync(cnt, st);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_noise_update: %s", cudaGetErrorString(e));
+    *active = n;
     return CY_OK;
 }

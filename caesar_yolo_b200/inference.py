@@ -52,7 +52,10 @@ class SFinder(object):
         self.save_tile_json = config.get('save_tile_catalog', False)
         self.save_tile_regions = config.get('save_tile_region', False)
         self.save_tile_img = config.get('save_tile_img', False)
-        self.measure_sources = bool(config.get('measure_sources', False))   # per-source measurements (opt-in)
+        # per-source measurements (opt-in); the local noise needs the peak and sum of the box, so it implies them
+        self.measure_noise = bool(config.get('measure_noise', False))
+        self.measure_sources = bool(config.get('measure_sources', False)) or self.measure_noise
+        self.noise_frame = int(config.get('noise_frame', 16))
         self.procId, self.nproc = _dist_info()
         self.timing = {}
         self.engine = None
@@ -199,20 +202,22 @@ class SFinder(object):
         recs['x1'] -= x0; recs['x2'] -= x0; recs['y1'] -= y0; recs['y2'] -= y0
         meas = None
         if self.measure_sources:   # in the coordinates of the catalog: the (sub-)image read, columns from x0
-            m = eng.measure(_as_sources(recs), dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0,
-                            y1 - y0)
-            meas = self._measurements(m, self.fits.header, x0, y0)
+            args = (_as_sources(recs), dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0)
+            m = eng.measure(*args)
+            noise = eng.measure_noise(*args, frame=self.noise_frame) if self.measure_noise else None
+            meas = self._measurements(m, self.fits.header, x0, y0, noise)
         self.timing['run_s'] = time.time() - t0
         return self._save_serial(recs, status, meas)
 
-    def _measurements(self, m, header, x0=0, y0=0):
+    def _measurements(self, m, header, x0=0, y0=0, noise=None):
         """Engine.measure output -> catalog.measurement_dicts with flux (beam area of the header) and the sky position
-        of the centroid (SIN / TAN WCS; x0, y0: offset of the catalog's pixel grid in the file)."""
+        of the centroid (SIN / TAN WCS; x0, y0: offset of the catalog's pixel grid in the file); noise: the
+        Engine.measure_noise output of the same sources, or None."""
         radec = fitsmeta.pixel_to_world(header, m['xc'] + x0, m['yc'] + y0)
         if radec is None:
             logger.warning("No RA---SIN/TAN, DEC--SIN/TAN celestial WCS in the image header (CTYPE1=%s, CTYPE2=%s): "
                            "ra/dec are written as null", header.get('CTYPE1'), header.get('CTYPE2'))
-        return catalog.measurement_dicts(m, fitsmeta.beam_area_pix(header), radec)
+        return catalog.measurement_dicts(m, fitsmeta.beam_area_pix(header), radec, noise)
 
     def _save_serial(self, recs, status, meas=None):
         self.results = {"image_id": self.image_id, "objs": catalog.records_to_objs(recs, self.class_names, meas=meas)}
@@ -275,7 +280,9 @@ class SFinder(object):
             if plane_dev is None:
                 logger.warning("Colour image: per-source measurements need a single-plane image and are not written")
             else:
-                meas = self._measurements(eng.measure(_as_sources(recs), plane_dev, W, False, 0, W, 0, H), {})
+                args = (_as_sources(recs), plane_dev, W, False, 0, W, 0, H)
+                noise = eng.measure_noise(*args, frame=self.noise_frame) if self.measure_noise else None
+                meas = self._measurements(eng.measure(*args), {}, noise=noise)
         self.timing['run_s'] = time.time() - t0
         return self._save_serial(recs, 0, meas)
 
@@ -338,8 +345,11 @@ class SFinder(object):
         meas = None
         if self.measure_sources:
             m = eng.measure_band(src, tiles, self.procId, self.nproc)
+            noise = None
+            if self.measure_noise:
+                noise = eng.measure_noise_band(src, tiles, self.noise_frame, self.procId, self.nproc)
             if self.procId == 0:
-                meas = self._measurements(m, self.fits.header)
+                meas = self._measurements(m, self.fits.header, noise=noise)
         self.timing['run_s'] = time.time() - t0
         if self.procId == 0:
             self.sources = {"sources": catalog.sources_to_dicts(src, self.class_names, meas)}

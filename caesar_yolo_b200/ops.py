@@ -383,5 +383,40 @@ def measure_combine(partials, world, src_dev, nsrc, ncols, out=None):
     return out[:nsrc * MEAS_DTYPE.itemsize]
 
 
+NOISE_PARTIAL_BYTES = ctypes.sizeof(_capi.NoisePartial)
+NOISE_DTYPE = np.dtype([('lo', '<f8'), ('hi', '<f8'), ('c', '<f8'), ('bkg', '<f8'), ('rms', '<f8'), ('nbkg', '<i8'),
+                        ('iters', '<i4'), ('done', '<i4')])
+NOISE_PARTIAL_DTYPE = np.dtype([('n', '<i8'), ('s1', '<f8'), ('s2', '<f8')])
+NOISE_MAX_PASSES = 6   # pass 0 and up to 5 clipping iterations
+assert NOISE_DTYPE.itemsize == ctypes.sizeof(_capi.NoiseState) and NOISE_PARTIAL_DTYPE.itemsize == NOISE_PARTIAL_BYTES
+
+
+def noise_init(src_dev, nsrc, ncols, row_begin, row_end, frame, state, unit_off):
+    """cy_noise_init.  state: uint8 device tensor of >= nsrc cy_noise_state; unit_off: int64 device tensor of >= nsrc + 1
+    elements.  Returns the number of work units (synchronises)."""
+    units = c_i64(0)
+    check(lib.cy_noise_init(ptr(src_dev), c_int(nsrc), c_int(ncols), c_int(row_begin), c_int(row_end), c_int(frame),
+                            ptr(state), ptr(unit_off), ctypes.byref(units), cur_stream()))
+    return units.value
+
+
+def noise_pass(img, row_stride, big_endian, row0, ncols, src_dev, nsrc, row_begin, row_end, frame, unit_off, units,
+               state, out):
+    """cy_noise_pass: one clipping pass over this range's rows -> out, uint8 device tensor of nsrc cy_noise_partial."""
+    check(lib.cy_noise_pass(ptr(img), c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0), c_int(ncols),
+                            ptr(src_dev), c_int(nsrc), c_int(row_begin), c_int(row_end), c_int(frame), ptr(unit_off),
+                            c_i64(units), ptr(state), ptr(out), cur_stream()))
+    return out
+
+
+def noise_update(partials, world, nsrc, state):
+    """cy_noise_update: partials [world * nsrc * 24] uint8 device (rank-major) -> state advanced by one pass.  Returns
+    the number of sources still active (synchronises)."""
+    active = c_int(0)
+    check(lib.cy_noise_update(ptr(partials), c_int(world), c_int(nsrc), ptr(state), ctypes.byref(active),
+                              cur_stream()))
+    return active.value
+
+
 def to_device_bytes(np_array, device):
     return torch.from_numpy(np_array.view(np.uint8).reshape(-1).copy()).to(device)

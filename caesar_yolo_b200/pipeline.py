@@ -354,6 +354,53 @@ class Engine(object):
             band, Y0 = self._get('meas_noband', (1,), torch.int32), r0
         return self.measure(sources, band, nx, big_endian, Y0, nx, r0, r1, world=world)
 
+    def measure_noise(self, sources, img, row_stride, big_endian, row0, ncols, row_begin, row_end, frame=16, world=1):
+        """Local background and noise of the catalog `sources` (ops.SRC_DTYPE): sigma-clipped mean / std of a frame of
+        `frame` pixels around each box, over rows [row_begin, row_end) of `img` (arguments as for Engine.measure;
+        cy_noise_init / cy_noise_pass / cy_noise_update).  One pass per clipping iteration, at most
+        ops.NOISE_MAX_PASSES; with world > 1 every rank passes the same catalog and its own rows, and the partials of
+        each pass are all-gathered in the group of the record exchange.  Every rank folds the same partials, so every
+        rank sees the same active count and runs the same passes.  Returns a structured array (ops.NOISE_DTYPE) whose
+        bkg, rms, nbkg, iters are final; self.noise_passes holds the number of passes run."""
+        src = np.ascontiguousarray(sources, dtype=ops.SRC_DTYPE)
+        n = len(src)
+        self.noise_passes = 0
+        if n == 0:
+            return np.zeros(0, dtype=ops.NOISE_DTYPE)
+        src_dev = ops.to_device_bytes(src, self.device)
+        e = self._mark()
+        state = self._get('noise_state', (n * ops.NOISE_DTYPE.itemsize,), torch.uint8)
+        off = self._get('noise_off', (n + 1,), torch.int64)
+        units = ops.noise_init(src_dev, n, ncols, row_begin, row_end, frame, state, off)
+        part = self._get('noise_part', (n * ops.NOISE_PARTIAL_BYTES,), torch.uint8)
+        allp = part
+        if world > 1:
+            import torch.distributed as dist
+            allp = self._get('noise_gather', (world * n * ops.NOISE_PARTIAL_BYTES,), torch.uint8)
+        active = n
+        while active:
+            if self.noise_passes == ops.NOISE_MAX_PASSES:
+                raise ops.CaesarB200Error("cy_noise_update: %d sources still active after %d passes"
+                                          % (active, self.noise_passes))
+            ops.noise_pass(img, row_stride, big_endian, row0, ncols, src_dev, n, row_begin, row_end, frame, off, units,
+                           state, part)
+            if world > 1:
+                dist.all_gather_into_tensor(allp, part)
+            active = ops.noise_update(allp, world, n, state)
+            self.noise_passes += 1
+        self._stage('noise', e)
+        self.launches += 3 + self.noise_passes * (3 + (1 if world > 1 else 0))
+        return state.cpu().numpy().view(ops.NOISE_DTYPE)
+
+    def measure_noise_band(self, sources, tiles, frame=16, rank=0, world=1):
+        """Engine.measure_noise over the rows this rank owns (measure_rows), read from the band of mosaic rows the last
+        run_image left in HBM.  The frames are thus clipped to the rows the run read, and no rank reads a row twice."""
+        r0, r1 = measure_rows(tiles, world)[rank]
+        band, Y0, _, nx, big_endian = self.band
+        if band is None:                     # a rank without tiles still takes part in every all-gather
+            band, Y0 = self._get('meas_noband', (1,), torch.int32), r0
+        return self.measure_noise(sources, band, nx, big_endian, Y0, nx, r0, r1, frame=frame, world=world)
+
     def _exchange_cap(self, world, need=0):
         """Records per rank slot of the all-gather: 48 per tile of the largest band (the catalogs of the synthetic
         mosaics hold ~20 per tile), grown on demand; kept across steps so the buffers are allocated once."""

@@ -281,6 +281,54 @@ int cy_measure_sources(const void* img, long long row_stride, int big_endian, in
 int cy_measure_combine(const cy_src_partial* partials, int world, const cy_source* src, int nsrc, int ncols,
                        cy_src_meas* meas, uintptr_t stream);
 
+/* Local background and noise of every source (not part of the reference).  The box of s is the integer rectangle
+ * [ceil x1, floor x2] x [ceil y1, floor y2] of the measurements above (a source whose box is empty has no frame).  Its
+ * frame is the box grown by F = `frame` pixels on every side, minus the box, clipped to columns [0, ncols) and to the
+ * rows the run measures; membership is decided in absolute pixel coordinates, so it does not depend on the row split.
+ * Non-finite pixels and 0 are masked, as for the box.  Mean-centred iterative sigma clipping, kappa = 3, at most 5
+ * iterations (astropy's sigma_clip defaults with cenfunc = 'mean', ddof = 0):
+ *   pass 0 takes the mean mu_0 and standard deviation sigma_0 of all unmasked frame pixels;
+ *   pass k >= 1 takes those of the pixels inside the intersection of [mu_j - 3 sigma_j, mu_j + 3 sigma_j], j < k
+ *   (inclusive bounds: astropy's nested rejection, restated as one interval per source, so a pass needs no per-pixel
+ *   state);
+ *   a source stops when pass k >= 1 keeps as many pixels as pass k - 1, after pass 5, or when pass 0 finds no pixel.
+ * bkg, rms: mean and standard deviation of the last kept set, nbkg its size, iters = k of the last pass (astropy's
+ * niterations; 0 for an empty frame).  The mean, not the median, is the centre: it is a sum, so it adds up over row
+ * ranges and ranks.  Pass k sums v - c and (v - c)^2 with c = 0 in pass 0 and c = mu_{k-1} after that, so the variance
+ * does not cancel on a pedestal: mu = c + s1 / n, sigma^2 = max(s2 / n - (s1 / n)^2, 0).
+ *
+ * Partial record of one source over one row range and one pass: every field adds.  24 bytes. */
+typedef struct {
+    int64_t n;                         /* kept frame pixels */
+    double s1, s2;                     /* sum of (v - c), (v - c)^2 */
+} cy_noise_partial;
+/* Clipping state of one source, the same on every rank.  While done = 0: [lo, hi] is the interval pass `iters` keeps
+ * (-inf, +inf before the first clip), c its shift, nbkg the pixels the previous pass kept.  Once done = 1: bkg, rms,
+ * nbkg, iters are final (bkg = rms = NaN when nbkg = 0).  56 bytes. */
+typedef struct {
+    double lo, hi, c;
+    double bkg, rms;
+    int64_t nbkg;
+    int32_t iters, done;
+} cy_noise_state;
+/* Sets state[nsrc] to pass 0 and writes the exclusive offsets unit_off[nsrc + 1] of the work units (up to 32 rows of one
+ * grown box inside [row_begin, row_end)), *units their count; the offsets serve every pass.  frame >= 1.  Synchronises
+ * the stream (the unit count is data dependent). */
+int cy_noise_init(const cy_source* src, int nsrc, int ncols, int row_begin, int row_end, int frame,
+                  cy_noise_state* state, long long* unit_off, long long* units, uintptr_t stream);
+/* One pass over rows [row_begin, row_end) of img (layout and row arguments as for cy_measure_sources; src, ncols, the
+ * rows, frame, unit_off and units as given to cy_noise_init): partials[nsrc] for the sources that are not done (the
+ * others are neither read nor written).  Rows inside the box's row span read the two side segments, other rows the
+ * full grown width; the unit partials of a source are folded in unit order. */
+int cy_noise_pass(const void* img, long long row_stride, int big_endian, int row0, int ncols, const cy_source* src,
+                  int nsrc, int row_begin, int row_end, int frame, const long long* unit_off, long long units,
+                  const cy_noise_state* state, cy_noise_partial* partials, uintptr_t stream);
+/* partials [world][nsrc] of one pass (all-gathered from `world` ranks that own disjoint row ranges) folded in rank order
+ * -> state advanced by one pass; *active: sources not yet done (the same on every rank, so every rank runs the same
+ * number of passes: at most 6).  Synchronises the stream. */
+int cy_noise_update(const cy_noise_partial* partials, int world, int nsrc, cy_noise_state* state, int* active,
+                    uintptr_t stream);
+
 /* ------------------------------------------------------------------------------------------------ whole path
  * FITS file -> merged catalog with no host-language orchestration: SFinder.run_parallel (caesar_yolo/inference.py:
  * 578-658; the serial SFinder.run :485-552 is the tile_x <= 0 case: the whole region is one tile), TileTask.find_sources

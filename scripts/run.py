@@ -69,9 +69,16 @@ def parse_args(argv=None):
                    help='B200 build only: 16-bit storage of weights/activations (default fp16; same tensor-core rate)')
     p.add_argument('--measure_sources', dest='measure_sources', action='store_true',
                    help='B200 build only: add peak, flux density, centroid, shape and sky position to every catalog source')
+    p.add_argument('--measure_noise', dest='measure_noise', action='store_true',
+                   help='B200 build only: add local background, rms, S/N, background-subtracted flux density and its '
+                        'error to every catalog source (implies --measure_sources)')
+    p.add_argument('--noise_frame', dest='noise_frame', type=int, default=16,
+                   help='B200 build only: width in pixels of the frame around each box that --measure_noise clips')
     p.add_argument('--detect_outfile', required=False, type=str, default="")
     p.add_argument('--detect_outfile_json', required=False, type=str, default="")
-    return p.parse_args(argv)
+    args = p.parse_args(argv)
+    args.measure_sources = args.measure_sources or args.measure_noise   # S/N and flux_bkgsub need the peak and sum
+    return args
 
 
 def validate_args(args):
@@ -93,6 +100,9 @@ def validate_args(args):
         return -1
     if args.weights == "" or not os.path.isfile(args.weights):
         logger.error("Given weight file %s not existing or not a file!" % args.weights)
+        return -1
+    if args.noise_frame < 1:
+        logger.error("Invalid noise_frame given (hint: give a frame width >= 1 pixel)!")
         return -1
     return 0
 
@@ -164,6 +174,7 @@ def main(argv=None):
         'draw_class_label_in_caption': args.draw_class_label_in_caption, 'save_plot': args.save_plots,
         'save_tile_catalog': args.save_tile_catalog, 'save_tile_region': args.save_tile_region,
         'save_tile_img': args.save_tile_img, 'precision': args.precision, 'measure_sources': args.measure_sources,
+        'measure_noise': args.measure_noise, 'noise_frame': args.noise_frame,
     })
     model = YOLO(args.weights, precision=args.precision)
     sfinder = SFinder(model, CONFIG)

@@ -9,6 +9,10 @@ pixels differs by reassociation only).
 
 usage: python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/measure_multirank.py
        (--backend gloo: the same with the ranks sharing one GPU)
+With --noise, every rank also runs Engine.measure_noise_band (one all-gather of the partials per clipping pass) and
+compares it with the single-rank run: nbkg, iters and the pass count exactly, bkg / rms within --rtol relative (bkg
+against max(|bkg|, rms)).
+
 Prints one JSON line on rank 0 with the largest relative difference per field and the verdict of every rank."""
 import argparse
 import json
@@ -52,6 +56,8 @@ def main():
     ap.add_argument('--rtol', type=float, default=1e-12)
     ap.add_argument('--backend', default='nccl', choices=['nccl', 'gloo'],
                     help='gloo lets several ranks share one GPU (NCCL needs one GPU per rank)')
+    ap.add_argument('--noise', action='store_true', help='also compare the local background / noise')
+    ap.add_argument('--noise_frame', type=int, default=16)
     a = ap.parse_args()
     import torch
     import torch.distributed as dist
@@ -78,13 +84,32 @@ def main():
     res = compare(meas, ref_meas)
     same_catalog = bool(src.tobytes() == ref.tobytes())
     ok = same_catalog and all(res[k + '_exact'] for k in EXACT) and all(res[k] <= a.rtol for k in FLOATS)
+    noise_res = None
+    if a.noise:
+        z = eng.measure_noise_band(src, tiles, a.noise_frame, rank, world)
+        passes = eng.noise_passes
+        zr = eng.measure_noise_band(ref, tiles, a.noise_frame)
+        noise_res = dict(passes=passes, single_rank_passes=eng.noise_passes,
+                         nbkg_exact=bool(np.array_equal(z['nbkg'], zr['nbkg'])),
+                         iters_exact=bool(np.array_equal(z['iters'], zr['iters'])))
+        for k in ('bkg', 'rms'):
+            x, y = z[k], zr[k]
+            same_nan = np.array_equal(np.isnan(x), np.isnan(y))
+            f = ~np.isnan(y)
+            scale = np.maximum(np.abs(x[f]), np.abs(y[f]))
+            if k == 'bkg':   # a mean near 0 is compared at the scale of the frame's spread
+                scale = np.maximum(scale, zr['rms'][f])
+            dd = np.abs(x[f] - y[f]) / np.where(scale > 0, scale, 1.0)
+            noise_res[k] = float(dd.max()) if (same_nan and dd.size) else (0.0 if same_nan else float('inf'))
+        ok = ok and noise_res['nbkg_exact'] and noise_res['iters_exact'] and passes == eng.noise_passes and \
+            noise_res['bkg'] <= a.rtol and noise_res['rms'] <= a.rtol
     flags = torch.tensor([1 if ok else 0], device=dev if a.backend == 'nccl' else 'cpu')
     dist.all_reduce(flags, op=dist.ReduceOp.MIN)
     if rank == 0:
         print(json.dumps(dict(world=world, backend=a.backend, gpus=torch.cuda.device_count(), mosaic=n,
                               sources=int(len(src)), rows_of_rank0=list(rows),
                               catalog_identical=same_catalog, max_rel_diff={k: res[k] for k in FLOATS},
-                              exact={k: res[k + '_exact'] for k in EXACT}, rtol=a.rtol,
+                              exact={k: res[k + '_exact'] for k in EXACT}, rtol=a.rtol, noise=noise_res,
                               matches_single_rank_on_every_rank=bool(int(flags[0])))), flush=True)
     dist.destroy_process_group()
     return 0 if int(flags[0]) else 1
