@@ -48,4 +48,9 @@ CONFIG = {
     #   mean / std of a frame of noise_frame pixels around each box
     'measure_noise': False,
     'noise_frame': 16,
+    # - Background and rms maps of the image (not in the reference; FITS input): the statistic of measure_noise over
+    #   boxes of bkg_box pixels on a lattice of step bkg_grid, interpolated bilinearly; bkgmap_<id>.fits, rmsmap_<id>.fits
+    'save_bkg_maps': False,
+    'bkg_box': 101,
+    'bkg_grid': 25,
 }

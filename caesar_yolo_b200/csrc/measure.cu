@@ -123,11 +123,10 @@ __device__ __forceinline__ int unit_source(const long long* __restrict__ off, in
     return lo;
 }
 
-// units per source (rows of the box grown by `grow`) -> exclusive offsets off[0..nsrc] (one CTA, chunks of
-// kScanThreads sources carried in order)
-__global__ void __launch_bounds__(kScanThreads) measure_units_scan_kernel(const cy_source* __restrict__ src, int nsrc,
-                                                                           int grow, int ncols, int row_begin,
-                                                                           int row_end, long long* __restrict__ off) {
+// units of items 0..n-1 (count(s)) -> exclusive offsets off[0..n] (one CTA of kScanThreads threads, chunks of
+// kScanThreads items carried in order)
+template <typename Count>
+__device__ __forceinline__ void scan_units(int nsrc, Count count, long long* __restrict__ off) {
     __shared__ long long warp_tot[kScanThreads / 32];
     __shared__ long long carry;
     const int t = threadIdx.x, lane = t & 31, w = t >> 5;
@@ -135,9 +134,7 @@ __global__ void __launch_bounds__(kScanThreads) measure_units_scan_kernel(const 
     __syncthreads();
     for (int base = 0; base < nsrc; base += kScanThreads) {
         const int s = base + t;
-        long long c = 0;
-        Box b;
-        if (s < nsrc && source_box(src[s], grow, ncols, row_begin, row_end, b)) c = (b.y1 - b.y0) / kUnitRows + 1;
+        const long long c = s < nsrc ? count(s) : 0;
         long long inc = c;
         for (int d = 1; d < 32; d <<= 1) {
             const long long v = __shfl_up_sync(0xffffffffu, inc, d);
@@ -153,6 +150,22 @@ __global__ void __launch_bounds__(kScanThreads) measure_units_scan_kernel(const 
         __syncthreads();
     }
     if (t == 0) off[nsrc] = carry;
+}
+
+struct SourceUnits {
+    const cy_source* src;
+    int grow, ncols, row_begin, row_end;
+    __device__ long long operator()(int s) const {
+        Box b;
+        return source_box(src[s], grow, ncols, row_begin, row_end, b) ? (b.y1 - b.y0) / kUnitRows + 1 : 0;
+    }
+};
+
+// units per source (rows of the box grown by `grow`) -> exclusive offsets off[0..nsrc]
+__global__ void __launch_bounds__(kScanThreads) measure_units_scan_kernel(const cy_source* __restrict__ src, int nsrc,
+                                                                           int grow, int ncols, int row_begin,
+                                                                           int row_end, long long* __restrict__ off) {
+    scan_units(nsrc, SourceUnits{src, grow, ncols, row_begin, row_end}, off);
 }
 
 // one CTA per unit: partial of up to kUnitRows rows of one box
@@ -278,6 +291,14 @@ __device__ __forceinline__ void nacc_merge(NAcc& a, const NAcc& b) {
     a.s2 += b.s2;
 }
 
+// decoded pixel value, NaN when masked: non-finite pixels and 0 (the masking rule of the box measurements)
+__device__ __forceinline__ float noise_pixel(const uint32_t* p, int big_endian) {
+    uint32_t raw = __ldg(p);
+    if (big_endian) raw = __byte_perm(raw, 0, 0x0123);
+    const float f = __uint_as_float(raw);
+    return (isfinite(f) && f != 0.0f) ? f : __int_as_float(0x7fc00000);
+}
+
 __global__ void noise_init_kernel(int nsrc, cy_noise_state* __restrict__ state) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= nsrc) return;
@@ -325,12 +346,8 @@ __global__ void __launch_bounds__(kThreads) noise_unit_kernel(const uint32_t* __
         const int nl = in_box ? side_l : g.x1 - g.x0 + 1, nr = in_box ? side_r : 0;
         for (int i = lane; i < nl + nr; i += 32) {
             const int x = i < nl ? g.x0 + i : r0 + (i - nl);
-            uint32_t raw = __ldg(row + x);
-            if (big_endian) raw = __byte_perm(raw, 0, 0x0123);
-            const float f = __uint_as_float(raw);
-            if (!isfinite(f) || f == 0.0f) continue;   // the masking rule of the box measurements
-            const double v = (double)f;
-            if (!(v >= lo && v <= hi)) continue;
+            const double v = (double)noise_pixel(row + x, big_endian);
+            if (!(v >= lo && v <= hi)) continue;       // false for a masked pixel (NaN)
             const double d = v - c;
             a.n += 1;
             a.s1 += d;
@@ -409,6 +426,201 @@ __global__ void noise_update_kernel(const cy_noise_partial* __restrict__ part, i
     }
     t.nbkg = a.n;
     state[s] = t;
+}
+
+// ---------------------------------------------------------------------------------------------- background maps
+// The sigma clipping above over the boxes of a node lattice (cy_bkg_grid_init / cy_bkg_grid_pass / cy_bkg_grid_maps).
+// A work unit is one chunk of <= kUnitRows rows of one node row and a group of kGridNodes adjacent node columns: the CTA
+// copies the columns its active nodes cover into shared memory once per chunk, slice by slice, and every warp folds
+// them into its nodes' sums.  Node rows overlap vertically (box / grid ~ 4 at the defaults); that re-read stays.
+
+constexpr int kGridNodes = 16;                          // node columns per unit: warp w takes nodes w and w + 8
+constexpr int kNodesPerWarp = kGridNodes / (kThreads / 32);
+constexpr int kSliceCols = 256;                         // columns of one shared-memory slice (32 KB with kUnitRows)
+
+// Node lattice of the region: columns [0, ncols) of the buffer, rows [R0, R1); rlo..rhi: the rows of this range
+// (inclusive; empty when rlo > rhi).  h is clipped to the region's larger side, which changes no box.
+struct Grid {
+    int ncols, R0, R1, g, h, nx, ny, ngroups, rlo, rhi;
+    __host__ __device__ int xnode(int i) const { return (int)min((long long)i * g, (long long)ncols - 1); }
+    __host__ __device__ int ynode(int j) const { return R0 + (int)min((long long)j * g, (long long)(R1 - R0) - 1); }
+    // rows of node row j inside this range, inclusive; false when none
+    __host__ __device__ bool rows(int j, int& a, int& b) const {
+        a = max(ynode(j) - h, rlo);
+        b = min(ynode(j) + h, rhi);
+        return a <= b;
+    }
+};
+
+static bool make_grid(int ncols, int R0, int R1, int row_begin, int row_end, int box, int grid, Grid& G) {
+    if (ncols < 1 || R1 <= R0 || row_begin < R0 || row_end < row_begin || row_end > R1 || box < 3 || !(box & 1) ||
+        grid < 1)
+        return false;
+    const int H = R1 - R0;
+    G.ncols = ncols;
+    G.R0 = R0;
+    G.R1 = R1;
+    G.g = grid;
+    G.h = min(box / 2, max(ncols, H));
+    G.nx = (int)(((long long)ncols - 1 + grid - 1) / grid) + 1;
+    G.ny = (int)(((long long)H - 1 + grid - 1) / grid) + 1;
+    G.ngroups = (G.nx + kGridNodes - 1) / kGridNodes;
+    G.rlo = row_begin;
+    G.rhi = row_end - 1;
+    return (long long)G.nx * G.ny <= 2147483647ll;
+}
+
+struct NodeRowUnits {
+    Grid G;
+    __device__ long long operator()(int j) const {
+        int a, b;
+        return G.rows(j, a, b) ? (long long)((b - a) / kUnitRows + 1) * G.ngroups : 0;
+    }
+};
+
+__global__ void __launch_bounds__(kScanThreads) bkg_units_scan_kernel(Grid G, long long* __restrict__ off) {
+    scan_units(G.ny, NodeRowUnits{G}, off);
+}
+
+// one CTA per unit: sums of (v - c), (v - c)^2 over the pixels of the unit's rows inside each active node's box and
+// kept interval -> unit_out[u * kGridNodes + k] for node column i0 + k.  A unit whose nodes are all done returns at once;
+// only the columns from the first to the last active node's box are read.
+__global__ void __launch_bounds__(kThreads) bkg_unit_kernel(const uint32_t* __restrict__ img, long long row_stride,
+                                                            int big_endian, int row0, Grid G,
+                                                            const long long* __restrict__ off,
+                                                            const cy_noise_state* __restrict__ state,
+                                                            cy_noise_partial* __restrict__ unit_out) {
+    __shared__ float tile[kUnitRows][kSliceCols];
+    __shared__ double s_lo[kGridNodes], s_hi[kGridNodes], s_c[kGridNodes];
+    __shared__ int s_active[kGridNodes];
+    const long long u = blockIdx.x;
+    const int j = unit_source(off, G.ny, u);
+    const long long local = u - off[j];
+    const int grp = (int)(local % G.ngroups), chunk = (int)(local / G.ngroups);
+    const int i0 = grp * kGridNodes, ni = min(kGridNodes, G.nx - i0);
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    if (threadIdx.x < kGridNodes) {
+        const int k = threadIdx.x;
+        int act = 0;
+        if (k < ni) {
+            const cy_noise_state& s = state[(long long)j * G.nx + i0 + k];
+            act = !s.done;
+            s_lo[k] = s.lo;
+            s_hi[k] = s.hi;
+            s_c[k] = s.c;
+        }
+        s_active[k] = act;
+    }
+    __syncthreads();
+    int ka = -1, kb = -1;
+    for (int k = 0; k < ni; ++k)
+        if (s_active[k]) {
+            if (ka < 0) ka = k;
+            kb = k;
+        }
+    if (ka < 0) return;
+    int a, b;
+    G.rows(j, a, b);
+    const int len = b - a + 1, nch = (b - a) / kUnitRows + 1;   // chunks of balanced size <= kUnitRows
+    const int ya = a + (int)((long long)chunk * len / nch);
+    const int nrows = a + (int)((long long)(chunk + 1) * len / nch) - ya;
+    const int cs = max(G.xnode(i0 + ka) - G.h, 0), ce = min(G.xnode(i0 + kb) + G.h, G.ncols - 1);
+    NAcc acc[kNodesPerWarp];
+#pragma unroll
+    for (int q = 0; q < kNodesPerWarp; ++q) acc[q] = {0, 0.0, 0.0};
+    for (int s0 = cs; s0 <= ce; s0 += kSliceCols) {
+        const int sw = min(kSliceCols, ce - s0 + 1);
+        for (int r = w; r < nrows; r += kThreads / 32) {
+            const uint32_t* row = img + (long long)(ya + r - row0) * row_stride + s0;
+            for (int c = lane; c < sw; c += 32) tile[r][c] = noise_pixel(row + c, big_endian);
+        }
+        __syncthreads();
+#pragma unroll
+        for (int q = 0; q < kNodesPerWarp; ++q) {
+            const int k = w + q * (kThreads / 32);
+            if (k >= ni || !s_active[k]) continue;
+            const int xk = G.xnode(i0 + k);
+            const int c0 = max(xk - G.h, s0), c1 = min(xk + G.h, s0 + sw - 1);
+            const double lo = s_lo[k], hi = s_hi[k], c = s_c[k];
+            for (int r = 0; r < nrows; ++r)
+                for (int x = c0 + lane; x <= c1; x += 32) {
+                    const double v = (double)tile[r][x - s0];
+                    if (!(v >= lo && v <= hi)) continue;   // false for a masked pixel (NaN)
+                    const double d = v - c;
+                    acc[q].n += 1;
+                    acc[q].s1 += d;
+                    acc[q].s2 += d * d;
+                }
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int q = 0; q < kNodesPerWarp; ++q) {
+        NAcc t = acc[q];
+        for (int d = 16; d > 0; d >>= 1) {
+            NAcc o;
+            o.n = __shfl_down_sync(0xffffffffu, t.n, d);
+            o.s1 = __shfl_down_sync(0xffffffffu, t.s1, d);
+            o.s2 = __shfl_down_sync(0xffffffffu, t.s2, d);
+            nacc_merge(t, o);
+        }
+        const int k = w + q * (kThreads / 32);
+        if (lane == 0 && k < ni && s_active[k]) {
+            cy_noise_partial& p = unit_out[u * kGridNodes + k];
+            p.n = t.n;
+            p.s1 = t.s1;
+            p.s2 = t.s2;
+        }
+    }
+}
+
+// unit partials of each active node, folded in chunk order -> one partial per node (zero without units)
+__global__ void bkg_fold_kernel(const cy_noise_partial* __restrict__ unit, const long long* __restrict__ off, Grid G,
+                                const cy_noise_state* __restrict__ state, cy_noise_partial* __restrict__ out) {
+    const long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= (long long)G.nx * G.ny || state[n].done) return;
+    const int j = (int)(n / G.nx), i = (int)(n % G.nx);
+    const long long nch = (off[j + 1] - off[j]) / G.ngroups;
+    NAcc a = {0, 0.0, 0.0};
+    for (long long c = 0; c < nch; ++c) {
+        const cy_noise_partial& p = unit[(off[j] + c * G.ngroups + i / kGridNodes) * kGridNodes + i % kGridNodes];
+        const NAcc b = {p.n, p.s1, p.s2};
+        nacc_merge(a, b);
+    }
+    out[n].n = a.n;
+    out[n].s1 = a.s1;
+    out[n].s2 = a.s2;
+}
+
+// bilinear weight of the finite corners, renormalised; NaN when they carry no weight
+__device__ __forceinline__ float interp_corners(double v00, double v01, double v10, double v11, double w00, double w01,
+                                                double w10, double w11) {
+    double s = 0.0, ws = 0.0;
+    if (!isnan(v00)) { s += w00 * v00; ws += w00; }
+    if (!isnan(v01)) { s += w01 * v01; ws += w01; }
+    if (!isnan(v10)) { s += w10 * v10; ws += w10; }
+    if (!isnan(v11)) { s += w11 * v11; ws += w11; }
+    return ws > 0.0 ? (float)(s / ws) : __int_as_float(0x7fc00000);
+}
+
+// one thread per map pixel: blockIdx.x = row - row_begin, blockIdx.y * blockDim.x + threadIdx.x = column
+__global__ void bkg_map_kernel(const cy_noise_state* __restrict__ state, Grid G, int row_begin,
+                               uint32_t* __restrict__ bkg, uint32_t* __restrict__ rms) {
+    const int x = blockIdx.y * blockDim.x + threadIdx.x;
+    if (x >= G.ncols) return;
+    const int y = row_begin + blockIdx.x;
+    const int i = G.nx >= 2 ? min(x / G.g, G.nx - 2) : 0, i1 = min(i + 1, G.nx - 1);   // x_i = i * g for i <= nx - 2
+    const int j = G.ny >= 2 ? min((y - G.R0) / G.g, G.ny - 2) : 0, j1 = min(j + 1, G.ny - 1);
+    const double t = i1 > i ? (double)(x - G.xnode(i)) / (double)(G.xnode(i1) - G.xnode(i)) : 0.0;
+    const double v = j1 > j ? (double)(y - G.ynode(j)) / (double)(G.ynode(j1) - G.ynode(j)) : 0.0;
+    const double w00 = (1.0 - t) * (1.0 - v), w01 = t * (1.0 - v), w10 = (1.0 - t) * v, w11 = t * v;
+    const cy_noise_state &a = state[(long long)j * G.nx + i], &b = state[(long long)j * G.nx + i1];
+    const cy_noise_state &c = state[(long long)j1 * G.nx + i], &d = state[(long long)j1 * G.nx + i1];
+    const float fb = interp_corners(a.bkg, b.bkg, c.bkg, d.bkg, w00, w01, w10, w11);
+    const float fr = interp_corners(a.rms, b.rms, c.rms, d.rms, w00, w01, w10, w11);
+    const long long o = (long long)blockIdx.x * G.ncols + x;
+    bkg[o] = __byte_perm(__float_as_uint(fb), 0, 0x0123);   // FITS byte order
+    rms[o] = __byte_perm(__float_as_uint(fr), 0, 0x0123);
 }
 
 }  // namespace
@@ -524,5 +736,65 @@ extern "C" int cy_noise_update(const cy_noise_partial* partials, int world, int 
     const cudaError_t e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_noise_update: %s", cudaGetErrorString(e));
     *active = n;
+    return CY_OK;
+}
+
+extern "C" int cy_bkg_grid_init(int ncols, int R0, int R1, int row_begin, int row_end, int box, int grid,
+                                cy_noise_state* state, long long* unit_off, long long* units, uintptr_t stream) {
+    Grid G;
+    if (!units || !make_grid(ncols, R0, R1, row_begin, row_end, box, grid, G))
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_init: invalid region, row range, box (odd, >= 3) or grid (>= 1)");
+    *units = 0;
+    if (!state || !unit_off) return set_error(CY_ERR_INVALID, "cy_bkg_grid_init: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long nodes = (long long)G.nx * G.ny;
+    noise_init_kernel<<<(unsigned)((nodes + 255) / 256), 256, 0, st>>>((int)nodes, state);
+    bkg_units_scan_kernel<<<1, kScanThreads, 0, st>>>(G, unit_off);
+    long long n = 0;   // the unit count is data dependent: bring it to the host
+    cudaMemcpyAsync(&n, unit_off + G.ny, sizeof(long long), cudaMemcpyDeviceToHost, st);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_init: %s", cudaGetErrorString(e));
+    if (n > 2147483647ll) return set_error(CY_ERR_INVALID, "cy_bkg_grid_init: %lld work units exceed one grid", n);
+    *units = n;
+    return CY_OK;
+}
+
+extern "C" int cy_bkg_grid_pass(const void* img, long long row_stride, int big_endian, int row0, int ncols, int R0,
+                                int R1, int row_begin, int row_end, int box, int grid, const long long* unit_off,
+                                long long units, const cy_noise_state* state, cy_noise_partial* partials,
+                                uintptr_t stream) {
+    Grid G;
+    if (!make_grid(ncols, R0, R1, row_begin, row_end, box, grid, G) || row_stride < ncols || row_begin < row0 ||
+        units < 0 || units > 2147483647ll)
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_pass: invalid image geometry, region, box, grid or unit count");
+    if (!unit_off || !state || !partials || (units > 0 && !img))
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_pass: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    cy_noise_partial* unit = nullptr;
+    if (units > 0 &&
+        cudaMallocAsync(&unit, (size_t)units * kGridNodes * sizeof(cy_noise_partial), st) != cudaSuccess)
+        return set_error(CY_ERR_NOMEM, "cy_bkg_grid_pass: no memory for %lld unit partials", units * kGridNodes);
+    if (units > 0)
+        bkg_unit_kernel<<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian, row0, G,
+                                                              unit_off, state, unit);
+    const long long nodes = (long long)G.nx * G.ny;
+    bkg_fold_kernel<<<(unsigned)((nodes + 255) / 256), 256, 0, st>>>(unit, unit_off, G, state, partials);
+    const cudaError_t e = cudaGetLastError();
+    if (unit) cudaFreeAsync(unit, st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_pass: %s", cudaGetErrorString(e));
+    return CY_OK;
+}
+
+extern "C" int cy_bkg_grid_maps(const cy_noise_state* state, int ncols, int R0, int R1, int row_begin, int row_end,
+                                int box, int grid, void* bkg, void* rms, uintptr_t stream) {
+    Grid G;
+    if (!make_grid(ncols, R0, R1, row_begin, row_end, box, grid, G) || (ncols + 255) / 256 > 65535)
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_maps: invalid region, row range, box or grid");
+    if (row_end == row_begin) return CY_OK;
+    if (!state || !bkg || !rms) return set_error(CY_ERR_INVALID, "cy_bkg_grid_maps: null argument");
+    bkg_map_kernel<<<dim3((unsigned)(row_end - row_begin), (unsigned)((ncols + 255) / 256)), 256, 0,
+                     (cudaStream_t)stream>>>(state, G, row_begin, (uint32_t*)bkg, (uint32_t*)rms);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_maps: %s", cudaGetErrorString(e));
     return CY_OK;
 }

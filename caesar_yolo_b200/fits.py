@@ -2,6 +2,8 @@
 Replaces utils.get_fits_header / read_fits / read_fits_crop of the reference (caesar_yolo/utils.py:150-164,
 193-246, 340-418): the pixel payload is handed to the GPU in its raw big-endian byte order (BITPIX -32) and decoded
 there (byte swap + non-finite -> 0 fused into the first load of the preprocessing kernels)."""
+import os
+
 import numpy as np
 
 _BITPIX_DTYPE = {8: ">u1", 16: ">i2", 32: ">i4", 64: ">i8", -32: ">f4", -64: ">f8"}
@@ -170,6 +172,94 @@ def write_fits(data, path):
         f.write(hdr.encode("ascii"))
         f.write(payload)
         f.write(b"\0" * (-len(payload) % 2880))
+
+
+def format_card(key, value, comment=""):
+    """One 80-character header card.  Logicals and numbers are right-justified to column 30 (fixed format; a float
+    whose shortest round-trip form is longer than 20 characters extends past it, which the free format allows); floats
+    always carry a '.' and an uppercase 'E' exponent; strings are quoted from column 11, embedded quotes doubled, and
+    padded to at least 8 characters."""
+    if isinstance(value, (bool, np.bool_)):
+        v = "%20s" % ("T" if value else "F")
+    elif isinstance(value, (int, np.integer)):
+        v = "%20d" % value
+    elif isinstance(value, (float, np.floating)):
+        if not np.isfinite(value):
+            raise ValueError("%s: a FITS header value must be finite" % key)
+        s = repr(float(value))
+        mant, _, exp = s.partition("e")
+        if "." not in mant:
+            mant += ".0"
+        v = "%20s" % (mant + ("E" + exp if exp else ""))
+    else:
+        v = "'%-8s'" % str(value).replace("'", "''")
+    c = "%-8s= %s" % (key, v)
+    if comment:
+        c += " / " + comment
+    if len(c) > 80:
+        raise ValueError("%s: card longer than 80 characters" % key)
+    return "%-80s" % c
+
+
+# cards of the image header that a map keeps: the celestial WCS of axes 1 and 2, the unit and the beam
+_WCS_AXIS_KEYS = ("CTYPE", "CRVAL", "CDELT", "CUNIT")
+_WCS_KEYS = ("CD1_1", "CD1_2", "CD2_1", "CD2_2", "PC1_1", "PC1_2", "PC2_1", "PC2_2", "CROTA2", "LONPOLE", "LATPOLE",
+             "RADESYS", "EQUINOX", "BUNIT", "BMAJ", "BMIN", "BPA")
+
+
+def map_header(h, nx, ny, x0=0, y0=0):
+    """Header (bytes, a multiple of 2880) of a 2-D BITPIX -32 map of nx x ny pixels whose pixel (0, 0) is pixel (x0, y0)
+    of the image with header dict h: the WCS cards of axes 1 and 2, BUNIT and the beam are copied, and CRPIX1/2 are
+    shifted by (x0, y0), so every map pixel has the sky position of the image pixel under it."""
+    cards = [format_card("SIMPLE", True, "conforms to FITS standard"), format_card("BITPIX", -32, "array data type"),
+             format_card("NAXIS", 2, "number of array dimensions"), format_card("NAXIS1", int(nx)),
+             format_card("NAXIS2", int(ny))]
+    for a, off in ((1, x0), (2, y0)):
+        for k in _WCS_AXIS_KEYS:
+            if "%s%d" % (k, a) in h:
+                cards.append(format_card("%s%d" % (k, a), h["%s%d" % (k, a)]))
+        if "CRPIX%d" % a in h:
+            cards.append(format_card("CRPIX%d" % a, h["CRPIX%d" % a] - off))
+    cards += [format_card(k, h[k]) for k in _WCS_KEYS if k in h]
+    cards.append("%-80s" % "END")
+    txt = "".join(cards)
+    return (txt + " " * (-len(txt) % 2880)).encode("ascii")
+
+
+def write_map_rows(path, header, rows, row_begin, nx, ny, rank=0, world=1, piece_bytes=1 << 26):
+    """Writes one FITS map in parallel by rows.  rows: this rank's map rows [row_begin, row_begin + len(rows)) as a
+    device tensor [n, nx] of 4-byte words already in FITS byte order; header: map_header bytes.  Rank 0 writes the
+    header and sizes the file (payload padded to 2880 bytes with zeros); after a barrier, every rank writes its rows
+    with pwrite through pinned staging in pieces of ~piece_bytes; a second barrier ends the call.  No rank holds more
+    than its own rows."""
+    import torch
+    if world > 1:
+        import torch.distributed as dist
+    if rank == 0:
+        payload = nx * ny * 4
+        with open(path, "wb") as f:
+            f.write(header)
+            f.truncate(len(header) + payload + (-payload % 2880))
+    if world > 1:
+        dist.barrier()
+    n = int(rows.shape[0]) if rows is not None else 0
+    if n:
+        step = max(1, piece_bytes // (nx * 4))
+        pin = torch.empty((min(step, n), nx), dtype=torch.int32, pin_memory=rows.is_cuda)
+        fd = os.open(path, os.O_WRONLY)
+        try:
+            for r in range(0, n, step):
+                k = min(step, n - r)
+                pin[:k].copy_(rows[r:r + k])
+                buf = memoryview(pin[:k].numpy()).cast("B")
+                off = len(header) + (row_begin + r) * nx * 4
+                done = 0
+                while done < len(buf):
+                    done += os.pwrite(fd, buf[done:], off + done)
+        finally:
+            os.close(fd)
+    if world > 1:
+        dist.barrier()
 
 
 def read_raster(path):

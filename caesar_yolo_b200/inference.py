@@ -56,6 +56,9 @@ class SFinder(object):
         self.measure_noise = bool(config.get('measure_noise', False))
         self.measure_sources = bool(config.get('measure_sources', False)) or self.measure_noise
         self.noise_frame = int(config.get('noise_frame', 16))
+        self.save_bkg_maps = bool(config.get('save_bkg_maps', False))
+        self.bkg_box = int(config.get('bkg_box', 101))
+        self.bkg_grid = int(config.get('bkg_grid', 25))
         self.procId, self.nproc = _dist_info()
         self.timing = {}
         self.engine = None
@@ -187,7 +190,7 @@ class SFinder(object):
         t0 = time.time()
         eng.begin(tiles)
         dev_img = None
-        if self._host_callable() is None or self.measure_sources:
+        if self._host_callable() is None or self.measure_sources or self.save_bkg_maps:
             img = self.fits.rows(y0, y1)
             dev_img = torch.from_numpy(np.array(img, copy=True).view(np.int32)).to(eng.device)   # memmap rows are read-only
         if self._host_callable() is not None:
@@ -206,6 +209,10 @@ class SFinder(object):
             m = eng.measure(*args)
             noise = eng.measure_noise(*args, frame=self.noise_frame) if self.measure_noise else None
             meas = self._measurements(m, self.fits.header, x0, y0, noise)
+        if self.save_bkg_maps:   # the region read: the crop, columns from x0
+            _, bkg, rms = eng.bkg_maps(dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0, 0,
+                                       y1 - y0, self.bkg_box, self.bkg_grid)
+            self._write_bkg_maps(bkg, rms, 0, (x0, y0, x1 - x0, y1 - y0))
         self.timing['run_s'] = time.time() - t0
         return self._save_serial(recs, status, meas)
 
@@ -218,6 +225,17 @@ class SFinder(object):
             logger.warning("No RA---SIN/TAN, DEC--SIN/TAN celestial WCS in the image header (CTYPE1=%s, CTYPE2=%s): "
                            "ra/dec are written as null", header.get('CTYPE1'), header.get('CTYPE2'))
         return catalog.measurement_dicts(m, fitsmeta.beam_area_pix(header), radec, noise)
+
+    def _write_bkg_maps(self, bkg, rms, row_begin, region):
+        """bkgmap_<id>.fits and rmsmap_<id>.fits in outdir: this rank's map rows (Engine.bkg_maps) of the region
+        (X0, R0, W, H), with the image's WCS shifted to the region."""
+        X0, R0, W, H = region
+        t0 = time.time()
+        hdr = fitsmeta.map_header(self.fits.header, W, H, X0, R0)
+        for name, rows in (('bkgmap_', bkg), ('rmsmap_', rms)):
+            fitsmeta.write_map_rows(os.path.join(self.outdir, name + str(self.image_id) + '.fits'), hdr, rows,
+                                    row_begin, W, H, self.procId, self.nproc)
+        self.timing['bkg_maps_write_s'] = time.time() - t0
 
     def _save_serial(self, recs, status, meas=None):
         self.results = {"image_id": self.image_id, "objs": catalog.records_to_objs(recs, self.class_names, meas=meas)}
@@ -276,6 +294,8 @@ class SFinder(object):
         packed, n = eng.finish()
         recs = packed.cpu().numpy().view(ops.REC_DTYPE).copy()
         meas = None
+        if self.save_bkg_maps:
+            logger.warning("Background and rms maps are written for FITS images only: none for %s", c['image_path'])
         if self.measure_sources:
             if plane_dev is None:
                 logger.warning("Colour image: per-source measurements need a single-plane image and are not written")
@@ -335,7 +355,8 @@ class SFinder(object):
             self._process_tiles_host_callable(eng, tiles, range(a, b), self._host_callable())
             src, n = eng.exchange_and_merge(self.nproc, rank0_only=rank0_only, rank=self.procId,
                                             on_local_records=hook)
-            if self.measure_sources:   # the tiles went through the host: bring this rank's rows to the GPU
+            # the tiles went through the host: bring this rank's rows to the GPU
+            if self.measure_sources or self.save_bkg_maps:
                 Y0, Y1 = (int(tiles['ymin'][a:b].min()), int(tiles['ymax'][a:b].max())) if b > a else (0, 0)
                 band = torch.from_numpy(np.array(self.fits.rows(Y0, Y1), copy=True).view(np.int32)).to(eng.device)
                 eng.band = (band if b > a else None, Y0, Y1, self.fits.nx, self.fits.is_raw_f32)
@@ -350,6 +371,9 @@ class SFinder(object):
                 noise = eng.measure_noise_band(src, tiles, self.noise_frame, self.procId, self.nproc)
             if self.procId == 0:
                 meas = self._measurements(m, self.fits.header, noise=noise)
+        if self.save_bkg_maps:   # every rank maps and writes its own rows; the catalog is not needed
+            _, bkg, rms, region, rows = eng.bkg_maps_band(tiles, self.bkg_box, self.bkg_grid, self.procId, self.nproc)
+            self._write_bkg_maps(bkg, rms, rows[0] - region[1], region)
         self.timing['run_s'] = time.time() - t0
         if self.procId == 0:
             self.sources = {"sources": catalog.sources_to_dicts(src, self.class_names, meas)}

@@ -418,5 +418,37 @@ def noise_update(partials, world, nsrc, state):
     return active.value
 
 
+def bkg_grid_nodes(n, grid):
+    """Node positions along one axis of n pixels with step `grid` (include/caesar_b200.h, background maps):
+    x_i = min(i * grid, n - 1), i = 0 .. ceil((n - 1) / grid)."""
+    return [min(i * grid, n - 1) for i in range(-(-(n - 1) // grid) + 1)]
+
+
+def bkg_grid_init(ncols, R0, R1, row_begin, row_end, box, grid, state, unit_off):
+    """cy_bkg_grid_init.  state: uint8 device tensor of >= Nx * Ny cy_noise_state; unit_off: int64 device tensor of
+    >= Ny + 1 elements.  Returns the number of work units (synchronises)."""
+    units = c_i64(0)
+    check(lib.cy_bkg_grid_init(c_int(ncols), c_int(R0), c_int(R1), c_int(row_begin), c_int(row_end), c_int(box),
+                               c_int(grid), ptr(state), ptr(unit_off), ctypes.byref(units), cur_stream()))
+    return units.value
+
+
+def bkg_grid_pass(img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box, grid, unit_off, units,
+                  state, out):
+    """cy_bkg_grid_pass: one clipping pass of the grid nodes over this range's rows -> out, uint8 device tensor of
+    Nx * Ny cy_noise_partial."""
+    check(lib.cy_bkg_grid_pass(ptr(img), c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0), c_int(ncols),
+                               c_int(R0), c_int(R1), c_int(row_begin), c_int(row_end), c_int(box), c_int(grid),
+                               ptr(unit_off), c_i64(units), ptr(state), ptr(out), cur_stream()))
+    return out
+
+
+def bkg_grid_maps(state, ncols, R0, R1, row_begin, row_end, box, grid, bkg, rms):
+    """cy_bkg_grid_maps: final node states -> rows [row_begin, row_end) of the bkg and rms maps (device tensors of
+    (row_end - row_begin) * ncols 4-byte words, big-endian float32)."""
+    check(lib.cy_bkg_grid_maps(ptr(state), c_int(ncols), c_int(R0), c_int(R1), c_int(row_begin), c_int(row_end),
+                               c_int(box), c_int(grid), ptr(bkg), ptr(rms), cur_stream()))
+
+
 def to_device_bytes(np_array, device):
     return torch.from_numpy(np_array.view(np.uint8).reshape(-1).copy()).to(device)

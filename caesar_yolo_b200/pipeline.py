@@ -401,6 +401,61 @@ class Engine(object):
             band, Y0 = self._get('meas_noband', (1,), torch.int32), r0
         return self.measure_noise(sources, band, nx, big_endian, Y0, nx, r0, r1, frame=frame, world=world)
 
+    def bkg_maps(self, img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box=101, grid=25, world=1):
+        """Background and rms maps of the region of columns [0, ncols) of `img` and rows [R0, R1) (node lattice,
+        statistic and interpolation: include/caesar_b200.h), over rows [row_begin, row_end) of `img` (arguments as for
+        Engine.measure; cy_bkg_grid_init / cy_bkg_grid_pass / cy_noise_update / cy_bkg_grid_maps).  With world > 1 every
+        rank passes the same region and its own rows, and the node partials of each pass are all-gathered in the group of
+        the record exchange, so every rank runs the same passes.  Returns (nodes, bkg, rms): the final node states
+        (ops.NOISE_DTYPE, shape [Ny, Nx]) and this range's map rows as int32 device tensors [row_end - row_begin, ncols]
+        holding big-endian float32; self.bkg_passes holds the number of passes run."""
+        nx, ny = len(ops.bkg_grid_nodes(ncols, grid)), len(ops.bkg_grid_nodes(R1 - R0, grid))
+        nodes = nx * ny
+        e = self._mark()
+        state = self._get('bkg_state', (nodes * ops.NOISE_DTYPE.itemsize,), torch.uint8)
+        off = self._get('bkg_off', (ny + 1,), torch.int64)
+        units = ops.bkg_grid_init(ncols, R0, R1, row_begin, row_end, box, grid, state, off)
+        part = self._get('bkg_part', (nodes * ops.NOISE_PARTIAL_BYTES,), torch.uint8)
+        allp = part
+        if world > 1:
+            import torch.distributed as dist
+            allp = self._get('bkg_gather', (world * nodes * ops.NOISE_PARTIAL_BYTES,), torch.uint8)
+        self.bkg_passes = 0
+        active = nodes
+        while active:
+            if self.bkg_passes == ops.NOISE_MAX_PASSES:
+                raise ops.CaesarB200Error("cy_noise_update: %d grid nodes still active after %d passes"
+                                          % (active, self.bkg_passes))
+            ops.bkg_grid_pass(img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box, grid, off,
+                              units, state, part)
+            if world > 1:
+                dist.all_gather_into_tensor(allp, part)
+            active = ops.noise_update(allp, world, nodes, state)
+            self.bkg_passes += 1
+        bkg = torch.empty((row_end - row_begin, ncols), dtype=torch.int32, device=self.device)
+        rms = torch.empty_like(bkg)
+        ops.bkg_grid_maps(state, ncols, R0, R1, row_begin, row_end, box, grid, bkg, rms)
+        self._stage('bkg_maps', e)
+        self.launches += 3 + self.bkg_passes * (3 + (1 if world > 1 else 0)) + 1
+        return state.cpu().numpy().view(ops.NOISE_DTYPE).reshape(ny, nx), bkg, rms
+
+    def bkg_maps_band(self, tiles, box=101, grid=25, rank=0, world=1):
+        """Engine.bkg_maps of the bounding box of the tile grid (columns [min xmin, max xmax), rows [min ymin,
+        max ymax)) over the rows this rank owns (measure_rows), read from the band of mosaic rows the last run_image
+        left in HBM.  Returns (nodes, bkg, rms, (X0, R0, W, H), (row_begin, row_end))."""
+        X0, X1 = int(tiles['xmin'].min()), int(tiles['xmax'].max())
+        R0, R1 = int(tiles['ymin'].min()), int(tiles['ymax'].max())
+        r0, r1 = measure_rows(tiles, world)[rank]
+        if r1 == r0:
+            r0 = r1 = R0
+        band, Y0, _, nx, big_endian = self.band
+        if band is None:                     # a rank without tiles still takes part in every all-gather
+            img, Y0 = self._get('meas_noband', (1,), torch.int32), r0
+        else:
+            img = band[:, X0:]
+        nodes, bkg, rms = self.bkg_maps(img, nx, big_endian, Y0, X1 - X0, R0, R1, r0, r1, box, grid, world)
+        return nodes, bkg, rms, (X0, R0, X1 - X0, R1 - R0), (r0, r1)
+
     def _exchange_cap(self, world, need=0):
         """Records per rank slot of the all-gather: 48 per tile of the largest band (the catalogs of the synthetic
         mosaics hold ~20 per tile), grown on demand; kept across steps so the buffers are allocated once."""

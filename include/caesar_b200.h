@@ -329,6 +329,38 @@ int cy_noise_pass(const void* img, long long row_stride, int big_endian, int row
 int cy_noise_update(const cy_noise_partial* partials, int world, int nsrc, cy_noise_state* state, int* active,
                     uintptr_t stream);
 
+/* Background and rms maps of an image region (not part of the reference).  The region is W = ncols columns (columns
+ * [0, ncols) of the buffer) by H = R1 - R0 rows (rows [R0, R1)); a run maps the pixels it read.
+ * Grid nodes: with step g = grid, node column i sits at x_i = min(i g, W - 1), i = 0 .. Nx - 1, Nx = ceil((W - 1) / g)
+ * + 1, and node row j at y_j = R0 + min(j g, H - 1), Ny alike from H: the first and last nodes lie on the region's
+ * edges, and W = 1 (H = 1) gives one node along that axis.  Node n = j Nx + i.  The box of a node is [x_i - h, x_i + h]
+ * x [y_j - h, y_j + h], h = box / 2, clipped to the region; box is odd and >= 3, grid >= 1.  Membership is decided in
+ * absolute pixel coordinates, so it does not depend on the row split.
+ * Node statistic: the one of cy_noise_state above, unchanged (unmasked box pixels, mean-centred sigma clipping, kappa =
+ * 3, at most 5 iterations; passes, partials and cy_noise_update as for the sources).  A node whose box has no unmasked
+ * pixel gets bkg = rms = NaN, like an empty frame.
+ * Map pixel (x, y): bilinear in fp64 between the nodes i, i + 1 and j, j + 1, where i is the largest index with x_i <= x
+ * clamped to Nx - 2 (0 when Nx = 1), t = (x - x_i) / (x_{i+1} - x_i) (0 when Nx = 1), and j, u alike along rows.  A
+ * corner whose value is NaN is dropped and the weights of the others renormalised; the pixel is NaN when the finite
+ * corners carry no weight.  The rms map interpolates the node rms (not the variance).  Stored as float32 in FITS byte
+ * order (big-endian, BITPIX -32). */
+
+/* Sets state[Nx * Ny] to pass 0 and writes the exclusive offsets unit_off[Ny + 1] of the work units of rows [row_begin,
+ * row_end) (R0 <= row_begin <= row_end <= R1; a unit is one chunk of <= 32 rows of one node row and 16 adjacent node
+ * columns), *units their count; the offsets serve every pass.  Synchronises the stream (for the unit count). */
+int cy_bkg_grid_init(int ncols, int R0, int R1, int row_begin, int row_end, int box, int grid, cy_noise_state* state,
+                     long long* unit_off, long long* units, uintptr_t stream);
+/* One clipping pass over rows [row_begin, row_end) of img (layout and row0 as for cy_measure_sources; the other
+ * arguments as given to cy_bkg_grid_init): partials[Nx * Ny] for the nodes that are not done.  Rank partials are folded
+ * with cy_noise_update(partials, world, Nx * Ny, state, &active, stream) until active = 0 (at most 6 passes). */
+int cy_bkg_grid_pass(const void* img, long long row_stride, int big_endian, int row0, int ncols, int R0, int R1,
+                     int row_begin, int row_end, int box, int grid, const long long* unit_off, long long units,
+                     const cy_noise_state* state, cy_noise_partial* partials, uintptr_t stream);
+/* Final node states -> rows [row_begin, row_end) of the bkg and rms maps: (row_end - row_begin) x ncols 4-byte words
+ * each, row-major, big-endian float32.  No pixel of the image is read. */
+int cy_bkg_grid_maps(const cy_noise_state* state, int ncols, int R0, int R1, int row_begin, int row_end, int box,
+                     int grid, void* bkg, void* rms, uintptr_t stream);
+
 /* ------------------------------------------------------------------------------------------------ whole path
  * FITS file -> merged catalog with no host-language orchestration: SFinder.run_parallel (caesar_yolo/inference.py:
  * 578-658; the serial SFinder.run :485-552 is the tile_x <= 0 case: the whole region is one tile), TileTask.find_sources

@@ -74,6 +74,13 @@ def parse_args(argv=None):
                         'error to every catalog source (implies --measure_sources)')
     p.add_argument('--noise_frame', dest='noise_frame', type=int, default=16,
                    help='B200 build only: width in pixels of the frame around each box that --measure_noise clips')
+    p.add_argument('--save_bkg_maps', dest='save_bkg_maps', action='store_true',
+                   help='B200 build only: write the background and rms maps of a FITS image (bkgmap_<id>.fits, '
+                        'rmsmap_<id>.fits)')
+    p.add_argument('--bkg_box', dest='bkg_box', type=int, default=101,
+                   help='B200 build only: side in pixels (odd, >= 3) of the box each --save_bkg_maps node clips')
+    p.add_argument('--bkg_grid', dest='bkg_grid', type=int, default=25,
+                   help='B200 build only: step in pixels (>= 1) of the --save_bkg_maps node lattice')
     p.add_argument('--detect_outfile', required=False, type=str, default="")
     p.add_argument('--detect_outfile_json', required=False, type=str, default="")
     args = p.parse_args(argv)
@@ -103,6 +110,12 @@ def validate_args(args):
         return -1
     if args.noise_frame < 1:
         logger.error("Invalid noise_frame given (hint: give a frame width >= 1 pixel)!")
+        return -1
+    if args.bkg_box < 3 or args.bkg_box % 2 == 0:
+        logger.error("Invalid bkg_box given (hint: give an odd box side >= 3 pixels)!")
+        return -1
+    if args.bkg_grid < 1:
+        logger.error("Invalid bkg_grid given (hint: give a grid step >= 1 pixel)!")
         return -1
     return 0
 
@@ -174,7 +187,8 @@ def main(argv=None):
         'draw_class_label_in_caption': args.draw_class_label_in_caption, 'save_plot': args.save_plots,
         'save_tile_catalog': args.save_tile_catalog, 'save_tile_region': args.save_tile_region,
         'save_tile_img': args.save_tile_img, 'precision': args.precision, 'measure_sources': args.measure_sources,
-        'measure_noise': args.measure_noise, 'noise_frame': args.noise_frame,
+        'measure_noise': args.measure_noise, 'noise_frame': args.noise_frame, 'save_bkg_maps': args.save_bkg_maps,
+        'bkg_box': args.bkg_box, 'bkg_grid': args.bkg_grid,
     })
     model = YOLO(args.weights, precision=args.precision)
     sfinder = SFinder(model, CONFIG)

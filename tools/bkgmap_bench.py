@@ -1,0 +1,163 @@
+#!/usr/bin/env python
+"""Cost of the background / rms maps (Engine.bkg_maps: cy_bkg_grid_init, the clipping passes, cy_bkg_grid_maps) on the
+benchmark workloads: BASELINE config 3 (16k^2 mosaic, tile step 1.0) and config 4 (32k^2, step 0.5), with bench.py's
+mosaic, model and thresholds, at the default box and grid.  For each: one pipeline.run_image (the band stays in HBM),
+then Engine.bkg_maps_band timed with CUDA events after a warm-up, next to the run_image step time on the same mosaic;
+each clipping pass is timed on its own with events; the two map files are written once with fits.write_map_rows and
+timed on the host clock.  Prints one JSON line per config with the card name and power limit beside the numbers.
+
+Algorithmic bytes of pass p: for every unit whose node group has an active node in pass p, the 4-byte pixels of its
+rows and of the columns from its first to its last active node's box (what bkg_unit_kernel reads), plus the unit
+partials written and folded.  The map kernel writes 8 bytes per pixel and reads no image pixel.
+
+    python tools/bkgmap_bench.py [--configs 3,4] [--reps 5] [--out DIR]
+"""
+import argparse
+import json
+import os
+import sys
+import tempfile
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+
+import bench  # noqa: E402  (mosaic generator, model and thresholds of the benchmark)
+from measure_bench import card  # noqa: E402
+
+GROUP, UNIT_ROWS, PARTIAL = 16, 32, 24
+
+
+def pass_bytes(nodes, W, H, box, grid):
+    """Bytes each pass reads / writes (module docstring), from the final node states: node n is active in passes
+    0 .. iters[n] (an empty node stops after pass 0)."""
+    from caesar_yolo_b200 import ops
+    h = box // 2
+    xs, ys = np.array(ops.bkg_grid_nodes(W, grid)), np.array(ops.bkg_grid_nodes(H, grid))
+    out = []
+    for p in range(int(nodes['iters'].max()) + 1):
+        act = nodes['iters'] >= p
+        total = 0
+        for j, y in enumerate(ys):
+            rows = min(y + h, H - 1) - max(y - h, 0) + 1
+            nch = (rows - 1) // UNIT_ROWS + 1
+            for g0 in range(0, len(xs), GROUP):
+                a = np.nonzero(act[j, g0:g0 + GROUP])[0]
+                if a.size == 0:
+                    continue
+                cols = min(xs[g0 + a[-1]] + h, W - 1) - max(xs[g0 + a[0]] - h, 0) + 1
+                total += rows * cols * 4 + nch * GROUP * PARTIAL * 2
+        out.append(float(total))
+    return out
+
+
+def run_config(cfg, reps, variant, box, grid):
+    import torch
+    from caesar_yolo_b200 import fits, ops, pipeline, weights as W
+    dev = torch.device('cuda:0')
+    torch.cuda.set_device(dev)
+    a = argparse.Namespace(mosaic=32768 if cfg == 4 else 16384)
+    step = 0.5 if cfg == 4 else 1.0
+    n = a.mosaic
+    _, host = bench.make_mosaic_pinned(a)
+    tiles = ops.generate_tiles(0, n - 1, 0, n - 1, 512, 512, step, step)
+    w = W.make_random_weights(variant, 5, seed=0, cls_bias=bench.CLS_BIAS.get(variant, -16.0))
+    eng = pipeline.Engine(w, pipeline.make_pp_config(**bench.PP_FLAGS), imgsz=640, score_thr=bench.SCORE_THR,
+                          iou_thr=bench.IOU_THR, thr_soft=bench.SOFT, thr_hard=bench.HARD, device=dev)
+    pipeline.run_image(eng, host, True, tiles)          # warm-up (plans, buffers)
+    torch.cuda.synchronize()
+    t0 = time.time()
+    k = 2
+    for _ in range(k):
+        pipeline.run_image(eng, host, True, tiles)
+    torch.cuda.synchronize()
+    step_ms = (time.time() - t0) * 1e3 / k
+    res = None
+    for _ in range(2):
+        res = eng.bkg_maps_band(tiles, box, grid)
+    nodes, bkg, rms, (X0, R0, Wd, Hd), rows = res
+    passes = eng.bkg_passes
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    torch.cuda.synchronize()
+    e0.record()
+    for _ in range(reps):
+        eng.bkg_maps_band(tiles, box, grid)
+    e1.record()
+    torch.cuda.synchronize()
+    call_ms = e0.elapsed_time(e1) / reps
+    # every pass on its own: the engine's loop restated with events around each cy_bkg_grid_pass
+    band, Y0, _, nx, be = eng.band
+    img = band[:, X0:]
+    nn = nodes.size
+    state = torch.empty((nn * ops.NOISE_DTYPE.itemsize,), dtype=torch.uint8, device=dev)
+    off = torch.empty((nodes.shape[0] + 1,), dtype=torch.int64, device=dev)
+    part = torch.empty((nn * ops.NOISE_PARTIAL_BYTES,), dtype=torch.uint8, device=dev)
+    pass_ms = [0.0] * passes
+    for _ in range(reps):
+        units = ops.bkg_grid_init(Wd, R0, R0 + Hd, rows[0], rows[1], box, grid, state, off)
+        for p in range(passes):
+            a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a0.record()
+            ops.bkg_grid_pass(img, nx, be, Y0, Wd, R0, R0 + Hd, rows[0], rows[1], box, grid, off, units, state, part)
+            a1.record()
+            ops.noise_update(part, 1, nn, state)
+            pass_ms[p] += a0.elapsed_time(a1) / reps
+    m0, m1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    m0.record()
+    for _ in range(reps):
+        ops.bkg_grid_maps(state, Wd, R0, R0 + Hd, rows[0], rows[1], box, grid, bkg, rms)
+    m1.record()
+    torch.cuda.synchronize()
+    map_ms = m0.elapsed_time(m1) / reps
+    nbytes = pass_bytes(nodes, Wd, Hd, box, grid)
+    with tempfile.TemporaryDirectory() as d:
+        hdr = fits.map_header({}, Wd, Hd, X0, R0)
+        t0 = time.time()
+        for name, m in (('bkgmap.fits', bkg), ('rmsmap.fits', rms)):
+            fits.write_map_rows(os.path.join(d, name), hdr, m, 0, Wd, Hd)
+        write_s = time.time() - t0
+    ok = nodes['nbkg'] > 0
+    return {"config": cfg, "mosaic": n, "tile_step": step, "bkg_box": box, "bkg_grid": grid,
+            "nodes": [int(nodes.shape[0]), int(nodes.shape[1])], "passes": passes,
+            "iters_histogram": np.bincount(nodes['iters'].ravel(), minlength=6).tolist(),
+            "bkg_maps_ms_per_call": round(call_ms, 3), "pass_ms": [round(x, 3) for x in pass_ms],
+            "map_rows_ms": round(map_ms, 3),
+            "pass_bytes": nbytes, "pass_gbs": [round(b / (t * 1e-3) / 1e9, 1) if t > 0 else None
+                                               for b, t in zip(nbytes, pass_ms)],
+            "map_bytes_written": 8 * Wd * Hd,
+            "run_image_step_ms": round(step_ms, 2), "bkg_maps_share_of_step": round(call_ms / step_ms, 4),
+            "file_write_s": round(write_s, 3), "file_bytes": 2 * (len(hdr) + 4 * Wd * Hd),
+            "median_node_rms": float(np.median(nodes['rms'][ok])) if ok.any() else None,
+            "note": "bkg_maps_ms_per_call: CUDA events around Engine.bkg_maps_band (unit plan, every pass with its host "
+                    "read of the active count, map rows, copy of the node states to the host); pass_ms: events around "
+                    "cy_bkg_grid_pass alone; file_write_s: host clock around both files (device -> pinned -> pwrite, "
+                    "one rank, a temporary directory on the local disk)"}
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument('--configs', default='3,4')
+    ap.add_argument('--reps', type=int, default=5)
+    ap.add_argument('--variant', default='l')
+    ap.add_argument('--bkg_box', type=int, default=101)
+    ap.add_argument('--bkg_grid', type=int, default=25)
+    ap.add_argument('--out', default=None, help='directory for bkgmap_bench.json')
+    a = ap.parse_args()
+    info = card()
+    lines = []
+    for c in [int(x) for x in a.configs.split(',')]:
+        r = run_config(c, a.reps, a.variant, a.bkg_box, a.bkg_grid)
+        r.update(info)
+        print(json.dumps(r), flush=True)
+        lines.append(r)
+    if a.out:
+        os.makedirs(a.out, exist_ok=True)
+        with open(os.path.join(a.out, 'bkgmap_bench.json'), 'w') as f:
+            json.dump(lines, f, indent=1)
+
+
+if __name__ == '__main__':
+    main()

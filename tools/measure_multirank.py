@@ -12,6 +12,10 @@ usage: python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.
 With --noise, every rank also runs Engine.measure_noise_band (one all-gather of the partials per clipping pass) and
 compares it with the single-rank run: nbkg, iters and the pass count exactly, bkg / rms within --rtol relative (bkg
 against max(|bkg|, rms)).
+With --maps, every rank also runs Engine.bkg_maps_band (the background / rms maps of the mosaic, one all-gather of the
+node partials per clipping pass) and compares it with the single-rank run: node nbkg, iters and the pass count exactly,
+node bkg / rms within --rtol relative (as for --noise), and its own rows of both maps within 1 float32 ulp of the same
+rows of the single-rank maps (NaN positions equal).
 
 Prints one JSON line on rank 0 with the largest relative difference per field and the verdict of every rank."""
 import argparse
@@ -58,6 +62,9 @@ def main():
                     help='gloo lets several ranks share one GPU (NCCL needs one GPU per rank)')
     ap.add_argument('--noise', action='store_true', help='also compare the local background / noise')
     ap.add_argument('--noise_frame', type=int, default=16)
+    ap.add_argument('--maps', action='store_true', help='also compare the background / rms maps')
+    ap.add_argument('--bkg_box', type=int, default=101)
+    ap.add_argument('--bkg_grid', type=int, default=25)
     a = ap.parse_args()
     import torch
     import torch.distributed as dist
@@ -103,13 +110,43 @@ def main():
             noise_res[k] = float(dd.max()) if (same_nan and dd.size) else (0.0 if same_nan else float('inf'))
         ok = ok and noise_res['nbkg_exact'] and noise_res['iters_exact'] and passes == eng.noise_passes and \
             noise_res['bkg'] <= a.rtol and noise_res['rms'] <= a.rtol
+    maps_res = None
+    if a.maps:
+        z, bkg, rms, _, (r0, r1) = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, rank, world)
+        passes = eng.bkg_passes
+        zr, bkg_r, rms_r, _, _ = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid)
+        maps_res = dict(passes=passes, single_rank_passes=eng.bkg_passes, nodes=int(z.size),
+                        nbkg_exact=bool(np.array_equal(z['nbkg'], zr['nbkg'])),
+                        iters_exact=bool(np.array_equal(z['iters'], zr['iters'])))
+        for k in ('bkg', 'rms'):
+            x, y = z[k].ravel(), zr[k].ravel()
+            same_nan = np.array_equal(np.isnan(x), np.isnan(y))
+            f = ~np.isnan(y)
+            scale = np.maximum(np.abs(x[f]), np.abs(y[f]))
+            if k == 'bkg':
+                scale = np.maximum(scale, zr['rms'].ravel()[f])
+            dd = np.abs(x[f] - y[f]) / np.where(scale > 0, scale, 1.0)
+            maps_res[k] = float(dd.max()) if (same_nan and dd.size) else (0.0 if same_nan else float('inf'))
+        ulp = 0.0
+        for mine, ref in ((bkg, bkg_r), (rms, rms_r)):
+            p = mine.cpu().numpy().view('>f4').astype(np.float64)
+            q = ref[r0 - tiles['ymin'].min():r1 - tiles['ymin'].min()].cpu().numpy().view('>f4').astype(np.float32)
+            if not np.array_equal(np.isnan(p), np.isnan(q)):
+                ulp = float('inf')
+                break
+            f = ~np.isnan(q)
+            if f.any():
+                ulp = max(ulp, float((np.abs(p[f] - q[f]) / np.spacing(np.abs(q[f]))).max()))
+        maps_res['map_max_ulp'] = ulp
+        ok = ok and maps_res['nbkg_exact'] and maps_res['iters_exact'] and passes == eng.bkg_passes and \
+            maps_res['bkg'] <= a.rtol and maps_res['rms'] <= a.rtol and ulp <= 1.0
     flags = torch.tensor([1 if ok else 0], device=dev if a.backend == 'nccl' else 'cpu')
     dist.all_reduce(flags, op=dist.ReduceOp.MIN)
     if rank == 0:
         print(json.dumps(dict(world=world, backend=a.backend, gpus=torch.cuda.device_count(), mosaic=n,
                               sources=int(len(src)), rows_of_rank0=list(rows),
                               catalog_identical=same_catalog, max_rel_diff={k: res[k] for k in FLOATS},
-                              exact={k: res[k + '_exact'] for k in EXACT}, rtol=a.rtol, noise=noise_res,
+                              exact={k: res[k + '_exact'] for k in EXACT}, rtol=a.rtol, noise=noise_res, maps=maps_res,
                               matches_single_rank_on_every_rank=bool(int(flags[0])))), flush=True)
     dist.destroy_process_group()
     return 0 if int(flags[0]) else 1
