@@ -119,6 +119,7 @@ SYMBOLS = [
     "cy_postprocess", "cy_nms_scratch_bytes", "cy_nms_batched", "cy_merge_tile", "cy_make_records",
     "cy_compact_scratch_bytes", "cy_compact_records", "cy_merge_global", "cy_measure_sources", "cy_measure_combine",
     "cy_noise_init", "cy_noise_pass", "cy_noise_update", "cy_bkg_grid_init", "cy_bkg_grid_pass", "cy_bkg_grid_maps",
+    "cy_source_mask", "cy_noise_pass_masked", "cy_bkg_grid_pass_masked", "cy_bkg_grid_probe_init", "cy_bkg_grid_fill",
     "cy_ctx_create", "cy_ctx_set_allgather", "cy_ctx_destroy", "cy_run_local", "cy_run_local_payload", "cy_ctx_records",
     "cy_ctx_pack_slot", "cy_ctx_unpack_slots", "cy_run_merge", "cy_run_mosaic", "cy_run_payload", "cy_ctx_info",
 ]

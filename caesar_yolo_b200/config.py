@@ -53,4 +53,7 @@ CONFIG = {
     'save_bkg_maps': False,
     'bkg_box': 101,
     'bkg_grid': 25,
+    # - Mask the catalog boxes out of the measure_noise frames and the save_bkg_maps node boxes (not in the reference);
+    #   map nodes left without pixels are filled from their neighbours.  Alone it changes nothing (one warning)
+    'bkg_mask_sources': False,
 }

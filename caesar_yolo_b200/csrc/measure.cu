@@ -316,13 +316,17 @@ __global__ void noise_init_kernel(int nsrc, cy_noise_state* __restrict__ state) 
 // one CTA per unit: sums of (v - c), (v - c)^2 over the frame pixels of up to kUnitRows rows of one grown box that lie
 // inside the source's kept interval [lo, hi].  Rows inside the box's row span read the two side segments, packed into
 // one run of lane indices; other rows read the full grown width.  A converged source's units return at once.
+// kMask: a pixel whose bit is set in the source mask (cy_source_mask over the same ncols and rows) is skipped before
+// its load; the unmasked instantiation does not touch `mask`.
+template <bool kMask>
 __global__ void __launch_bounds__(kThreads) noise_unit_kernel(const uint32_t* __restrict__ img, long long row_stride,
                                                               int big_endian, int row0, int ncols,
                                                               const cy_source* __restrict__ src, int nsrc,
                                                               int row_begin, int row_end, int frame,
                                                               const long long* __restrict__ off,
                                                               const cy_noise_state* __restrict__ state,
-                                                              cy_noise_partial* __restrict__ unit_out) {
+                                                              cy_noise_partial* __restrict__ unit_out,
+                                                              const uint32_t* __restrict__ mask) {
     __shared__ NAcc warp_acc[kThreads / 32];
     const long long u = blockIdx.x;
     const int s = unit_source(off, nsrc, u);
@@ -342,10 +346,12 @@ __global__ void __launch_bounds__(kThreads) noise_unit_kernel(const uint32_t* __
     NAcc a = {0, 0.0, 0.0};
     for (int y = ya + w; y <= yb; y += kThreads / 32) {
         const uint32_t* row = img + (long long)(y - row0) * row_stride;
+        const uint32_t* mrow = kMask ? mask + (long long)(y - row_begin) * ((ncols + 31) >> 5) : nullptr;
         const bool in_box = (double)y >= by0 && (double)y <= by1;
         const int nl = in_box ? side_l : g.x1 - g.x0 + 1, nr = in_box ? side_r : 0;
         for (int i = lane; i < nl + nr; i += 32) {
             const int x = i < nl ? g.x0 + i : r0 + (i - nl);
+            if (kMask && ((__ldg(mrow + (x >> 5)) >> (x & 31)) & 1u)) continue;
             const double v = (double)noise_pixel(row + x, big_endian);
             if (!(v >= lo && v <= hi)) continue;       // false for a masked pixel (NaN)
             const double d = v - c;
@@ -485,11 +491,16 @@ __global__ void __launch_bounds__(kScanThreads) bkg_units_scan_kernel(Grid G, lo
 // one CTA per unit: sums of (v - c), (v - c)^2 over the pixels of the unit's rows inside each active node's box and
 // kept interval -> unit_out[u * kGridNodes + k] for node column i0 + k.  A unit whose nodes are all done returns at once;
 // only the columns from the first to the last active node's box are read.
+// kMask: region pixel (x, y) is masked when bit x + mask_col0 of mask row y - G.rlo is set (mask_words words per row);
+// it enters the shared tile as NaN, so the fold loop is that of the unmasked instantiation, which does not touch `mask`.
+template <bool kMask>
 __global__ void __launch_bounds__(kThreads) bkg_unit_kernel(const uint32_t* __restrict__ img, long long row_stride,
                                                             int big_endian, int row0, Grid G,
                                                             const long long* __restrict__ off,
                                                             const cy_noise_state* __restrict__ state,
-                                                            cy_noise_partial* __restrict__ unit_out) {
+                                                            cy_noise_partial* __restrict__ unit_out,
+                                                            const uint32_t* __restrict__ mask, int mask_words,
+                                                            int mask_col0) {
     __shared__ float tile[kUnitRows][kSliceCols];
     __shared__ double s_lo[kGridNodes], s_hi[kGridNodes], s_c[kGridNodes];
     __shared__ int s_active[kGridNodes];
@@ -532,7 +543,16 @@ __global__ void __launch_bounds__(kThreads) bkg_unit_kernel(const uint32_t* __re
         const int sw = min(kSliceCols, ce - s0 + 1);
         for (int r = w; r < nrows; r += kThreads / 32) {
             const uint32_t* row = img + (long long)(ya + r - row0) * row_stride + s0;
-            for (int c = lane; c < sw; c += 32) tile[r][c] = noise_pixel(row + c, big_endian);
+            if (kMask) {
+                const uint32_t* mrow = mask + (long long)(ya + r - G.rlo) * mask_words;
+                for (int c = lane; c < sw; c += 32) {
+                    const int mx = s0 + c + mask_col0;
+                    tile[r][c] = ((__ldg(mrow + (mx >> 5)) >> (mx & 31)) & 1u) ? __int_as_float(0x7fc00000)
+                                                                              : noise_pixel(row + c, big_endian);
+                }
+            } else {
+                for (int c = lane; c < sw; c += 32) tile[r][c] = noise_pixel(row + c, big_endian);
+            }
         }
         __syncthreads();
 #pragma unroll
@@ -623,6 +643,110 @@ __global__ void bkg_map_kernel(const cy_noise_state* __restrict__ state, Grid G,
     rms[o] = __byte_perm(__float_as_uint(fr), 0, 0x0123);
 }
 
+// ---------------------------------------------------------------------------------------------- source mask
+// The union M of the catalog boxes as a bit mask (cy_source_mask): the units of measure_units_scan_kernel with grow = 0,
+// one CTA per unit; each thread ORs the bits of one (row, word) of the unit's rows into the mask.  OR does not depend on
+// the order, so overlapping boxes give the same bits whatever CTA runs first.
+__global__ void __launch_bounds__(kThreads) source_mask_kernel(const cy_source* __restrict__ src, int nsrc, int ncols,
+                                                               int row_begin, int row_end,
+                                                               const long long* __restrict__ off,
+                                                               uint32_t* __restrict__ mask) {
+    const long long u = blockIdx.x;
+    const int s = unit_source(off, nsrc, u);
+    Box b;
+    source_box(src[s], 0, ncols, row_begin, row_end, b);
+    const int ya = b.y0 + (int)(u - off[s]) * kUnitRows;
+    const int nrows = min(b.y1, ya + kUnitRows - 1) - ya + 1;
+    const int w0 = b.x0 >> 5, nw = (b.x1 >> 5) - w0 + 1, words = (ncols + 31) >> 5;
+    for (int t = threadIdx.x; t < nrows * nw; t += kThreads) {
+        const int r = t / nw, w = w0 + t % nw;
+        const int lo = max(b.x0 - 32 * w, 0), hi = min(b.x1 - 32 * w, 31);   // bits lo..hi of word w
+        const uint32_t bits = (hi - lo == 31 ? 0xffffffffu : ((1u << (hi - lo + 1)) - 1u)) << lo;
+        atomicOr(mask + (long long)(ya + r - row_begin) * words + w, bits);
+    }
+}
+
+// ---------------------------------------------------------------------------------------------- hole fill
+// Node classes of the fill (cy_bkg_grid_fill): a value (finite after clipping, or filled), an unfilled hole, blank.
+enum { kFillValue = 0, kFillHole = 1, kFillBlank = 2 };
+struct FillNode {
+    double bkg, rms;
+    int cls;
+};
+
+// probe state: pass 0 for the nodes without a value (nbkg = 0), done for the others; *nprobe counts the former
+__global__ void bkg_probe_init_kernel(const cy_noise_state* __restrict__ state, int nodes,
+                                      cy_noise_state* __restrict__ probe, int* __restrict__ nprobe) {
+    const int n = blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= nodes) return;
+    cy_noise_state t;
+    t.lo = -INFINITY;
+    t.hi = INFINITY;
+    t.c = 0.0;
+    t.bkg = t.rms = __longlong_as_double(0x7ff8000000000000ll);
+    t.nbkg = 0;
+    t.iters = 0;
+    t.done = state[n].nbkg > 0;
+    if (!t.done) atomicAdd(nprobe, 1);
+    probe[n] = t;
+}
+
+// final node states + the probe partials [world][nodes] (read for the nodes with nbkg = 0 only) -> fill nodes
+__global__ void bkg_fill_classify_kernel(const cy_noise_partial* __restrict__ part, int world, int nodes,
+                                         const cy_noise_state* __restrict__ state, FillNode* __restrict__ out) {
+    const int n = blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= nodes) return;
+    FillNode f;
+    f.bkg = state[n].bkg;
+    f.rms = state[n].rms;
+    f.cls = kFillValue;
+    if (state[n].nbkg == 0) {
+        long long k = 0;
+        for (int r = 0; r < world; ++r) k += part[(long long)r * nodes + n].n;
+        f.cls = k > 0 ? kFillHole : kFillBlank;
+    }
+    out[n] = f;
+}
+
+// one ring: every hole with a valued node among its 8 neighbours in `a` takes the mean of their values (summed in
+// row-major neighbour order) -> b; *changed counts the nodes filled in this ring
+__global__ void bkg_fill_ring_kernel(const FillNode* __restrict__ a, int nx, int ny, FillNode* __restrict__ b,
+                                     int* __restrict__ changed) {
+    const long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= (long long)nx * ny) return;
+    FillNode f = a[n];
+    if (f.cls == kFillHole) {
+        const int j = (int)(n / nx), i = (int)(n % nx);
+        double sb = 0.0, sr = 0.0;
+        int k = 0;
+        for (int dj = -1; dj <= 1; ++dj)
+            for (int di = -1; di <= 1; ++di) {
+                const int jj = j + dj, ii = i + di;
+                if ((dj == 0 && di == 0) || jj < 0 || jj >= ny || ii < 0 || ii >= nx) continue;
+                const FillNode& q = a[(long long)jj * nx + ii];
+                if (q.cls != kFillValue) continue;
+                sb += q.bkg;
+                sr += q.rms;
+                ++k;
+            }
+        if (k > 0) {
+            f.bkg = sb / k;
+            f.rms = sr / k;
+            f.cls = kFillValue;
+            atomicAdd(changed, 1);
+        }
+    }
+    b[n] = f;
+}
+
+// filled values -> the node states (nbkg stays 0, so a filled node can be recognised)
+__global__ void bkg_fill_store_kernel(const FillNode* __restrict__ a, int nodes, cy_noise_state* __restrict__ state) {
+    const int n = blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= nodes || state[n].nbkg > 0 || a[n].cls != kFillValue) return;
+    state[n].bkg = a[n].bkg;
+    state[n].rms = a[n].rms;
+}
+
 }  // namespace
 
 extern "C" int cy_measure_sources(const void* img, long long row_stride, int big_endian, int row0, int ncols,
@@ -694,29 +818,51 @@ extern "C" int cy_noise_init(const cy_source* src, int nsrc, int ncols, int row_
     return CY_OK;
 }
 
+static int noise_pass(const char* fn, const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                      const cy_source* src, int nsrc, int row_begin, int row_end, int frame, const long long* unit_off,
+                      long long units, const cy_noise_state* state, cy_noise_partial* partials, const uint32_t* mask,
+                      uintptr_t stream) {
+    if (nsrc < 0 || ncols <= 0 || row_stride < ncols || row_begin < row0 || row_end < row_begin || frame < 1 ||
+        units < 0 || units > 2147483647ll)
+        return set_error(CY_ERR_INVALID, "%s: invalid image geometry, row range, frame or unit count", fn);
+    if (nsrc == 0) return CY_OK;
+    if (!src || !unit_off || !state || !partials || (units > 0 && !img))
+        return set_error(CY_ERR_INVALID, "%s: null argument", fn);
+    cudaStream_t st = (cudaStream_t)stream;
+    cy_noise_partial* unit = nullptr;
+    if (units > 0 && cudaMallocAsync(&unit, (size_t)units * sizeof(cy_noise_partial), st) != cudaSuccess)
+        return set_error(CY_ERR_NOMEM, "%s: no memory for %lld unit partials", fn, units);
+    if (units > 0 && mask)
+        noise_unit_kernel<true><<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian,
+                                                                      row0, ncols, src, nsrc, row_begin, row_end,
+                                                                      frame, unit_off, state, unit, mask);
+    else if (units > 0)
+        noise_unit_kernel<false><<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian,
+                                                                       row0, ncols, src, nsrc, row_begin, row_end,
+                                                                       frame, unit_off, state, unit, nullptr);
+    noise_fold_kernel<<<(nsrc + 255) / 256, 256, 0, st>>>(unit, unit_off, nsrc, state, partials);
+    const cudaError_t e = cudaGetLastError();
+    if (unit) cudaFreeAsync(unit, st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "%s: %s", fn, cudaGetErrorString(e));
+    return CY_OK;
+}
+
 extern "C" int cy_noise_pass(const void* img, long long row_stride, int big_endian, int row0, int ncols,
                              const cy_source* src, int nsrc, int row_begin, int row_end, int frame,
                              const long long* unit_off, long long units, const cy_noise_state* state,
                              cy_noise_partial* partials, uintptr_t stream) {
-    if (nsrc < 0 || ncols <= 0 || row_stride < ncols || row_begin < row0 || row_end < row_begin || frame < 1 ||
-        units < 0 || units > 2147483647ll)
-        return set_error(CY_ERR_INVALID, "cy_noise_pass: invalid image geometry, row range, frame or unit count");
-    if (nsrc == 0) return CY_OK;
-    if (!src || !unit_off || !state || !partials || (units > 0 && !img))
-        return set_error(CY_ERR_INVALID, "cy_noise_pass: null argument");
-    cudaStream_t st = (cudaStream_t)stream;
-    cy_noise_partial* unit = nullptr;
-    if (units > 0 && cudaMallocAsync(&unit, (size_t)units * sizeof(cy_noise_partial), st) != cudaSuccess)
-        return set_error(CY_ERR_NOMEM, "cy_noise_pass: no memory for %lld unit partials", units);
-    if (units > 0)
-        noise_unit_kernel<<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian, row0,
-                                                                ncols, src, nsrc, row_begin, row_end, frame, unit_off,
-                                                                state, unit);
-    noise_fold_kernel<<<(nsrc + 255) / 256, 256, 0, st>>>(unit, unit_off, nsrc, state, partials);
-    const cudaError_t e = cudaGetLastError();
-    if (unit) cudaFreeAsync(unit, st);
-    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_noise_pass: %s", cudaGetErrorString(e));
-    return CY_OK;
+    return noise_pass("cy_noise_pass", img, row_stride, big_endian, row0, ncols, src, nsrc, row_begin, row_end, frame,
+                      unit_off, units, state, partials, nullptr, stream);
+}
+
+extern "C" int cy_noise_pass_masked(const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                                    const cy_source* src, int nsrc, int row_begin, int row_end, int frame,
+                                    const long long* unit_off, long long units, const cy_noise_state* state,
+                                    cy_noise_partial* partials, const uint32_t* mask, uintptr_t stream) {
+    if (units > 0 && row_end > row_begin && !mask)
+        return set_error(CY_ERR_INVALID, "cy_noise_pass_masked: null mask");
+    return noise_pass("cy_noise_pass_masked", img, row_stride, big_endian, row0, ncols, src, nsrc, row_begin, row_end,
+                      frame, unit_off, units, state, partials, row_end > row_begin ? mask : nullptr, stream);
 }
 
 extern "C" int cy_noise_update(const cy_noise_partial* partials, int world, int nsrc, cy_noise_state* state,
@@ -759,30 +905,57 @@ extern "C" int cy_bkg_grid_init(int ncols, int R0, int R1, int row_begin, int ro
     return CY_OK;
 }
 
-extern "C" int cy_bkg_grid_pass(const void* img, long long row_stride, int big_endian, int row0, int ncols, int R0,
-                                int R1, int row_begin, int row_end, int box, int grid, const long long* unit_off,
-                                long long units, const cy_noise_state* state, cy_noise_partial* partials,
-                                uintptr_t stream) {
+static int bkg_grid_pass(const char* fn, const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                         int R0, int R1, int row_begin, int row_end, int box, int grid, const long long* unit_off,
+                         long long units, const cy_noise_state* state, cy_noise_partial* partials,
+                         const uint32_t* mask, int mask_ncols, int mask_col0, uintptr_t stream) {
     Grid G;
     if (!make_grid(ncols, R0, R1, row_begin, row_end, box, grid, G) || row_stride < ncols || row_begin < row0 ||
         units < 0 || units > 2147483647ll)
-        return set_error(CY_ERR_INVALID, "cy_bkg_grid_pass: invalid image geometry, region, box, grid or unit count");
+        return set_error(CY_ERR_INVALID, "%s: invalid image geometry, region, box, grid or unit count", fn);
     if (!unit_off || !state || !partials || (units > 0 && !img))
-        return set_error(CY_ERR_INVALID, "cy_bkg_grid_pass: null argument");
+        return set_error(CY_ERR_INVALID, "%s: null argument", fn);
     cudaStream_t st = (cudaStream_t)stream;
     cy_noise_partial* unit = nullptr;
     if (units > 0 &&
         cudaMallocAsync(&unit, (size_t)units * kGridNodes * sizeof(cy_noise_partial), st) != cudaSuccess)
-        return set_error(CY_ERR_NOMEM, "cy_bkg_grid_pass: no memory for %lld unit partials", units * kGridNodes);
-    if (units > 0)
-        bkg_unit_kernel<<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian, row0, G,
-                                                              unit_off, state, unit);
+        return set_error(CY_ERR_NOMEM, "%s: no memory for %lld unit partials", fn, units * kGridNodes);
+    if (units > 0 && mask)
+        bkg_unit_kernel<true><<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian, row0,
+                                                                    G, unit_off, state, unit, mask,
+                                                                    (mask_ncols + 31) >> 5, mask_col0);
+    else if (units > 0)
+        bkg_unit_kernel<false><<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian, row0,
+                                                                     G, unit_off, state, unit, nullptr, 0, 0);
     const long long nodes = (long long)G.nx * G.ny;
     bkg_fold_kernel<<<(unsigned)((nodes + 255) / 256), 256, 0, st>>>(unit, unit_off, G, state, partials);
     const cudaError_t e = cudaGetLastError();
     if (unit) cudaFreeAsync(unit, st);
-    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_pass: %s", cudaGetErrorString(e));
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "%s: %s", fn, cudaGetErrorString(e));
     return CY_OK;
+}
+
+extern "C" int cy_bkg_grid_pass(const void* img, long long row_stride, int big_endian, int row0, int ncols, int R0,
+                                int R1, int row_begin, int row_end, int box, int grid, const long long* unit_off,
+                                long long units, const cy_noise_state* state, cy_noise_partial* partials,
+                                uintptr_t stream) {
+    return bkg_grid_pass("cy_bkg_grid_pass", img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box,
+                         grid, unit_off, units, state, partials, nullptr, 0, 0, stream);
+}
+
+extern "C" int cy_bkg_grid_pass_masked(const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                                       int R0, int R1, int row_begin, int row_end, int box, int grid,
+                                       const long long* unit_off, long long units, const cy_noise_state* state,
+                                       cy_noise_partial* partials, const uint32_t* mask, int mask_ncols,
+                                       int mask_col0, uintptr_t stream) {
+    if (mask_col0 < 0 || ncols <= 0 || mask_ncols < 1 || (long long)mask_col0 + ncols > mask_ncols)
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_pass_masked: the region's columns [%d, %lld) are not inside the "
+                         "mask's %d columns", mask_col0, (long long)mask_col0 + ncols, mask_ncols);
+    if (units > 0 && row_end > row_begin && !mask)
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_pass_masked: null mask");
+    return bkg_grid_pass("cy_bkg_grid_pass_masked", img, row_stride, big_endian, row0, ncols, R0, R1, row_begin,
+                         row_end, box, grid, unit_off, units, state, partials, row_end > row_begin ? mask : nullptr,
+                         mask_ncols, mask_col0, stream);
 }
 
 extern "C" int cy_bkg_grid_maps(const cy_noise_state* state, int ncols, int R0, int R1, int row_begin, int row_end,
@@ -796,5 +969,94 @@ extern "C" int cy_bkg_grid_maps(const cy_noise_state* state, int ncols, int R0, 
                      (cudaStream_t)stream>>>(state, G, row_begin, (uint32_t*)bkg, (uint32_t*)rms);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_maps: %s", cudaGetErrorString(e));
+    return CY_OK;
+}
+
+extern "C" int cy_source_mask(const cy_source* src, int nsrc, int ncols, int row_begin, int row_end, uint32_t* mask,
+                              uintptr_t stream) {
+    if (nsrc < 0 || ncols <= 0 || row_end < row_begin)
+        return set_error(CY_ERR_INVALID, "cy_source_mask: invalid source count, column count or row range");
+    const long long words = (long long)(row_end - row_begin) * ((ncols + 31) >> 5);
+    if (words == 0) return CY_OK;
+    if (!mask || (nsrc > 0 && !src)) return set_error(CY_ERR_INVALID, "cy_source_mask: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    CY_CUDA_CHECK(cudaMemsetAsync(mask, 0, (size_t)words * sizeof(uint32_t), st));
+    if (nsrc == 0) return CY_OK;
+    long long* off = nullptr;
+    CY_CUDA_CHECK(cudaMallocAsync(&off, (size_t)(nsrc + 1) * sizeof(long long), st));
+    measure_units_scan_kernel<<<1, kScanThreads, 0, st>>>(src, nsrc, 0, ncols, row_begin, row_end, off);
+    long long units = 0;   // the unit count is data dependent: bring it to the host
+    cudaMemcpyAsync(&units, off + nsrc, sizeof(long long), cudaMemcpyDeviceToHost, st);
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess && units > 2147483647ll) {
+        cudaFreeAsync(off, st);
+        return set_error(CY_ERR_INVALID, "cy_source_mask: %lld work units exceed one grid", units);
+    }
+    if (e == cudaSuccess && units > 0)
+        source_mask_kernel<<<(unsigned)units, kThreads, 0, st>>>(src, nsrc, ncols, row_begin, row_end, off, mask);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    cudaFreeAsync(off, st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_source_mask: %s", cudaGetErrorString(e));
+    return CY_OK;
+}
+
+extern "C" int cy_bkg_grid_probe_init(const cy_noise_state* state, int nodes, cy_noise_state* probe, int* nprobe,
+                                      uintptr_t stream) {
+    if (nodes < 1 || !nprobe) return set_error(CY_ERR_INVALID, "cy_bkg_grid_probe_init: invalid arguments");
+    *nprobe = 0;
+    if (!state || !probe) return set_error(CY_ERR_INVALID, "cy_bkg_grid_probe_init: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    int* cnt = nullptr;
+    CY_CUDA_CHECK(cudaMallocAsync(&cnt, sizeof(int), st));
+    cudaMemsetAsync(cnt, 0, sizeof(int), st);
+    bkg_probe_init_kernel<<<(nodes + 255) / 256, 256, 0, st>>>(state, nodes, probe, cnt);
+    int n = 0;
+    cudaMemcpyAsync(&n, cnt, sizeof(int), cudaMemcpyDeviceToHost, st);
+    cudaFreeAsync(cnt, st);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_probe_init: %s", cudaGetErrorString(e));
+    *nprobe = n;
+    return CY_OK;
+}
+
+extern "C" int cy_bkg_grid_fill(const cy_noise_partial* probe_partials, int world, int nx, int ny,
+                                cy_noise_state* state, int* filled, uintptr_t stream) {
+    if (world < 1 || nx < 1 || ny < 1 || (long long)nx * ny > 2147483647ll || !filled)
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_fill: invalid arguments");
+    *filled = 0;
+    if (!probe_partials || !state) return set_error(CY_ERR_INVALID, "cy_bkg_grid_fill: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int nodes = nx * ny, blocks = (nodes + 255) / 256;
+    FillNode* buf = nullptr;
+    int* cnt = nullptr;
+    CY_CUDA_CHECK(cudaMallocAsync(&buf, 2 * (size_t)nodes * sizeof(FillNode), st));
+    if (cudaMallocAsync(&cnt, sizeof(int), st) != cudaSuccess) {
+        cudaFreeAsync(buf, st);
+        return set_error(CY_ERR_NOMEM, "cy_bkg_grid_fill: no memory for the ring counter");
+    }
+    FillNode *a = buf, *b = buf + nodes;
+    bkg_fill_classify_kernel<<<blocks, 256, 0, st>>>(probe_partials, world, nodes, state, a);
+    cudaError_t e = cudaSuccess;
+    int total = 0;
+    for (;;) {   // a ring fills at least one node or ends the fill: at most nodes + 1 rings
+        cudaMemsetAsync(cnt, 0, sizeof(int), st);
+        bkg_fill_ring_kernel<<<blocks, 256, 0, st>>>(a, nx, ny, b, cnt);
+        int changed = 0;
+        cudaMemcpyAsync(&changed, cnt, sizeof(int), cudaMemcpyDeviceToHost, st);
+        e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess || changed == 0) break;
+        total += changed;
+        FillNode* t = a;
+        a = b;
+        b = t;
+    }
+    if (e == cudaSuccess) {
+        bkg_fill_store_kernel<<<blocks, 256, 0, st>>>(a, nodes, state);
+        e = cudaGetLastError();
+    }
+    cudaFreeAsync(cnt, st);
+    cudaFreeAsync(buf, st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_fill: %s", cudaGetErrorString(e));
+    *filled = total;
     return CY_OK;
 }

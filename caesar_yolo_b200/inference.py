@@ -59,6 +59,12 @@ class SFinder(object):
         self.save_bkg_maps = bool(config.get('save_bkg_maps', False))
         self.bkg_box = int(config.get('bkg_box', 101))
         self.bkg_grid = int(config.get('bkg_grid', 25))
+        # the catalog boxes masked out of the noise frames and the map nodes; only these two consumers use the mask
+        self.bkg_mask_sources = bool(config.get('bkg_mask_sources', False))
+        if self.bkg_mask_sources and not (self.measure_noise or self.save_bkg_maps):
+            logger.warning("bkg_mask_sources masks the catalog boxes out of the measure_noise frames and the "
+                           "save_bkg_maps nodes: with neither option on it changes nothing")
+            self.bkg_mask_sources = False
         self.procId, self.nproc = _dist_info()
         self.timing = {}
         self.engine = None
@@ -204,14 +210,16 @@ class SFinder(object):
         recs = recs.copy()
         recs['x1'] -= x0; recs['x2'] -= x0; recs['y1'] -= y0; recs['y2'] -= y0
         meas = None
+        # one mask of the catalog boxes over the crop, for the frames and the map nodes alike
+        mask = eng.source_mask(_as_sources(recs), x1 - x0, 0, y1 - y0) if self.bkg_mask_sources else None
         if self.measure_sources:   # in the coordinates of the catalog: the (sub-)image read, columns from x0
             args = (_as_sources(recs), dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0)
             m = eng.measure(*args)
-            noise = eng.measure_noise(*args, frame=self.noise_frame) if self.measure_noise else None
+            noise = eng.measure_noise(*args, frame=self.noise_frame, mask=mask) if self.measure_noise else None
             meas = self._measurements(m, self.fits.header, x0, y0, noise)
         if self.save_bkg_maps:   # the region read: the crop, columns from x0
             _, bkg, rms = eng.bkg_maps(dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0, 0,
-                                       y1 - y0, self.bkg_box, self.bkg_grid)
+                                       y1 - y0, self.bkg_box, self.bkg_grid, mask=mask)
             self._write_bkg_maps(bkg, rms, 0, (x0, y0, x1 - x0, y1 - y0))
         self.timing['run_s'] = time.time() - t0
         return self._save_serial(recs, status, meas)
@@ -231,7 +239,7 @@ class SFinder(object):
         (X0, R0, W, H), with the image's WCS shifted to the region."""
         X0, R0, W, H = region
         t0 = time.time()
-        hdr = fitsmeta.map_header(self.fits.header, W, H, X0, R0)
+        hdr = fitsmeta.map_header(self.fits.header, W, H, X0, R0, bkgmask=self.bkg_mask_sources)
         for name, rows in (('bkgmap_', bkg), ('rmsmap_', rms)):
             fitsmeta.write_map_rows(os.path.join(self.outdir, name + str(self.image_id) + '.fits'), hdr, rows,
                                     row_begin, W, H, self.procId, self.nproc)
@@ -301,7 +309,8 @@ class SFinder(object):
                 logger.warning("Colour image: per-source measurements need a single-plane image and are not written")
             else:
                 args = (_as_sources(recs), plane_dev, W, False, 0, W, 0, H)
-                noise = eng.measure_noise(*args, frame=self.noise_frame) if self.measure_noise else None
+                mask = eng.source_mask(args[0], W, 0, H) if self.bkg_mask_sources and self.measure_noise else None
+                noise = eng.measure_noise(*args, frame=self.noise_frame, mask=mask) if self.measure_noise else None
                 meas = self._measurements(eng.measure(*args), {}, noise=noise)
         self.timing['run_s'] = time.time() - t0
         return self._save_serial(recs, 0, meas)
@@ -345,8 +354,8 @@ class SFinder(object):
                 st = eng.tile_status[a:b].cpu().numpy()
                 catalog.write_tile_outputs(recs, tiles, np.arange(a, b), st, self.class_names, self.image_id,
                                            self.outdir, self.save_tile_json, self.save_tile_regions)
-        # measurements need the catalog on every rank (each measures its own rows)
-        rank0_only = not self.measure_sources
+        # measurements and masked maps need the catalog on every rank (each measures or masks its own rows)
+        rank0_only = not (self.measure_sources or (self.save_bkg_maps and self.bkg_mask_sources))
         if self._host_callable() is not None:
             from .pipeline import split_tile_rows
             eng.begin(tiles)
@@ -364,15 +373,18 @@ class SFinder(object):
             src, n = run_image(eng, img, self.fits.is_raw_f32, tiles, rank=self.procId, world=self.nproc,
                                on_rank0_only=rank0_only, on_local_records=hook)
         meas = None
+        # one mask of the catalog boxes over this rank's rows, for the frames and the map nodes alike
+        mask = eng.source_mask_band(src, tiles, self.procId, self.nproc) if self.bkg_mask_sources else None
         if self.measure_sources:
             m = eng.measure_band(src, tiles, self.procId, self.nproc)
             noise = None
             if self.measure_noise:
-                noise = eng.measure_noise_band(src, tiles, self.noise_frame, self.procId, self.nproc)
+                noise = eng.measure_noise_band(src, tiles, self.noise_frame, self.procId, self.nproc, mask=mask)
             if self.procId == 0:
                 meas = self._measurements(m, self.fits.header, noise=noise)
-        if self.save_bkg_maps:   # every rank maps and writes its own rows; the catalog is not needed
-            _, bkg, rms, region, rows = eng.bkg_maps_band(tiles, self.bkg_box, self.bkg_grid, self.procId, self.nproc)
+        if self.save_bkg_maps:   # every rank maps and writes its own rows; unmasked maps need no catalog
+            _, bkg, rms, region, rows = eng.bkg_maps_band(tiles, self.bkg_box, self.bkg_grid, self.procId, self.nproc,
+                                                          mask=mask)
             self._write_bkg_maps(bkg, rms, rows[0] - region[1], region)
         self.timing['run_s'] = time.time() - t0
         if self.procId == 0:

@@ -409,6 +409,34 @@ def noise_pass(img, row_stride, big_endian, row0, ncols, src_dev, nsrc, row_begi
     return out
 
 
+def noise_pass_masked(img, row_stride, big_endian, row0, ncols, src_dev, nsrc, row_begin, row_end, frame, unit_off,
+                      units, state, out, mask):
+    """cy_noise_pass_masked: noise_pass with the frame pixels in the source mask (source_mask of the same sources,
+    ncols and rows) masked."""
+    check(lib.cy_noise_pass_masked(ptr(img), c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0),
+                                   c_int(ncols), ptr(src_dev), c_int(nsrc), c_int(row_begin), c_int(row_end),
+                                   c_int(frame), ptr(unit_off), c_i64(units), ptr(state), ptr(out), ptr(mask),
+                                   cur_stream()))
+    return out
+
+
+def source_mask_words(ncols):
+    """uint32 words per row of a source mask of ncols columns."""
+    return (ncols + 31) // 32
+
+
+def source_mask(src_dev, nsrc, ncols, row_begin, row_end, out=None):
+    """cy_source_mask: bit mask of the union of the catalog boxes over columns [0, ncols) and rows [row_begin, row_end)
+    -> int32 device tensor [row_end - row_begin, source_mask_words(ncols)] (bit x & 31 of word x >> 5 of row
+    y - row_begin: pixel (x, y) lies in a box; synchronises)."""
+    shape = (row_end - row_begin, source_mask_words(ncols))
+    if out is None:
+        out = torch.empty(shape, dtype=torch.int32, device=src_dev.device)
+    check(lib.cy_source_mask(ptr(src_dev), c_int(nsrc), c_int(ncols), c_int(row_begin), c_int(row_end), ptr(out),
+                             cur_stream()))
+    return out
+
+
 def noise_update(partials, world, nsrc, state):
     """cy_noise_update: partials [world * nsrc * 24] uint8 device (rank-major) -> state advanced by one pass.  Returns
     the number of sources still active (synchronises)."""
@@ -441,6 +469,34 @@ def bkg_grid_pass(img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, r
                                c_int(R0), c_int(R1), c_int(row_begin), c_int(row_end), c_int(box), c_int(grid),
                                ptr(unit_off), c_i64(units), ptr(state), ptr(out), cur_stream()))
     return out
+
+
+def bkg_grid_pass_masked(img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box, grid, unit_off,
+                         units, state, out, mask, mask_ncols, mask_col0=0):
+    """cy_bkg_grid_pass_masked: bkg_grid_pass with the node-box pixels in the source mask masked; mask: source_mask of
+    rows [row_begin, row_end) over mask_ncols columns, region column x = mask column x + mask_col0."""
+    check(lib.cy_bkg_grid_pass_masked(ptr(img), c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0),
+                                      c_int(ncols), c_int(R0), c_int(R1), c_int(row_begin), c_int(row_end), c_int(box),
+                                      c_int(grid), ptr(unit_off), c_i64(units), ptr(state), ptr(out), ptr(mask),
+                                      c_int(mask_ncols), c_int(mask_col0), cur_stream()))
+    return out
+
+
+def bkg_grid_probe_init(state, nodes, probe):
+    """cy_bkg_grid_probe_init: probe state (uint8 device tensor of >= nodes cy_noise_state) with the nodes of nbkg = 0
+    active.  Returns their count (synchronises)."""
+    n = c_int(0)
+    check(lib.cy_bkg_grid_probe_init(ptr(state), c_int(nodes), ptr(probe), ctypes.byref(n), cur_stream()))
+    return n.value
+
+
+def bkg_grid_fill(probe_partials, world, nx, ny, state):
+    """cy_bkg_grid_fill: probe partials [world * Nx * Ny * 24] uint8 device (rank-major) -> the holes of the node states
+    filled in rings.  Returns the number of nodes filled (synchronises once per ring)."""
+    n = c_int(0)
+    check(lib.cy_bkg_grid_fill(ptr(probe_partials), c_int(world), c_int(nx), c_int(ny), ptr(state), ctypes.byref(n),
+                               cur_stream()))
+    return n.value
 
 
 def bkg_grid_maps(state, ncols, R0, R1, row_begin, row_end, box, grid, bkg, rms):

@@ -42,11 +42,22 @@ def make_pp_config(enabled=True, subtract_bkg=False, sigma_bkg=3.0, use_box_mask
 import os
 import time
 
+from typing import NamedTuple
+
 import numpy as np
 import torch
 
 from . import ops
 from ._capi import CaesarB200Error, Letterbox
+
+
+class SourceMask(NamedTuple):
+    """Engine.source_mask: the bit mask of rows [row_begin, row_end) (int32 device tensor [rows, ceil(ncols / 32)],
+    layout: ops.source_mask) and the columns and rows it was built over, which its consumers check."""
+    bits: torch.Tensor
+    ncols: int
+    row_begin: int
+    row_end: int
 
 
 class Engine(object):
@@ -354,19 +365,45 @@ class Engine(object):
             band, Y0 = self._get('meas_noband', (1,), torch.int32), r0
         return self.measure(sources, band, nx, big_endian, Y0, nx, r0, r1, world=world)
 
-    def measure_noise(self, sources, img, row_stride, big_endian, row0, ncols, row_begin, row_end, frame=16, world=1):
+    def source_mask(self, sources, ncols, row_begin, row_end):
+        """Bit mask of the union of the boxes of the catalog `sources` (ops.SRC_DTYPE) over columns [0, ncols) and rows
+        [row_begin, row_end) (cy_source_mask; layout: ops.source_mask) -> SourceMask.  A run builds it once over the rows
+        it measures and passes it to measure_noise and bkg_maps, so both leave the catalog boxes out of their
+        statistics."""
+        src = np.ascontiguousarray(sources, dtype=ops.SRC_DTYPE)
+        e = self._mark()
+        out = torch.empty((row_end - row_begin, ops.source_mask_words(ncols)), dtype=torch.int32, device=self.device)
+        mask = ops.source_mask(ops.to_device_bytes(src, self.device), len(src), ncols, row_begin, row_end, out=out)
+        self._stage('source_mask', e)
+        self.launches += 3 if len(src) else 1
+        return SourceMask(mask, ncols, row_begin, row_end)
+
+    def source_mask_band(self, sources, tiles, rank=0, world=1):
+        """Engine.source_mask over the image columns and the rows this rank owns (measure_rows): the mask that
+        measure_noise_band and bkg_maps_band take."""
+        r0, r1 = measure_rows(tiles, world)[rank]
+        return self.source_mask(sources, self.band[3], r0, r1)
+
+    def measure_noise(self, sources, img, row_stride, big_endian, row0, ncols, row_begin, row_end, frame=16, world=1,
+                      mask=None):
         """Local background and noise of the catalog `sources` (ops.SRC_DTYPE): sigma-clipped mean / std of a frame of
         `frame` pixels around each box, over rows [row_begin, row_end) of `img` (arguments as for Engine.measure;
         cy_noise_init / cy_noise_pass / cy_noise_update).  One pass per clipping iteration, at most
         ops.NOISE_MAX_PASSES; with world > 1 every rank passes the same catalog and its own rows, and the partials of
         each pass are all-gathered in the group of the record exchange.  Every rank folds the same partials, so every
-        rank sees the same active count and runs the same passes.  Returns a structured array (ops.NOISE_DTYPE) whose
-        bkg, rms, nbkg, iters are final; self.noise_passes holds the number of passes run."""
+        rank sees the same active count and runs the same passes.  mask: Engine.source_mask of the same catalog, ncols
+        and rows, or None; with it, the frame pixels inside any catalog box are masked (cy_noise_pass_masked).  Returns
+        a structured array (ops.NOISE_DTYPE) whose bkg, rms, nbkg, iters are final; self.noise_passes holds the number
+        of passes run."""
         src = np.ascontiguousarray(sources, dtype=ops.SRC_DTYPE)
         n = len(src)
         self.noise_passes = 0
         if n == 0:
             return np.zeros(0, dtype=ops.NOISE_DTYPE)
+        if mask is not None and (mask.ncols, mask.row_begin, mask.row_end) != (ncols, row_begin, row_end):
+            raise CaesarB200Error("Engine.measure_noise: a mask of %d columns, rows [%d, %d) for a frame of %d columns, "
+                                  "rows [%d, %d)" % (mask.ncols, mask.row_begin, mask.row_end, ncols, row_begin,
+                                                     row_end))
         src_dev = ops.to_device_bytes(src, self.device)
         e = self._mark()
         state = self._get('noise_state', (n * ops.NOISE_DTYPE.itemsize,), torch.uint8)
@@ -382,8 +419,12 @@ class Engine(object):
             if self.noise_passes == ops.NOISE_MAX_PASSES:
                 raise ops.CaesarB200Error("cy_noise_update: %d sources still active after %d passes"
                                           % (active, self.noise_passes))
-            ops.noise_pass(img, row_stride, big_endian, row0, ncols, src_dev, n, row_begin, row_end, frame, off, units,
-                           state, part)
+            if mask is None:
+                ops.noise_pass(img, row_stride, big_endian, row0, ncols, src_dev, n, row_begin, row_end, frame, off,
+                               units, state, part)
+            else:
+                ops.noise_pass_masked(img, row_stride, big_endian, row0, ncols, src_dev, n, row_begin, row_end, frame,
+                                      off, units, state, part, mask.bits)
             if world > 1:
                 dist.all_gather_into_tensor(allp, part)
             active = ops.noise_update(allp, world, n, state)
@@ -392,25 +433,35 @@ class Engine(object):
         self.launches += 3 + self.noise_passes * (3 + (1 if world > 1 else 0))
         return state.cpu().numpy().view(ops.NOISE_DTYPE)
 
-    def measure_noise_band(self, sources, tiles, frame=16, rank=0, world=1):
+    def measure_noise_band(self, sources, tiles, frame=16, rank=0, world=1, mask=None):
         """Engine.measure_noise over the rows this rank owns (measure_rows), read from the band of mosaic rows the last
-        run_image left in HBM.  The frames are thus clipped to the rows the run read, and no rank reads a row twice."""
+        run_image left in HBM.  The frames are thus clipped to the rows the run read, and no rank reads a row twice.
+        mask: Engine.source_mask_band of the same catalog, or None."""
         r0, r1 = measure_rows(tiles, world)[rank]
         band, Y0, _, nx, big_endian = self.band
         if band is None:                     # a rank without tiles still takes part in every all-gather
             band, Y0 = self._get('meas_noband', (1,), torch.int32), r0
-        return self.measure_noise(sources, band, nx, big_endian, Y0, nx, r0, r1, frame=frame, world=world)
+        return self.measure_noise(sources, band, nx, big_endian, Y0, nx, r0, r1, frame=frame, world=world, mask=mask)
 
-    def bkg_maps(self, img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box=101, grid=25, world=1):
+    def bkg_maps(self, img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box=101, grid=25, world=1,
+                 mask=None, mask_col0=0):
         """Background and rms maps of the region of columns [0, ncols) of `img` and rows [R0, R1) (node lattice,
         statistic and interpolation: include/caesar_b200.h), over rows [row_begin, row_end) of `img` (arguments as for
         Engine.measure; cy_bkg_grid_init / cy_bkg_grid_pass / cy_noise_update / cy_bkg_grid_maps).  With world > 1 every
         rank passes the same region and its own rows, and the node partials of each pass are all-gathered in the group of
-        the record exchange, so every rank runs the same passes.  Returns (nodes, bkg, rms): the final node states
-        (ops.NOISE_DTYPE, shape [Ny, Nx]) and this range's map rows as int32 device tensors [row_end - row_begin, ncols]
-        holding big-endian float32; self.bkg_passes holds the number of passes run."""
+        the record exchange, so every rank runs the same passes.  mask: Engine.source_mask of rows [row_begin, row_end),
+        region column x being mask column x + mask_col0, or None.  With it, the node-box pixels inside any catalog box
+        are masked (cy_bkg_grid_pass_masked), and the nodes left without a pixel whose box holds data are filled from
+        their neighbours (cy_bkg_grid_probe_init, one unmasked pass of the probe, cy_bkg_grid_fill); self.bkg_holes_filled
+        holds their count.  Returns (nodes, bkg, rms): the final node states (ops.NOISE_DTYPE, shape [Ny, Nx]) and this
+        range's map rows as int32 device tensors [row_end - row_begin, ncols] holding big-endian float32;
+        self.bkg_passes holds the number of clipping passes run."""
         nx, ny = len(ops.bkg_grid_nodes(ncols, grid)), len(ops.bkg_grid_nodes(R1 - R0, grid))
         nodes = nx * ny
+        if mask is not None and (mask.row_end - mask.row_begin != row_end - row_begin or
+                                 (row_end > row_begin and mask.row_begin != row_begin)):
+            raise CaesarB200Error("Engine.bkg_maps: a mask of rows [%d, %d) for rows [%d, %d)"
+                                  % (mask.row_begin, mask.row_end, row_begin, row_end))
         e = self._mark()
         state = self._get('bkg_state', (nodes * ops.NOISE_DTYPE.itemsize,), torch.uint8)
         off = self._get('bkg_off', (ny + 1,), torch.int64)
@@ -426,12 +477,27 @@ class Engine(object):
             if self.bkg_passes == ops.NOISE_MAX_PASSES:
                 raise ops.CaesarB200Error("cy_noise_update: %d grid nodes still active after %d passes"
                                           % (active, self.bkg_passes))
-            ops.bkg_grid_pass(img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box, grid, off,
-                              units, state, part)
+            if mask is None:
+                ops.bkg_grid_pass(img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box, grid, off,
+                                  units, state, part)
+            else:
+                ops.bkg_grid_pass_masked(img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box,
+                                         grid, off, units, state, part, mask.bits, mask.ncols, mask_col0)
             if world > 1:
                 dist.all_gather_into_tensor(allp, part)
             active = ops.noise_update(allp, world, nodes, state)
             self.bkg_passes += 1
+        self.bkg_holes_filled = 0
+        if mask is not None:   # the node states are the same on every rank, and so is the probe count
+            probe = self._get('bkg_probe', (nodes * ops.NOISE_DTYPE.itemsize,), torch.uint8)
+            if ops.bkg_grid_probe_init(state, nodes, probe):
+                ops.bkg_grid_pass(img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box, grid, off,
+                                  units, probe, part)
+                if world > 1:
+                    dist.all_gather_into_tensor(allp, part)
+                self.bkg_holes_filled = ops.bkg_grid_fill(allp, world, nx, ny, state)
+                self.launches += 3 + (1 if world > 1 else 0) + 2
+            self.launches += 1
         bkg = torch.empty((row_end - row_begin, ncols), dtype=torch.int32, device=self.device)
         rms = torch.empty_like(bkg)
         ops.bkg_grid_maps(state, ncols, R0, R1, row_begin, row_end, box, grid, bkg, rms)
@@ -439,10 +505,11 @@ class Engine(object):
         self.launches += 3 + self.bkg_passes * (3 + (1 if world > 1 else 0)) + 1
         return state.cpu().numpy().view(ops.NOISE_DTYPE).reshape(ny, nx), bkg, rms
 
-    def bkg_maps_band(self, tiles, box=101, grid=25, rank=0, world=1):
+    def bkg_maps_band(self, tiles, box=101, grid=25, rank=0, world=1, mask=None):
         """Engine.bkg_maps of the bounding box of the tile grid (columns [min xmin, max xmax), rows [min ymin,
         max ymax)) over the rows this rank owns (measure_rows), read from the band of mosaic rows the last run_image
-        left in HBM.  Returns (nodes, bkg, rms, (X0, R0, W, H), (row_begin, row_end))."""
+        left in HBM.  mask: Engine.source_mask_band (image columns, so the region starts at its column X0), or None.
+        Returns (nodes, bkg, rms, (X0, R0, W, H), (row_begin, row_end))."""
         X0, X1 = int(tiles['xmin'].min()), int(tiles['xmax'].max())
         R0, R1 = int(tiles['ymin'].min()), int(tiles['ymax'].max())
         r0, r1 = measure_rows(tiles, world)[rank]
@@ -453,7 +520,8 @@ class Engine(object):
             img, Y0 = self._get('meas_noband', (1,), torch.int32), r0
         else:
             img = band[:, X0:]
-        nodes, bkg, rms = self.bkg_maps(img, nx, big_endian, Y0, X1 - X0, R0, R1, r0, r1, box, grid, world)
+        nodes, bkg, rms = self.bkg_maps(img, nx, big_endian, Y0, X1 - X0, R0, R1, r0, r1, box, grid, world, mask=mask,
+                                        mask_col0=X0)
         return nodes, bkg, rms, (X0, R0, X1 - X0, R1 - R0), (r0, r1)
 
     def _exchange_cap(self, world, need=0):

@@ -329,6 +329,26 @@ int cy_noise_pass(const void* img, long long row_stride, int big_endian, int row
 int cy_noise_update(const cy_noise_partial* partials, int world, int nsrc, cy_noise_state* state, int* active,
                     uintptr_t stream);
 
+/* Source mask (opt-in, not part of the reference).  M is the union over all sources of the integer boxes [ceil x1,
+ * floor x2] x [ceil y1, floor y2], the rule of the box measurements; an empty box or NaN coordinates add nothing, and
+ * the boxes are not dilated.  Membership is decided in absolute pixel coordinates, so M does not depend on the row
+ * split.  With the mask, a frame pixel (cy_noise_pass_masked) or a node-box pixel (cy_bkg_grid_pass_masked) in M is
+ * masked exactly like a non-finite or 0 pixel.  A frame already excludes its own box, so the mask removes the boxes of
+ * its neighbours; a frame left empty gives nbkg = 0 and NaN bkg / rms, as above.  The per-source statistics and the
+ * maps of one run use the same M, so they still compare directly.
+ * Layout: rows [row_begin, row_end) of the image, (row_end - row_begin) x ceil(ncols / 32) uint32 words, row-major;
+ * bit (x & 31) of word (x >> 5) of mask row y - row_begin is set when pixel (x, y) is in M; bits past ncols are 0.
+ * Writes the mask of columns [0, ncols) and rows [row_begin, row_end) for the nsrc sources src[] (device): zeroed first,
+ * then the bits of every box ORed in (work units of up to 32 rows of one box, so the result does not depend on the
+ * order).  Synchronises the stream (the unit count is data dependent). */
+int cy_source_mask(const cy_source* src, int nsrc, int ncols, int row_begin, int row_end, uint32_t* mask,
+                   uintptr_t stream);
+/* cy_noise_pass with the frame pixels in M masked; mask: cy_source_mask of the same src, ncols and rows. */
+int cy_noise_pass_masked(const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                         const cy_source* src, int nsrc, int row_begin, int row_end, int frame,
+                         const long long* unit_off, long long units, const cy_noise_state* state,
+                         cy_noise_partial* partials, const uint32_t* mask, uintptr_t stream);
+
 /* Background and rms maps of an image region (not part of the reference).  The region is W = ncols columns (columns
  * [0, ncols) of the buffer) by H = R1 - R0 rows (rows [R0, R1)); a run maps the pixels it read.
  * Grid nodes: with step g = grid, node column i sits at x_i = min(i g, W - 1), i = 0 .. Nx - 1, Nx = ceil((W - 1) / g)
@@ -356,6 +376,33 @@ int cy_bkg_grid_init(int ncols, int R0, int R1, int row_begin, int row_end, int 
 int cy_bkg_grid_pass(const void* img, long long row_stride, int big_endian, int row0, int ncols, int R0, int R1,
                      int row_begin, int row_end, int box, int grid, const long long* unit_off, long long units,
                      const cy_noise_state* state, cy_noise_partial* partials, uintptr_t stream);
+/* cy_bkg_grid_pass with the node-box pixels in M masked.  mask: cy_source_mask of rows [row_begin, row_end) over
+ * mask_ncols columns; region column x is mask column x + mask_col0 (0 <= mask_col0, mask_col0 + ncols <= mask_ncols), so
+ * a region that starts at column X0 of a wider mask passes mask_col0 = X0. */
+int cy_bkg_grid_pass_masked(const void* img, long long row_stride, int big_endian, int row0, int ncols, int R0, int R1,
+                            int row_begin, int row_end, int box, int grid, const long long* unit_off, long long units,
+                            const cy_noise_state* state, cy_noise_partial* partials, const uint32_t* mask,
+                            int mask_ncols, int mask_col0, uintptr_t stream);
+/* Hole fill of a masked lattice.  After the masked passes every node is one of:
+ *   finite: nbkg > 0;
+ *   hole:   nbkg = 0, but its box holds at least one data pixel (finite and non-zero) when M is ignored;
+ *   blank:  its box holds no data pixel (the NaN borders of a mosaic).
+ * Ring k fills every unfilled hole that has a finite or already-filled node among its 8 lattice neighbours with the fp64
+ * mean of those neighbours' bkg and, separately, rms as they stood after ring k - 1, summed in row-major neighbour order
+ * (deterministic).  Rings repeat until no node changes.  Blank nodes are never filled and never feed the fill, so NaN
+ * borders do not spread; holes with no path to a finite node stay NaN; a filled node keeps nbkg = 0.  The map
+ * interpolation above is unchanged.  Catalog bkg / rms are never filled.
+ * Probe: sets probe[nodes] to pass 0 for the nodes with nbkg = 0 of the final states `state` and to done for the
+ * others, *nprobe the count of the former (the same on every rank).  When it is not 0, one unmasked cy_bkg_grid_pass
+ * of the probe (same arguments and unit plan as the passes; only the boxes of the probed nodes are read) gives each
+ * probed node's data-pixel count n; the partials are all-gathered like those of a pass.  Synchronises the stream. */
+int cy_bkg_grid_probe_init(const cy_noise_state* state, int nodes, cy_noise_state* probe, int* nprobe,
+                           uintptr_t stream);
+/* Fill: probe partials [world][Nx * Ny] folded in rank order (n > 0: hole) -> the holes of state[Nx * Ny] filled in
+ * rings; *filled: the nodes filled.  Every rank fills the same replicated states identically.  Synchronises the stream
+ * once per ring. */
+int cy_bkg_grid_fill(const cy_noise_partial* probe_partials, int world, int nx, int ny, cy_noise_state* state,
+                     int* filled, uintptr_t stream);
 /* Final node states -> rows [row_begin, row_end) of the bkg and rms maps: (row_end - row_begin) x ncols 4-byte words
  * each, row-major, big-endian float32.  No pixel of the image is read. */
 int cy_bkg_grid_maps(const cy_noise_state* state, int ncols, int R0, int R1, int row_begin, int row_end, int box,

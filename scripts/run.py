@@ -81,6 +81,9 @@ def parse_args(argv=None):
                    help='B200 build only: side in pixels (odd, >= 3) of the box each --save_bkg_maps node clips')
     p.add_argument('--bkg_grid', dest='bkg_grid', type=int, default=25,
                    help='B200 build only: step in pixels (>= 1) of the --save_bkg_maps node lattice')
+    p.add_argument('--bkg_mask_sources', dest='bkg_mask_sources', action='store_true',
+                   help='B200 build only: mask the catalog boxes out of the --measure_noise frames and the '
+                        '--save_bkg_maps node boxes, and fill the map nodes left without pixels from their neighbours')
     p.add_argument('--detect_outfile', required=False, type=str, default="")
     p.add_argument('--detect_outfile_json', required=False, type=str, default="")
     args = p.parse_args(argv)
@@ -188,7 +191,7 @@ def main(argv=None):
         'save_tile_catalog': args.save_tile_catalog, 'save_tile_region': args.save_tile_region,
         'save_tile_img': args.save_tile_img, 'precision': args.precision, 'measure_sources': args.measure_sources,
         'measure_noise': args.measure_noise, 'noise_frame': args.noise_frame, 'save_bkg_maps': args.save_bkg_maps,
-        'bkg_box': args.bkg_box, 'bkg_grid': args.bkg_grid,
+        'bkg_box': args.bkg_box, 'bkg_grid': args.bkg_grid, 'bkg_mask_sources': args.bkg_mask_sources,
     })
     model = YOLO(args.weights, precision=args.precision)
     sfinder = SFinder(model, CONFIG)

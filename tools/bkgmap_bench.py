@@ -10,7 +10,14 @@ Algorithmic bytes of pass p: for every unit whose node group has an active node 
 rows and of the columns from its first to its last active node's box (what bkg_unit_kernel reads), plus the unit
 partials written and folded.  The map kernel writes 8 bytes per pixel and reads no image pixel.
 
-    python tools/bkgmap_bench.py [--configs 3,4] [--reps 5] [--out DIR]
+With --mask, the source mask is timed as well on the catalog of the same run_image: the mask build
+(Engine.source_mask_band), the masked map call (Engine.bkg_maps_band with the mask: masked passes, probe and fill), the
+probe and fill alone (events around cy_bkg_grid_probe_init, the probe pass and cy_bkg_grid_fill, restated from the final
+masked states), and the local noise of the catalog with and without the mask (Engine.measure_noise_band).  The masked and
+unmasked calls alternate within each repetition, so both see the same machine state.  It reports the masked pixel
+fraction, the nodes left without pixels and the holes filled, and writes r05_bkgmask_bench.json to --out.
+
+    python tools/bkgmap_bench.py [--configs 3,4] [--reps 5] [--mask] [--out DIR]
 """
 import argparse
 import json
@@ -72,7 +79,7 @@ def run_config(cfg, reps, variant, box, grid):
     t0 = time.time()
     k = 2
     for _ in range(k):
-        pipeline.run_image(eng, host, True, tiles)
+        src, _ = pipeline.run_image(eng, host, True, tiles)
     torch.cuda.synchronize()
     step_ms = (time.time() - t0) * 1e3 / k
     res = None
@@ -137,6 +144,93 @@ def run_config(cfg, reps, variant, box, grid):
                     "one rank, a temporary directory on the local disk)"}
 
 
+def _events(fn, reps):
+    """ms per call of fn over reps calls, CUDA events around each call (fn synchronises inside: host reads)."""
+    import torch
+    t = 0.0
+    for _ in range(reps):
+        a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a0.record()
+        fn()
+        a1.record()
+        torch.cuda.synchronize()
+        t += a0.elapsed_time(a1)
+    return t / reps
+
+
+def mask_config(cfg, reps, variant, box, grid, frame=16):
+    """The --mask measurements of one config (module docstring)."""
+    import torch
+    from caesar_yolo_b200 import ops, pipeline, weights as W
+    dev = torch.device('cuda:0')
+    torch.cuda.set_device(dev)
+    a = argparse.Namespace(mosaic=32768 if cfg == 4 else 16384)
+    step = 0.5 if cfg == 4 else 1.0
+    n = a.mosaic
+    _, host = bench.make_mosaic_pinned(a)
+    tiles = ops.generate_tiles(0, n - 1, 0, n - 1, 512, 512, step, step)
+    w = W.make_random_weights(variant, 5, seed=0, cls_bias=bench.CLS_BIAS.get(variant, -16.0))
+    eng = pipeline.Engine(w, pipeline.make_pp_config(**bench.PP_FLAGS), imgsz=640, score_thr=bench.SCORE_THR,
+                          iou_thr=bench.IOU_THR, thr_soft=bench.SOFT, thr_hard=bench.HARD, device=dev)
+    src, _ = pipeline.run_image(eng, host, True, tiles)
+    mask = eng.source_mask_band(src, tiles)              # warm-up of every call timed below
+    plain = eng.bkg_maps_band(tiles, box, grid)[0]
+    nodes, _, _, (X0, R0, Wd, Hd), rows = eng.bkg_maps_band(tiles, box, grid, mask=mask)
+    passes, filled = eng.bkg_passes, eng.bkg_holes_filled
+    eng.measure_noise_band(src, tiles, frame)
+    eng.measure_noise_band(src, tiles, frame, mask=mask)
+    ms = dict(mask=0.0, maps=0.0, maps_masked=0.0, noise=0.0, noise_masked=0.0)
+    for _ in range(reps):                                # the masked and unmasked calls alternate
+        ms['mask'] += _events(lambda: eng.source_mask_band(src, tiles), 1) / reps
+        ms['maps'] += _events(lambda: eng.bkg_maps_band(tiles, box, grid), 1) / reps
+        ms['maps_masked'] += _events(lambda: eng.bkg_maps_band(tiles, box, grid, mask=mask), 1) / reps
+        ms['noise'] += _events(lambda: eng.measure_noise_band(src, tiles, frame), 1) / reps
+        ms['noise_masked'] += _events(lambda: eng.measure_noise_band(src, tiles, frame, mask=mask), 1) / reps
+    noise_passes = eng.noise_passes
+    # probe and fill alone, from the final masked states (restated: the masked passes, then a copy of the states)
+    band, Y0, _, nx, be = eng.band
+    img = band[:, X0:]
+    nn = nodes.size
+    state = torch.empty((nn * ops.NOISE_DTYPE.itemsize,), dtype=torch.uint8, device=dev)
+    probe = torch.empty_like(state)
+    off = torch.empty((nodes.shape[0] + 1,), dtype=torch.int64, device=dev)
+    part = torch.empty((nn * ops.NOISE_PARTIAL_BYTES,), dtype=torch.uint8, device=dev)
+    units = ops.bkg_grid_init(Wd, R0, R0 + Hd, rows[0], rows[1], box, grid, state, off)
+    active = nn
+    while active:
+        ops.bkg_grid_pass_masked(img, nx, be, Y0, Wd, R0, R0 + Hd, rows[0], rows[1], box, grid, off, units, state, part,
+                                 mask.bits, mask.ncols, X0)
+        active = ops.noise_update(part, 1, nn, state)
+    saved = state.clone()
+
+    def probe_fill():
+        state.copy_(saved)
+        if ops.bkg_grid_probe_init(state, nn, probe):
+            ops.bkg_grid_pass(img, nx, be, Y0, Wd, R0, R0 + Hd, rows[0], rows[1], box, grid, off, units, probe, part)
+            ops.bkg_grid_fill(part, 1, nodes.shape[1], nodes.shape[0], state)
+    probe_fill()
+    probe_ms = _events(probe_fill, reps)
+    assert state.cpu().numpy().view(ops.NOISE_DTYPE).tobytes() == nodes.tobytes()
+    mbits = 0
+    mh = mask.bits.cpu().numpy().view(np.uint8)
+    for r in range(0, mh.shape[0], 1024):
+        mbits += int(np.unpackbits(mh[r:r + 1024]).sum())
+    masked_frac = mbits / float(mh.shape[0] * nx)
+    return {"config": cfg, "mosaic": n, "tile_step": step, "bkg_box": box, "bkg_grid": grid, "noise_frame": frame,
+            "sources": int(len(src)), "masked_pixel_fraction": round(masked_frac, 5),
+            "nodes": [int(nodes.shape[0]), int(nodes.shape[1])], "passes_masked": passes,
+            "nodes_without_pixels_unmasked": int(np.sum(plain['nbkg'] == 0)),
+            "nodes_without_pixels_masked": int(np.sum(nodes['nbkg'] == 0)), "holes_filled": int(filled),
+            "noise_passes": noise_passes,
+            "source_mask_ms": round(ms['mask'], 3), "bkg_maps_ms": round(ms['maps'], 3),
+            "bkg_maps_masked_ms": round(ms['maps_masked'], 3), "probe_fill_ms": round(probe_ms, 3),
+            "noise_ms": round(ms['noise'], 3), "noise_masked_ms": round(ms['noise_masked'], 3),
+            "note": "CUDA events around each call, synchronised after it; the masked and unmasked calls alternate in "
+                    "every repetition.  bkg_maps_masked_ms includes the masked passes, the probe and the fill, not the "
+                    "mask build (source_mask_ms, built once per run); probe_fill_ms: cy_bkg_grid_probe_init, the probe "
+                    "pass and cy_bkg_grid_fill from the final masked states"}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--configs', default='3,4')
@@ -144,18 +238,20 @@ def main():
     ap.add_argument('--variant', default='l')
     ap.add_argument('--bkg_box', type=int, default=101)
     ap.add_argument('--bkg_grid', type=int, default=25)
-    ap.add_argument('--out', default=None, help='directory for bkgmap_bench.json')
+    ap.add_argument('--mask', action='store_true', help='time the source mask (module docstring)')
+    ap.add_argument('--out', default=None, help='directory for bkgmap_bench.json (r05_bkgmask_bench.json with --mask)')
     a = ap.parse_args()
     info = card()
     lines = []
     for c in [int(x) for x in a.configs.split(',')]:
-        r = run_config(c, a.reps, a.variant, a.bkg_box, a.bkg_grid)
+        r = (mask_config if a.mask else run_config)(c, a.reps, a.variant, a.bkg_box, a.bkg_grid)
         r.update(info)
         print(json.dumps(r), flush=True)
         lines.append(r)
     if a.out:
         os.makedirs(a.out, exist_ok=True)
-        with open(os.path.join(a.out, 'bkgmap_bench.json'), 'w') as f:
+        name = 'r05_bkgmask_bench.json' if a.mask else 'bkgmap_bench.json'
+        with open(os.path.join(a.out, name), 'w') as f:
             json.dump(lines, f, indent=1)
 
 

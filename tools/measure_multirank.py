@@ -16,6 +16,9 @@ With --maps, every rank also runs Engine.bkg_maps_band (the background / rms map
 node partials per clipping pass) and compares it with the single-rank run: node nbkg, iters and the pass count exactly,
 node bkg / rms within --rtol relative (as for --noise), and its own rows of both maps within 1 float32 ulp of the same
 rows of the single-rank maps (NaN positions equal).
+With --mask, --noise and --maps run with the source mask of the catalog (Engine.source_mask_band, built once per run over
+the rank's rows); the map comparison then also requires the same set of filled nodes (nbkg = 0 with a finite value) and
+the same count of holes filled.
 
 Prints one JSON line on rank 0 with the largest relative difference per field and the verdict of every rank."""
 import argparse
@@ -65,6 +68,7 @@ def main():
     ap.add_argument('--maps', action='store_true', help='also compare the background / rms maps')
     ap.add_argument('--bkg_box', type=int, default=101)
     ap.add_argument('--bkg_grid', type=int, default=25)
+    ap.add_argument('--mask', action='store_true', help='run --noise and --maps with the source mask')
     a = ap.parse_args()
     import torch
     import torch.distributed as dist
@@ -91,11 +95,13 @@ def main():
     res = compare(meas, ref_meas)
     same_catalog = bool(src.tobytes() == ref.tobytes())
     ok = same_catalog and all(res[k + '_exact'] for k in EXACT) and all(res[k] <= a.rtol for k in FLOATS)
+    mask = eng.source_mask_band(src, tiles, rank, world) if a.mask else None
+    ref_mask = eng.source_mask_band(ref, tiles) if a.mask else None
     noise_res = None
     if a.noise:
-        z = eng.measure_noise_band(src, tiles, a.noise_frame, rank, world)
+        z = eng.measure_noise_band(src, tiles, a.noise_frame, rank, world, mask=mask)
         passes = eng.noise_passes
-        zr = eng.measure_noise_band(ref, tiles, a.noise_frame)
+        zr = eng.measure_noise_band(ref, tiles, a.noise_frame, mask=ref_mask)
         noise_res = dict(passes=passes, single_rank_passes=eng.noise_passes,
                          nbkg_exact=bool(np.array_equal(z['nbkg'], zr['nbkg'])),
                          iters_exact=bool(np.array_equal(z['iters'], zr['iters'])))
@@ -112,12 +118,17 @@ def main():
             noise_res['bkg'] <= a.rtol and noise_res['rms'] <= a.rtol
     maps_res = None
     if a.maps:
-        z, bkg, rms, _, (r0, r1) = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, rank, world)
-        passes = eng.bkg_passes
-        zr, bkg_r, rms_r, _, _ = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid)
+        z, bkg, rms, _, (r0, r1) = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, rank, world, mask=mask)
+        passes, filled = eng.bkg_passes, eng.bkg_holes_filled
+        zr, bkg_r, rms_r, _, _ = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, mask=ref_mask)
         maps_res = dict(passes=passes, single_rank_passes=eng.bkg_passes, nodes=int(z.size),
                         nbkg_exact=bool(np.array_equal(z['nbkg'], zr['nbkg'])),
                         iters_exact=bool(np.array_equal(z['iters'], zr['iters'])))
+        if a.mask:
+            maps_res.update(holes_filled=filled, single_rank_holes_filled=eng.bkg_holes_filled,
+                            filled_set_exact=bool(np.array_equal((z['nbkg'] == 0) & ~np.isnan(z['bkg']),
+                                                                 (zr['nbkg'] == 0) & ~np.isnan(zr['bkg']))))
+            ok = ok and maps_res['filled_set_exact'] and filled == eng.bkg_holes_filled
         for k in ('bkg', 'rms'):
             x, y = z[k].ravel(), zr[k].ravel()
             same_nan = np.array_equal(np.isnan(x), np.isnan(y))
