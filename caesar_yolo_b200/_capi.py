@@ -100,8 +100,14 @@ class NoiseState(ctypes.Structure):
                 ("nbkg", c_i64), ("iters", ctypes.c_int32), ("done", ctypes.c_int32)]
 
 
+class SelectState(ctypes.Structure):
+    """cy_select_state: median select of one source or node (prefixes and ranks of the two middle ranks)."""
+    _fields_ = [("prefix", ctypes.c_uint32 * 2), ("rank", c_i64 * 2), ("n", c_i64), ("split", ctypes.c_int32),
+                ("round", ctypes.c_int32)]
+
+
 assert ctypes.sizeof(SrcPartial) == 80 and ctypes.sizeof(SrcMeas) == 80
-assert ctypes.sizeof(NoisePartial) == 24 and ctypes.sizeof(NoiseState) == 56
+assert ctypes.sizeof(NoisePartial) == 24 and ctypes.sizeof(NoiseState) == 56 and ctypes.sizeof(SelectState) == 40
 
 
 ALLGATHER_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t,
@@ -120,6 +126,8 @@ SYMBOLS = [
     "cy_compact_scratch_bytes", "cy_compact_records", "cy_merge_global", "cy_measure_sources", "cy_measure_combine",
     "cy_noise_init", "cy_noise_pass", "cy_noise_update", "cy_bkg_grid_init", "cy_bkg_grid_pass", "cy_bkg_grid_maps",
     "cy_source_mask", "cy_noise_pass_masked", "cy_bkg_grid_pass_masked", "cy_bkg_grid_probe_init", "cy_bkg_grid_fill",
+    "cy_noise_pass_median", "cy_noise_pass_median_masked", "cy_bkg_grid_pass_median", "cy_bkg_grid_pass_median_masked",
+    "cy_median_update",
     "cy_ctx_create", "cy_ctx_set_allgather", "cy_ctx_destroy", "cy_run_local", "cy_run_local_payload", "cy_ctx_records",
     "cy_ctx_pack_slot", "cy_ctx_unpack_slots", "cy_run_merge", "cy_run_mosaic", "cy_run_payload", "cy_ctx_info",
 ]

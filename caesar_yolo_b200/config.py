@@ -56,4 +56,7 @@ CONFIG = {
     # - Mask the catalog boxes out of the measure_noise frames and the save_bkg_maps node boxes (not in the reference);
     #   map nodes left without pixels are filled from their neighbours.  Alone it changes nothing (one warning)
     'bkg_mask_sources': False,
+    # - Centre of the sigma clipping of measure_noise and save_bkg_maps (not in the reference): 'mean' or 'median'
+    #   (astropy's sigma_clipped_stats default; bkg is then the clipped median).  Alone it changes nothing (one warning)
+    'bkg_estimator': 'mean',
 }

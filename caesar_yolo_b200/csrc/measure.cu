@@ -299,6 +299,54 @@ __device__ __forceinline__ float noise_pixel(const uint32_t* p, int big_endian) 
     return (isfinite(f) && f != 0.0f) ? f : __int_as_float(0x7fc00000);
 }
 
+// ---- median select (cy_noise_pass_median, cy_bkg_grid_pass_median, cy_median_update).  A kept pixel's key is the
+// order-preserving map of its float32 bits (negative: all bits flipped; positive: sign bit set; 0 and non-finite values
+// are masked).  Round r counts byte r (from the top) of the keys whose top 8r bits equal the prefix of a middle rank:
+// slots [0, 256) for the lower middle rank, [256, 512) for the upper one once their prefixes differ.
+constexpr int kSelectBins = 256;
+constexpr int kSelectSlots = 2 * kSelectBins;
+constexpr int kSelectRounds = 4;
+
+__device__ __forceinline__ uint32_t float_key(uint32_t bits) {
+    return (bits & 0x80000000u) ? ~bits : (bits | 0x80000000u);
+}
+
+__device__ __forceinline__ uint32_t key_bits(uint32_t key) {
+    return (key & 0x80000000u) ? (key & 0x7fffffffu) : ~key;
+}
+
+struct Select {
+    uint32_t p0, p1;
+    int round, split, shift;   // shift = 32 - 8 round: the prefix of a key is key >> shift (round >= 1)
+};
+
+__device__ __forceinline__ Select select_load(const cy_select_state& t, int round) {
+    return Select{t.prefix[0], t.prefix[1], round, round > 0 ? t.split : 0, 32 - 8 * round};
+}
+
+// the kept pixel with float bits `bits` -> its slot, counted once per distinct slot of the warp (all 32 lanes call)
+__device__ __forceinline__ void select_count(uint32_t* h, const Select& q, bool keep, uint32_t bits) {
+    int slot = -1;
+    if (keep) {
+        const uint32_t key = float_key(bits);
+        if (q.round == 0) {
+            slot = (int)(key >> 24);
+        } else {
+            const uint32_t pre = key >> q.shift, b = (key >> (q.shift - 8)) & 255u;
+            if (pre == q.p0) slot = (int)b;
+            else if (q.split && pre == q.p1) slot = kSelectBins + (int)b;
+        }
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, slot);
+    if (slot >= 0 && (int)(threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(h + slot, (uint32_t)__popc(peers));
+}
+
+// shared slots -> the global histogram of the source or node (integer adds: any order gives the same counts)
+__device__ __forceinline__ void select_flush(const uint32_t* h, uint32_t* __restrict__ out, int t, int nt) {
+    for (int i = t; i < kSelectSlots; i += nt)
+        if (h[i]) atomicAdd(out + i, h[i]);
+}
+
 __global__ void noise_init_kernel(int nsrc, cy_noise_state* __restrict__ state) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= nsrc) return;
@@ -318,7 +366,10 @@ __global__ void noise_init_kernel(int nsrc, cy_noise_state* __restrict__ state) 
 // one run of lane indices; other rows read the full grown width.  A converged source's units return at once.
 // kMask: a pixel whose bit is set in the source mask (cy_source_mask over the same ncols and rows) is skipped before
 // its load; the unmasked instantiation does not touch `mask`.
-template <bool kMask>
+// kMedian: one digit round of the median select (select_count): round 0 also sums the moments, rounds 1..3 only count;
+// the CTA's histogram goes to hist[s * kSelectSlots ..] with integer atomics.  The mean instantiation does not touch
+// sel, round or hist.
+template <bool kMask, bool kMedian = false>
 __global__ void __launch_bounds__(kThreads) noise_unit_kernel(const uint32_t* __restrict__ img, long long row_stride,
                                                               int big_endian, int row0, int ncols,
                                                               const cy_source* __restrict__ src, int nsrc,
@@ -326,7 +377,9 @@ __global__ void __launch_bounds__(kThreads) noise_unit_kernel(const uint32_t* __
                                                               const long long* __restrict__ off,
                                                               const cy_noise_state* __restrict__ state,
                                                               cy_noise_partial* __restrict__ unit_out,
-                                                              const uint32_t* __restrict__ mask) {
+                                                              const uint32_t* __restrict__ mask,
+                                                              const cy_select_state* __restrict__ sel = nullptr,
+                                                              int round = 0, uint32_t* __restrict__ hist = nullptr) {
     __shared__ NAcc warp_acc[kThreads / 32];
     const long long u = blockIdx.x;
     const int s = unit_source(off, nsrc, u);
@@ -344,20 +397,51 @@ __global__ void __launch_bounds__(kThreads) noise_unit_kernel(const uint32_t* __
     const int yb = min(g.y1, ya + kUnitRows - 1);
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     NAcc a = {0, 0.0, 0.0};
-    for (int y = ya + w; y <= yb; y += kThreads / 32) {
-        const uint32_t* row = img + (long long)(y - row0) * row_stride;
-        const uint32_t* mrow = kMask ? mask + (long long)(y - row_begin) * ((ncols + 31) >> 5) : nullptr;
-        const bool in_box = (double)y >= by0 && (double)y <= by1;
-        const int nl = in_box ? side_l : g.x1 - g.x0 + 1, nr = in_box ? side_r : 0;
-        for (int i = lane; i < nl + nr; i += 32) {
-            const int x = i < nl ? g.x0 + i : r0 + (i - nl);
-            if (kMask && ((__ldg(mrow + (x >> 5)) >> (x & 31)) & 1u)) continue;
-            const double v = (double)noise_pixel(row + x, big_endian);
-            if (!(v >= lo && v <= hi)) continue;       // false for a masked pixel (NaN)
-            const double d = v - c;
-            a.n += 1;
-            a.s1 += d;
-            a.s2 += d * d;
+    if constexpr (kMedian) {
+        __shared__ uint32_t s_hist[kSelectSlots];
+        for (int i = threadIdx.x; i < kSelectSlots; i += kThreads) s_hist[i] = 0;
+        __syncthreads();
+        const Select q = select_load(sel[s], round);
+        for (int y = ya + w; y <= yb; y += kThreads / 32) {
+            const uint32_t* row = img + (long long)(y - row0) * row_stride;
+            const uint32_t* mrow = kMask ? mask + (long long)(y - row_begin) * ((ncols + 31) >> 5) : nullptr;
+            const bool in_box = (double)y >= by0 && (double)y <= by1;
+            const int nl = in_box ? side_l : g.x1 - g.x0 + 1, nr = in_box ? side_r : 0;
+            for (int i0 = 0; i0 < nl + nr; i0 += 32) {   // the warp stays converged for select_count
+                const int i = i0 + lane, x = i < nl ? g.x0 + i : r0 + (i - nl);
+                float f = __int_as_float(0x7fc00000);
+                if (i < nl + nr && !(kMask && ((__ldg(mrow + (x >> 5)) >> (x & 31)) & 1u)))
+                    f = noise_pixel(row + x, big_endian);
+                const double v = (double)f;
+                const bool keep = v >= lo && v <= hi;   // false for a masked pixel (NaN)
+                if (keep && round == 0) {
+                    const double d = v - c;
+                    a.n += 1;
+                    a.s1 += d;
+                    a.s2 += d * d;
+                }
+                select_count(s_hist, q, keep, __float_as_uint(f));
+            }
+        }
+        __syncthreads();
+        select_flush(s_hist, hist + (long long)s * kSelectSlots, threadIdx.x, kThreads);
+        if (round != 0) return;
+    } else {
+        for (int y = ya + w; y <= yb; y += kThreads / 32) {
+            const uint32_t* row = img + (long long)(y - row0) * row_stride;
+            const uint32_t* mrow = kMask ? mask + (long long)(y - row_begin) * ((ncols + 31) >> 5) : nullptr;
+            const bool in_box = (double)y >= by0 && (double)y <= by1;
+            const int nl = in_box ? side_l : g.x1 - g.x0 + 1, nr = in_box ? side_r : 0;
+            for (int i = lane; i < nl + nr; i += 32) {
+                const int x = i < nl ? g.x0 + i : r0 + (i - nl);
+                if (kMask && ((__ldg(mrow + (x >> 5)) >> (x & 31)) & 1u)) continue;
+                const double v = (double)noise_pixel(row + x, big_endian);
+                if (!(v >= lo && v <= hi)) continue;       // false for a masked pixel (NaN)
+                const double d = v - c;
+                a.n += 1;
+                a.s1 += d;
+                a.s2 += d * d;
+            }
         }
     }
     for (int d = 16; d > 0; d >>= 1) {
@@ -434,6 +518,89 @@ __global__ void noise_update_kernel(const cy_noise_partial* __restrict__ part, i
     state[s] = t;
 }
 
+// Walks the bins of one digit: the bin that holds rank `rank` (0-based) of the counted keys; rank becomes the rank
+// inside that bin and the bin is appended to the prefix.
+__device__ __forceinline__ void select_pick(const uint32_t* __restrict__ h, int64_t& rank, uint32_t& prefix) {
+    int b = 0;
+    long long below = 0;
+    for (; b < kSelectBins - 1; ++b) {
+        const long long c = h[b];
+        if (rank < below + c) break;
+        below += c;
+    }
+    rank -= below;
+    prefix = (prefix << 8) | (uint32_t)b;
+}
+
+// Round `round` of pass k, after the histograms of every rank are summed.  Round 0 also folds the moment partials
+// [world][n] in rank order (as noise_update_kernel): an empty set or n_k = n_{k-1} stops the source here (the set did
+// not change, so its median is the shift c = m_{k-1}); otherwise the middle ranks of the n_k kept pixels are set.
+// Every round picks the bins of both ranks; round 3 has their full keys, finalises m_k and advances the state like
+// noise_update_kernel with the median as the centre.  cnt[0] counts the sources that go on, cnt[1] the sets of
+// 2^32 pixels or more (their uint32 bins can wrap).
+__global__ void median_update_kernel(const cy_noise_partial* __restrict__ part, int world,
+                                     const uint32_t* __restrict__ hist, int nsrc, cy_noise_state* __restrict__ state,
+                                     cy_select_state* __restrict__ sel, int round, int* __restrict__ cnt) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= nsrc) return;
+    cy_noise_state t = state[s];
+    if (t.done) return;
+    cy_select_state q = sel[s];
+    const int k = t.iters;   // index of the pass
+    if (round == 0) {
+        NAcc a = {0, 0.0, 0.0};
+        for (int r = 0; r < world; ++r) {
+            const cy_noise_partial& p = part[(long long)r * nsrc + s];
+            const NAcc b = {p.n, p.s1, p.s2};
+            nacc_merge(a, b);
+        }
+        if (a.n == 0) {
+            t.nbkg = 0;
+            t.bkg = t.rms = __longlong_as_double(0x7ff8000000000000ll);
+            t.done = 1;
+            state[s] = t;
+            return;
+        }
+        const double m1 = a.s1 / (double)a.n;
+        t.rms = sqrt(fmax(a.s2 / (double)a.n - m1 * m1, 0.0));
+        if (k >= 1 && a.n == t.nbkg) {
+            t.bkg = t.c;
+            t.done = 1;
+            state[s] = t;
+            return;
+        }
+        state[s] = t;
+        q.n = a.n;
+        q.rank[0] = (a.n - 1) / 2;   // x_((n-1)/2) and x_(n/2): the same rank for odd n
+        q.rank[1] = a.n / 2;
+        q.prefix[0] = q.prefix[1] = 0;
+        q.split = 0;
+    }
+    const uint32_t* h = hist + (long long)s * kSelectSlots;
+    select_pick(h, q.rank[0], q.prefix[0]);
+    select_pick(q.split ? h + kSelectBins : h, q.rank[1], q.prefix[1]);
+    q.split = q.prefix[0] != q.prefix[1];
+    q.round = round;
+    sel[s] = q;
+    if (round < kSelectRounds - 1) return;
+    if (q.n > 0xffffffffll) atomicAdd(cnt + 1, 1);
+    const double m = ((double)__uint_as_float(key_bits(q.prefix[0])) +
+                      (double)__uint_as_float(key_bits(q.prefix[1]))) / 2.0;   // np.median of the fp64 values
+    const double sd = t.rms;
+    t.bkg = m;
+    if (k == kClipMaxIters) {
+        t.done = 1;
+    } else {
+        t.lo = fmax(t.lo, m - kClipSigma * sd);
+        t.hi = fmin(t.hi, m + kClipSigma * sd);
+        t.c = m;
+        t.iters = k + 1;
+        atomicAdd(cnt, 1);
+    }
+    t.nbkg = q.n;
+    state[s] = t;
+}
+
 // ---------------------------------------------------------------------------------------------- background maps
 // The sigma clipping above over the boxes of a node lattice (cy_bkg_grid_init / cy_bkg_grid_pass / cy_bkg_grid_maps).
 // A work unit is one chunk of <= kUnitRows rows of one node row and a group of kGridNodes adjacent node columns: the CTA
@@ -443,6 +610,7 @@ __global__ void noise_update_kernel(const cy_noise_partial* __restrict__ part, i
 constexpr int kGridNodes = 16;                          // node columns per unit: warp w takes nodes w and w + 8
 constexpr int kNodesPerWarp = kGridNodes / (kThreads / 32);
 constexpr int kSliceCols = 256;                         // columns of one shared-memory slice (32 KB with kUnitRows)
+constexpr int kBkgSelectSmem = (kGridNodes * kSelectSlots + 3 * kGridNodes) * 4;   // median select: 32.2 KB
 
 // Node lattice of the region: columns [0, ncols) of the buffer, rows [R0, R1); rlo..rhi: the rows of this range
 // (inclusive; empty when rlo > rhi).  h is clipped to the region's larger side, which changes no box.
@@ -493,14 +661,18 @@ __global__ void __launch_bounds__(kScanThreads) bkg_units_scan_kernel(Grid G, lo
 // only the columns from the first to the last active node's box are read.
 // kMask: region pixel (x, y) is masked when bit x + mask_col0 of mask row y - G.rlo is set (mask_words words per row);
 // it enters the shared tile as NaN, so the fold loop is that of the unmasked instantiation, which does not touch `mask`.
-template <bool kMask>
+// kMedian: one digit round of the median select, as for noise_unit_kernel; the kGridNodes histograms and the nodes'
+// prefixes live in kBkgSelectSmem bytes of dynamic shared memory, and a node's slots go to hist[n * kSelectSlots ..].
+template <bool kMask, bool kMedian = false>
 __global__ void __launch_bounds__(kThreads) bkg_unit_kernel(const uint32_t* __restrict__ img, long long row_stride,
                                                             int big_endian, int row0, Grid G,
                                                             const long long* __restrict__ off,
                                                             const cy_noise_state* __restrict__ state,
                                                             cy_noise_partial* __restrict__ unit_out,
                                                             const uint32_t* __restrict__ mask, int mask_words,
-                                                            int mask_col0) {
+                                                            int mask_col0,
+                                                            const cy_select_state* __restrict__ sel = nullptr,
+                                                            int round = 0, uint32_t* __restrict__ hist = nullptr) {
     __shared__ float tile[kUnitRows][kSliceCols];
     __shared__ double s_lo[kGridNodes], s_hi[kGridNodes], s_c[kGridNodes];
     __shared__ int s_active[kGridNodes];
@@ -521,6 +693,17 @@ __global__ void __launch_bounds__(kThreads) bkg_unit_kernel(const uint32_t* __re
             s_c[k] = s.c;
         }
         s_active[k] = act;
+    }
+    if constexpr (kMedian) {
+        extern __shared__ uint32_t s_sel[];   // [kGridNodes][kSelectSlots] counts, then p0, p1, split per node
+        for (int i = threadIdx.x; i < kGridNodes * kSelectSlots; i += kThreads) s_sel[i] = 0;
+        if (threadIdx.x < kGridNodes && (int)threadIdx.x < ni) {
+            const cy_select_state& t = sel[(long long)j * G.nx + i0 + threadIdx.x];
+            uint32_t* p = s_sel + kGridNodes * kSelectSlots + threadIdx.x;
+            p[0] = t.prefix[0];
+            p[kGridNodes] = t.prefix[1];
+            p[2 * kGridNodes] = t.split;
+        }
     }
     __syncthreads();
     int ka = -1, kb = -1;
@@ -562,17 +745,47 @@ __global__ void __launch_bounds__(kThreads) bkg_unit_kernel(const uint32_t* __re
             const int xk = G.xnode(i0 + k);
             const int c0 = max(xk - G.h, s0), c1 = min(xk + G.h, s0 + sw - 1);
             const double lo = s_lo[k], hi = s_hi[k], c = s_c[k];
-            for (int r = 0; r < nrows; ++r)
-                for (int x = c0 + lane; x <= c1; x += 32) {
-                    const double v = (double)tile[r][x - s0];
-                    if (!(v >= lo && v <= hi)) continue;   // false for a masked pixel (NaN)
-                    const double d = v - c;
-                    acc[q].n += 1;
-                    acc[q].s1 += d;
-                    acc[q].s2 += d * d;
+            if constexpr (kMedian) {
+                extern __shared__ uint32_t s_sel[];
+                const uint32_t* p = s_sel + kGridNodes * kSelectSlots + k;
+                const Select sq{p[0], p[kGridNodes], round, round > 0 ? (int)p[2 * kGridNodes] : 0, 32 - 8 * round};
+                uint32_t* h = s_sel + k * kSelectSlots;
+                const int nseg = (c1 - c0) / 32 + 1;   // one loop, so the warp stays converged for select_count
+                for (int t = 0; t < nrows * nseg; ++t) {
+                    const int r = t / nseg, x = c0 + (t - r * nseg) * 32 + lane;
+                    const float f = x <= c1 ? tile[r][x - s0] : __int_as_float(0x7fc00000);
+                    const double v = (double)f;
+                    const bool keep = v >= lo && v <= hi;   // false for a masked pixel (NaN)
+                    if (keep && round == 0) {
+                        const double d = v - c;
+                        acc[q].n += 1;
+                        acc[q].s1 += d;
+                        acc[q].s2 += d * d;
+                    }
+                    select_count(h, sq, keep, __float_as_uint(f));
                 }
+            } else {
+                for (int r = 0; r < nrows; ++r)
+                    for (int x = c0 + lane; x <= c1; x += 32) {
+                        const double v = (double)tile[r][x - s0];
+                        if (!(v >= lo && v <= hi)) continue;   // false for a masked pixel (NaN)
+                        const double d = v - c;
+                        acc[q].n += 1;
+                        acc[q].s1 += d;
+                        acc[q].s2 += d * d;
+                    }
+            }
         }
         __syncthreads();
+    }
+    if constexpr (kMedian) {   // the loop ends with a barrier: every count is in
+        extern __shared__ uint32_t s_sel[];
+        for (int i = threadIdx.x; i < kGridNodes * kSelectSlots; i += kThreads) {
+            const int k = i / kSelectSlots;
+            if (k < ni && s_active[k] && s_sel[i])
+                atomicAdd(hist + ((long long)j * G.nx + i0 + k) * kSelectSlots + i % kSelectSlots, s_sel[i]);
+        }
+        if (round != 0) return;
     }
 #pragma unroll
     for (int q = 0; q < kNodesPerWarp; ++q) {
@@ -818,21 +1031,36 @@ extern "C" int cy_noise_init(const cy_source* src, int nsrc, int ncols, int row_
     return CY_OK;
 }
 
+// sel == nullptr: a pass of the mean; otherwise round `round` of a median pass (hist zeroed, then counted; the moment
+// partials are written in round 0 only)
 static int noise_pass(const char* fn, const void* img, long long row_stride, int big_endian, int row0, int ncols,
                       const cy_source* src, int nsrc, int row_begin, int row_end, int frame, const long long* unit_off,
                       long long units, const cy_noise_state* state, cy_noise_partial* partials, const uint32_t* mask,
-                      uintptr_t stream) {
+                      uintptr_t stream, const cy_select_state* sel = nullptr, int round = 0, uint32_t* hist = nullptr) {
     if (nsrc < 0 || ncols <= 0 || row_stride < ncols || row_begin < row0 || row_end < row_begin || frame < 1 ||
-        units < 0 || units > 2147483647ll)
-        return set_error(CY_ERR_INVALID, "%s: invalid image geometry, row range, frame or unit count", fn);
+        units < 0 || units > 2147483647ll || round < 0 || round >= kSelectRounds)
+        return set_error(CY_ERR_INVALID, "%s: invalid image geometry, row range, frame, unit count or round", fn);
     if (nsrc == 0) return CY_OK;
     if (!src || !unit_off || !state || !partials || (units > 0 && !img))
         return set_error(CY_ERR_INVALID, "%s: null argument", fn);
     cudaStream_t st = (cudaStream_t)stream;
+    if (sel) CY_CUDA_CHECK(cudaMemsetAsync(hist, 0, (size_t)nsrc * kSelectSlots * sizeof(uint32_t), st));
+    const bool moments = !sel || round == 0;
     cy_noise_partial* unit = nullptr;
-    if (units > 0 && cudaMallocAsync(&unit, (size_t)units * sizeof(cy_noise_partial), st) != cudaSuccess)
+    if (moments && units > 0 && cudaMallocAsync(&unit, (size_t)units * sizeof(cy_noise_partial), st) != cudaSuccess)
         return set_error(CY_ERR_NOMEM, "%s: no memory for %lld unit partials", fn, units);
-    if (units > 0 && mask)
+    const uint32_t* I = (const uint32_t*)img;
+    if (units > 0 && sel && mask)
+        noise_unit_kernel<true, true><<<(unsigned)units, kThreads, 0, st>>>(I, row_stride, big_endian, row0, ncols,
+                                                                            src, nsrc, row_begin, row_end, frame,
+                                                                            unit_off, state, unit, mask, sel, round,
+                                                                            hist);
+    else if (units > 0 && sel)
+        noise_unit_kernel<false, true><<<(unsigned)units, kThreads, 0, st>>>(I, row_stride, big_endian, row0, ncols,
+                                                                             src, nsrc, row_begin, row_end, frame,
+                                                                             unit_off, state, unit, nullptr, sel,
+                                                                             round, hist);
+    else if (units > 0 && mask)
         noise_unit_kernel<true><<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian,
                                                                       row0, ncols, src, nsrc, row_begin, row_end,
                                                                       frame, unit_off, state, unit, mask);
@@ -840,7 +1068,7 @@ static int noise_pass(const char* fn, const void* img, long long row_stride, int
         noise_unit_kernel<false><<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian,
                                                                        row0, ncols, src, nsrc, row_begin, row_end,
                                                                        frame, unit_off, state, unit, nullptr);
-    noise_fold_kernel<<<(nsrc + 255) / 256, 256, 0, st>>>(unit, unit_off, nsrc, state, partials);
+    if (moments) noise_fold_kernel<<<(nsrc + 255) / 256, 256, 0, st>>>(unit, unit_off, nsrc, state, partials);
     const cudaError_t e = cudaGetLastError();
     if (unit) cudaFreeAsync(unit, st);
     if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "%s: %s", fn, cudaGetErrorString(e));
@@ -863,6 +1091,64 @@ extern "C" int cy_noise_pass_masked(const void* img, long long row_stride, int b
         return set_error(CY_ERR_INVALID, "cy_noise_pass_masked: null mask");
     return noise_pass("cy_noise_pass_masked", img, row_stride, big_endian, row0, ncols, src, nsrc, row_begin, row_end,
                       frame, unit_off, units, state, partials, row_end > row_begin ? mask : nullptr, stream);
+}
+
+static int median_args(const char* fn, const cy_select_state* sel, uint32_t* hist) {
+    if (!sel || !hist) return set_error(CY_ERR_INVALID, "%s: null select state or histogram", fn);
+    return CY_OK;
+}
+
+extern "C" int cy_noise_pass_median(const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                                    const cy_source* src, int nsrc, int row_begin, int row_end, int frame,
+                                    const long long* unit_off, long long units, const cy_noise_state* state,
+                                    const cy_select_state* sel, int round, cy_noise_partial* partials,
+                                    uint32_t* hist, uintptr_t stream) {
+    if (nsrc > 0 && median_args("cy_noise_pass_median", sel, hist)) return CY_ERR_INVALID;
+    return noise_pass("cy_noise_pass_median", img, row_stride, big_endian, row0, ncols, src, nsrc, row_begin, row_end,
+                      frame, unit_off, units, state, partials, nullptr, stream, sel, round, hist);
+}
+
+extern "C" int cy_noise_pass_median_masked(const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                                           const cy_source* src, int nsrc, int row_begin, int row_end, int frame,
+                                           const long long* unit_off, long long units, const cy_noise_state* state,
+                                           const cy_select_state* sel, int round, cy_noise_partial* partials,
+                                           uint32_t* hist, const uint32_t* mask, uintptr_t stream) {
+    if (units > 0 && row_end > row_begin && !mask)
+        return set_error(CY_ERR_INVALID, "cy_noise_pass_median_masked: null mask");
+    if (nsrc > 0 && median_args("cy_noise_pass_median_masked", sel, hist)) return CY_ERR_INVALID;
+    return noise_pass("cy_noise_pass_median_masked", img, row_stride, big_endian, row0, ncols, src, nsrc, row_begin,
+                      row_end, frame, unit_off, units, state, partials, row_end > row_begin ? mask : nullptr, stream,
+                      sel, round, hist);
+}
+
+extern "C" int cy_median_update(const cy_noise_partial* partials, int world, const uint32_t* hist, int n,
+                                cy_noise_state* state, cy_select_state* sel, int round, int* active,
+                                uintptr_t stream) {
+    if (world < 1 || n < 0 || round < 0 || round >= kSelectRounds || (round == kSelectRounds - 1 && !active))
+        return set_error(CY_ERR_INVALID, "cy_median_update: invalid arguments");
+    if (active) *active = 0;
+    if (n == 0) return CY_OK;
+    if (!partials || !hist || !state || !sel) return set_error(CY_ERR_INVALID, "cy_median_update: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (round < kSelectRounds - 1) {
+        median_update_kernel<<<(n + 255) / 256, 256, 0, st>>>(partials, world, hist, n, state, sel, round, nullptr);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_median_update: %s", cudaGetErrorString(e));
+        return CY_OK;
+    }
+    int* cnt = nullptr;
+    CY_CUDA_CHECK(cudaMallocAsync(&cnt, 2 * sizeof(int), st));
+    cudaMemsetAsync(cnt, 0, 2 * sizeof(int), st);
+    median_update_kernel<<<(n + 255) / 256, 256, 0, st>>>(partials, world, hist, n, state, sel, round, cnt);
+    int h[2] = {0, 0};
+    cudaMemcpyAsync(h, cnt, 2 * sizeof(int), cudaMemcpyDeviceToHost, st);
+    cudaFreeAsync(cnt, st);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_median_update: %s", cudaGetErrorString(e));
+    if (h[1] > 0)
+        return set_error(CY_ERR_INVALID, "cy_median_update: %d frames or node boxes keep 2^32 pixels or more", h[1]);
+    *active = h[0];
+    return CY_OK;
 }
 
 extern "C" int cy_noise_update(const cy_noise_partial* partials, int world, int nsrc, cy_noise_state* state,
@@ -905,30 +1191,42 @@ extern "C" int cy_bkg_grid_init(int ncols, int R0, int R1, int row_begin, int ro
     return CY_OK;
 }
 
+// sel == nullptr: a pass of the mean; otherwise round `round` of a median pass, as for noise_pass
 static int bkg_grid_pass(const char* fn, const void* img, long long row_stride, int big_endian, int row0, int ncols,
                          int R0, int R1, int row_begin, int row_end, int box, int grid, const long long* unit_off,
                          long long units, const cy_noise_state* state, cy_noise_partial* partials,
-                         const uint32_t* mask, int mask_ncols, int mask_col0, uintptr_t stream) {
+                         const uint32_t* mask, int mask_ncols, int mask_col0, uintptr_t stream,
+                         const cy_select_state* sel = nullptr, int round = 0, uint32_t* hist = nullptr) {
     Grid G;
     if (!make_grid(ncols, R0, R1, row_begin, row_end, box, grid, G) || row_stride < ncols || row_begin < row0 ||
-        units < 0 || units > 2147483647ll)
-        return set_error(CY_ERR_INVALID, "%s: invalid image geometry, region, box, grid or unit count", fn);
+        units < 0 || units > 2147483647ll || round < 0 || round >= kSelectRounds)
+        return set_error(CY_ERR_INVALID, "%s: invalid image geometry, region, box, grid, unit count or round", fn);
     if (!unit_off || !state || !partials || (units > 0 && !img))
         return set_error(CY_ERR_INVALID, "%s: null argument", fn);
     cudaStream_t st = (cudaStream_t)stream;
+    const long long nodes = (long long)G.nx * G.ny;
+    if (sel) CY_CUDA_CHECK(cudaMemsetAsync(hist, 0, (size_t)nodes * kSelectSlots * sizeof(uint32_t), st));
+    const bool moments = !sel || round == 0;
     cy_noise_partial* unit = nullptr;
-    if (units > 0 &&
+    if (moments && units > 0 &&
         cudaMallocAsync(&unit, (size_t)units * kGridNodes * sizeof(cy_noise_partial), st) != cudaSuccess)
         return set_error(CY_ERR_NOMEM, "%s: no memory for %lld unit partials", fn, units * kGridNodes);
-    if (units > 0 && mask)
+    const uint32_t* I = (const uint32_t*)img;
+    const int words = (mask_ncols + 31) >> 5;
+    if (units > 0 && sel) {
+        auto k = mask ? bkg_unit_kernel<true, true> : bkg_unit_kernel<false, true>;
+        CY_CUDA_CHECK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kBkgSelectSmem));
+        k<<<(unsigned)units, kThreads, kBkgSelectSmem, st>>>(I, row_stride, big_endian, row0, G, unit_off, state, unit,
+                                                            mask, mask ? words : 0, mask ? mask_col0 : 0, sel, round,
+                                                            hist);
+    } else if (units > 0 && mask)
         bkg_unit_kernel<true><<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian, row0,
                                                                     G, unit_off, state, unit, mask,
                                                                     (mask_ncols + 31) >> 5, mask_col0);
     else if (units > 0)
         bkg_unit_kernel<false><<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian, row0,
                                                                      G, unit_off, state, unit, nullptr, 0, 0);
-    const long long nodes = (long long)G.nx * G.ny;
-    bkg_fold_kernel<<<(unsigned)((nodes + 255) / 256), 256, 0, st>>>(unit, unit_off, G, state, partials);
+    if (moments) bkg_fold_kernel<<<(unsigned)((nodes + 255) / 256), 256, 0, st>>>(unit, unit_off, G, state, partials);
     const cudaError_t e = cudaGetLastError();
     if (unit) cudaFreeAsync(unit, st);
     if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "%s: %s", fn, cudaGetErrorString(e));
@@ -956,6 +1254,34 @@ extern "C" int cy_bkg_grid_pass_masked(const void* img, long long row_stride, in
     return bkg_grid_pass("cy_bkg_grid_pass_masked", img, row_stride, big_endian, row0, ncols, R0, R1, row_begin,
                          row_end, box, grid, unit_off, units, state, partials, row_end > row_begin ? mask : nullptr,
                          mask_ncols, mask_col0, stream);
+}
+
+extern "C" int cy_bkg_grid_pass_median(const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                                       int R0, int R1, int row_begin, int row_end, int box, int grid,
+                                       const long long* unit_off, long long units, const cy_noise_state* state,
+                                       const cy_select_state* sel, int round, cy_noise_partial* partials,
+                                       uint32_t* hist, uintptr_t stream) {
+    if (median_args("cy_bkg_grid_pass_median", sel, hist)) return CY_ERR_INVALID;
+    return bkg_grid_pass("cy_bkg_grid_pass_median", img, row_stride, big_endian, row0, ncols, R0, R1, row_begin,
+                         row_end, box, grid, unit_off, units, state, partials, nullptr, 0, 0, stream, sel, round,
+                         hist);
+}
+
+extern "C" int cy_bkg_grid_pass_median_masked(const void* img, long long row_stride, int big_endian, int row0,
+                                              int ncols, int R0, int R1, int row_begin, int row_end, int box, int grid,
+                                              const long long* unit_off, long long units,
+                                              const cy_noise_state* state, const cy_select_state* sel, int round,
+                                              cy_noise_partial* partials, uint32_t* hist, const uint32_t* mask,
+                                              int mask_ncols, int mask_col0, uintptr_t stream) {
+    if (mask_col0 < 0 || ncols <= 0 || mask_ncols < 1 || (long long)mask_col0 + ncols > mask_ncols)
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_pass_median_masked: the region's columns [%d, %lld) are not "
+                         "inside the mask's %d columns", mask_col0, (long long)mask_col0 + ncols, mask_ncols);
+    if (units > 0 && row_end > row_begin && !mask)
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_pass_median_masked: null mask");
+    if (median_args("cy_bkg_grid_pass_median_masked", sel, hist)) return CY_ERR_INVALID;
+    return bkg_grid_pass("cy_bkg_grid_pass_median_masked", img, row_stride, big_endian, row0, ncols, R0, R1,
+                         row_begin, row_end, box, grid, unit_off, units, state, partials,
+                         row_end > row_begin ? mask : nullptr, mask_ncols, mask_col0, stream, sel, round, hist);
 }
 
 extern "C" int cy_bkg_grid_maps(const cy_noise_state* state, int ncols, int R0, int R1, int row_begin, int row_end,

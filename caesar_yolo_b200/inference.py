@@ -65,6 +65,15 @@ class SFinder(object):
             logger.warning("bkg_mask_sources masks the catalog boxes out of the measure_noise frames and the "
                            "save_bkg_maps nodes: with neither option on it changes nothing")
             self.bkg_mask_sources = False
+        # the centre of the clipping of both consumers, so the per-source statistics and the maps still compare
+        self.bkg_estimator = config.get('bkg_estimator', 'mean')
+        if self.bkg_estimator not in ops.BKG_ESTIMATORS:
+            raise ValueError("bkg_estimator must be one of %s, not %r" % (", ".join(ops.BKG_ESTIMATORS),
+                                                                          self.bkg_estimator))
+        if self.bkg_estimator != 'mean' and not (self.measure_noise or self.save_bkg_maps):
+            logger.warning("bkg_estimator sets the centre of the measure_noise and save_bkg_maps clipping: with neither "
+                           "option on it changes nothing")
+            self.bkg_estimator = 'mean'
         self.procId, self.nproc = _dist_info()
         self.timing = {}
         self.engine = None
@@ -215,11 +224,12 @@ class SFinder(object):
         if self.measure_sources:   # in the coordinates of the catalog: the (sub-)image read, columns from x0
             args = (_as_sources(recs), dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0)
             m = eng.measure(*args)
-            noise = eng.measure_noise(*args, frame=self.noise_frame, mask=mask) if self.measure_noise else None
+            noise = eng.measure_noise(*args, frame=self.noise_frame, mask=mask,
+                                      estimator=self.bkg_estimator) if self.measure_noise else None
             meas = self._measurements(m, self.fits.header, x0, y0, noise)
         if self.save_bkg_maps:   # the region read: the crop, columns from x0
             _, bkg, rms = eng.bkg_maps(dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0, 0,
-                                       y1 - y0, self.bkg_box, self.bkg_grid, mask=mask)
+                                       y1 - y0, self.bkg_box, self.bkg_grid, mask=mask, estimator=self.bkg_estimator)
             self._write_bkg_maps(bkg, rms, 0, (x0, y0, x1 - x0, y1 - y0))
         self.timing['run_s'] = time.time() - t0
         return self._save_serial(recs, status, meas)
@@ -239,7 +249,8 @@ class SFinder(object):
         (X0, R0, W, H), with the image's WCS shifted to the region."""
         X0, R0, W, H = region
         t0 = time.time()
-        hdr = fitsmeta.map_header(self.fits.header, W, H, X0, R0, bkgmask=self.bkg_mask_sources)
+        hdr = fitsmeta.map_header(self.fits.header, W, H, X0, R0, bkgmask=self.bkg_mask_sources,
+                                  bkgest=self.bkg_estimator)
         for name, rows in (('bkgmap_', bkg), ('rmsmap_', rms)):
             fitsmeta.write_map_rows(os.path.join(self.outdir, name + str(self.image_id) + '.fits'), hdr, rows,
                                     row_begin, W, H, self.procId, self.nproc)
@@ -310,7 +321,8 @@ class SFinder(object):
             else:
                 args = (_as_sources(recs), plane_dev, W, False, 0, W, 0, H)
                 mask = eng.source_mask(args[0], W, 0, H) if self.bkg_mask_sources and self.measure_noise else None
-                noise = eng.measure_noise(*args, frame=self.noise_frame, mask=mask) if self.measure_noise else None
+                noise = eng.measure_noise(*args, frame=self.noise_frame, mask=mask,
+                                          estimator=self.bkg_estimator) if self.measure_noise else None
                 meas = self._measurements(eng.measure(*args), {}, noise=noise)
         self.timing['run_s'] = time.time() - t0
         return self._save_serial(recs, 0, meas)
@@ -379,12 +391,13 @@ class SFinder(object):
             m = eng.measure_band(src, tiles, self.procId, self.nproc)
             noise = None
             if self.measure_noise:
-                noise = eng.measure_noise_band(src, tiles, self.noise_frame, self.procId, self.nproc, mask=mask)
+                noise = eng.measure_noise_band(src, tiles, self.noise_frame, self.procId, self.nproc, mask=mask,
+                                               estimator=self.bkg_estimator)
             if self.procId == 0:
                 meas = self._measurements(m, self.fits.header, noise=noise)
         if self.save_bkg_maps:   # every rank maps and writes its own rows; unmasked maps need no catalog
             _, bkg, rms, region, rows = eng.bkg_maps_band(tiles, self.bkg_box, self.bkg_grid, self.procId, self.nproc,
-                                                          mask=mask)
+                                                          mask=mask, estimator=self.bkg_estimator)
             self._write_bkg_maps(bkg, rms, rows[0] - region[1], region)
         self.timing['run_s'] = time.time() - t0
         if self.procId == 0:

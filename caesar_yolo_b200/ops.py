@@ -446,6 +446,52 @@ def noise_update(partials, world, nsrc, state):
     return active.value
 
 
+BKG_ESTIMATORS = ('mean', 'median')
+SELECT_BYTES = ctypes.sizeof(_capi.SelectState)
+SELECT_SLOTS = 512    # uint32 histogram slots per source or node: 256 bins for each of the two middle ranks
+SELECT_ROUNDS = 4     # 8-bit digit rounds of the median select per clipping pass
+
+
+def noise_pass_median(img, row_stride, big_endian, row0, ncols, src_dev, nsrc, row_begin, row_end, frame, unit_off,
+                      units, state, sel, rnd, out, hist, mask=None):
+    """cy_noise_pass_median[_masked]: round rnd of a median pass over this range's rows -> hist (int32 device tensor of
+    nsrc * SELECT_SLOTS uint32 counts) and, in round 0, out (as noise_pass).  mask: source_mask, or None."""
+    args = [ptr(img), c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0), c_int(ncols), ptr(src_dev),
+            c_int(nsrc), c_int(row_begin), c_int(row_end), c_int(frame), ptr(unit_off), c_i64(units), ptr(state),
+            ptr(sel), c_int(rnd), ptr(out), ptr(hist)]
+    if mask is None:
+        check(lib.cy_noise_pass_median(*args, cur_stream()))
+    else:
+        check(lib.cy_noise_pass_median_masked(*args, ptr(mask), cur_stream()))
+
+
+def bkg_grid_pass_median(img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box, grid, unit_off,
+                         units, state, sel, rnd, out, hist, mask=None, mask_ncols=0, mask_col0=0):
+    """cy_bkg_grid_pass_median[_masked]: round rnd of a median pass of the grid nodes -> hist (Nx * Ny * SELECT_SLOTS
+    counts) and, in round 0, out (as bkg_grid_pass).  mask: as for bkg_grid_pass_masked, or None."""
+    args = [ptr(img), c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0), c_int(ncols), c_int(R0),
+            c_int(R1), c_int(row_begin), c_int(row_end), c_int(box), c_int(grid), ptr(unit_off), c_i64(units),
+            ptr(state), ptr(sel), c_int(rnd), ptr(out), ptr(hist)]
+    if mask is None:
+        check(lib.cy_bkg_grid_pass_median(*args, cur_stream()))
+    else:
+        check(lib.cy_bkg_grid_pass_median_masked(*args, ptr(mask), c_int(mask_ncols), c_int(mask_col0), cur_stream()))
+
+
+def median_update(partials, world, hist, n, state, sel, rnd):
+    """cy_median_update: round rnd of a median pass, with hist summed over the ranks (and, in round 0, the partials
+    [world * n * 24] gathered in rank order).  Returns the number still active after the last round (synchronises),
+    None after the others (no synchronisation)."""
+    if rnd < SELECT_ROUNDS - 1:
+        check(lib.cy_median_update(ptr(partials), c_int(world), ptr(hist), c_int(n), ptr(state), ptr(sel), c_int(rnd),
+                                   None, cur_stream()))
+        return None
+    active = c_int(0)
+    check(lib.cy_median_update(ptr(partials), c_int(world), ptr(hist), c_int(n), ptr(state), ptr(sel), c_int(rnd),
+                               ctypes.byref(active), cur_stream()))
+    return active.value
+
+
 def bkg_grid_nodes(n, grid):
     """Node positions along one axis of n pixels with step `grid` (include/caesar_b200.h, background maps):
     x_i = min(i * grid, n - 1), i = 0 .. ceil((n - 1) / grid)."""

@@ -385,7 +385,7 @@ class Engine(object):
         return self.source_mask(sources, self.band[3], r0, r1)
 
     def measure_noise(self, sources, img, row_stride, big_endian, row0, ncols, row_begin, row_end, frame=16, world=1,
-                      mask=None):
+                      mask=None, estimator='mean'):
         """Local background and noise of the catalog `sources` (ops.SRC_DTYPE): sigma-clipped mean / std of a frame of
         `frame` pixels around each box, over rows [row_begin, row_end) of `img` (arguments as for Engine.measure;
         cy_noise_init / cy_noise_pass / cy_noise_update).  One pass per clipping iteration, at most
@@ -394,7 +394,9 @@ class Engine(object):
         rank sees the same active count and runs the same passes.  mask: Engine.source_mask of the same catalog, ncols
         and rows, or None; with it, the frame pixels inside any catalog box are masked (cy_noise_pass_masked).  Returns
         a structured array (ops.NOISE_DTYPE) whose bkg, rms, nbkg, iters are final; self.noise_passes holds the number
-        of passes run."""
+        of passes run.  estimator: 'mean' (mean-centred clipping) or 'median' (median-centred, bkg = the median of the
+        last set; every pass is ops.SELECT_ROUNDS rounds, see Engine._median_passes)."""
+        _check_estimator('Engine.measure_noise', estimator)
         src = np.ascontiguousarray(sources, dtype=ops.SRC_DTYPE)
         n = len(src)
         self.noise_passes = 0
@@ -414,6 +416,14 @@ class Engine(object):
         if world > 1:
             import torch.distributed as dist
             allp = self._get('noise_gather', (world * n * ops.NOISE_PARTIAL_BYTES,), torch.uint8)
+        if estimator == 'median':
+            def run_round(sel, rnd, hist):
+                ops.noise_pass_median(img, row_stride, big_endian, row0, ncols, src_dev, n, row_begin, row_end, frame,
+                                      off, units, state, sel, rnd, part, hist, None if mask is None else mask.bits)
+            self.noise_passes = self._median_passes('noise', n, state, part, allp, world, run_round, 'sources')
+            self._stage('noise', e)
+            self.launches += 3 + self.noise_passes * (9 + (5 if world > 1 else 0))
+            return state.cpu().numpy().view(ops.NOISE_DTYPE)
         active = n
         while active:
             if self.noise_passes == ops.NOISE_MAX_PASSES:
@@ -433,18 +443,44 @@ class Engine(object):
         self.launches += 3 + self.noise_passes * (3 + (1 if world > 1 else 0))
         return state.cpu().numpy().view(ops.NOISE_DTYPE)
 
-    def measure_noise_band(self, sources, tiles, frame=16, rank=0, world=1, mask=None):
+    def _median_passes(self, tag, n, state, part, allp, world, run_round, what):
+        """Median-centred clipping passes of n sources or nodes until none is active: each pass is ops.SELECT_ROUNDS
+        digit rounds of run_round(sel, rnd, hist) and cy_median_update.  With world > 1 the round-0 moment partials
+        are all-gathered (folded in rank order, as for the mean) and the uint32 histograms are summed with one
+        all-reduce per round: integer sums are exact in any order.  The active count is read once per pass.  Returns
+        the number of passes."""
+        sel = self._get(tag + '_sel', (n * ops.SELECT_BYTES,), torch.uint8)
+        hist = self._get(tag + '_hist', (n * ops.SELECT_SLOTS,), torch.int32)
+        if world > 1:
+            import torch.distributed as dist
+        passes, active = 0, n
+        while active:
+            if passes == ops.NOISE_MAX_PASSES:
+                raise ops.CaesarB200Error("cy_median_update: %d %s still active after %d passes"
+                                          % (active, what, passes))
+            for rnd in range(ops.SELECT_ROUNDS):
+                run_round(sel, rnd, hist)
+                if world > 1:
+                    if rnd == 0:
+                        dist.all_gather_into_tensor(allp, part)
+                    dist.all_reduce(hist)
+                active = ops.median_update(allp, world, hist, n, state, sel, rnd)
+            passes += 1
+        return passes
+
+    def measure_noise_band(self, sources, tiles, frame=16, rank=0, world=1, mask=None, estimator='mean'):
         """Engine.measure_noise over the rows this rank owns (measure_rows), read from the band of mosaic rows the last
         run_image left in HBM.  The frames are thus clipped to the rows the run read, and no rank reads a row twice.
-        mask: Engine.source_mask_band of the same catalog, or None."""
+        mask: Engine.source_mask_band of the same catalog, or None; estimator as for Engine.measure_noise."""
         r0, r1 = measure_rows(tiles, world)[rank]
         band, Y0, _, nx, big_endian = self.band
         if band is None:                     # a rank without tiles still takes part in every all-gather
             band, Y0 = self._get('meas_noband', (1,), torch.int32), r0
-        return self.measure_noise(sources, band, nx, big_endian, Y0, nx, r0, r1, frame=frame, world=world, mask=mask)
+        return self.measure_noise(sources, band, nx, big_endian, Y0, nx, r0, r1, frame=frame, world=world, mask=mask,
+                                  estimator=estimator)
 
     def bkg_maps(self, img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box=101, grid=25, world=1,
-                 mask=None, mask_col0=0):
+                 mask=None, mask_col0=0, estimator='mean'):
         """Background and rms maps of the region of columns [0, ncols) of `img` and rows [R0, R1) (node lattice,
         statistic and interpolation: include/caesar_b200.h), over rows [row_begin, row_end) of `img` (arguments as for
         Engine.measure; cy_bkg_grid_init / cy_bkg_grid_pass / cy_noise_update / cy_bkg_grid_maps).  With world > 1 every
@@ -455,7 +491,9 @@ class Engine(object):
         their neighbours (cy_bkg_grid_probe_init, one unmasked pass of the probe, cy_bkg_grid_fill); self.bkg_holes_filled
         holds their count.  Returns (nodes, bkg, rms): the final node states (ops.NOISE_DTYPE, shape [Ny, Nx]) and this
         range's map rows as int32 device tensors [row_end - row_begin, ncols] holding big-endian float32;
-        self.bkg_passes holds the number of clipping passes run."""
+        self.bkg_passes holds the number of clipping passes run.  estimator: as for Engine.measure_noise, so the maps and
+        the per-source statistics of one run compare directly."""
+        _check_estimator('Engine.bkg_maps', estimator)
         nx, ny = len(ops.bkg_grid_nodes(ncols, grid)), len(ops.bkg_grid_nodes(R1 - R0, grid))
         nodes = nx * ny
         if mask is not None and (mask.row_end - mask.row_begin != row_end - row_begin or
@@ -472,7 +510,15 @@ class Engine(object):
             import torch.distributed as dist
             allp = self._get('bkg_gather', (world * nodes * ops.NOISE_PARTIAL_BYTES,), torch.uint8)
         self.bkg_passes = 0
-        active = nodes
+        active = 0 if estimator == 'median' else nodes
+        if estimator == 'median':
+            def run_round(sel, rnd, hist):
+                ops.bkg_grid_pass_median(img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box, grid,
+                                         off, units, state, sel, rnd, part, hist,
+                                         None if mask is None else mask.bits, 0 if mask is None else mask.ncols,
+                                         mask_col0)
+            self.bkg_passes = self._median_passes('bkg', nodes, state, part, allp, world, run_round, 'grid nodes')
+            self.launches += self.bkg_passes * (6 + (4 if world > 1 else 0))   # the rounds beyond the mean's pass
         while active:
             if self.bkg_passes == ops.NOISE_MAX_PASSES:
                 raise ops.CaesarB200Error("cy_noise_update: %d grid nodes still active after %d passes"
@@ -505,10 +551,11 @@ class Engine(object):
         self.launches += 3 + self.bkg_passes * (3 + (1 if world > 1 else 0)) + 1
         return state.cpu().numpy().view(ops.NOISE_DTYPE).reshape(ny, nx), bkg, rms
 
-    def bkg_maps_band(self, tiles, box=101, grid=25, rank=0, world=1, mask=None):
+    def bkg_maps_band(self, tiles, box=101, grid=25, rank=0, world=1, mask=None, estimator='mean'):
         """Engine.bkg_maps of the bounding box of the tile grid (columns [min xmin, max xmax), rows [min ymin,
         max ymax)) over the rows this rank owns (measure_rows), read from the band of mosaic rows the last run_image
-        left in HBM.  mask: Engine.source_mask_band (image columns, so the region starts at its column X0), or None.
+        left in HBM.  mask: Engine.source_mask_band (image columns, so the region starts at its column X0), or None;
+        estimator as for Engine.bkg_maps.
         Returns (nodes, bkg, rms, (X0, R0, W, H), (row_begin, row_end))."""
         X0, X1 = int(tiles['xmin'].min()), int(tiles['xmax'].max())
         R0, R1 = int(tiles['ymin'].min()), int(tiles['ymax'].max())
@@ -521,7 +568,7 @@ class Engine(object):
         else:
             img = band[:, X0:]
         nodes, bkg, rms = self.bkg_maps(img, nx, big_endian, Y0, X1 - X0, R0, R1, r0, r1, box, grid, world, mask=mask,
-                                        mask_col0=X0)
+                                        mask_col0=X0, estimator=estimator)
         return nodes, bkg, rms, (X0, R0, X1 - X0, R1 - R0), (r0, r1)
 
     def _exchange_cap(self, world, need=0):
@@ -533,6 +580,11 @@ class Engine(object):
         want = min(want, self.T * ops.MAX_DET)
         self._buf['xcap'] = want
         return want
+
+
+def _check_estimator(fn, estimator):
+    if estimator not in ops.BKG_ESTIMATORS:
+        raise CaesarB200Error("%s: estimator %r is not one of %s" % (fn, estimator, ", ".join(ops.BKG_ESTIMATORS)))
 
 
 def piece_end(r0, y_end, rows_per_piece, y_stop):

@@ -286,15 +286,16 @@ int cy_measure_combine(const cy_src_partial* partials, int world, const cy_sourc
  * frame is the box grown by F = `frame` pixels on every side, minus the box, clipped to columns [0, ncols) and to the
  * rows the run measures; membership is decided in absolute pixel coordinates, so it does not depend on the row split.
  * Non-finite pixels and 0 are masked, as for the box.  Mean-centred iterative sigma clipping, kappa = 3, at most 5
- * iterations (astropy's sigma_clip defaults with cenfunc = 'mean', ddof = 0):
+ * iterations (astropy's sigma_clip with cenfunc = 'mean', ddof = 0; astropy's default centre, the median, is the
+ * median estimator below):
  *   pass 0 takes the mean mu_0 and standard deviation sigma_0 of all unmasked frame pixels;
  *   pass k >= 1 takes those of the pixels inside the intersection of [mu_j - 3 sigma_j, mu_j + 3 sigma_j], j < k
  *   (inclusive bounds: astropy's nested rejection, restated as one interval per source, so a pass needs no per-pixel
  *   state);
  *   a source stops when pass k >= 1 keeps as many pixels as pass k - 1, after pass 5, or when pass 0 finds no pixel.
  * bkg, rms: mean and standard deviation of the last kept set, nbkg its size, iters = k of the last pass (astropy's
- * niterations; 0 for an empty frame).  The mean, not the median, is the centre: it is a sum, so it adds up over row
- * ranges and ranks.  Pass k sums v - c and (v - c)^2 with c = 0 in pass 0 and c = mu_{k-1} after that, so the variance
+ * niterations; 0 for an empty frame).  The mean is the default centre: it is a sum, so it adds up over row ranges and
+ * ranks.  Pass k sums v - c and (v - c)^2 with c = 0 in pass 0 and c = mu_{k-1} after that, so the variance
  * does not cancel on a pedestal: mu = c + s1 / n, sigma^2 = max(s2 / n - (s1 / n)^2, 0).
  *
  * Partial record of one source over one row range and one pass: every field adds.  24 bytes. */
@@ -329,6 +330,46 @@ int cy_noise_pass(const void* img, long long row_stride, int big_endian, int row
 int cy_noise_update(const cy_noise_partial* partials, int world, int nsrc, cy_noise_state* state, int* active,
                     uintptr_t stream);
 
+/* Median estimator (opt-in, bkg_estimator = 'median'; not part of the reference).  The same pixel sets, frames, node
+ * boxes and mask rules as above, clipped around the median: astropy's sigma_clipped_stats defaults (cenfunc = 'median',
+ * stdfunc = 'std', ddof = 0, sigma = 3, maxiters = 5).
+ *   Set 0 is all unmasked pixels.  Pass k takes n_k, the median m_k and the standard deviation sigma_k of set k; set
+ *   k + 1 = set k intersected with [m_k - 3 sigma_k, m_k + 3 sigma_k] (inclusive bounds, one interval per source).
+ *   A source stops when n_k = n_{k-1} for k >= 1 (the set did not change: m_k = m_{k-1}), after pass 5, or when set k
+ *   is empty.  bkg = m of the last set, rms = sigma of the last set, nbkg its size, iters as above.
+ *   Median of n values x_(0) <= ... <= x_(n-1): x_((n-1)/2) for odd n, (x_(n/2-1) + x_(n/2)) / 2 in fp64 for even n,
+ *   which is np.median of the float64 values.  sigma is summed about the shift c = m_{k-1} (0 in pass 0), as above.
+ * The median is selected exactly by radix select on the order-preserving key of the float32 bits (negative values:
+ * every bit flipped; positive values: the sign bit set).  A pass is 4 digit rounds of 8 bits.  Round 0 reads set k and
+ * writes the moment partials of the mean path together with the 256-bin histogram of the top key byte; round r >= 1
+ * counts byte r of the kept keys whose top 8r bits equal the prefix of a middle rank.  The two middle ranks of an even
+ * n may part at some digit; both prefixes are followed, in slots [0, 256) and [256, 512).  The histograms are uint32
+ * counts, so they add exactly in any order over work units, row ranges and ranks (sum them across ranks, e.g. with an
+ * all-reduce): the median does not depend on the row split.  A set of 2^32 pixels or more is refused.
+ * Select state of one source or node, the same on every rank.  40 bytes. */
+typedef struct {
+    uint32_t prefix[2];                /* top 8 (round + 1) key bits of the lower / upper middle rank */
+    int64_t rank[2];                   /* their ranks among the kept keys that share the prefix */
+    int64_t n;                         /* n_k, the size of set k */
+    int32_t split;                     /* the two prefixes differ */
+    int32_t round;                     /* last round picked */
+} cy_select_state;
+/* Round `round` (0..3) of a median pass: hist[nsrc * 512] (uint32, device) is zeroed and filled with this range's
+ * counts; in round 0 partials[nsrc] are written as by cy_noise_pass (the other rounds leave them).  The other arguments
+ * as for cy_noise_pass; sel as left by cy_median_update. */
+int cy_noise_pass_median(const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                         const cy_source* src, int nsrc, int row_begin, int row_end, int frame,
+                         const long long* unit_off, long long units, const cy_noise_state* state,
+                         const cy_select_state* sel, int round, cy_noise_partial* partials, uint32_t* hist,
+                         uintptr_t stream);
+/* round r of a pass, after the histograms of all ranks are summed into hist[n * 512] (and, in round 0, the partials
+ * [world][n] all-gathered): round 0 folds the partials in rank order and stops the sources whose set is empty or
+ * unchanged; every round picks the bins of the middle ranks; round 3 finalises m_k and advances the states (as
+ * cy_noise_update does for the mean), synchronises the stream and sets *active (rounds 0..2 do not synchronise and
+ * leave *active alone; active may be NULL there).  n: sources, or the Nx * Ny nodes of a lattice. */
+int cy_median_update(const cy_noise_partial* partials, int world, const uint32_t* hist, int n, cy_noise_state* state,
+                     cy_select_state* sel, int round, int* active, uintptr_t stream);
+
 /* Source mask (opt-in, not part of the reference).  M is the union over all sources of the integer boxes [ceil x1,
  * floor x2] x [ceil y1, floor y2], the rule of the box measurements; an empty box or NaN coordinates add nothing, and
  * the boxes are not dilated.  Membership is decided in absolute pixel coordinates, so M does not depend on the row
@@ -348,6 +389,13 @@ int cy_noise_pass_masked(const void* img, long long row_stride, int big_endian, 
                          const cy_source* src, int nsrc, int row_begin, int row_end, int frame,
                          const long long* unit_off, long long units, const cy_noise_state* state,
                          cy_noise_partial* partials, const uint32_t* mask, uintptr_t stream);
+
+/* cy_noise_pass_median with the frame pixels in M masked. */
+int cy_noise_pass_median_masked(const void* img, long long row_stride, int big_endian, int row0, int ncols,
+                                const cy_source* src, int nsrc, int row_begin, int row_end, int frame,
+                                const long long* unit_off, long long units, const cy_noise_state* state,
+                                const cy_select_state* sel, int round, cy_noise_partial* partials, uint32_t* hist,
+                                const uint32_t* mask, uintptr_t stream);
 
 /* Background and rms maps of an image region (not part of the reference).  The region is W = ncols columns (columns
  * [0, ncols) of the buffer) by H = R1 - R0 rows (rows [R0, R1)); a run maps the pixels it read.
@@ -383,6 +431,19 @@ int cy_bkg_grid_pass_masked(const void* img, long long row_stride, int big_endia
                             int row_begin, int row_end, int box, int grid, const long long* unit_off, long long units,
                             const cy_noise_state* state, cy_noise_partial* partials, const uint32_t* mask,
                             int mask_ncols, int mask_col0, uintptr_t stream);
+/* Round `round` of a median pass of the lattice (median estimator above): hist[Nx * Ny * 512] as for
+ * cy_noise_pass_median, the other arguments as for cy_bkg_grid_pass; rounds are folded with cy_median_update(partials,
+ * world, hist, Nx * Ny, state, sel, round, &active, stream).  The hole probe and fill run unchanged on the median
+ * states (the probe is an unmasked cy_bkg_grid_pass: it only counts). */
+int cy_bkg_grid_pass_median(const void* img, long long row_stride, int big_endian, int row0, int ncols, int R0, int R1,
+                            int row_begin, int row_end, int box, int grid, const long long* unit_off, long long units,
+                            const cy_noise_state* state, const cy_select_state* sel, int round,
+                            cy_noise_partial* partials, uint32_t* hist, uintptr_t stream);
+int cy_bkg_grid_pass_median_masked(const void* img, long long row_stride, int big_endian, int row0, int ncols, int R0,
+                                   int R1, int row_begin, int row_end, int box, int grid, const long long* unit_off,
+                                   long long units, const cy_noise_state* state, const cy_select_state* sel,
+                                   int round, cy_noise_partial* partials, uint32_t* hist, const uint32_t* mask,
+                                   int mask_ncols, int mask_col0, uintptr_t stream);
 /* Hole fill of a masked lattice.  After the masked passes every node is one of:
  *   finite: nbkg > 0;
  *   hole:   nbkg = 0, but its box holds at least one data pixel (finite and non-zero) when M is ignored;

@@ -84,6 +84,9 @@ def parse_args(argv=None):
     p.add_argument('--bkg_mask_sources', dest='bkg_mask_sources', action='store_true',
                    help='B200 build only: mask the catalog boxes out of the --measure_noise frames and the '
                         '--save_bkg_maps node boxes, and fill the map nodes left without pixels from their neighbours')
+    p.add_argument('--bkg_estimator', dest='bkg_estimator', type=str, default='mean', choices=['mean', 'median'],
+                   help='B200 build only: centre of the --measure_noise and --save_bkg_maps sigma clipping (median: '
+                        "astropy's sigma_clipped_stats default; bkg is the clipped median)")
     p.add_argument('--detect_outfile', required=False, type=str, default="")
     p.add_argument('--detect_outfile_json', required=False, type=str, default="")
     args = p.parse_args(argv)
@@ -119,6 +122,9 @@ def validate_args(args):
         return -1
     if args.bkg_grid < 1:
         logger.error("Invalid bkg_grid given (hint: give a grid step >= 1 pixel)!")
+        return -1
+    if args.bkg_estimator not in ('mean', 'median'):
+        logger.error("Invalid bkg_estimator given (hint: give mean or median)!")
         return -1
     return 0
 
@@ -192,6 +198,7 @@ def main(argv=None):
         'save_tile_img': args.save_tile_img, 'precision': args.precision, 'measure_sources': args.measure_sources,
         'measure_noise': args.measure_noise, 'noise_frame': args.noise_frame, 'save_bkg_maps': args.save_bkg_maps,
         'bkg_box': args.bkg_box, 'bkg_grid': args.bkg_grid, 'bkg_mask_sources': args.bkg_mask_sources,
+        'bkg_estimator': args.bkg_estimator,
     })
     model = YOLO(args.weights, precision=args.precision)
     sfinder = SFinder(model, CONFIG)

@@ -17,7 +17,12 @@ masked states), and the local noise of the catalog with and without the mask (En
 unmasked calls alternate within each repetition, so both see the same machine state.  It reports the masked pixel
 fraction, the nodes left without pixels and the holes filled, and writes r05_bkgmask_bench.json to --out.
 
-    python tools/bkgmap_bench.py [--configs 3,4] [--reps 5] [--mask] [--out DIR]
+With --estimator median, the median estimator is timed against the mean on the catalog of the same run_image:
+Engine.measure_noise_band and Engine.bkg_maps_band, each unmasked and with the source mask, the median and the mean
+calls alternating within each repetition.  It reports the pass counts, the bytes of the select histograms and how far
+the median and mean node bkg lie apart, and writes r06_bkgmedian_bench.json to --out.
+
+    python tools/bkgmap_bench.py [--configs 3,4] [--reps 5] [--mask | --estimator median] [--out DIR]
 """
 import argparse
 import json
@@ -231,6 +236,53 @@ def mask_config(cfg, reps, variant, box, grid, frame=16):
                     "pass and cy_bkg_grid_fill from the final masked states"}
 
 
+def median_config(cfg, reps, variant, box, grid, frame=16):
+    """The --estimator median measurements of one config (module docstring)."""
+    import torch
+    from caesar_yolo_b200 import ops, pipeline, weights as W
+    dev = torch.device('cuda:0')
+    torch.cuda.set_device(dev)
+    a = argparse.Namespace(mosaic=32768 if cfg == 4 else 16384)
+    step = 0.5 if cfg == 4 else 1.0
+    n = a.mosaic
+    _, host = bench.make_mosaic_pinned(a)
+    tiles = ops.generate_tiles(0, n - 1, 0, n - 1, 512, 512, step, step)
+    w = W.make_random_weights(variant, 5, seed=0, cls_bias=bench.CLS_BIAS.get(variant, -16.0))
+    eng = pipeline.Engine(w, pipeline.make_pp_config(**bench.PP_FLAGS), imgsz=640, score_thr=bench.SCORE_THR,
+                          iou_thr=bench.IOU_THR, thr_soft=bench.SOFT, thr_hard=bench.HARD, device=dev)
+    src, _ = pipeline.run_image(eng, host, True, tiles)
+    mask = eng.source_mask_band(src, tiles)
+    calls = {}
+    for est in ('mean', 'median'):
+        for m in (None, mask):
+            tag = est + ('_masked' if m is not None else '')
+            calls['noise_' + tag] = (lambda e=est, mm=m: eng.measure_noise_band(src, tiles, frame, mask=mm,
+                                                                                estimator=e))
+            calls['maps_' + tag] = (lambda e=est, mm=m: eng.bkg_maps_band(tiles, box, grid, mask=mm, estimator=e))
+    out, passes = {}, {}
+    for k, fn in calls.items():                          # warm-up of every call timed below
+        out[k] = fn()
+        passes[k] = eng.noise_passes if k.startswith('noise') else eng.bkg_passes
+    ms = {k: 0.0 for k in calls}
+    for _ in range(reps):                                # the median and mean calls alternate
+        for k, fn in calls.items():
+            ms[k] += _events(fn, 1) / reps
+    nodes_mean, nodes_med = out['maps_mean'][0], out['maps_median'][0]
+    ok = (nodes_mean['nbkg'] > 0) & (nodes_med['nbkg'] > 0)
+    dz = np.abs(nodes_med['bkg'][ok] - nodes_mean['bkg'][ok]) / nodes_mean['rms'][ok]
+    return {"config": cfg, "mosaic": n, "tile_step": step, "bkg_box": box, "bkg_grid": grid, "noise_frame": frame,
+            "sources": int(len(src)), "nodes": [int(nodes_med.shape[0]), int(nodes_med.shape[1])],
+            "passes": passes, "ms": {k: round(v, 3) for k, v in ms.items()},
+            "median_over_mean": {k: round(ms[k.replace('mean', 'median')] / ms[k], 2) for k in ms if 'mean' in k},
+            "select_histogram_bytes": {"noise": len(src) * ops.SELECT_SLOTS * 4,
+                                       "maps": int(nodes_med.size) * ops.SELECT_SLOTS * 4},
+            "node_bkg_median_minus_mean_over_rms": {"median": float(np.median(dz)), "max": float(dz.max())},
+            "note": "CUDA events around each call, synchronised after it (Engine.measure_noise_band / bkg_maps_band: "
+                    "unit plan, every pass with its host read of the active count; the median passes are 4 digit "
+                    "rounds each); the median and mean calls alternate in every repetition; the masked calls include "
+                    "the probe and fill of the maps, not the mask build (built once)"}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--configs', default='3,4')
@@ -239,18 +291,23 @@ def main():
     ap.add_argument('--bkg_box', type=int, default=101)
     ap.add_argument('--bkg_grid', type=int, default=25)
     ap.add_argument('--mask', action='store_true', help='time the source mask (module docstring)')
-    ap.add_argument('--out', default=None, help='directory for bkgmap_bench.json (r05_bkgmask_bench.json with --mask)')
+    ap.add_argument('--estimator', default='mean', choices=['mean', 'median'],
+                    help='median: time the median estimator against the mean (module docstring)')
+    ap.add_argument('--out', default=None, help='directory for bkgmap_bench.json (r05_bkgmask_bench.json with --mask, '
+                                                 'r06_bkgmedian_bench.json with --estimator median)')
     a = ap.parse_args()
     info = card()
     lines = []
     for c in [int(x) for x in a.configs.split(',')]:
-        r = (mask_config if a.mask else run_config)(c, a.reps, a.variant, a.bkg_box, a.bkg_grid)
+        fn = median_config if a.estimator == 'median' else mask_config if a.mask else run_config
+        r = fn(c, a.reps, a.variant, a.bkg_box, a.bkg_grid)
         r.update(info)
         print(json.dumps(r), flush=True)
         lines.append(r)
     if a.out:
         os.makedirs(a.out, exist_ok=True)
-        name = 'r05_bkgmask_bench.json' if a.mask else 'bkgmap_bench.json'
+        name = 'r06_bkgmedian_bench.json' if a.estimator == 'median' else \
+            'r05_bkgmask_bench.json' if a.mask else 'bkgmap_bench.json'
         with open(os.path.join(a.out, name), 'w') as f:
             json.dump(lines, f, indent=1)
 

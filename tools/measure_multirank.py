@@ -19,6 +19,8 @@ rows of the single-rank maps (NaN positions equal).
 With --mask, --noise and --maps run with the source mask of the catalog (Engine.source_mask_band, built once per run over
 the rank's rows); the map comparison then also requires the same set of filled nodes (nbkg = 0 with a finite value) and
 the same count of holes filled.
+With --estimator median, --noise and --maps clip around the median (histograms summed with one all-reduce per digit
+round); bkg, nbkg, iters and the pass count must then be identical to the single-rank run, rms within --rtol.
 
 Prints one JSON line on rank 0 with the largest relative difference per field and the verdict of every rank."""
 import argparse
@@ -69,6 +71,8 @@ def main():
     ap.add_argument('--bkg_box', type=int, default=101)
     ap.add_argument('--bkg_grid', type=int, default=25)
     ap.add_argument('--mask', action='store_true', help='run --noise and --maps with the source mask')
+    ap.add_argument('--estimator', default='mean', choices=['mean', 'median'],
+                    help='centre of the --noise and --maps clipping')
     a = ap.parse_args()
     import torch
     import torch.distributed as dist
@@ -99,9 +103,9 @@ def main():
     ref_mask = eng.source_mask_band(ref, tiles) if a.mask else None
     noise_res = None
     if a.noise:
-        z = eng.measure_noise_band(src, tiles, a.noise_frame, rank, world, mask=mask)
+        z = eng.measure_noise_band(src, tiles, a.noise_frame, rank, world, mask=mask, estimator=a.estimator)
         passes = eng.noise_passes
-        zr = eng.measure_noise_band(ref, tiles, a.noise_frame, mask=ref_mask)
+        zr = eng.measure_noise_band(ref, tiles, a.noise_frame, mask=ref_mask, estimator=a.estimator)
         noise_res = dict(passes=passes, single_rank_passes=eng.noise_passes,
                          nbkg_exact=bool(np.array_equal(z['nbkg'], zr['nbkg'])),
                          iters_exact=bool(np.array_equal(z['iters'], zr['iters'])))
@@ -114,13 +118,16 @@ def main():
                 scale = np.maximum(scale, zr['rms'][f])
             dd = np.abs(x[f] - y[f]) / np.where(scale > 0, scale, 1.0)
             noise_res[k] = float(dd.max()) if (same_nan and dd.size) else (0.0 if same_nan else float('inf'))
+        noise_res['bkg_identical'] = bool(np.array_equal(z['bkg'], zr['bkg'], equal_nan=True))
         ok = ok and noise_res['nbkg_exact'] and noise_res['iters_exact'] and passes == eng.noise_passes and \
-            noise_res['bkg'] <= a.rtol and noise_res['rms'] <= a.rtol
+            noise_res['bkg'] <= a.rtol and noise_res['rms'] <= a.rtol and \
+            (a.estimator == 'mean' or noise_res['bkg_identical'])
     maps_res = None
     if a.maps:
-        z, bkg, rms, _, (r0, r1) = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, rank, world, mask=mask)
+        z, bkg, rms, _, (r0, r1) = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, rank, world, mask=mask,
+                                                     estimator=a.estimator)
         passes, filled = eng.bkg_passes, eng.bkg_holes_filled
-        zr, bkg_r, rms_r, _, _ = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, mask=ref_mask)
+        zr, bkg_r, rms_r, _, _ = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, mask=ref_mask, estimator=a.estimator)
         maps_res = dict(passes=passes, single_rank_passes=eng.bkg_passes, nodes=int(z.size),
                         nbkg_exact=bool(np.array_equal(z['nbkg'], zr['nbkg'])),
                         iters_exact=bool(np.array_equal(z['iters'], zr['iters'])))
@@ -149,15 +156,18 @@ def main():
             if f.any():
                 ulp = max(ulp, float((np.abs(p[f] - q[f]) / np.spacing(np.abs(q[f]))).max()))
         maps_res['map_max_ulp'] = ulp
+        maps_res['bkg_identical'] = bool(np.array_equal(z['bkg'], zr['bkg'], equal_nan=True))
         ok = ok and maps_res['nbkg_exact'] and maps_res['iters_exact'] and passes == eng.bkg_passes and \
-            maps_res['bkg'] <= a.rtol and maps_res['rms'] <= a.rtol and ulp <= 1.0
+            maps_res['bkg'] <= a.rtol and maps_res['rms'] <= a.rtol and ulp <= 1.0 and \
+            (a.estimator == 'mean' or maps_res['bkg_identical'])
     flags = torch.tensor([1 if ok else 0], device=dev if a.backend == 'nccl' else 'cpu')
     dist.all_reduce(flags, op=dist.ReduceOp.MIN)
     if rank == 0:
         print(json.dumps(dict(world=world, backend=a.backend, gpus=torch.cuda.device_count(), mosaic=n,
                               sources=int(len(src)), rows_of_rank0=list(rows),
                               catalog_identical=same_catalog, max_rel_diff={k: res[k] for k in FLOATS},
-                              exact={k: res[k + '_exact'] for k in EXACT}, rtol=a.rtol, noise=noise_res, maps=maps_res,
+                              exact={k: res[k + '_exact'] for k in EXACT}, rtol=a.rtol, estimator=a.estimator,
+                              noise=noise_res, maps=maps_res,
                               matches_single_rank_on_every_rank=bool(int(flags[0])))), flush=True)
     dist.destroy_process_group()
     return 0 if int(flags[0]) else 1
