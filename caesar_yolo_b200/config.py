@@ -53,6 +53,9 @@ CONFIG = {
     'save_bkg_maps': False,
     'bkg_box': 101,
     'bkg_grid': 25,
+    # - Background-subtracted and S/N maps of the image (not in the reference; FITS input; implies save_bkg_maps):
+    #   (image - bkg) and (image - bkg) / rms at every pixel of the bkg / rms maps; resmap_<id>.fits, snrmap_<id>.fits
+    'save_snr_maps': False,
     # - Mask the catalog boxes out of the measure_noise frames and the save_bkg_maps node boxes (not in the reference);
     #   map nodes left without pixels are filled from their neighbours.  Alone it changes nothing (one warning)
     'bkg_mask_sources': False,

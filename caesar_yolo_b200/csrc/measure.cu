@@ -836,12 +836,10 @@ __device__ __forceinline__ float interp_corners(double v00, double v01, double v
     return ws > 0.0 ? (float)(s / ws) : __int_as_float(0x7fc00000);
 }
 
-// one thread per map pixel: blockIdx.x = row - row_begin, blockIdx.y * blockDim.x + threadIdx.x = column
-__global__ void bkg_map_kernel(const cy_noise_state* __restrict__ state, Grid G, int row_begin,
-                               uint32_t* __restrict__ bkg, uint32_t* __restrict__ rms) {
-    const int x = blockIdx.y * blockDim.x + threadIdx.x;
-    if (x >= G.ncols) return;
-    const int y = row_begin + blockIdx.x;
+// the bkg and rms map values of region pixel (x, y): the corners and weights of its lattice cell, then interp_corners.
+// bkg_map_kernel and snr_map_kernel both take them from here, so the two agree to the bit.
+__device__ __forceinline__ void map_pixel(const cy_noise_state* __restrict__ state, const Grid& G, int x, int y,
+                                          float& fb, float& fr) {
     const int i = G.nx >= 2 ? min(x / G.g, G.nx - 2) : 0, i1 = min(i + 1, G.nx - 1);   // x_i = i * g for i <= nx - 2
     const int j = G.ny >= 2 ? min((y - G.R0) / G.g, G.ny - 2) : 0, j1 = min(j + 1, G.ny - 1);
     const double t = i1 > i ? (double)(x - G.xnode(i)) / (double)(G.xnode(i1) - G.xnode(i)) : 0.0;
@@ -849,11 +847,43 @@ __global__ void bkg_map_kernel(const cy_noise_state* __restrict__ state, Grid G,
     const double w00 = (1.0 - t) * (1.0 - v), w01 = t * (1.0 - v), w10 = (1.0 - t) * v, w11 = t * v;
     const cy_noise_state &a = state[(long long)j * G.nx + i], &b = state[(long long)j * G.nx + i1];
     const cy_noise_state &c = state[(long long)j1 * G.nx + i], &d = state[(long long)j1 * G.nx + i1];
-    const float fb = interp_corners(a.bkg, b.bkg, c.bkg, d.bkg, w00, w01, w10, w11);
-    const float fr = interp_corners(a.rms, b.rms, c.rms, d.rms, w00, w01, w10, w11);
+    fb = interp_corners(a.bkg, b.bkg, c.bkg, d.bkg, w00, w01, w10, w11);
+    fr = interp_corners(a.rms, b.rms, c.rms, d.rms, w00, w01, w10, w11);
+}
+
+// one thread per map pixel: blockIdx.x = row - row_begin, blockIdx.y * blockDim.x + threadIdx.x = column
+__global__ void bkg_map_kernel(const cy_noise_state* __restrict__ state, Grid G, int row_begin,
+                               uint32_t* __restrict__ bkg, uint32_t* __restrict__ rms) {
+    const int x = blockIdx.y * blockDim.x + threadIdx.x;
+    if (x >= G.ncols) return;
+    float fb, fr;
+    map_pixel(state, G, x, row_begin + blockIdx.x, fb, fr);
     const long long o = (long long)blockIdx.x * G.ncols + x;
     bkg[o] = __byte_perm(__float_as_uint(fb), 0, 0x0123);   // FITS byte order
     rms[o] = __byte_perm(__float_as_uint(fr), 0, 0x0123);
+}
+
+// background-subtracted and S/N maps (cy_bkg_grid_snr_maps), the grid of bkg_map_kernel: each thread reads its image
+// pixel once (a warp reads 32 adjacent words of one row) and writes res = v - bkg and snr = (v - bkg) / rms, both in
+// fp64 and rounded once.  NaN: a masked pixel or a NaN bkg in both maps; a NaN or non-positive rms in snr only.
+__global__ void snr_map_kernel(const uint32_t* __restrict__ img, long long row_stride, int big_endian, int row0,
+                               const cy_noise_state* __restrict__ state, Grid G, int row_begin,
+                               uint32_t* __restrict__ res, uint32_t* __restrict__ snr) {
+    const int x = blockIdx.y * blockDim.x + threadIdx.x;
+    if (x >= G.ncols) return;
+    const int y = row_begin + blockIdx.x;
+    const float v = noise_pixel(img + (long long)(y - row0) * row_stride + x, big_endian);
+    float fb, fr;
+    map_pixel(state, G, x, y, fb, fr);
+    float r = __int_as_float(0x7fc00000), s = r;
+    if (!isnan(v) && !isnan(fb)) {
+        const double d = (double)v - (double)fb;
+        r = (float)d;
+        if (fr > 0.0f) s = (float)(d / (double)fr);   // false for NaN
+    }
+    const long long o = (long long)blockIdx.x * G.ncols + x;
+    res[o] = __byte_perm(__float_as_uint(r), 0, 0x0123);   // FITS byte order
+    snr[o] = __byte_perm(__float_as_uint(s), 0, 0x0123);
 }
 
 // ---------------------------------------------------------------------------------------------- source mask
@@ -1295,6 +1325,23 @@ extern "C" int cy_bkg_grid_maps(const cy_noise_state* state, int ncols, int R0, 
                      (cudaStream_t)stream>>>(state, G, row_begin, (uint32_t*)bkg, (uint32_t*)rms);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_maps: %s", cudaGetErrorString(e));
+    return CY_OK;
+}
+
+extern "C" int cy_bkg_grid_snr_maps(const cy_noise_state* state, const void* img, long long row_stride, int big_endian,
+                                    int row0, int ncols, int R0, int R1, int row_begin, int row_end, int box, int grid,
+                                    void* res, void* snr, uintptr_t stream) {
+    Grid G;
+    if (!make_grid(ncols, R0, R1, row_begin, row_end, box, grid, G) || (ncols + 255) / 256 > 65535 ||
+        row_stride < ncols || row_begin < row0)
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_snr_maps: invalid image geometry, region, row range, box or grid");
+    if (row_end == row_begin) return CY_OK;
+    if (!state || !img || !res || !snr) return set_error(CY_ERR_INVALID, "cy_bkg_grid_snr_maps: null argument");
+    snr_map_kernel<<<dim3((unsigned)(row_end - row_begin), (unsigned)((ncols + 255) / 256)), 256, 0,
+                     (cudaStream_t)stream>>>((const uint32_t*)img, row_stride, big_endian, row0, state, G, row_begin,
+                                             (uint32_t*)res, (uint32_t*)snr);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_snr_maps: %s", cudaGetErrorString(e));
     return CY_OK;
 }
 

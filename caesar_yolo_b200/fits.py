@@ -207,12 +207,13 @@ _WCS_KEYS = ("CD1_1", "CD1_2", "CD2_1", "CD2_2", "PC1_1", "PC1_2", "PC2_1", "PC2
              "RADESYS", "EQUINOX", "BUNIT", "BMAJ", "BMIN", "BPA")
 
 
-def map_header(h, nx, ny, x0=0, y0=0, bkgmask=False, bkgest='mean'):
+def map_header(h, nx, ny, x0=0, y0=0, bkgmask=False, bkgest='mean', bunit=True):
     """Header (bytes, a multiple of 2880) of a 2-D BITPIX -32 map of nx x ny pixels whose pixel (0, 0) is pixel (x0, y0)
     of the image with header dict h: the WCS cards of axes 1 and 2, BUNIT and the beam are copied, and CRPIX1/2 are
     shifted by (x0, y0), so every map pixel has the sky position of the image pixel under it.  bkgmask: the catalog
     boxes were masked out of the node boxes (card BKGMASK = T; no card otherwise).  bkgest: the centre of the node
-    clipping; 'median' writes BKGEST = 'MEDIAN', the mean writes no card."""
+    clipping; 'median' writes BKGEST = 'MEDIAN', the mean writes no card.  bunit=False leaves BUNIT out, for a map
+    without the image's unit (the S/N map)."""
     cards = [format_card("SIMPLE", True, "conforms to FITS standard"), format_card("BITPIX", -32, "array data type"),
              format_card("NAXIS", 2, "number of array dimensions"), format_card("NAXIS1", int(nx)),
              format_card("NAXIS2", int(ny))]
@@ -222,7 +223,7 @@ def map_header(h, nx, ny, x0=0, y0=0, bkgmask=False, bkgest='mean'):
                 cards.append(format_card("%s%d" % (k, a), h["%s%d" % (k, a)]))
         if "CRPIX%d" % a in h:
             cards.append(format_card("CRPIX%d" % a, h["CRPIX%d" % a] - off))
-    cards += [format_card(k, h[k]) for k in _WCS_KEYS if k in h]
+    cards += [format_card(k, h[k]) for k in _WCS_KEYS if k in h and (bunit or k != "BUNIT")]
     if bkgmask:
         cards.append(format_card("BKGMASK", True, "catalog boxes masked out of the node boxes"))
     if bkgest == 'median':

@@ -56,7 +56,9 @@ class SFinder(object):
         self.measure_noise = bool(config.get('measure_noise', False))
         self.measure_sources = bool(config.get('measure_sources', False)) or self.measure_noise
         self.noise_frame = int(config.get('noise_frame', 16))
-        self.save_bkg_maps = bool(config.get('save_bkg_maps', False))
+        # the background-subtracted and S/N maps are made from the node states of the bkg / rms maps, so they imply them
+        self.save_snr_maps = bool(config.get('save_snr_maps', False))
+        self.save_bkg_maps = bool(config.get('save_bkg_maps', False)) or self.save_snr_maps
         self.bkg_box = int(config.get('bkg_box', 101))
         self.bkg_grid = int(config.get('bkg_grid', 25))
         # the catalog boxes masked out of the noise frames and the map nodes; only these two consumers use the mask
@@ -228,9 +230,15 @@ class SFinder(object):
                                       estimator=self.bkg_estimator) if self.measure_noise else None
             meas = self._measurements(m, self.fits.header, x0, y0, noise)
         if self.save_bkg_maps:   # the region read: the crop, columns from x0
-            _, bkg, rms = eng.bkg_maps(dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0, 0,
-                                       y1 - y0, self.bkg_box, self.bkg_grid, mask=mask, estimator=self.bkg_estimator)
-            self._write_bkg_maps(bkg, rms, 0, (x0, y0, x1 - x0, y1 - y0))
+            args = (dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0, 0, y1 - y0,
+                    self.bkg_box, self.bkg_grid)
+            nodes, bkg, rms = eng.bkg_maps(*args, mask=mask, estimator=self.bkg_estimator)
+            region = (x0, y0, x1 - x0, y1 - y0)
+            self._write_maps('bkg_maps_write_s', (('bkgmap_', bkg, True), ('rmsmap_', rms, True)), 0, region)
+            del bkg, rms   # freed before res / snr are allocated: no more than two region maps at a time
+            if self.save_snr_maps:
+                res, snr = eng.snr_maps(nodes, *args)
+                self._write_maps('snr_maps_write_s', (('resmap_', res, True), ('snrmap_', snr, False)), 0, region)
         self.timing['run_s'] = time.time() - t0
         return self._save_serial(recs, status, meas)
 
@@ -244,17 +252,18 @@ class SFinder(object):
                            "ra/dec are written as null", header.get('CTYPE1'), header.get('CTYPE2'))
         return catalog.measurement_dicts(m, fitsmeta.beam_area_pix(header), radec, noise)
 
-    def _write_bkg_maps(self, bkg, rms, row_begin, region):
-        """bkgmap_<id>.fits and rmsmap_<id>.fits in outdir: this rank's map rows (Engine.bkg_maps) of the region
-        (X0, R0, W, H), with the image's WCS shifted to the region."""
+    def _write_maps(self, timing_key, maps, row_begin, region):
+        """<prefix><id>.fits in outdir for each (prefix, rows, bunit) of maps: this rank's map rows of the region
+        (X0, R0, W, H), with the image's WCS shifted to the region; bunit=False leaves BUNIT out (a dimensionless
+        map)."""
         X0, R0, W, H = region
         t0 = time.time()
-        hdr = fitsmeta.map_header(self.fits.header, W, H, X0, R0, bkgmask=self.bkg_mask_sources,
-                                  bkgest=self.bkg_estimator)
-        for name, rows in (('bkgmap_', bkg), ('rmsmap_', rms)):
+        for name, rows, bunit in maps:
+            hdr = fitsmeta.map_header(self.fits.header, W, H, X0, R0, bkgmask=self.bkg_mask_sources,
+                                      bkgest=self.bkg_estimator, bunit=bunit)
             fitsmeta.write_map_rows(os.path.join(self.outdir, name + str(self.image_id) + '.fits'), hdr, rows,
                                     row_begin, W, H, self.procId, self.nproc)
-        self.timing['bkg_maps_write_s'] = time.time() - t0
+        self.timing[timing_key] = time.time() - t0
 
     def _save_serial(self, recs, status, meas=None):
         self.results = {"image_id": self.image_id, "objs": catalog.records_to_objs(recs, self.class_names, meas=meas)}
@@ -314,7 +323,9 @@ class SFinder(object):
         recs = packed.cpu().numpy().view(ops.REC_DTYPE).copy()
         meas = None
         if self.save_bkg_maps:
-            logger.warning("Background and rms maps are written for FITS images only: none for %s", c['image_path'])
+            logger.warning("%s maps are written for FITS images only: none for %s",
+                           "Background, rms, background-subtracted and S/N" if self.save_snr_maps
+                           else "Background and rms", c['image_path'])
         if self.measure_sources:
             if plane_dev is None:
                 logger.warning("Colour image: per-source measurements need a single-plane image and are not written")
@@ -396,9 +407,15 @@ class SFinder(object):
             if self.procId == 0:
                 meas = self._measurements(m, self.fits.header, noise=noise)
         if self.save_bkg_maps:   # every rank maps and writes its own rows; unmasked maps need no catalog
-            _, bkg, rms, region, rows = eng.bkg_maps_band(tiles, self.bkg_box, self.bkg_grid, self.procId, self.nproc,
-                                                          mask=mask, estimator=self.bkg_estimator)
-            self._write_bkg_maps(bkg, rms, rows[0] - region[1], region)
+            nodes, bkg, rms, region, rows = eng.bkg_maps_band(tiles, self.bkg_box, self.bkg_grid, self.procId,
+                                                              self.nproc, mask=mask, estimator=self.bkg_estimator)
+            self._write_maps('bkg_maps_write_s', (('bkgmap_', bkg, True), ('rmsmap_', rms, True)),
+                             rows[0] - region[1], region)
+            del bkg, rms   # freed before res / snr are allocated: no more than two region maps at a time
+            if self.save_snr_maps:   # the same rows of the band, no collective
+                res, snr, _, _ = eng.snr_maps_band(nodes, tiles, self.bkg_box, self.bkg_grid, self.procId, self.nproc)
+                self._write_maps('snr_maps_write_s', (('resmap_', res, True), ('snrmap_', snr, False)),
+                                 rows[0] - region[1], region)
         self.timing['run_s'] = time.time() - t0
         if self.procId == 0:
             self.sources = {"sources": catalog.sources_to_dicts(src, self.class_names, meas)}

@@ -552,5 +552,14 @@ def bkg_grid_maps(state, ncols, R0, R1, row_begin, row_end, box, grid, bkg, rms)
                                c_int(box), c_int(grid), ptr(bkg), ptr(rms), cur_stream()))
 
 
+def bkg_grid_snr_maps(state, img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box, grid, res,
+                      snr):
+    """cy_bkg_grid_snr_maps: final node states and this range's image rows (layout as for bkg_grid_pass) -> rows
+    [row_begin, row_end) of the background-subtracted and S/N maps (device tensors as for bkg_grid_maps)."""
+    check(lib.cy_bkg_grid_snr_maps(ptr(state), ptr(img), c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0),
+                                   c_int(ncols), c_int(R0), c_int(R1), c_int(row_begin), c_int(row_end), c_int(box),
+                                   c_int(grid), ptr(res), ptr(snr), cur_stream()))
+
+
 def to_device_bytes(np_array, device):
     return torch.from_numpy(np_array.view(np.uint8).reshape(-1).copy()).to(device)

@@ -557,6 +557,15 @@ class Engine(object):
         left in HBM.  mask: Engine.source_mask_band (image columns, so the region starts at its column X0), or None;
         estimator as for Engine.bkg_maps.
         Returns (nodes, bkg, rms, (X0, R0, W, H), (row_begin, row_end))."""
+        img, nx, big_endian, Y0, (X0, R0, W, H), (r0, r1) = self._map_band(tiles, rank, world)
+        nodes, bkg, rms = self.bkg_maps(img, nx, big_endian, Y0, W, R0, R0 + H, r0, r1, box, grid, world, mask=mask,
+                                        mask_col0=X0, estimator=estimator)
+        return nodes, bkg, rms, (X0, R0, W, H), (r0, r1)
+
+    def _map_band(self, tiles, rank, world):
+        """The map region of a tiled run, (X0, R0, W, H): the bounding box of the tile grid; this rank's rows of it
+        (measure_rows, [R0, R0) when it has none); and where they are read: (img, row_stride, big_endian, row0, region,
+        rows), img being the band of mosaic rows the last run_image left in HBM from column X0."""
         X0, X1 = int(tiles['xmin'].min()), int(tiles['xmax'].max())
         R0, R1 = int(tiles['ymin'].min()), int(tiles['ymax'].max())
         r0, r1 = measure_rows(tiles, world)[rank]
@@ -567,9 +576,34 @@ class Engine(object):
             img, Y0 = self._get('meas_noband', (1,), torch.int32), r0
         else:
             img = band[:, X0:]
-        nodes, bkg, rms = self.bkg_maps(img, nx, big_endian, Y0, X1 - X0, R0, R1, r0, r1, box, grid, world, mask=mask,
-                                        mask_col0=X0, estimator=estimator)
-        return nodes, bkg, rms, (X0, R0, X1 - X0, R1 - R0), (r0, r1)
+        return img, nx, big_endian, Y0, (X0, R0, X1 - X0, R1 - R0), (r0, r1)
+
+    def snr_maps(self, nodes, img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box=101, grid=25):
+        """Background-subtracted and S/N maps (definition: include/caesar_b200.h) of the region of Engine.bkg_maps over
+        rows [row_begin, row_end) of `img` (the same arguments), from `nodes`, the final node states Engine.bkg_maps
+        returned (cy_bkg_grid_snr_maps).  One pass over the rows and no collective: each rank maps its own rows.
+        Returns (res, snr): int32 device tensors [row_end - row_begin, ncols] holding big-endian float32."""
+        nx, ny = len(ops.bkg_grid_nodes(ncols, grid)), len(ops.bkg_grid_nodes(R1 - R0, grid))
+        nodes = np.ascontiguousarray(nodes, dtype=ops.NOISE_DTYPE)
+        if nodes.shape != (ny, nx):
+            raise CaesarB200Error("Engine.snr_maps: node states of shape %s for a lattice of %d x %d nodes"
+                                  % (nodes.shape, ny, nx))
+        e = self._mark()
+        res = torch.empty((row_end - row_begin, ncols), dtype=torch.int32, device=self.device)
+        snr = torch.empty_like(res)
+        ops.bkg_grid_snr_maps(ops.to_device_bytes(nodes, self.device), img, row_stride, big_endian, row0, ncols, R0, R1,
+                              row_begin, row_end, box, grid, res, snr)
+        self._stage('snr_maps', e)
+        self.launches += 1
+        return res, snr
+
+    def snr_maps_band(self, nodes, tiles, box=101, grid=25, rank=0, world=1):
+        """Engine.snr_maps of the region and rows of Engine.bkg_maps_band (the same band of mosaic rows in HBM, so the
+        file is not read again), from the node states it returned.  Returns (res, snr, (X0, R0, W, H), (row_begin,
+        row_end))."""
+        img, nx, big_endian, Y0, (X0, R0, W, H), (r0, r1) = self._map_band(tiles, rank, world)
+        res, snr = self.snr_maps(nodes, img, nx, big_endian, Y0, W, R0, R0 + H, r0, r1, box, grid)
+        return res, snr, (X0, R0, W, H), (r0, r1)
 
     def _exchange_cap(self, world, need=0):
         """Records per rank slot of the all-gather: 48 per tile of the largest band (the catalogs of the synthetic

@@ -411,7 +411,13 @@ int cy_noise_pass_median_masked(const void* img, long long row_stride, int big_e
  * clamped to Nx - 2 (0 when Nx = 1), t = (x - x_i) / (x_{i+1} - x_i) (0 when Nx = 1), and j, u alike along rows.  A
  * corner whose value is NaN is dropped and the weights of the others renormalised; the pixel is NaN when the finite
  * corners carry no weight.  The rms map interpolates the node rms (not the variance).  Stored as float32 in FITS byte
- * order (big-endian, BITPIX -32). */
+ * order (big-endian, BITPIX -32).
+ * Background-subtracted and S/N maps (opt-in): at map pixel (x, y), v is the image pixel decoded as for the noise
+ * statistics (byte order applied; non-finite and 0 are masked), fb and fr the float32 values of the bkg and rms maps
+ * at that pixel, to the bit (same interpolation, NaN corners dropped alike).
+ *   res = (float)((double)v - (double)fb),  snr = (float)(((double)v - (double)fb) / (double)fr).
+ * A masked v or a NaN fb gives NaN in both maps; a NaN fr or fr <= 0 gives NaN in snr only.  The source mask M is not
+ * applied to these maps (sources show in them; M only shaped the nodes).  Stored like the bkg and rms maps. */
 
 /* Sets state[Nx * Ny] to pass 0 and writes the exclusive offsets unit_off[Ny + 1] of the work units of rows [row_begin,
  * row_end) (R0 <= row_begin <= row_end <= R1; a unit is one chunk of <= 32 rows of one node row and 16 adjacent node
@@ -468,6 +474,13 @@ int cy_bkg_grid_fill(const cy_noise_partial* probe_partials, int world, int nx, 
  * each, row-major, big-endian float32.  No pixel of the image is read. */
 int cy_bkg_grid_maps(const cy_noise_state* state, int ncols, int R0, int R1, int row_begin, int row_end, int box,
                      int grid, void* bkg, void* rms, uintptr_t stream);
+/* Final node states and rows [row_begin, row_end) of img (layout, row0 and region columns as for cy_bkg_grid_pass)
+ * -> the same rows of the background-subtracted (res) and S/N (snr) maps above: (row_end - row_begin) x ncols 4-byte
+ * words each, row-major, big-endian float32.  One pass: every image pixel of the rows is read once; no collective (each
+ * rank maps its own rows).  The other arguments as for cy_bkg_grid_maps. */
+int cy_bkg_grid_snr_maps(const cy_noise_state* state, const void* img, long long row_stride, int big_endian, int row0,
+                         int ncols, int R0, int R1, int row_begin, int row_end, int box, int grid, void* res, void* snr,
+                         uintptr_t stream);
 
 /* ------------------------------------------------------------------------------------------------ whole path
  * FITS file -> merged catalog with no host-language orchestration: SFinder.run_parallel (caesar_yolo/inference.py:

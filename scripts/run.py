@@ -77,6 +77,9 @@ def parse_args(argv=None):
     p.add_argument('--save_bkg_maps', dest='save_bkg_maps', action='store_true',
                    help='B200 build only: write the background and rms maps of a FITS image (bkgmap_<id>.fits, '
                         'rmsmap_<id>.fits)')
+    p.add_argument('--save_snr_maps', dest='save_snr_maps', action='store_true',
+                   help='B200 build only: also write the background-subtracted and S/N maps of a FITS image '
+                        '(resmap_<id>.fits, snrmap_<id>.fits; implies --save_bkg_maps)')
     p.add_argument('--bkg_box', dest='bkg_box', type=int, default=101,
                    help='B200 build only: side in pixels (odd, >= 3) of the box each --save_bkg_maps node clips')
     p.add_argument('--bkg_grid', dest='bkg_grid', type=int, default=25,
@@ -91,6 +94,7 @@ def parse_args(argv=None):
     p.add_argument('--detect_outfile_json', required=False, type=str, default="")
     args = p.parse_args(argv)
     args.measure_sources = args.measure_sources or args.measure_noise   # S/N and flux_bkgsub need the peak and sum
+    args.save_bkg_maps = args.save_bkg_maps or args.save_snr_maps       # res / snr are made from the bkg / rms nodes
     return args
 
 
@@ -198,7 +202,7 @@ def main(argv=None):
         'save_tile_img': args.save_tile_img, 'precision': args.precision, 'measure_sources': args.measure_sources,
         'measure_noise': args.measure_noise, 'noise_frame': args.noise_frame, 'save_bkg_maps': args.save_bkg_maps,
         'bkg_box': args.bkg_box, 'bkg_grid': args.bkg_grid, 'bkg_mask_sources': args.bkg_mask_sources,
-        'bkg_estimator': args.bkg_estimator,
+        'bkg_estimator': args.bkg_estimator, 'save_snr_maps': args.save_snr_maps,
     })
     model = YOLO(args.weights, precision=args.precision)
     sfinder = SFinder(model, CONFIG)

@@ -22,7 +22,14 @@ Engine.measure_noise_band and Engine.bkg_maps_band, each unmasked and with the s
 calls alternating within each repetition.  It reports the pass counts, the bytes of the select histograms and how far
 the median and mean node bkg lie apart, and writes r06_bkgmedian_bench.json to --out.
 
-    python tools/bkgmap_bench.py [--configs 3,4] [--reps 5] [--mask | --estimator median] [--out DIR]
+With --snr, the background-subtracted and S/N maps are timed from the final node states of the same run_image's band:
+cy_bkg_grid_snr_maps alone (CUDA events around --reps launches into preallocated rows, after a warm-up; the 12 bytes per
+pixel of a 16k^2 or 32k^2 region are far more than the 126 MB L2, so every launch reads and writes HBM), alternating with
+cy_bkg_grid_maps into the same kind of rows, and the Engine.snr_maps_band call (row allocation and node upload included).
+Algorithmic bytes: 4 read and 8 written per pixel, plus the bkg and rms of every node once.  The two files are written
+once and timed on the host clock.  Writes r07_snrmap_bench.json to --out.
+
+    python tools/bkgmap_bench.py [--configs 3,4] [--reps 5] [--mask | --estimator median | --snr] [--out DIR]
 """
 import argparse
 import json
@@ -283,6 +290,72 @@ def median_config(cfg, reps, variant, box, grid, frame=16):
                     "the probe and fill of the maps, not the mask build (built once)"}
 
 
+def snr_config(cfg, reps, variant, box, grid):
+    """The --snr measurements of one config (module docstring)."""
+    import torch
+    from caesar_yolo_b200 import fits, ops, pipeline, weights as W
+    dev = torch.device('cuda:0')
+    torch.cuda.set_device(dev)
+    a = argparse.Namespace(mosaic=32768 if cfg == 4 else 16384)
+    step = 0.5 if cfg == 4 else 1.0
+    n = a.mosaic
+    _, host = bench.make_mosaic_pinned(a)
+    tiles = ops.generate_tiles(0, n - 1, 0, n - 1, 512, 512, step, step)
+    w = W.make_random_weights(variant, 5, seed=0, cls_bias=bench.CLS_BIAS.get(variant, -16.0))
+    eng = pipeline.Engine(w, pipeline.make_pp_config(**bench.PP_FLAGS), imgsz=640, score_thr=bench.SCORE_THR,
+                          iou_thr=bench.IOU_THR, thr_soft=bench.SOFT, thr_hard=bench.HARD, device=dev)
+    pipeline.run_image(eng, host, True, tiles)
+    nodes, bkg, rms, (X0, R0, Wd, Hd), rows = eng.bkg_maps_band(tiles, box, grid)
+    res, snr, _, _ = eng.snr_maps_band(nodes, tiles, box, grid)          # warm-up of the Engine call
+    band, Y0, _, nx, be = eng.band
+    img = band[:, X0:]
+    state = ops.to_device_bytes(nodes, dev)
+    res2, snr2 = torch.empty_like(res), torch.empty_like(snr)
+
+    def snr_call():
+        ops.bkg_grid_snr_maps(state, img, nx, be, Y0, Wd, R0, R0 + Hd, rows[0], rows[1], box, grid, res2, snr2)
+
+    def map_call():
+        ops.bkg_grid_maps(state, Wd, R0, R0 + Hd, rows[0], rows[1], box, grid, bkg, rms)
+    snr_call()
+    map_call()
+    torch.cuda.synchronize()
+    same = bool(torch.equal(res, res2) and torch.equal(snr, snr2))
+    ms = dict(snr=0.0, maps=0.0, engine=0.0)
+    for _ in range(reps):                                # the two kernels alternate, reps launches each
+        for k, fn in (('snr', snr_call), ('maps', map_call)):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(reps):
+                fn()
+            e1.record()
+            torch.cuda.synchronize()
+            ms[k] += e0.elapsed_time(e1) / (reps * reps)
+        ms['engine'] += _events(lambda: eng.snr_maps_band(nodes, tiles, box, grid), 1) / reps
+    pix = Wd * (rows[1] - rows[0])
+    snr_bytes = 12 * pix + 16 * nodes.size
+    with tempfile.TemporaryDirectory() as d:
+        t0 = time.time()
+        for name, m, unit in (('resmap.fits', res, True), ('snrmap.fits', snr, False)):
+            fits.write_map_rows(os.path.join(d, name), fits.map_header({}, Wd, Hd, X0, R0, bunit=unit), m, 0, Wd, Hd)
+        write_s = time.time() - t0
+    f = snr.cpu().numpy().view('>f4')
+    finite = float(np.isfinite(f).mean())
+    return {"config": cfg, "mosaic": n, "tile_step": step, "bkg_box": box, "bkg_grid": grid,
+            "nodes": [int(nodes.shape[0]), int(nodes.shape[1])], "pixels": pix,
+            "snr_kernel_ms": round(ms['snr'], 3), "snr_bytes": snr_bytes,
+            "snr_tb_s": round(snr_bytes / (ms['snr'] * 1e-3) / 1e12, 2),
+            "bkg_map_kernel_ms": round(ms['maps'], 3), "bkg_map_bytes": 8 * pix + 16 * nodes.size,
+            "bkg_map_tb_s": round((8 * pix + 16 * nodes.size) / (ms['maps'] * 1e-3) / 1e12, 2),
+            "snr_maps_band_ms": round(ms['engine'], 3), "engine_and_kernel_bytes_identical": same,
+            "snr_finite_fraction": round(finite, 5), "file_write_s": round(write_s, 3),
+            "note": "snr_kernel_ms / bkg_map_kernel_ms: CUDA events around back-to-back launches of cy_bkg_grid_snr_maps "
+                    "/ cy_bkg_grid_maps into preallocated rows, the two alternating per repetition; bytes: 4 read + 8 "
+                    "written per pixel (8 written for the bkg / rms maps) + 16 per node; snr_maps_band_ms: events "
+                    "around Engine.snr_maps_band (row allocation, node upload, kernel); file_write_s: host clock "
+                    "around both files (one rank, a temporary directory on the local disk)"}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--configs', default='3,4')
@@ -293,20 +366,23 @@ def main():
     ap.add_argument('--mask', action='store_true', help='time the source mask (module docstring)')
     ap.add_argument('--estimator', default='mean', choices=['mean', 'median'],
                     help='median: time the median estimator against the mean (module docstring)')
+    ap.add_argument('--snr', action='store_true', help='time the background-subtracted and S/N maps (module docstring)')
     ap.add_argument('--out', default=None, help='directory for bkgmap_bench.json (r05_bkgmask_bench.json with --mask, '
-                                                 'r06_bkgmedian_bench.json with --estimator median)')
+                                                 'r06_bkgmedian_bench.json with --estimator median, '
+                                                 'r07_snrmap_bench.json with --snr)')
     a = ap.parse_args()
     info = card()
     lines = []
     for c in [int(x) for x in a.configs.split(',')]:
-        fn = median_config if a.estimator == 'median' else mask_config if a.mask else run_config
+        fn = snr_config if a.snr else median_config if a.estimator == 'median' else mask_config if a.mask else \
+            run_config
         r = fn(c, a.reps, a.variant, a.bkg_box, a.bkg_grid)
         r.update(info)
         print(json.dumps(r), flush=True)
         lines.append(r)
     if a.out:
         os.makedirs(a.out, exist_ok=True)
-        name = 'r06_bkgmedian_bench.json' if a.estimator == 'median' else \
+        name = 'r07_snrmap_bench.json' if a.snr else 'r06_bkgmedian_bench.json' if a.estimator == 'median' else \
             'r05_bkgmask_bench.json' if a.mask else 'bkgmap_bench.json'
         with open(os.path.join(a.out, name), 'w') as f:
             json.dump(lines, f, indent=1)

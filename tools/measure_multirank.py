@@ -21,6 +21,13 @@ the rank's rows); the map comparison then also requires the same set of filled n
 the same count of holes filled.
 With --estimator median, --noise and --maps clip around the median (histograms summed with one all-reduce per digit
 round); bkg, nbkg, iters and the pass count must then be identical to the single-rank run, rms within --rtol.
+With --snr, every rank also runs Engine.bkg_maps_band and Engine.snr_maps_band (the background-subtracted and S/N maps of
+its own rows, no collective beyond the node passes), with --mask and --estimator as given.  Its rows of both maps must be
+byte-identical to the same rows of one single-rank call on the same node states (the maps do not depend on the row
+split).  Against the single-rank run (its own node passes), they must be byte-identical when the node bkg / rms are; with
+the mean estimator the node sums are folded in another order over 2 ranks, so the node values, and with them res / snr,
+may differ in the last bits: the tool then reports the largest difference in float32 ulps (within the 1 ulp of the --maps
+check, compounded by the division).
 
 Prints one JSON line on rank 0 with the largest relative difference per field and the verdict of every rank."""
 import argparse
@@ -72,7 +79,8 @@ def main():
     ap.add_argument('--bkg_grid', type=int, default=25)
     ap.add_argument('--mask', action='store_true', help='run --noise and --maps with the source mask')
     ap.add_argument('--estimator', default='mean', choices=['mean', 'median'],
-                    help='centre of the --noise and --maps clipping')
+                    help='centre of the --noise, --maps and --snr clipping')
+    ap.add_argument('--snr', action='store_true', help='also compare the background-subtracted and S/N maps')
     a = ap.parse_args()
     import torch
     import torch.distributed as dist
@@ -160,6 +168,27 @@ def main():
         ok = ok and maps_res['nbkg_exact'] and maps_res['iters_exact'] and passes == eng.bkg_passes and \
             maps_res['bkg'] <= a.rtol and maps_res['rms'] <= a.rtol and ulp <= 1.0 and \
             (a.estimator == 'mean' or maps_res['bkg_identical'])
+    snr_res = None
+    if a.snr:
+        z = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, rank, world, mask=mask, estimator=a.estimator)[0]
+        res_m, snr_m, _, (r0, r1) = eng.snr_maps_band(z, tiles, a.bkg_box, a.bkg_grid, rank, world)
+        zr = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, mask=ref_mask, estimator=a.estimator)[0]
+        y0 = int(tiles['ymin'].min())
+        res_s, snr_s, _, _ = eng.snr_maps_band(z, tiles, a.bkg_box, a.bkg_grid)   # the same nodes, all rows at once
+        split_ok = bool(torch.equal(res_m, res_s[r0 - y0:r1 - y0]) and torch.equal(snr_m, snr_s[r0 - y0:r1 - y0]))
+        res_r, snr_r, _, _ = eng.snr_maps_band(zr, tiles, a.bkg_box, a.bkg_grid)
+        same_nodes = all(z[k].tobytes() == zr[k].tobytes() for k in ('bkg', 'rms'))
+        snr_res = dict(rows=[r0, r1], row_split_identical=split_ok, node_bkg_rms_identical=same_nodes,
+                       res_identical=bool(torch.equal(res_m, res_r[r0 - y0:r1 - y0])),
+                       snr_identical=bool(torch.equal(snr_m, snr_r[r0 - y0:r1 - y0])))
+        for k, mine, ref_rows in (('res', res_m, res_r), ('snr', snr_m, snr_r)):
+            p = mine.cpu().numpy().view('>f4').astype(np.float64)
+            q = ref_rows[r0 - y0:r1 - y0].cpu().numpy().view('>f4').astype(np.float32)
+            f = ~np.isnan(q)
+            same_nan = np.array_equal(np.isnan(p), ~f)
+            ulp = float((np.abs(p[f] - q[f]) / np.spacing(np.abs(q[f]))).max()) if f.any() else 0.0
+            snr_res[k + '_max_ulp'] = ulp if same_nan else float('inf')
+        ok = ok and split_ok and (not same_nodes or (snr_res['res_identical'] and snr_res['snr_identical']))
     flags = torch.tensor([1 if ok else 0], device=dev if a.backend == 'nccl' else 'cpu')
     dist.all_reduce(flags, op=dist.ReduceOp.MIN)
     if rank == 0:
@@ -167,7 +196,7 @@ def main():
                               sources=int(len(src)), rows_of_rank0=list(rows),
                               catalog_identical=same_catalog, max_rel_diff={k: res[k] for k in FLOATS},
                               exact={k: res[k + '_exact'] for k in EXACT}, rtol=a.rtol, estimator=a.estimator,
-                              noise=noise_res, maps=maps_res,
+                              noise=noise_res, maps=maps_res, snr=snr_res,
                               matches_single_rank_on_every_rank=bool(int(flags[0])))), flush=True)
     dist.destroy_process_group()
     return 0 if int(flags[0]) else 1
