@@ -62,4 +62,11 @@ CONFIG = {
     # - Centre of the sigma clipping of measure_noise and save_bkg_maps (not in the reference): 'mean' or 'median'
     #   (astropy's sigma_clipped_stats default; bkg is then the clipped median).  Alone it changes nothing (one warning)
     'bkg_estimator': 'mean',
+    # - Catalog completeness by injection and recovery (not in the reference; FITS input): inject_sources beam-shaped
+    #   point sources per round at empty positions, with S/N log-uniform in inject_snr_range against the rms map of the
+    #   save_bkg_maps options, detected again; inject_<id>.json.  0: off
+    'inject_sources': 0,
+    'inject_rounds': 1,
+    'inject_snr_range': (3.0, 100.0),
+    'inject_seed': 0,
 }

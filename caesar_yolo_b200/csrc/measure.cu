@@ -990,6 +990,53 @@ __global__ void bkg_fill_store_kernel(const FillNode* __restrict__ a, int nodes,
     state[n].rms = a[n].rms;
 }
 
+// ---------------------------------------------------------------------------------------------- injection
+// Beam-shaped point sources added to the rows in HBM (cy_inject_sources) and taken out again (cy_inject_restore).  One
+// CTA per injection; thread k of the footprint's (2 rx + 1) (2 ry + 1) pixels is slot word k of the injection's slot
+// in `saved`, so restore writes back exactly the words inject saved.  Footprints of one call are disjoint: no two CTAs
+// touch the same word.  The Gaussian is evaluated with explicit round-to-nearest operations (no FMA contraction), so a
+// host restatement in fp64 gives the same bits up to the last bit of exp.
+template <bool kRestore>
+__global__ void __launch_bounds__(kThreads) inject_kernel(uint32_t* __restrict__ img, long long row_stride,
+                                                          int big_endian, int row0, int ncols, int row_begin,
+                                                          int row_end, const cy_injection* __restrict__ inj, int rx,
+                                                          int ry, double ixx, double ixy2, double iyy,
+                                                          uint32_t* __restrict__ saved) {
+    const cy_injection q = inj[blockIdx.x];
+    const int fw = 2 * rx + 1, nfp = fw * (2 * ry + 1);
+    uint32_t* slot = saved + (long long)blockIdx.x * nfp;
+    for (int k = threadIdx.x; k < nfp; k += blockDim.x) {
+        const int x = q.cx - rx + k % fw, y = q.cy - ry + k / fw;
+        if (x < 0 || x >= ncols || y < row_begin || y >= row_end) continue;
+        uint32_t* p = img + (long long)(y - row0) * row_stride + x;
+        if (kRestore) {
+            *p = slot[k];
+            continue;
+        }
+        const uint32_t w = *p;
+        slot[k] = w;
+        const float v = __uint_as_float(big_endian ? __byte_perm(w, 0, 0x0123) : w);
+        if (!isfinite(v) || v == 0.0f) continue;                       // masked: the word stays
+        const double dx = __dsub_rn((double)x, q.x), dy = __dsub_rn((double)y, q.y);
+        const double quad = __dadd_rn(__dadd_rn(__dmul_rn(__dmul_rn(ixx, dx), dx), __dmul_rn(__dmul_rn(ixy2, dx), dy)),
+                                      __dmul_rn(__dmul_rn(iyy, dy), dy));
+        const float out = (float)__dadd_rn((double)v, __dmul_rn(q.peak, exp(__dmul_rn(-0.5, quad))));
+        *p = big_endian ? __byte_perm(__float_as_uint(out), 0, 0x0123) : __float_as_uint(out);
+    }
+}
+
+// bkg and rms map values at n region pixels (cy_bkg_grid_sample): map_pixel, so they are the maps' bits
+__global__ void bkg_sample_kernel(const cy_noise_state* __restrict__ state, Grid G, const int32_t* __restrict__ xy,
+                                  int n, float* __restrict__ bkg, float* __restrict__ rms) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int x = xy[2 * i], y = xy[2 * i + 1];
+    float fb = __int_as_float(0x7fc00000), fr = fb;
+    if (x >= 0 && x < G.ncols && y >= G.R0 && y < G.R1) map_pixel(state, G, x, y, fb, fr);
+    bkg[i] = fb;
+    rms[i] = fr;
+}
+
 }  // namespace
 
 extern "C" int cy_measure_sources(const void* img, long long row_stride, int big_endian, int row0, int ncols,
@@ -1431,5 +1478,58 @@ extern "C" int cy_bkg_grid_fill(const cy_noise_partial* probe_partials, int worl
     cudaFreeAsync(buf, st);
     if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_fill: %s", cudaGetErrorString(e));
     *filled = total;
+    return CY_OK;
+}
+
+static int inject_args(const char* fn, const void* img, long long row_stride, int row0, int ncols, int row_begin,
+                       int row_end, const cy_injection* inj, int ninj, int rx, int ry, const void* saved) {
+    if (ninj < 0 || ncols <= 0 || row_stride < ncols || row_begin < row0 || row_end < row_begin || rx < 0 || ry < 0 ||
+        (long long)(2 * rx + 1) * (2 * ry + 1) > 2147483647ll)
+        return set_error(CY_ERR_INVALID, "%s: invalid image geometry, row range, injection count or footprint", fn);
+    if (ninj > 0 && row_end > row_begin && (!img || !inj || !saved))
+        return set_error(CY_ERR_INVALID, "%s: null argument", fn);
+    return CY_OK;
+}
+
+extern "C" int cy_inject_sources(void* img, long long row_stride, int big_endian, int row0, int ncols, int row_begin,
+                                 int row_end, const cy_injection* inj, int ninj, int rx, int ry, double ixx, double ixy,
+                                 double iyy, uint32_t* saved, uintptr_t stream) {
+    if (int rc = inject_args("cy_inject_sources", img, row_stride, row0, ncols, row_begin, row_end, inj, ninj, rx, ry,
+                             saved))
+        return rc;
+    if (ninj == 0 || row_end == row_begin) return CY_OK;
+    inject_kernel<false><<<(unsigned)ninj, kThreads, 0, (cudaStream_t)stream>>>(
+        (uint32_t*)img, row_stride, big_endian, row0, ncols, row_begin, row_end, inj, rx, ry, ixx, 2.0 * ixy, iyy,
+        saved);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_inject_sources: %s", cudaGetErrorString(e));
+    return CY_OK;
+}
+
+extern "C" int cy_inject_restore(void* img, long long row_stride, int row0, int ncols, int row_begin, int row_end,
+                                 const cy_injection* inj, int ninj, int rx, int ry, const uint32_t* saved,
+                                 uintptr_t stream) {
+    if (int rc = inject_args("cy_inject_restore", img, row_stride, row0, ncols, row_begin, row_end, inj, ninj, rx, ry,
+                             saved))
+        return rc;
+    if (ninj == 0 || row_end == row_begin) return CY_OK;
+    inject_kernel<true><<<(unsigned)ninj, kThreads, 0, (cudaStream_t)stream>>>(
+        (uint32_t*)img, row_stride, 0, row0, ncols, row_begin, row_end, inj, rx, ry, 0.0, 0.0, 0.0,
+        (uint32_t*)saved);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_inject_restore: %s", cudaGetErrorString(e));
+    return CY_OK;
+}
+
+extern "C" int cy_bkg_grid_sample(const cy_noise_state* state, int ncols, int R0, int R1, int box, int grid,
+                                  const int32_t* xy, int n, float* bkg, float* rms, uintptr_t stream) {
+    Grid G;
+    if (n < 0 || !make_grid(ncols, R0, R1, R0, R1, box, grid, G))
+        return set_error(CY_ERR_INVALID, "cy_bkg_grid_sample: invalid region, box, grid or pixel count");
+    if (n == 0) return CY_OK;
+    if (!state || !xy || !bkg || !rms) return set_error(CY_ERR_INVALID, "cy_bkg_grid_sample: null argument");
+    bkg_sample_kernel<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(state, G, xy, n, bkg, rms);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_sample: %s", cudaGetErrorString(e));
     return CY_OK;
 }

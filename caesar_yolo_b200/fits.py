@@ -109,6 +109,29 @@ def beam_area_pix(h):
     return area / det
 
 
+def beam_cov_pix(h):
+    """Covariance (2x2, pixels^2) of the Gaussian restoring beam in pixel axes: C_sky = R diag(s_maj^2, s_min^2) R^T
+    with s = FWHM / (2 sqrt(2 ln 2)) of BMAJ / BMIN (degrees) and the major axis along (sin BPA, cos BPA) in the
+    intermediate world axes x = east, y = north (BPA: degrees east of north, 0 when absent); C_pix = M^-1 C_sky M^-T,
+    M = pixel_scale_matrix.  None when the beam cards or the pixel scale are missing or degenerate."""
+    m = pixel_scale_matrix(h)
+    if m is None or "BMAJ" not in h or "BMIN" not in h:
+        return None
+    k = 2.0 * np.sqrt(2.0 * np.log(2.0))
+    smaj, smin = float(h["BMAJ"]) / k, float(h["BMIN"]) / k
+    pa = np.radians(float(h.get("BPA", 0.0)))
+    u = np.array([np.sin(pa), np.cos(pa)])
+    v = np.array([np.cos(pa), -np.sin(pa)])
+    c_sky = smaj * smaj * np.outer(u, u) + smin * smin * np.outer(v, v)
+    det = float(np.linalg.det(m))
+    if not (smaj > 0 and smin > 0 and np.isfinite(smaj) and np.isfinite(smin) and det != 0 and np.isfinite(det)
+            and np.isfinite(pa)):
+        return None
+    mi = np.linalg.inv(m)
+    c = mi @ c_sky @ mi.T
+    return 0.5 * (c + c.T)
+
+
 def celestial_projection(h):
     """'SIN' or 'TAN' when CTYPE1/2 are RA---SIN / DEC--SIN or RA---TAN / DEC--TAN, else None."""
     t1, t2 = str(h.get("CTYPE1", "")).strip().upper(), str(h.get("CTYPE2", "")).strip().upper()

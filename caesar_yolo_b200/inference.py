@@ -5,6 +5,7 @@ Differences by design (B200-first): tiles are processed in batches on the GPU in
 tile; ranks are torch.distributed ranks (one per GPU) that own contiguous bands of tile rows instead of mpi4py
 round-robin workers; the gather is one NCCL all-gather of 32-byte records; the neighbour table and both merges are
 native/CUDA.  Catalog content and order equal the reference run with nproc=1."""
+import json
 import logging
 import os
 import time
@@ -12,7 +13,7 @@ import time
 import numpy as np
 import torch
 
-from . import catalog, fits as fitsmeta, ops
+from . import catalog, fits as fitsmeta, inject, ops
 from .fits import FitsImage
 from .pipeline import Engine, make_pp_config, run_image
 from .preprocessing import DataPreprocessor
@@ -33,6 +34,16 @@ def _as_sources(recs):
     for k in ('x1', 'y1', 'x2', 'y2', 'score', 'cls', 'flags', 'tile_id'):
         src[k] = recs[k]
     return src
+
+
+def check_inject_options(n, rounds, snr_range):
+    """Raises ValueError for an injection count < 0, rounds < 1 or an S/N range that is not (lo, hi), 0 < lo <= hi."""
+    if n < 0:
+        raise ValueError("inject_sources must be >= 0, not %d" % n)
+    if rounds < 1:
+        raise ValueError("inject_rounds must be >= 1, not %d" % rounds)
+    if len(snr_range) != 2 or not (0 < snr_range[0] <= snr_range[1]) or not np.isfinite(snr_range[1]):
+        raise ValueError("inject_snr_range must be (lo, hi) with 0 < lo <= hi, not %r" % (snr_range,))
 
 
 class SFinder(object):
@@ -63,7 +74,13 @@ class SFinder(object):
         self.bkg_grid = int(config.get('bkg_grid', 25))
         # the catalog boxes masked out of the noise frames and the map nodes; only these two consumers use the mask
         self.bkg_mask_sources = bool(config.get('bkg_mask_sources', False))
-        if self.bkg_mask_sources and not (self.measure_noise or self.save_bkg_maps):
+        # completeness by injection and recovery: the injected S/N is set by the rms map of the same options
+        self.inject_sources = int(config.get('inject_sources', 0))
+        self.inject_rounds = int(config.get('inject_rounds', 1))
+        self.inject_snr_range = tuple(float(v) for v in config.get('inject_snr_range', (3.0, 100.0)))
+        self.inject_seed = int(config.get('inject_seed', 0))
+        check_inject_options(self.inject_sources, self.inject_rounds, self.inject_snr_range)
+        if self.bkg_mask_sources and not (self.measure_noise or self.save_bkg_maps or self.inject_sources):
             logger.warning("bkg_mask_sources masks the catalog boxes out of the measure_noise frames and the "
                            "save_bkg_maps nodes: with neither option on it changes nothing")
             self.bkg_mask_sources = False
@@ -72,7 +89,7 @@ class SFinder(object):
         if self.bkg_estimator not in ops.BKG_ESTIMATORS:
             raise ValueError("bkg_estimator must be one of %s, not %r" % (", ".join(ops.BKG_ESTIMATORS),
                                                                           self.bkg_estimator))
-        if self.bkg_estimator != 'mean' and not (self.measure_noise or self.save_bkg_maps):
+        if self.bkg_estimator != 'mean' and not (self.measure_noise or self.save_bkg_maps or self.inject_sources):
             logger.warning("bkg_estimator sets the centre of the measure_noise and save_bkg_maps clipping: with neither "
                            "option on it changes nothing")
             self.bkg_estimator = 'mean'
@@ -201,6 +218,9 @@ class SFinder(object):
             x0, x1, y0, y1 = c['image_xmin'], c['image_xmax'], c['image_ymin'], c['image_ymax']
             if min(x0, x1, y0, y1) < 0 or x1 <= x0 or y1 <= y0:
                 return -1
+        cov = self._inject_beam()
+        if cov is False:
+            return -1
         eng = self._engine()
         tiles = np.zeros(1, dtype=ops.TILE_DTYPE)
         tiles[0] = (x0, x1, y0, y1)
@@ -240,7 +260,86 @@ class SFinder(object):
                 res, snr = eng.snr_maps(nodes, *args)
                 self._write_maps('snr_maps_write_s', (('resmap_', res, True), ('snrmap_', snr, False)), 0, region)
         self.timing['run_s'] = time.time() - t0
-        return self._save_serial(recs, status, meas)
+        status = self._save_serial(recs, status, meas)
+        if cov is not None:   # after every other output: the rounds change none of them
+            t1 = time.time()
+            if not self.save_bkg_maps:
+                args = (dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0, 0, y1 - y0,
+                        self.bkg_box, self.bkg_grid)
+                nodes, _, _ = eng.bkg_maps(*args, mask=mask, estimator=self.bkg_estimator, maps=False)
+            crop = np.zeros(1, dtype=ops.TILE_DTYPE)
+            crop[0] = (0, x1 - x0, 0, y1 - y0)
+
+            def rerun(ids):
+                if len(ids):
+                    eng.process_tiles(dev_img, self.fits.nx, self.fits.is_raw_f32, 0, y0, [0])
+
+            def merge():
+                p, _ = eng.finish()
+                r = p.cpu().numpy().view(ops.REC_DTYPE).copy()
+                r['x1'] -= x0; r['x2'] -= x0; r['y1'] -= y0; r['y2'] -= y0
+                return _as_sources(r)
+            plan = inject.Plan(region=(0, 0, x1 - x0, y1 - y0), catalog=_as_sources(recs), tiles=crop, my_tiles=(0, 1),
+                               target=(dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0),
+                               x_off=0, centre_masked=self._centre_masked(x0, y0),
+                               sample_rms=lambda cx, cy: eng.sample_bkg_maps(nodes, x1 - x0, 0, y1 - y0, self.bkg_box,
+                                                                             self.bkg_grid, cx, cy)[1],
+                               rerun=rerun, merge=merge)
+            self._inject_rounds(plan, cov)
+            self.timing['inject_s'] = time.time() - t1
+        return status
+
+    # ------------------------------------------------------------------------------------------------------
+    def _inject_beam(self):
+        """C_pix of the beam when the run injects sources (fits.beam_cov_pix), None when it does not, False (after
+        logging an error) when the header has no beam or pixel scale.  PNG / JPG input and a foreign preprocess_fcn
+        (it reads its tiles from the file, so it would not see the injection) log one warning and inject nothing."""
+        if not self.inject_sources:
+            return None
+        if self.fits is None:
+            logger.warning("Source injection needs a FITS image: no injection into %s", self.config['image_path'])
+            return None
+        if self._host_callable() is not None:
+            logger.warning("Source injection needs the CUDA preprocessing chain (a foreign preprocess_fcn reads its "
+                           "tiles from the file and would not see the injected sources): no injection")
+            return None
+        cov = fitsmeta.beam_cov_pix(self.fits.header)
+        if cov is None:
+            logger.error("Source injection needs the beam (BMAJ, BMIN) and the pixel scale (CDELT or CD) in the image "
+                         "header")
+            return False
+        return cov
+
+    def _centre_masked(self, x0, y0):
+        """centre_masked(cx, cy) of the injection placement: pixel (cx + x0, cy + y0) of the file is 0 or
+        non-finite (decoded as the rows the run read)."""
+        def f(cx, cy):
+            v = np.asarray(self.fits.raw[np.asarray(cy) + y0, np.asarray(cx) + x0]).astype(np.float32)
+            if not self.fits.is_raw_f32:
+                v = v * np.float32(self.fits.bscale) + np.float32(self.fits.bzero)
+            return ~np.isfinite(v) | (v == 0)
+        return f
+
+    def _inject_rounds(self, plan, cov):
+        """inject.run_rounds on the plan; rank 0 writes inject_<image_id>.json.  The per-tile debug outputs are off
+        during the rounds."""
+        eng = self.engine
+        keep = eng.tile_status, eng.tile_img_sink
+        eng.tile_status, eng.tile_img_sink = None, None
+        try:
+            out = inject.run_rounds(eng, plan, self.inject_sources, self.inject_rounds, self.inject_snr_range,
+                                    self.inject_seed, cov, self.class_names, rank=self.procId)
+        finally:
+            eng.tile_status, eng.tile_img_sink = keep
+        if self.procId != 0:
+            return
+        params = {'seed': self.inject_seed, 'rounds': self.inject_rounds, 'n': self.inject_sources,
+                  'snr_range': list(self.inject_snr_range), 'cov_pix': [[float(v) for v in row] for row in cov],
+                  'footprint': list(inject.footprint_half(cov)), 'bkg_estimator': self.bkg_estimator,
+                  'bkg_mask_sources': self.bkg_mask_sources, 'bkg_box': self.bkg_box, 'bkg_grid': self.bkg_grid}
+        doc = inject.report(self.image_id, out[0], out[1], params)
+        with open(os.path.join(self.outdir, 'inject_' + str(self.image_id) + '.json'), 'w') as f:
+            json.dump(doc, f, indent=1)
 
     def _measurements(self, m, header, x0=0, y0=0, noise=None):
         """Engine.measure output -> catalog.measurement_dicts with flux (beam area of the header) and the sky position
@@ -322,6 +421,8 @@ class SFinder(object):
         packed, n = eng.finish()
         recs = packed.cpu().numpy().view(ops.REC_DTYPE).copy()
         meas = None
+        if self.inject_sources:
+            logger.warning("Source injection needs a FITS image: no injection into %s", c['image_path'])
         if self.save_bkg_maps:
             logger.warning("%s maps are written for FITS images only: none for %s",
                            "Background, rms, background-subtracted and S/N" if self.save_snr_maps
@@ -358,6 +459,9 @@ class SFinder(object):
             logger.error("Too many tasks per worker (%d > %d), increase --max_ntasks_per_worker or the GPU count",
                          ntasks_max, c['max_ntasks_per_worker'])
             return -1
+        cov = self._inject_beam()
+        if cov is False:
+            return -1
         eng = self._engine()
         img = self.fits   # raw big-endian float32 rows are read from the file into pinned staging (pipeline._RowSource)
         # per-tile debug files (inference.py:218-229): every rank writes the files of its own tiles
@@ -378,7 +482,7 @@ class SFinder(object):
                 catalog.write_tile_outputs(recs, tiles, np.arange(a, b), st, self.class_names, self.image_id,
                                            self.outdir, self.save_tile_json, self.save_tile_regions)
         # measurements and masked maps need the catalog on every rank (each measures or masks its own rows)
-        rank0_only = not (self.measure_sources or (self.save_bkg_maps and self.bkg_mask_sources))
+        rank0_only = not (self.measure_sources or (self.save_bkg_maps and self.bkg_mask_sources) or cov is not None)
         if self._host_callable() is not None:
             from .pipeline import split_tile_rows
             eng.begin(tiles)
@@ -421,6 +525,15 @@ class SFinder(object):
             self.sources = {"sources": catalog.sources_to_dicts(src, self.class_names, meas)}
             self.save()
             logger.info("Run completed in %d seconds", int(time.time() - t0))
+        if cov is not None:   # after every other output: the rounds change none of them
+            t1 = time.time()
+            if not self.save_bkg_maps:
+                nodes = eng.bkg_maps_band(tiles, self.bkg_box, self.bkg_grid, self.procId, self.nproc, mask=mask,
+                                          estimator=self.bkg_estimator, maps=False)[0]
+            plan = inject.tiled_plan(eng, tiles, src, nodes, self.bkg_box, self.bkg_grid, self._centre_masked(0, 0),
+                                     self.procId, self.nproc)
+            self._inject_rounds(plan, cov)
+            self.timing['inject_s'] = time.time() - t1
         return 0
 
     def save(self):

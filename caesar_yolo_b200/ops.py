@@ -561,5 +561,35 @@ def bkg_grid_snr_maps(state, img, row_stride, big_endian, row0, ncols, R0, R1, r
                                    c_int(grid), ptr(res), ptr(snr), cur_stream()))
 
 
+def bkg_grid_sample(state, ncols, R0, R1, box, grid, xy):
+    """cy_bkg_grid_sample: final node states (uint8 device tensor) and region pixels xy (int32 device tensor [n, 2] of
+    (region column, row)) -> (bkg, rms) float32 device tensors [n], the map values there to the bit (NaN outside)."""
+    n = int(xy.shape[0])
+    bkg = torch.empty((n,), dtype=torch.float32, device=xy.device)
+    rms = torch.empty_like(bkg)
+    check(lib.cy_bkg_grid_sample(ptr(state), c_int(ncols), c_int(R0), c_int(R1), c_int(box), c_int(grid), ptr(xy),
+                                 c_int(n), ptr(bkg), ptr(rms), cur_stream()))
+    return bkg, rms
+
+
+INJ_DTYPE = np.dtype([('x', '<f8'), ('y', '<f8'), ('peak', '<f8'), ('cx', '<i4'), ('cy', '<i4')])   # cy_injection
+
+
+def inject_sources(img, row_stride, big_endian, row0, ncols, row_begin, row_end, inj_dev, ninj, rx, ry, icov, saved):
+    """cy_inject_sources: the ninj injections inj_dev (uint8 device tensor of INJ_DTYPE records) added to rows
+    [row_begin, row_end) of img (layout as for measure_sources); icov = (ixx, ixy, iyy) of C_pix^-1; saved: int32
+    device tensor of >= ninj (2 rx + 1)(2 ry + 1) words that receives the original words."""
+    check(lib.cy_inject_sources(ptr(img), c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0), c_int(ncols),
+                                c_int(row_begin), c_int(row_end), ptr(inj_dev), c_int(ninj), c_int(rx), c_int(ry),
+                                c_double(icov[0]), c_double(icov[1]), c_double(icov[2]), ptr(saved), cur_stream()))
+
+
+def inject_restore(img, row_stride, row0, ncols, row_begin, row_end, inj_dev, ninj, rx, ry, saved):
+    """cy_inject_restore: the words inject_sources saved (same arguments) written back."""
+    check(lib.cy_inject_restore(ptr(img), c_i64(row_stride), c_int(row0), c_int(ncols), c_int(row_begin),
+                                c_int(row_end), ptr(inj_dev), c_int(ninj), c_int(rx), c_int(ry), ptr(saved),
+                                cur_stream()))
+
+
 def to_device_bytes(np_array, device):
     return torch.from_numpy(np_array.view(np.uint8).reshape(-1).copy()).to(device)

@@ -480,7 +480,7 @@ class Engine(object):
                                   estimator=estimator)
 
     def bkg_maps(self, img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box=101, grid=25, world=1,
-                 mask=None, mask_col0=0, estimator='mean'):
+                 mask=None, mask_col0=0, estimator='mean', maps=True):
         """Background and rms maps of the region of columns [0, ncols) of `img` and rows [R0, R1) (node lattice,
         statistic and interpolation: include/caesar_b200.h), over rows [row_begin, row_end) of `img` (arguments as for
         Engine.measure; cy_bkg_grid_init / cy_bkg_grid_pass / cy_noise_update / cy_bkg_grid_maps).  With world > 1 every
@@ -492,7 +492,8 @@ class Engine(object):
         holds their count.  Returns (nodes, bkg, rms): the final node states (ops.NOISE_DTYPE, shape [Ny, Nx]) and this
         range's map rows as int32 device tensors [row_end - row_begin, ncols] holding big-endian float32;
         self.bkg_passes holds the number of clipping passes run.  estimator: as for Engine.measure_noise, so the maps and
-        the per-source statistics of one run compare directly."""
+        the per-source statistics of one run compare directly.  maps=False: the node states alone (bkg = rms = None);
+        no map row is allocated or written."""
         _check_estimator('Engine.bkg_maps', estimator)
         nx, ny = len(ops.bkg_grid_nodes(ncols, grid)), len(ops.bkg_grid_nodes(R1 - R0, grid))
         nodes = nx * ny
@@ -544,22 +545,24 @@ class Engine(object):
                 self.bkg_holes_filled = ops.bkg_grid_fill(allp, world, nx, ny, state)
                 self.launches += 3 + (1 if world > 1 else 0) + 2
             self.launches += 1
-        bkg = torch.empty((row_end - row_begin, ncols), dtype=torch.int32, device=self.device)
-        rms = torch.empty_like(bkg)
-        ops.bkg_grid_maps(state, ncols, R0, R1, row_begin, row_end, box, grid, bkg, rms)
+        bkg = rms = None
+        if maps:
+            bkg = torch.empty((row_end - row_begin, ncols), dtype=torch.int32, device=self.device)
+            rms = torch.empty_like(bkg)
+            ops.bkg_grid_maps(state, ncols, R0, R1, row_begin, row_end, box, grid, bkg, rms)
         self._stage('bkg_maps', e)
-        self.launches += 3 + self.bkg_passes * (3 + (1 if world > 1 else 0)) + 1
+        self.launches += 3 + self.bkg_passes * (3 + (1 if world > 1 else 0)) + (1 if maps else 0)
         return state.cpu().numpy().view(ops.NOISE_DTYPE).reshape(ny, nx), bkg, rms
 
-    def bkg_maps_band(self, tiles, box=101, grid=25, rank=0, world=1, mask=None, estimator='mean'):
+    def bkg_maps_band(self, tiles, box=101, grid=25, rank=0, world=1, mask=None, estimator='mean', maps=True):
         """Engine.bkg_maps of the bounding box of the tile grid (columns [min xmin, max xmax), rows [min ymin,
         max ymax)) over the rows this rank owns (measure_rows), read from the band of mosaic rows the last run_image
         left in HBM.  mask: Engine.source_mask_band (image columns, so the region starts at its column X0), or None;
-        estimator as for Engine.bkg_maps.
+        estimator and maps as for Engine.bkg_maps.
         Returns (nodes, bkg, rms, (X0, R0, W, H), (row_begin, row_end))."""
         img, nx, big_endian, Y0, (X0, R0, W, H), (r0, r1) = self._map_band(tiles, rank, world)
         nodes, bkg, rms = self.bkg_maps(img, nx, big_endian, Y0, W, R0, R0 + H, r0, r1, box, grid, world, mask=mask,
-                                        mask_col0=X0, estimator=estimator)
+                                        mask_col0=X0, estimator=estimator, maps=maps)
         return nodes, bkg, rms, (X0, R0, W, H), (r0, r1)
 
     def _map_band(self, tiles, rank, world):
@@ -604,6 +607,55 @@ class Engine(object):
         img, nx, big_endian, Y0, (X0, R0, W, H), (r0, r1) = self._map_band(tiles, rank, world)
         res, snr = self.snr_maps(nodes, img, nx, big_endian, Y0, W, R0, R0 + H, r0, r1, box, grid)
         return res, snr, (X0, R0, W, H), (r0, r1)
+
+    def sample_bkg_maps(self, nodes, ncols, R0, R1, box, grid, x, y):
+        """The bkg and rms map values (float32 numpy arrays) at region pixels (x[k] region column, y[k] row) of the
+        lattice of Engine.bkg_maps(ncols, R0, R1, box, grid) with the final node states `nodes` it returned
+        (cy_bkg_grid_sample): the bits of the maps there, without writing a map row.  NaN outside the region."""
+        nodes = np.ascontiguousarray(nodes, dtype=ops.NOISE_DTYPE)
+        if nodes.size != len(ops.bkg_grid_nodes(ncols, grid)) * len(ops.bkg_grid_nodes(R1 - R0, grid)):
+            raise CaesarB200Error("Engine.sample_bkg_maps: %d node states for a lattice of %d x %d nodes"
+                                  % (nodes.size, len(ops.bkg_grid_nodes(R1 - R0, grid)),
+                                     len(ops.bkg_grid_nodes(ncols, grid))))
+        xy = np.ascontiguousarray(np.stack([np.asarray(x, np.int32), np.asarray(y, np.int32)], axis=1))
+        e = self._mark()
+        bkg, rms = ops.bkg_grid_sample(ops.to_device_bytes(nodes, self.device), ncols, R0, R1, box, grid,
+                                       torch.from_numpy(xy).to(self.device))
+        self._stage('bkg_sample', e)
+        self.launches += 1
+        return bkg.cpu().numpy(), rms.cpu().numpy()
+
+    def inject(self, img, row_stride, big_endian, row0, ncols, row_begin, row_end, inj, rx, ry, icov):
+        """Adds the injections `inj` (numpy ops.INJ_DTYPE, disjoint footprints of half sizes rx, ry) to rows
+        [row_begin, row_end) of `img` (arguments as for Engine.measure; cy_inject_sources); icov: (ixx, ixy, iyy) of
+        C_pix^-1.  Returns the handle Engine.restore takes to put the original words back."""
+        inj = np.ascontiguousarray(inj, dtype=ops.INJ_DTYPE)
+        n = len(inj)
+        inj_dev = ops.to_device_bytes(inj, self.device) if n else None
+        saved = self._get('inj_saved', (max(n, 1) * (2 * rx + 1) * (2 * ry + 1),), torch.int32)
+        e = self._mark()
+        ops.inject_sources(img, row_stride, big_endian, row0, ncols, row_begin, row_end, inj_dev, n, rx, ry, icov,
+                           saved)
+        self._stage('inject', e)
+        self.launches += 1 if n else 0
+        return (img, row_stride, row0, ncols, row_begin, row_end, inj_dev, n, rx, ry, saved)
+
+    def restore(self, handle):
+        """Writes back the words Engine.inject saved (cy_inject_restore): the rows are bit-identical to before."""
+        e = self._mark()
+        ops.inject_restore(*handle)
+        self._stage('restore', e)
+        self.launches += 1 if handle[7] else 0
+
+    def snapshot_records(self):
+        """Copies of the per-tile record slots and counts, which Engine.restore_records puts back: a rerun of some
+        tiles through process_tiles overwrites their slots only, so the snapshot undoes it."""
+        return self.rec_slots.clone(), self.nrec.clone()
+
+    def restore_records(self, snap):
+        self.rec_slots.copy_(snap[0])
+        self.nrec.copy_(snap[1])
+        self.launches += 2
 
     def _exchange_cap(self, world, need=0):
         """Records per rank slot of the all-gather: 48 per tile of the largest band (the catalogs of the synthetic

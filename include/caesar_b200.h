@@ -481,6 +481,42 @@ int cy_bkg_grid_maps(const cy_noise_state* state, int ncols, int R0, int R1, int
 int cy_bkg_grid_snr_maps(const cy_noise_state* state, const void* img, long long row_stride, int big_endian, int row0,
                          int ncols, int R0, int R1, int row_begin, int row_end, int box, int grid, void* res, void* snr,
                          uintptr_t stream);
+/* Final node states -> the bkg and rms map values at n region pixels xy[2 k] = x (region column), xy[2 k + 1] = y
+ * (row, R0 <= y < R1), bit for bit the float32 values cy_bkg_grid_maps writes there (native byte order); a pixel
+ * outside the region gives NaN.  The arguments as for cy_bkg_grid_maps; no map row is written. */
+int cy_bkg_grid_sample(const cy_noise_state* state, int ncols, int R0, int R1, int box, int grid, const int32_t* xy,
+                       int n, float* bkg, float* rms, uintptr_t stream);
+
+/* Source injection (opt-in, inject_sources; not part of the reference): completeness by injection and recovery.
+ * Beam: C_sky = R diag(s_maj^2, s_min^2) R^T, s = FWHM / (2 sqrt(2 ln 2)) of BMAJ / BMIN (degrees), the major axis
+ *   along (sin BPA, cos BPA) in intermediate world axes (x = east, y = north; BPA 0 when absent); C_pix = M^-1 C_sky
+ *   M^-T, M the pixel scale matrix (CD, or CDELT with PC or CROTA2).  The host passes C_pix^-1 = [[ixx, ixy], [ixy, iyy]].
+ * Injection k: centre (x_k, y_k) in fp64 pixels of the buffer's frame, peak A_k, (c_x, c_y) = (floor(x_k + 1/2),
+ *   floor(y_k + 1/2)).  Footprint: [c_x - rx, c_x + rx] x [c_y - ry, c_y + ry], rx = ceil(4 sqrt(C_xx)), ry = ceil(4
+ *   sqrt(C_yy)).  A footprint pixel (x, y) with word w decodes to v as for the noise statistics (byte order applied;
+ *   non-finite and 0 are masked).  A masked pixel keeps w; otherwise it becomes, in the buffer's byte order,
+ *     (float)((double)v + A_k exp(-0.5 q)),  q = (ixx dx) dx + ((2 ixy) dx) dy + (iyy dy) dy,
+ *   dx = x - x_k, dy = y - y_k, every operation rounded to nearest in fp64 in this order (no fused multiply-add).
+ * S/N: snr_k log-uniform in [lo, hi], A_k = snr_k rms_k, rms_k the float32 rms map value at (c_x, c_y)
+ *   (cy_bkg_grid_sample of the node states of the bkg / rms maps, same options).
+ * Placement (host): uniform candidates over the map region, rejected when the footprint leaves the region, the centre
+ *   pixel is masked, rms_k is NaN or <= 0, the footprint meets the integer box of a catalog source or a footprint
+ *   already placed in the round; at most 20 N candidates per round.  Footprints of a round are disjoint. */
+typedef struct {
+    double x, y;                       /* centre, fp64 pixels of the buffer's frame (x: buffer column, y: image row) */
+    double peak;                       /* A_k, in the image's unit */
+    int32_t cx, cy;                    /* floor(x + 1/2), floor(y + 1/2) */
+} cy_injection;
+/* Adds the ninj injections inj[] (device) over rows [row_begin, row_end) of img (layout and row0 as for
+ * cy_measure_sources; columns [0, ncols)): one CTA per injection over its footprint cut by the columns and rows.  Each
+ * word of the cut footprint is first saved to saved[k (2 rx + 1)(2 ry + 1) + (y - c_y + ry)(2 rx + 1) + x - c_x + rx]
+ * (device, ninj (2 rx + 1)(2 ry + 1) words), then written as above.  The footprints must be disjoint. */
+int cy_inject_sources(void* img, long long row_stride, int big_endian, int row0, int ncols, int row_begin, int row_end,
+                      const cy_injection* inj, int ninj, int rx, int ry, double ixx, double ixy, double iyy,
+                      uint32_t* saved, uintptr_t stream);
+/* Scatters the words cy_inject_sources saved (same img, rows, inj, rx, ry) back: the rows are bit-identical to before. */
+int cy_inject_restore(void* img, long long row_stride, int row0, int ncols, int row_begin, int row_end,
+                      const cy_injection* inj, int ninj, int rx, int ry, const uint32_t* saved, uintptr_t stream);
 
 /* ------------------------------------------------------------------------------------------------ whole path
  * FITS file -> merged catalog with no host-language orchestration: SFinder.run_parallel (caesar_yolo/inference.py:

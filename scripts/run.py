@@ -90,6 +90,17 @@ def parse_args(argv=None):
     p.add_argument('--bkg_estimator', dest='bkg_estimator', type=str, default='mean', choices=['mean', 'median'],
                    help='B200 build only: centre of the --measure_noise and --save_bkg_maps sigma clipping (median: '
                         "astropy's sigma_clipped_stats default; bkg is the clipped median)")
+    p.add_argument('--inject_sources', dest='inject_sources', type=int, default=0,
+                   help='B200 build only: estimate the catalog completeness of a FITS image by injecting this many '
+                        'beam-shaped point sources per round at empty positions and detecting them again '
+                        '(inject_<id>.json; 0: off)')
+    p.add_argument('--inject_rounds', dest='inject_rounds', type=int, default=1,
+                   help='B200 build only: rounds of --inject_sources, each from the original image')
+    p.add_argument('--inject_snr_range', dest='inject_snr_range', type=str, default='3,100',
+                   help='B200 build only: lo,hi (0 < lo <= hi) of the log-uniform S/N of the injected sources, '
+                        'against the rms map of the --save_bkg_maps options')
+    p.add_argument('--inject_seed', dest='inject_seed', type=int, default=0,
+                   help='B200 build only: seed of the --inject_sources placement')
     p.add_argument('--detect_outfile', required=False, type=str, default="")
     p.add_argument('--detect_outfile_json', required=False, type=str, default="")
     args = p.parse_args(argv)
@@ -130,7 +141,28 @@ def validate_args(args):
     if args.bkg_estimator not in ('mean', 'median'):
         logger.error("Invalid bkg_estimator given (hint: give mean or median)!")
         return -1
+    if args.inject_sources < 0:
+        logger.error("Invalid inject_sources given (hint: give a count >= 0)!")
+        return -1
+    if args.inject_rounds < 1:
+        logger.error("Invalid inject_rounds given (hint: give a round count >= 1)!")
+        return -1
+    if parse_snr_range(args.inject_snr_range) is None:
+        logger.error("Invalid inject_snr_range given (hint: give lo,hi with 0 < lo <= hi)!")
+        return -1
     return 0
+
+
+def parse_snr_range(txt):
+    """'lo,hi' -> (lo, hi) with 0 < lo <= hi, both finite; None otherwise."""
+    parts = txt.split(',')
+    try:
+        lo, hi = (float(v) for v in parts) if len(parts) == 2 else (None, None)
+    except ValueError:
+        return None
+    if lo is None or not (0 < lo <= hi < float('inf')):
+        return None
+    return lo, hi
 
 
 def build_stages(args):
@@ -203,6 +235,8 @@ def main(argv=None):
         'measure_noise': args.measure_noise, 'noise_frame': args.noise_frame, 'save_bkg_maps': args.save_bkg_maps,
         'bkg_box': args.bkg_box, 'bkg_grid': args.bkg_grid, 'bkg_mask_sources': args.bkg_mask_sources,
         'bkg_estimator': args.bkg_estimator, 'save_snr_maps': args.save_snr_maps,
+        'inject_sources': args.inject_sources, 'inject_rounds': args.inject_rounds,
+        'inject_snr_range': parse_snr_range(args.inject_snr_range), 'inject_seed': args.inject_seed,
     })
     model = YOLO(args.weights, precision=args.precision)
     sfinder = SFinder(model, CONFIG)

@@ -29,6 +29,11 @@ the mean estimator the node sums are folded in another order over 2 ranks, so th
 may differ in the last bits: the tool then reports the largest difference in float32 ulps (within the 1 ulp of the --maps
 check, compounded by the division).
 
+With --inject, every rank also runs --inject_rounds rounds of --inject_n source injections (inject.run_rounds, the
+steps of SFinder with inject_sources, with --mask and --estimator as given) after a run over all ranks and after a
+single-rank run.  The placements must be identical; with --estimator median the whole result (every injection, its
+match and the per-round counts) must be; with the mean the node rms may differ in the last bits over another row split
+(see --snr), so the tool reports the largest relative difference of the peaks and how many matches differ.
 Prints one JSON line on rank 0 with the largest relative difference per field and the verdict of every rank."""
 import argparse
 import json
@@ -65,6 +70,39 @@ def compare(m, r):
     return out
 
 
+def inject_rounds(a, eng, host, tiles, rank, world):
+    """--inject: source-injection rounds of the run over `world` ranks and of the single-rank run (run_image, node
+    states of the maps, inject.run_rounds with --mask and --estimator).  On rank 0: the placements must be identical;
+    with the median estimator the whole result must be; with the mean the node rms may differ in the last bits over
+    another row split, so the largest peak difference and the injections whose match differs are reported."""
+    from caesar_yolo_b200 import fits, inject, pipeline
+    words = host.numpy().view(np.uint32)
+
+    def centre_masked(cx, cy):
+        v = words[cy, cx].byteswap().view(np.float32)
+        return ~np.isfinite(v) | (v == 0)
+    cov = fits.beam_cov_pix({"BMAJ": 0.0025, "BMIN": 0.002, "BPA": 30.0, "CDELT1": -0.0004, "CDELT2": 0.0004})
+    out = []
+    for r, w in ((rank, world), (0, 1)):
+        src, _ = pipeline.run_image(eng, host, True, tiles, rank=r, world=w, on_rank0_only=False)
+        mask = eng.source_mask_band(src, tiles, r, w) if a.mask else None
+        nodes = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, r, w, mask=mask, estimator=a.estimator, maps=False)[0]
+        plan = inject.tiled_plan(eng, tiles, src, nodes, a.bkg_box, a.bkg_grid, centre_masked, r, w)
+        out.append(inject.run_rounds(eng, plan, a.inject_n, a.inject_rounds, (3.0, 100.0), 0, cov, eng.names,
+                                     rank=r))
+    if rank != 0:
+        return None
+    (im, rm), (i1, r1) = out
+    key = ('round', 'x', 'y', 'snr')
+    same_place = [tuple(d[k] for k in key) for d in im] == [tuple(d[k] for k in key) for d in i1]
+    identical = json.dumps([im, rm]) == json.dumps([i1, r1])
+    peak = max([abs(p['peak'] - q['peak']) / max(abs(q['peak']), 1e-30) for p, q in zip(im, i1)] or [0.0])
+    differ = sum(1 for p, q in zip(im, i1) if (p['recovered'], p['source']) != (q['recovered'], q['source']))
+    return dict(injections=len(im), placements_identical=same_place, result_identical=identical,
+                max_rel_peak_diff=peak, matches_differing=differ, rounds=rm, single_rank_rounds=r1,
+                ok=bool(same_place and (a.estimator == 'mean' or identical)))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--mosaic', type=int, default=16384)
@@ -81,6 +119,9 @@ def main():
     ap.add_argument('--estimator', default='mean', choices=['mean', 'median'],
                     help='centre of the --noise, --maps and --snr clipping')
     ap.add_argument('--snr', action='store_true', help='also compare the background-subtracted and S/N maps')
+    ap.add_argument('--inject', action='store_true', help='also compare source-injection rounds')
+    ap.add_argument('--inject_n', type=int, default=1024)
+    ap.add_argument('--inject_rounds', type=int, default=2)
     a = ap.parse_args()
     import torch
     import torch.distributed as dist
@@ -189,6 +230,10 @@ def main():
             ulp = float((np.abs(p[f] - q[f]) / np.spacing(np.abs(q[f]))).max()) if f.any() else 0.0
             snr_res[k + '_max_ulp'] = ulp if same_nan else float('inf')
         ok = ok and split_ok and (not same_nodes or (snr_res['res_identical'] and snr_res['snr_identical']))
+    inject_res = None
+    if a.inject:
+        inject_res = inject_rounds(a, eng, host, tiles, rank, world)
+        ok = ok and (rank != 0 or inject_res['ok'])
     flags = torch.tensor([1 if ok else 0], device=dev if a.backend == 'nccl' else 'cpu')
     dist.all_reduce(flags, op=dist.ReduceOp.MIN)
     if rank == 0:
@@ -196,7 +241,7 @@ def main():
                               sources=int(len(src)), rows_of_rank0=list(rows),
                               catalog_identical=same_catalog, max_rel_diff={k: res[k] for k in FLOATS},
                               exact={k: res[k + '_exact'] for k in EXACT}, rtol=a.rtol, estimator=a.estimator,
-                              noise=noise_res, maps=maps_res, snr=snr_res,
+                              noise=noise_res, maps=maps_res, snr=snr_res, inject=inject_res,
                               matches_single_rank_on_every_rank=bool(int(flags[0])))), flush=True)
     dist.destroy_process_group()
     return 0 if int(flags[0]) else 1
