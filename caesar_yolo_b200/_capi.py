@@ -125,7 +125,8 @@ SYMBOLS = [
     "cy_postprocess", "cy_nms_scratch_bytes", "cy_nms_batched", "cy_merge_tile", "cy_make_records",
     "cy_compact_scratch_bytes", "cy_compact_records", "cy_merge_global", "cy_measure_sources", "cy_measure_combine",
     "cy_noise_init", "cy_noise_pass", "cy_noise_update", "cy_bkg_grid_init", "cy_bkg_grid_pass", "cy_bkg_grid_maps",
-    "cy_bkg_grid_snr_maps", "cy_bkg_grid_sample", "cy_inject_sources", "cy_inject_restore",
+    "cy_bkg_grid_snr_maps", "cy_bkg_grid_sample", "cy_inject_sources", "cy_inject_restore", "cy_negate_rows",
+    "cy_source_peak_snr",
     "cy_source_mask", "cy_noise_pass_masked", "cy_bkg_grid_pass_masked", "cy_bkg_grid_probe_init", "cy_bkg_grid_fill",
     "cy_noise_pass_median", "cy_noise_pass_median_masked", "cy_bkg_grid_pass_median", "cy_bkg_grid_pass_median_masked",
     "cy_median_update",

@@ -69,4 +69,8 @@ CONFIG = {
     'inject_rounds': 1,
     'inject_snr_range': (3.0, 100.0),
     'inject_seed': 0,
+    # - Catalog reliability from the inverted image (not in the reference; FITS input): the catalog of -I, the peak S/N
+    #   of both catalogs against the S/N map of the save_bkg_maps options, tables over inject_snr_range and the score;
+    #   reliability_<id>.json (and .reg with save_region)
+    'reliability': False,
 }

@@ -863,9 +863,20 @@ __global__ void bkg_map_kernel(const cy_noise_state* __restrict__ state, Grid G,
     rms[o] = __byte_perm(__float_as_uint(fr), 0, 0x0123);
 }
 
+// res = v - bkg and snr = (v - bkg) / rms of one pixel, both in fp64 and rounded once.  NaN: a masked pixel (v NaN) or a
+// NaN bkg in both; a NaN or non-positive rms in snr only.  snr_map_kernel and peak_snr_kernel both take them from here.
+__device__ __forceinline__ void res_snr(float v, float fb, float fr, float& r, float& s) {
+    r = __int_as_float(0x7fc00000);
+    s = r;
+    if (!isnan(v) && !isnan(fb)) {
+        const double d = (double)v - (double)fb;
+        r = (float)d;
+        if (fr > 0.0f) s = (float)(d / (double)fr);   // false for NaN
+    }
+}
+
 // background-subtracted and S/N maps (cy_bkg_grid_snr_maps), the grid of bkg_map_kernel: each thread reads its image
-// pixel once (a warp reads 32 adjacent words of one row) and writes res = v - bkg and snr = (v - bkg) / rms, both in
-// fp64 and rounded once.  NaN: a masked pixel or a NaN bkg in both maps; a NaN or non-positive rms in snr only.
+// pixel once (a warp reads 32 adjacent words of one row) and writes res and snr (res_snr).
 __global__ void snr_map_kernel(const uint32_t* __restrict__ img, long long row_stride, int big_endian, int row0,
                                const cy_noise_state* __restrict__ state, Grid G, int row_begin,
                                uint32_t* __restrict__ res, uint32_t* __restrict__ snr) {
@@ -875,12 +886,8 @@ __global__ void snr_map_kernel(const uint32_t* __restrict__ img, long long row_s
     const float v = noise_pixel(img + (long long)(y - row0) * row_stride + x, big_endian);
     float fb, fr;
     map_pixel(state, G, x, y, fb, fr);
-    float r = __int_as_float(0x7fc00000), s = r;
-    if (!isnan(v) && !isnan(fb)) {
-        const double d = (double)v - (double)fb;
-        r = (float)d;
-        if (fr > 0.0f) s = (float)(d / (double)fr);   // false for NaN
-    }
+    float r, s;
+    res_snr(v, fb, fr, r, s);
     const long long o = (long long)blockIdx.x * G.ncols + x;
     res[o] = __byte_perm(__float_as_uint(r), 0, 0x0123);   // FITS byte order
     snr[o] = __byte_perm(__float_as_uint(s), 0, 0x0123);
@@ -1035,6 +1042,93 @@ __global__ void bkg_sample_kernel(const cy_noise_state* __restrict__ state, Grid
     if (x >= 0 && x < G.ncols && y >= G.R0 && y < G.R1) map_pixel(state, G, x, y, fb, fr);
     bkg[i] = fb;
     rms[i] = fr;
+}
+
+// ---------------------------------------------------------------------------------------------- reliability
+// The inverted image (cy_negate_rows) and the peak S/N of the catalog boxes (cy_source_peak_snr).
+
+// w with its sign flipped when it decodes to a finite non-zero value; masked words (0, -0, NaN, +-inf) stay
+__device__ __forceinline__ uint32_t negate_word(uint32_t w, int big_endian) {
+    const uint32_t mag = (big_endian ? __byte_perm(w, 0, 0x0123) : w) & 0x7fffffffu;
+    return (mag != 0u && mag < 0x7f800000u) ? w ^ (big_endian ? 0x80u : 0x80000000u) : w;
+}
+
+constexpr int kNegateUnroll = 4;   // 16-byte vectors in flight per thread
+
+// one CTA per row (blockIdx.x = row - row_begin) over words [0, ncols): a scalar head up to the row's first 16-byte
+// boundary, 16-byte vectors, a scalar tail.  Rows need not be aligned (a crop starts at any column), and no word at
+// column >= ncols is touched.
+__global__ void __launch_bounds__(kThreads) negate_kernel(uint32_t* __restrict__ img, long long row_stride,
+                                                          int big_endian, int row0, int ncols, int row_begin) {
+    uint32_t* row = img + (long long)(row_begin + (int)blockIdx.x - row0) * row_stride;
+    const int head = min(ncols, (int)(((16u - ((uint32_t)(uintptr_t)row & 15u)) & 15u) >> 2));
+    const int nvec = (ncols - head) >> 2, tail = head + 4 * nvec;
+    const int t = threadIdx.x;
+    if (t < head) row[t] = negate_word(row[t], big_endian);
+    if (tail + t < ncols) row[tail + t] = negate_word(row[tail + t], big_endian);
+    uint4* v = reinterpret_cast<uint4*>(row + head);
+    for (int i0 = 0; i0 < nvec; i0 += kNegateUnroll * kThreads) {
+        uint4 q[kNegateUnroll];
+#pragma unroll
+        for (int k = 0; k < kNegateUnroll; ++k) {
+            const int i = i0 + k * kThreads + t;
+            if (i < nvec) q[k] = v[i];
+        }
+#pragma unroll
+        for (int k = 0; k < kNegateUnroll; ++k) {
+            const int i = i0 + k * kThreads + t;
+            if (i >= nvec) continue;
+            q[k].x = negate_word(q[k].x, big_endian);
+            q[k].y = negate_word(q[k].y, big_endian);
+            q[k].z = negate_word(q[k].z, big_endian);
+            q[k].w = negate_word(q[k].w, big_endian);
+            v[i] = q[k];
+        }
+    }
+}
+
+// one CTA per unit of measure_units_scan_kernel (grow 0, catalog columns [0, ncols + col_off)): every pixel of the
+// unit's rows of the box that lies in the region (region column = catalog column - col_off) gets the snr of
+// snr_map_kernel.  The largest sign * snr wins, ties to the lowest row-major region index: the key (float_key of the
+// value, with -0 read as +0) << 32 | ~index is folded by max, within the CTA and by a 64-bit atomicMax across units,
+// which gives the same bits in any order.  0 (no key is 0) means no pixel.
+__global__ void __launch_bounds__(kThreads) peak_snr_kernel(const uint32_t* __restrict__ img, long long row_stride,
+                                                            int big_endian, int row0,
+                                                            const cy_noise_state* __restrict__ state, Grid G,
+                                                            int col_off, const cy_source* __restrict__ src, int nsrc,
+                                                            int negative, int row_begin, int row_end,
+                                                            const long long* __restrict__ off,
+                                                            unsigned long long* __restrict__ peaks) {
+    const long long u = blockIdx.x;
+    const int s = unit_source(off, nsrc, u);
+    Box b;
+    source_box(src[s], 0, G.ncols + col_off, row_begin, row_end, b);
+    const int ya = b.y0 + (int)(u - off[s]) * kUnitRows;
+    const int yb = min(b.y1, ya + kUnitRows - 1);
+    const int xa = max(b.x0, col_off) - col_off, xb = b.x1 - col_off;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    unsigned long long best = 0;
+    for (int y = ya + w; y <= yb; y += kThreads / 32) {
+        const uint32_t* row = img + (long long)(y - row0) * row_stride;
+        const uint32_t base = (uint32_t)(y - G.R0) * (uint32_t)G.ncols;   // < 2^32: checked by the entry
+        for (int x = xa + lane; x <= xb; x += 32) {
+            const float v = noise_pixel(row + x, big_endian);
+            if (isnan(v)) continue;                         // masked: snr is NaN
+            float fb, fr, r, q;
+            map_pixel(state, G, x, y, fb, fr);
+            res_snr(v, fb, fr, r, q);
+            if (isnan(q)) continue;
+            uint32_t bits = __float_as_uint(q) ^ (negative ? 0x80000000u : 0u);
+            if ((bits & 0x7fffffffu) == 0u) bits = 0u;
+            const unsigned long long key = ((unsigned long long)float_key(bits) << 32) | (0xffffffffu - (base + x));
+            best = key > best ? key : best;
+        }
+    }
+    for (int d = 16; d > 0; d >>= 1) {
+        const unsigned long long o = __shfl_down_sync(0xffffffffu, best, d);
+        best = o > best ? o : best;
+    }
+    if (lane == 0 && best) atomicMax(peaks + s, best);
 }
 
 }  // namespace
@@ -1531,5 +1625,57 @@ extern "C" int cy_bkg_grid_sample(const cy_noise_state* state, int ncols, int R0
     bkg_sample_kernel<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(state, G, xy, n, bkg, rms);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_bkg_grid_sample: %s", cudaGetErrorString(e));
+    return CY_OK;
+}
+
+extern "C" int cy_negate_rows(void* img, long long row_stride, int big_endian, int row0, int ncols, int row_begin,
+                              int row_end, uintptr_t stream) {
+    if (ncols <= 0 || row_stride < ncols || row_begin < row0 || row_end < row_begin)
+        return set_error(CY_ERR_INVALID, "cy_negate_rows: invalid image geometry or row range");
+    if (row_end == row_begin) return CY_OK;
+    if (!img) return set_error(CY_ERR_INVALID, "cy_negate_rows: null argument");
+    if ((uintptr_t)img & 3u) return set_error(CY_ERR_INVALID, "cy_negate_rows: image not 4-byte aligned");
+    negate_kernel<<<(unsigned)(row_end - row_begin), kThreads, 0, (cudaStream_t)stream>>>(
+        (uint32_t*)img, row_stride, big_endian, row0, ncols, row_begin);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_negate_rows: %s", cudaGetErrorString(e));
+    return CY_OK;
+}
+
+extern "C" int cy_source_peak_snr(const cy_noise_state* state, int ncols, int R0, int R1, int box, int grid,
+                                  const void* img, long long row_stride, int big_endian, int row0, int col_off,
+                                  const cy_source* src, int nsrc, int sign, int row_begin, int row_end,
+                                  unsigned long long* peaks, uintptr_t stream) {
+    Grid G;
+    if (nsrc < 0 || !make_grid(ncols, R0, R1, row_begin, row_end, box, grid, G) || row_stride < ncols ||
+        row_begin < row0 || col_off < 0 || (long long)ncols + col_off > 2147483647ll || (sign != 1 && sign != -1))
+        return set_error(CY_ERR_INVALID, "cy_source_peak_snr: invalid image geometry, region, row range, box, grid, "
+                                         "column offset, source count or sign");
+    if ((long long)ncols * (R1 - R0) > 4294967295ll)
+        return set_error(CY_ERR_INVALID, "cy_source_peak_snr: a region of %lld pixels (the index has 32 bits)",
+                         (long long)ncols * (R1 - R0));
+    if (nsrc == 0) return CY_OK;
+    if (!state || !src || !peaks || (row_end > row_begin && !img))
+        return set_error(CY_ERR_INVALID, "cy_source_peak_snr: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    CY_CUDA_CHECK(cudaMemsetAsync(peaks, 0, (size_t)nsrc * sizeof(unsigned long long), st));
+    if (row_end == row_begin) return CY_OK;
+    long long* off = nullptr;
+    CY_CUDA_CHECK(cudaMallocAsync(&off, (size_t)(nsrc + 1) * sizeof(long long), st));
+    measure_units_scan_kernel<<<1, kScanThreads, 0, st>>>(src, nsrc, 0, ncols + col_off, row_begin, row_end, off);
+    long long units = 0;   // the unit count is data dependent: bring it to the host
+    cudaMemcpyAsync(&units, off + nsrc, sizeof(long long), cudaMemcpyDeviceToHost, st);
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess && units > 2147483647ll) {
+        cudaFreeAsync(off, st);
+        return set_error(CY_ERR_INVALID, "cy_source_peak_snr: %lld work units exceed one grid", units);
+    }
+    if (e == cudaSuccess && units > 0)
+        peak_snr_kernel<<<(unsigned)units, kThreads, 0, st>>>((const uint32_t*)img, row_stride, big_endian, row0, state,
+                                                              G, col_off, src, nsrc, sign < 0, row_begin, row_end, off,
+                                                              peaks);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    cudaFreeAsync(off, st);
+    if (e != cudaSuccess) return set_error(CY_ERR_CUDA, "cy_source_peak_snr: %s", cudaGetErrorString(e));
     return CY_OK;
 }

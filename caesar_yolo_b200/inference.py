@@ -13,7 +13,7 @@ import time
 import numpy as np
 import torch
 
-from . import catalog, fits as fitsmeta, inject, ops
+from . import catalog, fits as fitsmeta, inject, ops, reliability
 from .fits import FitsImage
 from .pipeline import Engine, make_pp_config, run_image
 from .preprocessing import DataPreprocessor
@@ -80,7 +80,10 @@ class SFinder(object):
         self.inject_snr_range = tuple(float(v) for v in config.get('inject_snr_range', (3.0, 100.0)))
         self.inject_seed = int(config.get('inject_seed', 0))
         check_inject_options(self.inject_sources, self.inject_rounds, self.inject_snr_range)
-        if self.bkg_mask_sources and not (self.measure_noise or self.save_bkg_maps or self.inject_sources):
+        # reliability from the inverted image: the peak S/N of both catalogs is read from the S/N map of the same options
+        self.reliability = bool(config.get('reliability', False))
+        if self.bkg_mask_sources and not (self.measure_noise or self.save_bkg_maps or self.inject_sources or
+                                          self.reliability):
             logger.warning("bkg_mask_sources masks the catalog boxes out of the measure_noise frames and the "
                            "save_bkg_maps nodes: with neither option on it changes nothing")
             self.bkg_mask_sources = False
@@ -89,7 +92,8 @@ class SFinder(object):
         if self.bkg_estimator not in ops.BKG_ESTIMATORS:
             raise ValueError("bkg_estimator must be one of %s, not %r" % (", ".join(ops.BKG_ESTIMATORS),
                                                                           self.bkg_estimator))
-        if self.bkg_estimator != 'mean' and not (self.measure_noise or self.save_bkg_maps or self.inject_sources):
+        if self.bkg_estimator != 'mean' and not (self.measure_noise or self.save_bkg_maps or self.inject_sources or
+                                                 self.reliability):
             logger.warning("bkg_estimator sets the centre of the measure_noise and save_bkg_maps clipping: with neither "
                            "option on it changes nothing")
             self.bkg_estimator = 'mean'
@@ -221,6 +225,7 @@ class SFinder(object):
         cov = self._inject_beam()
         if cov is False:
             return -1
+        rel = self._reliability_on()
         eng = self._engine()
         tiles = np.zeros(1, dtype=ops.TILE_DTYPE)
         tiles[0] = (x0, x1, y0, y1)
@@ -249,44 +254,51 @@ class SFinder(object):
             noise = eng.measure_noise(*args, frame=self.noise_frame, mask=mask,
                                       estimator=self.bkg_estimator) if self.measure_noise else None
             meas = self._measurements(m, self.fits.header, x0, y0, noise)
-        if self.save_bkg_maps:   # the region read: the crop, columns from x0
-            args = (dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0, 0, y1 - y0,
-                    self.bkg_box, self.bkg_grid)
-            nodes, bkg, rms = eng.bkg_maps(*args, mask=mask, estimator=self.bkg_estimator)
+        nodes = None
+        # the map region: the crop read, columns from x0
+        margs = (None if dev_img is None else dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0,
+                 y1 - y0, 0, y1 - y0, self.bkg_box, self.bkg_grid)
+        if self.save_bkg_maps:
+            nodes, bkg, rms = eng.bkg_maps(*margs, mask=mask, estimator=self.bkg_estimator)
             region = (x0, y0, x1 - x0, y1 - y0)
             self._write_maps('bkg_maps_write_s', (('bkgmap_', bkg, True), ('rmsmap_', rms, True)), 0, region)
             del bkg, rms   # freed before res / snr are allocated: no more than two region maps at a time
             if self.save_snr_maps:
-                res, snr = eng.snr_maps(nodes, *args)
+                res, snr = eng.snr_maps(nodes, *margs)
                 self._write_maps('snr_maps_write_s', (('resmap_', res, True), ('snrmap_', snr, False)), 0, region)
         self.timing['run_s'] = time.time() - t0
         status = self._save_serial(recs, status, meas)
+        crop = np.zeros(1, dtype=ops.TILE_DTYPE)
+        crop[0] = (0, x1 - x0, 0, y1 - y0)
+
+        def rerun(ids):
+            if len(ids):
+                eng.process_tiles(dev_img, self.fits.nx, self.fits.is_raw_f32, 0, y0, [0])
+
+        def merge():
+            p, _ = eng.finish()
+            r = p.cpu().numpy().view(ops.REC_DTYPE).copy()
+            r['x1'] -= x0; r['x2'] -= x0; r['y1'] -= y0; r['y2'] -= y0
+            return _as_sources(r)
         if cov is not None:   # after every other output: the rounds change none of them
             t1 = time.time()
-            if not self.save_bkg_maps:
-                args = (dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0, 0, y1 - y0,
-                        self.bkg_box, self.bkg_grid)
-                nodes, _, _ = eng.bkg_maps(*args, mask=mask, estimator=self.bkg_estimator, maps=False)
-            crop = np.zeros(1, dtype=ops.TILE_DTYPE)
-            crop[0] = (0, x1 - x0, 0, y1 - y0)
-
-            def rerun(ids):
-                if len(ids):
-                    eng.process_tiles(dev_img, self.fits.nx, self.fits.is_raw_f32, 0, y0, [0])
-
-            def merge():
-                p, _ = eng.finish()
-                r = p.cpu().numpy().view(ops.REC_DTYPE).copy()
-                r['x1'] -= x0; r['x2'] -= x0; r['y1'] -= y0; r['y2'] -= y0
-                return _as_sources(r)
+            if nodes is None:
+                nodes, _, _ = eng.bkg_maps(*margs, mask=mask, estimator=self.bkg_estimator, maps=False)
             plan = inject.Plan(region=(0, 0, x1 - x0, y1 - y0), catalog=_as_sources(recs), tiles=crop, my_tiles=(0, 1),
-                               target=(dev_img[:, x0:], self.fits.nx, self.fits.is_raw_f32, 0, x1 - x0, 0, y1 - y0),
-                               x_off=0, centre_masked=self._centre_masked(x0, y0),
+                               target=margs[:7], x_off=0, centre_masked=self._centre_masked(x0, y0),
                                sample_rms=lambda cx, cy: eng.sample_bkg_maps(nodes, x1 - x0, 0, y1 - y0, self.bkg_box,
                                                                              self.bkg_grid, cx, cy)[1],
                                rerun=rerun, merge=merge)
             self._inject_rounds(plan, cov)
             self.timing['inject_s'] = time.time() - t1
+        if rel:   # after every other output, the injection included: it changes none of them
+            t1 = time.time()
+            if nodes is None:
+                nodes, _, _ = eng.bkg_maps(*margs, mask=mask, estimator=self.bkg_estimator, maps=False)
+            plan = inject.Plan(catalog=_as_sources(recs), tiles=crop, my_tiles=(0, 1), target=margs[:7], rerun=rerun,
+                               merge=merge, peak_snr=lambda src, sign: eng.peak_snr(nodes, src, *margs, sign=sign))
+            self._reliability(plan, merged_key=False)
+            self.timing['reliability_s'] = time.time() - t1
         return status
 
     # ------------------------------------------------------------------------------------------------------
@@ -340,6 +352,44 @@ class SFinder(object):
         doc = inject.report(self.image_id, out[0], out[1], params)
         with open(os.path.join(self.outdir, 'inject_' + str(self.image_id) + '.json'), 'w') as f:
             json.dump(doc, f, indent=1)
+
+    def _reliability_on(self):
+        """True when the run estimates the reliability.  PNG / JPG input and a foreign preprocess_fcn (it reads its
+        tiles from the file, so it would not see the negated rows) log one warning and estimate nothing."""
+        if not self.reliability:
+            return False
+        if self.fits is None:
+            logger.warning("The reliability estimate needs a FITS image: none for %s", self.config['image_path'])
+            return False
+        if self._host_callable() is not None:
+            logger.warning("The reliability estimate needs the CUDA preprocessing chain (a foreign preprocess_fcn reads "
+                           "its tiles from the file and would not see the inverted image): none")
+            return False
+        return True
+
+    def _reliability(self, plan, merged_key):
+        """reliability.run on the plan; rank 0 writes reliability_<image_id>.json and, with save_region,
+        reliability_<image_id>.reg (the negative detections).  The per-tile debug outputs are off during the rerun."""
+        eng = self.engine
+        keep = eng.tile_status, eng.tile_img_sink
+        eng.tile_status, eng.tile_img_sink = None, None
+        try:
+            neg, pos_peak, neg_peak = reliability.run(eng, plan)
+        finally:
+            eng.tile_status, eng.tile_img_sink = keep
+        if self.procId != 0:
+            return
+        params = {'snr_range': list(self.inject_snr_range), 'score_thr': float(self.config['score_thr']),
+                  'bkg_estimator': self.bkg_estimator, 'bkg_mask_sources': self.bkg_mask_sources,
+                  'bkg_box': self.bkg_box, 'bkg_grid': self.bkg_grid}
+        doc = reliability.report(self.image_id, plan.catalog, neg, pos_peak, neg_peak, self.class_names, params,
+                                 len(plan.tiles))
+        with open(os.path.join(self.outdir, 'reliability_' + str(self.image_id) + '.json'), 'w') as f:
+            json.dump(doc, f, indent=1)
+        if self.write_to_ds9:
+            catalog.write_ds9(doc['negative_detections'],
+                              os.path.join(self.outdir, 'reliability_' + str(self.image_id) + '.reg'),
+                              merged_key=merged_key)
 
     def _measurements(self, m, header, x0=0, y0=0, noise=None):
         """Engine.measure output -> catalog.measurement_dicts with flux (beam area of the header) and the sky position
@@ -423,6 +473,7 @@ class SFinder(object):
         meas = None
         if self.inject_sources:
             logger.warning("Source injection needs a FITS image: no injection into %s", c['image_path'])
+        self._reliability_on()
         if self.save_bkg_maps:
             logger.warning("%s maps are written for FITS images only: none for %s",
                            "Background, rms, background-subtracted and S/N" if self.save_snr_maps
@@ -462,6 +513,7 @@ class SFinder(object):
         cov = self._inject_beam()
         if cov is False:
             return -1
+        rel = self._reliability_on()
         eng = self._engine()
         img = self.fits   # raw big-endian float32 rows are read from the file into pinned staging (pipeline._RowSource)
         # per-tile debug files (inference.py:218-229): every rank writes the files of its own tiles
@@ -481,8 +533,10 @@ class SFinder(object):
                 st = eng.tile_status[a:b].cpu().numpy()
                 catalog.write_tile_outputs(recs, tiles, np.arange(a, b), st, self.class_names, self.image_id,
                                            self.outdir, self.save_tile_json, self.save_tile_regions)
-        # measurements and masked maps need the catalog on every rank (each measures or masks its own rows)
-        rank0_only = not (self.measure_sources or (self.save_bkg_maps and self.bkg_mask_sources) or cov is not None)
+        # measurements, masked maps, injection and reliability need the catalog on every rank (each measures or masks
+        # its own rows)
+        rank0_only = not (self.measure_sources or (self.save_bkg_maps and self.bkg_mask_sources) or cov is not None or
+                          rel)
         if self._host_callable() is not None:
             from .pipeline import split_tile_rows
             eng.begin(tiles)
@@ -500,6 +554,7 @@ class SFinder(object):
             src, n = run_image(eng, img, self.fits.is_raw_f32, tiles, rank=self.procId, world=self.nproc,
                                on_rank0_only=rank0_only, on_local_records=hook)
         meas = None
+        nodes = None
         # one mask of the catalog boxes over this rank's rows, for the frames and the map nodes alike
         mask = eng.source_mask_band(src, tiles, self.procId, self.nproc) if self.bkg_mask_sources else None
         if self.measure_sources:
@@ -527,13 +582,21 @@ class SFinder(object):
             logger.info("Run completed in %d seconds", int(time.time() - t0))
         if cov is not None:   # after every other output: the rounds change none of them
             t1 = time.time()
-            if not self.save_bkg_maps:
+            if nodes is None:
                 nodes = eng.bkg_maps_band(tiles, self.bkg_box, self.bkg_grid, self.procId, self.nproc, mask=mask,
                                           estimator=self.bkg_estimator, maps=False)[0]
             plan = inject.tiled_plan(eng, tiles, src, nodes, self.bkg_box, self.bkg_grid, self._centre_masked(0, 0),
                                      self.procId, self.nproc)
             self._inject_rounds(plan, cov)
             self.timing['inject_s'] = time.time() - t1
+        if rel:   # after every other output, the injection included: it changes none of them
+            t1 = time.time()
+            if nodes is None:
+                nodes = eng.bkg_maps_band(tiles, self.bkg_box, self.bkg_grid, self.procId, self.nproc, mask=mask,
+                                          estimator=self.bkg_estimator, maps=False)[0]
+            plan = reliability.tiled_plan(eng, tiles, src, nodes, self.bkg_box, self.bkg_grid, self.procId, self.nproc)
+            self._reliability(plan, merged_key=True)
+            self.timing['reliability_s'] = time.time() - t1
         return 0
 
     def save(self):

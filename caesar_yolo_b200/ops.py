@@ -591,5 +591,39 @@ def inject_restore(img, row_stride, row0, ncols, row_begin, row_end, inj_dev, ni
                                 cur_stream()))
 
 
+def negate_rows(img, row_stride, big_endian, row0, ncols, row_begin, row_end):
+    """cy_negate_rows: the sign of every finite non-zero pixel of columns [0, ncols) of rows [row_begin, row_end) of img
+    (layout as for measure_sources) flipped in place; masked words keep their bits."""
+    check(lib.cy_negate_rows(ptr(img), c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0), c_int(ncols),
+                             c_int(row_begin), c_int(row_end), cur_stream()))
+
+
+def source_peak_snr(state, ncols, R0, R1, box, grid, img, row_stride, big_endian, row0, col_off, src_dev, nsrc, sign,
+                    row_begin, row_end, out):
+    """cy_source_peak_snr: peak S/N keys of the nsrc sources src_dev (uint8 device tensor of SRC_DTYPE records) over
+    rows [row_begin, row_end) of the region of bkg_grid_snr_maps, region column = catalog column - col_off -> out
+    (int64 device tensor [nsrc], holding the unsigned keys; decode with peak_snr_decode after an unsigned max fold)."""
+    check(lib.cy_source_peak_snr(ptr(state), c_int(ncols), c_int(R0), c_int(R1), c_int(box), c_int(grid), ptr(img),
+                                 c_i64(row_stride), c_int(1 if big_endian else 0), c_int(row0), c_int(col_off),
+                                 ptr(src_dev), c_int(nsrc), c_int(sign), c_int(row_begin), c_int(row_end), ptr(out),
+                                 cur_stream()))
+    return out
+
+
+def peak_snr_decode(keys, ncols, R0, col_off=0):
+    """Folded keys of cy_source_peak_snr (uint64 numpy) -> (snr float32, x int64, y int64) in catalog coordinates;
+    NaN and -1 where the key is 0 (no pixel)."""
+    keys = np.asarray(keys, np.uint64)
+    hi = (keys >> np.uint64(32)).astype(np.uint32)
+    bits = np.where(hi & np.uint32(0x80000000), hi & np.uint32(0x7fffffff), ~hi).astype(np.uint32)
+    idx = (np.uint64(0xffffffff) - (keys & np.uint64(0xffffffff))).astype(np.int64)
+    none = keys == 0
+    snr = bits.view(np.float32).copy()
+    snr[none] = np.nan
+    x = np.where(none, -1, idx % ncols + col_off)
+    y = np.where(none, -1, idx // ncols + R0)
+    return snr, x, y
+
+
 def to_device_bytes(np_array, device):
     return torch.from_numpy(np_array.view(np.uint8).reshape(-1).copy()).to(device)

@@ -647,6 +647,56 @@ class Engine(object):
         self._stage('restore', e)
         self.launches += 1 if handle[7] else 0
 
+    def negate(self, img, row_stride, big_endian, row0, ncols, row_begin, row_end):
+        """Inverts rows [row_begin, row_end), columns [0, ncols) of `img` in place (arguments as for Engine.measure;
+        cy_negate_rows): every finite non-zero pixel changes sign, masked words stay.  A second call restores the rows
+        bit for bit."""
+        e = self._mark()
+        ops.negate_rows(img, row_stride, big_endian, row0, ncols, row_begin, row_end)
+        self._stage('negate', e)
+        self.launches += 1 if row_end > row_begin else 0
+
+    def peak_snr(self, nodes, sources, img, row_stride, big_endian, row0, ncols, R0, R1, row_begin, row_end, box=101,
+                 grid=25, col_off=0, sign=1, world=1):
+        """Peak S/N of the catalog `sources` (ops.SRC_DTYPE, sign +1) or of the negative catalog (sign -1) against the
+        S/N map of the region of Engine.snr_maps (the same arguments) with the final node states `nodes`, over rows
+        [row_begin, row_end) of `img` (definition: include/caesar_b200.h; cy_source_peak_snr).  Catalog column c is
+        region column c - col_off.  No map row is written.  With world > 1 every rank passes the same catalog and its
+        own rows; the partial keys are all-gathered in the group of the record exchange and folded by their maximum,
+        which is exact in any order.  Returns (snr float32, x, y int64 arrays): the value and its pixel in catalog
+        coordinates, NaN and -1 where no pixel qualifies."""
+        src = np.ascontiguousarray(sources, dtype=ops.SRC_DTYPE)
+        n = len(src)
+        nx, ny = len(ops.bkg_grid_nodes(ncols, grid)), len(ops.bkg_grid_nodes(R1 - R0, grid))
+        nodes = np.ascontiguousarray(nodes, dtype=ops.NOISE_DTYPE)
+        if nodes.size != nx * ny:
+            raise CaesarB200Error("Engine.peak_snr: %d node states for a lattice of %d x %d nodes"
+                                  % (nodes.size, ny, nx))
+        if n == 0:
+            return np.zeros(0, np.float32), np.zeros(0, np.int64), np.zeros(0, np.int64)
+        e = self._mark()
+        part = self._get('peak_part', (n,), torch.int64)
+        ops.source_peak_snr(ops.to_device_bytes(nodes, self.device), ncols, R0, R1, box, grid, img, row_stride,
+                            big_endian, row0, col_off, ops.to_device_bytes(src, self.device), n, sign, row_begin,
+                            row_end, part)
+        if world > 1:
+            import torch.distributed as dist
+            allp = self._get('peak_gather', (world * n,), torch.int64)
+            dist.all_gather_into_tensor(allp, part)
+        else:
+            allp = part
+        keys = allp.cpu().numpy().view(np.uint64).reshape(world, n).max(axis=0)
+        self._stage('peak_snr', e)
+        self.launches += 3 + (1 if world > 1 else 0)
+        return ops.peak_snr_decode(keys, ncols, R0, col_off)
+
+    def peak_snr_band(self, nodes, sources, tiles, box=101, grid=25, sign=1, rank=0, world=1):
+        """Engine.peak_snr over the region and rows of Engine.bkg_maps_band (this rank's rows, measure_rows, of the band
+        the last run_image left in HBM), from the node states it returned; the catalog in image coordinates."""
+        img, nx, big_endian, Y0, (X0, R0, W, H), (r0, r1) = self._map_band(tiles, rank, world)
+        return self.peak_snr(nodes, sources, img, nx, big_endian, Y0, W, R0, R0 + H, r0, r1, box, grid, col_off=X0,
+                             sign=sign, world=world)
+
     def snapshot_records(self):
         """Copies of the per-tile record slots and counts, which Engine.restore_records puts back: a rerun of some
         tiles through process_tiles overwrites their slots only, so the snapshot undoes it."""

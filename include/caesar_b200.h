@@ -518,6 +518,41 @@ int cy_inject_sources(void* img, long long row_stride, int big_endian, int row0,
 int cy_inject_restore(void* img, long long row_stride, int row0, int ncols, int row_begin, int row_end,
                       const cy_injection* inj, int ninj, int rx, int ry, const uint32_t* saved, uintptr_t stream);
 
+/* Reliability (opt-in, reliability; not part of the reference): the false detections the catalog holds, estimated by
+ * detecting sources in the inverted image.  Real sources are positive; noise and most artefacts are symmetric about 0.
+ * Negation: the inverted image is I with every word whose decoded value v (as for the noise statistics: byte order
+ *   applied, non-finite and 0 masked) is finite and non-zero replaced by -v, i.e. the float32 sign bit flipped in the
+ *   buffer's byte order.  Masked words (0, -0, NaN, +-inf) keep their bits, so both images have the same masks, and
+ *   negating twice restores the rows bit for bit.
+ * Negative catalog: the catalog a normal run of the same configuration gives on the inverted image.  A tile's records
+ *   depend on its own pixels only, so every tile of a rank detected again on the negated rows gives it byte for byte.
+ * Peak S/N of a source of sign s (+1: the catalog, -1: the negative catalog): the maximum of s snr(x, y) over the
+ *   pixels of its integer box [ceil x1, floor x2] x [ceil y1, floor y2] that lie in the map region and where snr is not
+ *   NaN; snr(x, y) = (float)(((double)v - fb) / fr) is the S/N map of cy_bkg_grid_snr_maps of this run's final node
+ *   states (the save_bkg_maps options).  -0 counts as +0; ties go to the first pixel in row-major order.  NaN, with no
+ *   position, when no pixel qualifies.  Both catalogs are measured against the noise of the original image.  Without
+ *   the source mask this is the S/N map of a run on the inverted image, bit for bit: the clipping with either
+ *   estimator, the hole fill and the interpolation are odd under negation in round-to-nearest arithmetic (bkg -> -bkg,
+ *   rms unchanged; a zero difference is +0 in both images).
+ * Tables (host): the completeness table's NBINS log-spaced bins over the injection S/N range [lo, hi]: n_pos, n_neg and
+ *   reliability = 1 - n_neg / n_pos (not clipped; null when n_pos = 0); the same counts for S/N >= each lower edge;
+ *   the counts below lo, above hi and NaN; the same cumulative table against the detection score at thresholds
+ *   score_thr + k (1 - score_thr) / 10, k = 0..9; the class counts of both catalogs. */
+/* Negates (as above) columns [0, ncols) of rows [row_begin, row_end) of img in place (layout and row0 as for
+ * cy_measure_sources; img 4-byte aligned).  No other word is touched. */
+int cy_negate_rows(void* img, long long row_stride, int big_endian, int row0, int ncols, int row_begin, int row_end,
+                   uintptr_t stream);
+/* Peak S/N partial of each of the nsrc sources src[] (device; catalog coordinates, sign = +1 or -1) over rows
+ * [row_begin, row_end) of the region of cy_bkg_grid_snr_maps (state, ncols, R0, R1, box, grid; img, row_stride,
+ * big_endian, row0 as there, img pointing at region column 0); region column = catalog column - col_off (col_off >= 0).
+ * peaks[k] (device) = 0 when no pixel of these rows qualifies, otherwise (float_key(bits of s snr) << 32) |
+ * (0xffffffff - ((y - R0) ncols + x)) of the winning pixel (x: region column), float_key as for the median select.
+ * The partials of any split of the rows (row ranges, ranks) fold to the same key by an unsigned maximum.  Refuses a
+ * region of 2^32 pixels or more. */
+int cy_source_peak_snr(const cy_noise_state* state, int ncols, int R0, int R1, int box, int grid, const void* img,
+                       long long row_stride, int big_endian, int row0, int col_off, const cy_source* src, int nsrc,
+                       int sign, int row_begin, int row_end, unsigned long long* peaks, uintptr_t stream);
+
 /* ------------------------------------------------------------------------------------------------ whole path
  * FITS file -> merged catalog with no host-language orchestration: SFinder.run_parallel (caesar_yolo/inference.py:
  * 578-658; the serial SFinder.run :485-552 is the tile_x <= 0 case: the whole region is one tile), TileTask.find_sources

@@ -101,6 +101,10 @@ def parse_args(argv=None):
                         'against the rms map of the --save_bkg_maps options')
     p.add_argument('--inject_seed', dest='inject_seed', type=int, default=0,
                    help='B200 build only: seed of the --inject_sources placement')
+    p.add_argument('--reliability', dest='reliability', action='store_true',
+                   help='B200 build only: estimate the catalog reliability of a FITS image by detecting sources in the '
+                        'inverted image (reliability_<id>.json; S/N bins of --inject_snr_range against the S/N map of '
+                        'the --save_bkg_maps options)')
     p.add_argument('--detect_outfile', required=False, type=str, default="")
     p.add_argument('--detect_outfile_json', required=False, type=str, default="")
     args = p.parse_args(argv)
@@ -237,6 +241,7 @@ def main(argv=None):
         'bkg_estimator': args.bkg_estimator, 'save_snr_maps': args.save_snr_maps,
         'inject_sources': args.inject_sources, 'inject_rounds': args.inject_rounds,
         'inject_snr_range': parse_snr_range(args.inject_snr_range), 'inject_seed': args.inject_seed,
+        'reliability': args.reliability,
     })
     model = YOLO(args.weights, precision=args.precision)
     sfinder = SFinder(model, CONFIG)

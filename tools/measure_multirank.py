@@ -34,6 +34,11 @@ steps of SFinder with inject_sources, with --mask and --estimator as given) afte
 single-rank run.  The placements must be identical; with --estimator median the whole result (every injection, its
 match and the per-round counts) must be; with the mean the node rms may differ in the last bits over another row split
 (see --snr), so the tool reports the largest relative difference of the peaks and how many matches differ.
+With --reliability, every rank also runs the reliability estimate (reliability.run, the steps of SFinder with
+reliability, with --mask and --estimator as given) after a run over all ranks and after a single-rank run.  The negative
+catalog must be byte for byte identical; with --estimator median the peak S/N of both catalogs must be too; with the
+mean the node values may differ in the last bits over another row split (see --snr), so the tool reports the largest
+relative difference of the peak S/N and how many peak pixels differ.
 Prints one JSON line on rank 0 with the largest relative difference per field and the verdict of every rank."""
 import argparse
 import json
@@ -103,6 +108,39 @@ def inject_rounds(a, eng, host, tiles, rank, world):
                 ok=bool(same_place and (a.estimator == 'mean' or identical)))
 
 
+def reliability_runs(a, eng, host, tiles, rank, world):
+    """--reliability: the negative catalog and the peak S/N of both catalogs of the run over `world` ranks and of the
+    single-rank run (run_image, node states of the maps, reliability.run with --mask and --estimator).  On rank 0: the
+    negative catalogs must be identical, and with the median estimator the peak S/N (value and pixel) too."""
+    from caesar_yolo_b200 import pipeline, reliability
+    out = []
+    for r, w in ((rank, world), (0, 1)):
+        src, _ = pipeline.run_image(eng, host, True, tiles, rank=r, world=w, on_rank0_only=False)
+        mask = eng.source_mask_band(src, tiles, r, w) if a.mask else None
+        nodes = eng.bkg_maps_band(tiles, a.bkg_box, a.bkg_grid, r, w, mask=mask, estimator=a.estimator, maps=False)[0]
+        plan = reliability.tiled_plan(eng, tiles, src, nodes, a.bkg_box, a.bkg_grid, r, w)
+        neg, pos_peak, neg_peak = reliability.run(eng, plan)
+        out.append((np.array(neg, copy=True), pos_peak, neg_peak))
+    if rank != 0:
+        return None
+    (nm, pm, qm), (n1, p1, q1) = out
+    same_neg = nm.tobytes() == n1.tobytes()
+    res = dict(negative_sources=int(len(n1)), negative_catalog_identical=same_neg)
+    for name, m, o in (('catalog', pm, p1), ('negative', qm, q1)):
+        if len(m[0]) != len(o[0]):
+            res[name + '_snr_identical'] = False
+            continue
+        fin = np.isfinite(o[0])
+        res[name + '_snr_identical'] = bool(np.array_equal(m[0].view(np.uint32), o[0].view(np.uint32)) and
+                                            np.array_equal(m[1], o[1]) and np.array_equal(m[2], o[2]))
+        d = np.abs(m[0][fin].astype(np.float64) - o[0][fin]) / np.maximum(np.abs(o[0][fin]), 1e-30)
+        res[name + '_max_rel_snr_diff'] = float(d.max()) if len(d) else 0.0
+        res[name + '_peak_pixels_differing'] = int(((m[1] != o[1]) | (m[2] != o[2])).sum())
+    res['ok'] = bool(same_neg and (a.estimator == 'mean' or (res.get('catalog_snr_identical') and
+                                                            res.get('negative_snr_identical'))))
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--mosaic', type=int, default=16384)
@@ -122,6 +160,7 @@ def main():
     ap.add_argument('--inject', action='store_true', help='also compare source-injection rounds')
     ap.add_argument('--inject_n', type=int, default=1024)
     ap.add_argument('--inject_rounds', type=int, default=2)
+    ap.add_argument('--reliability', action='store_true', help='also compare the reliability estimate')
     a = ap.parse_args()
     import torch
     import torch.distributed as dist
@@ -234,6 +273,10 @@ def main():
     if a.inject:
         inject_res = inject_rounds(a, eng, host, tiles, rank, world)
         ok = ok and (rank != 0 or inject_res['ok'])
+    rel_res = None
+    if a.reliability:
+        rel_res = reliability_runs(a, eng, host, tiles, rank, world)
+        ok = ok and (rank != 0 or rel_res['ok'])
     flags = torch.tensor([1 if ok else 0], device=dev if a.backend == 'nccl' else 'cpu')
     dist.all_reduce(flags, op=dist.ReduceOp.MIN)
     if rank == 0:
@@ -242,6 +285,7 @@ def main():
                               catalog_identical=same_catalog, max_rel_diff={k: res[k] for k in FLOATS},
                               exact={k: res[k + '_exact'] for k in EXACT}, rtol=a.rtol, estimator=a.estimator,
                               noise=noise_res, maps=maps_res, snr=snr_res, inject=inject_res,
+                              reliability=rel_res,
                               matches_single_rank_on_every_rank=bool(int(flags[0])))), flush=True)
     dist.destroy_process_group()
     return 0 if int(flags[0]) else 1
